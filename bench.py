@@ -22,6 +22,11 @@ launches are one CUDA graph, timed with CUDA events around the replay, max over 
 
 Prints ONE JSON line (rank 0).  Keys follow the driver contract, plus `roofline`, `roofline_fp32`,
 `cpu_baseline`, `e2e`, `clocks`, `gpu_launches`, `l2_flushed`, `l2_resident`, `rollout`.
+
+`--dump-outputs DIR` (C2 only) also writes what the last timed step returned to its caller -- observation, reward,
+terminated, truncated of the batch it stepped, rank 0 -- as DIR/<name>.npy (float32), so that two builds can be compared
+output for output: actions and seeds depend only on the arguments.  Nothing is written into the source tree (it may be
+read-only): log files go to a temporary directory and no bytecode is cached.
 """
 from __future__ import annotations
 
@@ -129,7 +134,21 @@ def cpu_kind():
     return "reference" if ref_shim.reference_available() else "port"
 
 
-_REF_LOG_DIR = None
+_LOG_DIR = None
+
+
+def _log_dir():
+    """One scratch log directory per process: the reference opens a log file per env (env.py:23-31), this package's
+    single-env face one when an episode ends; neither belongs in the working directory."""
+    global _LOG_DIR
+    if _LOG_DIR is None:
+        import atexit
+        import shutil
+        import tempfile
+
+        _LOG_DIR = tempfile.mkdtemp(prefix="evac_bench_logs_")
+        atexit.register(shutil.rmtree, _LOG_DIR, ignore_errors=True)
+    return _LOG_DIR
 
 
 def _make_cpu_env(kind, n_ped, env_kw=None, wrap_kw=None):
@@ -138,21 +157,13 @@ def _make_cpu_env(kind, n_ped, env_kw=None, wrap_kw=None):
         kw["number_of_pedestrians"] = n_ped
     WRAP_KW_ = WRAP_KW if wrap_kw is None else wrap_kw
     if kind == "reference":
-        import tempfile
         import warnings
 
         from oracle import ref_shim
 
         warnings.filterwarnings("ignore")
         ref = ref_shim.load_reference()
-        global _REF_LOG_DIR
-        if _REF_LOG_DIR is None:  # one scratch log directory per process (the reference opens a log file per env, env.py:23-31)
-            import atexit
-            import shutil
-
-            _REF_LOG_DIR = tempfile.mkdtemp(prefix="evac_ref_logs_")
-            atexit.register(shutil.rmtree, _REF_LOG_DIR, ignore_errors=True)
-        cfg = ref.EnvConfig(wandb_enabled=False, giff_freq=10 ** 9, path_logs=_REF_LOG_DIR, **kw)
+        cfg = ref.EnvConfig(wandb_enabled=False, giff_freq=10 ** 9, path_logs=_log_dir(), **kw)
         return ref.setup_env(cfg, ref.EnvWrappersConfig(**WRAP_KW_))
     from oracle.evac_oracle import OracleConfig, OracleEnv
 
@@ -193,14 +204,14 @@ def _cpu_worker(args, n_ped=None, kind="port"):
     for _ in range(steps):
         one_step()
     dt = time.perf_counter() - t0
-    global _REF_LOG_DIR
-    if _REF_LOG_DIR is not None:  # (forked workers leave through os._exit: atexit handlers do not run there)
+    global _LOG_DIR
+    if _LOG_DIR is not None:  # (forked workers leave through os._exit: atexit handlers do not run there)
         import logging
         import shutil
 
         logging.shutdown()
-        shutil.rmtree(_REF_LOG_DIR, ignore_errors=True)
-        _REF_LOG_DIR = None
+        shutil.rmtree(_LOG_DIR, ignore_errors=True)
+        _LOG_DIR = None
     return dt
 
 
@@ -245,7 +256,8 @@ def c1_leg(dev, seeds=8, steps=2000):
                 if arm == "cpu":
                     env = _make_cpu_env(kind, None, env_kw=dict(number_of_pedestrians=N_PED), wrap_kw=wrap)
                 else:
-                    env = eb.setup_env(eb.EnvConfig(number_of_pedestrians=N_PED, wandb_enabled=False), eb.EnvWrappersConfig(**wrap), device=dev)
+                    env = eb.setup_env(eb.EnvConfig(number_of_pedestrians=N_PED, wandb_enabled=False, path_logs=_log_dir()),
+                                       eb.EnvWrappersConfig(**wrap), device=dev)
                 np.random.seed(seed)
                 rs = np.random.RandomState(1000 + seed)
                 acts = rs.uniform(-1, 1, size=(steps, 2)).astype(np.float32)
@@ -268,12 +280,12 @@ def c1_leg(dev, seeds=8, steps=2000):
         cpu, gpu = float(np.median(rates["cpu"])), float(np.median(rates["gpu"]))
         out["cases"][name] = {"cpu_env_steps_per_s": cpu, "gpu_single_env_steps_per_s": gpu, "cpu_us_per_step": 1e6 / cpu,
                               "gpu_single_env_us_per_step": 1e6 / gpu, "speedup_single_env": gpu / cpu}
-    global _REF_LOG_DIR
-    if _REF_LOG_DIR is not None:
+    global _LOG_DIR
+    if _LOG_DIR is not None:
         import shutil
 
-        shutil.rmtree(_REF_LOG_DIR, ignore_errors=True)
-        _REF_LOG_DIR = None
+        shutil.rmtree(_LOG_DIR, ignore_errors=True)
+        _LOG_DIR = None
     return out
 
 
@@ -428,7 +440,7 @@ def run_ours(args):
     with torch.cuda.stream(side):
         with torch.cuda.graph(graph_a, stream=side):
             for s in range(K):
-                sets[s % R].unwrapped.step(actions[W + s])
+                last = sets[s % R].unwrapped.step(actions[W + s])  # (the batch's own output buffers: every replay refills them)
     torch.cuda.synchronize(dev)
     # kernel nodes recorded into the graph (the library counts launches at capture time) = launches of the K timed steps
     launches = sum(x.unwrapped.launch_count for x in sets) - launches0
@@ -473,6 +485,9 @@ def run_ours(args):
                             "on 12 decoy batches (L2 turned over), event, the K timed steps, event")
         except Exception:  # pragma: no cover
             pass
+    if args.dump_outputs and rank == 0:  # the last timed step's results, before any other leg reuses the batches
+        obs, reward, terminated, truncated, _ = last
+        dump_outputs(args.dump_outputs, {"obs": obs, "reward": reward, "terminated": terminated, "truncated": truncated})
     del graph_b
     del graph_a
     restore(env)
@@ -659,6 +674,24 @@ def _build_id():
     from evacuation_b200 import _native as nat
 
     return nat.build_id()
+
+
+DUMP_BYTES = 64 * 10 ** 6 - 4096  # at most 64 MB in all, .npy headers included
+DUMP_SAMPLE_SEED = 0
+
+
+def dump_outputs(directory, arrays):
+    """Write every [E, ...] tensor as <directory>/<name>.npy in float32 (flags as 0 / 1).  When they exceed DUMP_BYTES in
+    all, the same fixed, seeded sample of environments (rows, ascending) is kept from each."""
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    rows = len(next(iter(arrays.values())))
+    keep = min(rows, DUMP_BYTES // (sum(a.nbytes for a in arrays.values()) // rows))
+    if keep < rows:
+        idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(rows, size=keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, f"{k}.npy"), a)
 
 
 def pairwise_probe(device_index):
@@ -957,7 +990,12 @@ def main():
     ap.add_argument("--no-c5", action="store_true", help="skip the C5 leg (65536 envs in total with the policy in the loop)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--workload", default="c2", choices=["c2", "c5"], help="c2 = the bench line; c5 = config 5 with the policy in the loop")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (C2, rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs writes the outputs of the C2 path (--impl ours --workload c2)")
     if args.impl == "reference":
         run_reference_arm(args)
     elif args.workload == "c5":
@@ -967,4 +1005,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # (the tree may be read-only)
     main()

@@ -325,6 +325,31 @@ def test_bench_reference_arm_prints_one_contract_line(force_port):
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_bench_dump_outputs_are_float32_and_a_fixed_sample_under_64_mb(tmp_path):
+    """`bench.py --dump-outputs`: one <name>.npy per array in float32 (flags as 0 / 1); above 64 MB in all, the same
+    seeded sample of environments (ascending) is kept from every array, and the same one on every run."""
+    import torch
+
+    import bench
+
+    E = 65536  # 65536 x (62 x 6 + 2) x 4 bytes = 98 MB
+    arrays = {"obs": torch.rand((E, 62, 6), generator=torch.Generator().manual_seed(0)),
+              "reward": torch.arange(E, dtype=torch.float32), "terminated": torch.arange(E) % 3 == 0}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["obs.npy", "reward.npy", "terminated.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 * 10 ** 6
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    rows = got["reward"].astype(np.int64)  # the reward column holds the environment index
+    assert all(a.dtype == np.float32 and len(a) == len(rows) for a in got.values())
+    assert E // 2 < len(rows) < E and np.all(np.diff(rows) > 0)
+    np.testing.assert_array_equal(got["obs"], arrays["obs"].numpy()[rows])
+    np.testing.assert_array_equal(got["terminated"], (rows % 3 == 0).astype(np.float32))
+    for f in files:
+        np.testing.assert_array_equal(np.load(tmp_path / "b" / f), got[f[:-4]])
+
+
 def test_bind_host_to_device_never_raises():
     """The NUMA helper is opt-in plumbing for the host face: without NVML (this container) or on a single-node host it
     must report what it did and leave the process affinity usable."""
