@@ -140,7 +140,7 @@ def load() -> C.CDLL:
     if lib.evac_abi_version() != EVAC_ABI_VERSION:
         raise EvacNativeError("libevac_b200.so ABI version mismatch; rebuild")
     got = lib.evac_build_id().decode()
-    if got != want and not os.environ.get("EVAC_B200_LIB"):  # (EVAC_B200_LIB: an explicitly chosen kernel-variant build)
+    if got != want and not os.environ.get("EVAC_B200_LIB"):  # (EVAC_B200_LIB: an explicitly chosen library built elsewhere)
         raise EvacNativeError(f"{LIB_PATH} was built from other sources (build id {got}, tree {want}); rebuild")
     _lib = lib
     return lib

@@ -19,7 +19,7 @@ import sys
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
-LIB_PATH = os.environ.get("EVAC_B200_LIB") or os.path.join(PKG_DIR, "libevac_b200.so")  # override: kernel-variant experiments
+LIB_PATH = os.environ.get("EVAC_B200_LIB") or os.path.join(PKG_DIR, "libevac_b200.so")  # override: a library built elsewhere (A/B runs)
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 _ID_MARKER = b"EVAC_BUILD_ID="
@@ -78,9 +78,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     objs, procs = [], []
     for src in sources():  # one nvcc per translation unit, in parallel
         obj = os.path.join(CSRC, os.path.splitext(os.path.basename(src))[0] + ".o")
-        obj = obj[:-2] + os.environ.get("EVAC_B200_OBJ_TAG", "") + ".o"
-        cmd = [nvcc, *NVCC_FLAGS, f'-DEVAC_BUILD_ID="{build_id}"', *os.environ.get("EVAC_B200_NVCC_EXTRA", "").split(),
-               *(["-Xptxas=-v"] if verbose else []), "-c", "-o", obj, src]
+        cmd = [nvcc, *NVCC_FLAGS, f'-DEVAC_BUILD_ID="{build_id}"', *(["-Xptxas=-v"] if verbose else []), "-c", "-o", obj, src]
         if verbose:
             print(" ".join(cmd), file=sys.stderr)
         objs.append(obj)

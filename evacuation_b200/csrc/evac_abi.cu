@@ -71,10 +71,8 @@ struct EvacHandle {
   int threads = 0, ppt = 0;
   int num_sms = 0;
   int cells_x = 0, cells_y = 0, cell_reach = 1;  // > 0: cell-list neighbour search (multi-warp fp32 shapes)
-  int cell_pair_walk = 1;        // paired walk of the sorted slots (EVAC_CELL_PAIR_WALK=0: one slot per thread)
+  int cell_pair_walk = 1;        // paired walk of the sorted slots (0: one slot per thread)
   int cluster = 1;               // > 1: one environment per thread-block cluster of this many 1024 x 4 CTAs (N > 4096, evac_cluster.cuh)
-  bool warp_kernel = true;       // N <= 64 fp32: evac_warp_kernel (false: the generic kernel, EVAC_WARP_KERNEL=generic)
-  int warps_per_cta = 1;         // environments per CTA of evac_warp_kernel (EVAC_WARP_WPC = 1 | 2 | 4 | 8)
 };
 
 // smallest double b such that sqrt(v) >= t for every v >= b  <=>  (v < b) == (sqrt(v) < t)
@@ -152,7 +150,7 @@ static int launch_step_t(EvacHandle* h, const KArgs<real>& a, cudaStream_t st) {
   auto kern = evac_step_kernel<real, THREADS, PPT>;
   if (smem > 48 * 1024 && attr_set[h->device & 15] < smem) {
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // the whole unified L1 / shared-memory array as shared memory: lets two 113 KB CTAs of the 512 x 8 shape share an SM
+    // the whole unified L1 / shared-memory array as shared memory
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     attr_set[h->device & 15] = smem;
   }
@@ -191,39 +189,22 @@ static int launch_cluster_t(EvacHandle* h, const KArgs<float>& a, cudaStream_t s
 }
 
 static void pick_shape(int n, int* threads, int* ppt) {
-  const char* shape = getenv("EVAC_SHAPE_64");  // A/B switch for N <= 64: "64x1" or "32x2" (default)
-  if (n <= 64 && shape && strcmp(shape, "64x1") == 0) { *threads = 64; *ppt = 1; }
-  else if (n <= 64) { *threads = 32; *ppt = 2; }
+  if (n <= 64) { *threads = 32; *ppt = 2; }
   else if (n <= 128) { *threads = 128; *ppt = 1; }
   else if (n <= 256) { *threads = 256; *ppt = 1; }
   else if (n <= 512) { *threads = 256; *ppt = 2; }
   else if (n <= 1024) { *threads = 512; *ppt = 2; }
   else if (n <= 2048) { *threads = 512; *ppt = 4; }
-  else if (n <= 4096) {
-    // 1024 x 4 = one CTA per SM; EVAC_SHAPE_4096=512x8: two co-resident CTAs per SM (113 KB of shared memory each, 64 registers):
-    // 256 environments are then ONE wave on 148 SMs instead of 1.73, and a CTA's barrier stalls are filled by its neighbour
-    const char* s4 = getenv("EVAC_SHAPE_4096");
-    if (s4 && strcmp(s4, "512x8") == 0) { *threads = 512; *ppt = 8; } else { *threads = 1024; *ppt = 4; }
-  }
+  else if (n <= 4096) { *threads = 1024; *ppt = 4; }  // one CTA per SM
   else { *threads = 1024; *ppt = 8; }  // up to 8192: the sorted tile (16 B per pedestrian) + cell list still fit one SM's shared memory
 }
 
-// N <= 64, float32: the dedicated one-warp kernel (evac_warp.cuh), observation encoding resolved at compile time.
-// EVAC_WARP_KERNEL=generic selects evac_step_kernel<float,32,2> instead (A/B measurements).
-template <int WPC>
-static void launch_warp_t(const KArgs<float>& a, cudaStream_t st) {
-  const int grid = (a.E + WPC - 1) / WPC;
-  if (a.positions == POS_REL && a.statuses == STAT_OHE && a.obs_type == OBS_BOX) evac_warp_kernel<WMODE_REL_OHE_BOX, WPC><<<grid, 32 * WPC, 0, st>>>(a);
-  else if (a.positions == POS_GRAV) evac_warp_kernel<WMODE_GRAV, WPC><<<grid, 32 * WPC, 0, st>>>(a);
-  else evac_warp_kernel<WMODE_GENERIC, WPC><<<grid, 32 * WPC, 0, st>>>(a);
-}
+// N <= 64, float32: the dedicated one-warp kernel (evac_warp.cuh), observation encoding resolved at compile time.  One
+// environment per CTA: measured on B200 at 4096 envs with 1 / 2 / 4 / 8 environments per CTA, 14.0 / 14.4 / 14.4 / 14.9 us.
 static int launch_warp(EvacHandle* h, const KArgs<float>& a, cudaStream_t st) {
-  switch (h->warps_per_cta) {  // measured on B200 (tools/wpc_sweep.sh): 1 is the fastest at 4096 envs (14.0 / 14.4 / 14.4 / 14.9 us)
-    case 2: launch_warp_t<2>(a, st); break;
-    case 4: launch_warp_t<4>(a, st); break;
-    case 8: launch_warp_t<8>(a, st); break;
-    default: launch_warp_t<1>(a, st); break;
-  }
+  if (a.positions == POS_REL && a.statuses == STAT_OHE && a.obs_type == OBS_BOX) evac_warp_kernel<WMODE_REL_OHE_BOX><<<a.E, 32, 0, st>>>(a);
+  else if (a.positions == POS_GRAV) evac_warp_kernel<WMODE_GRAV><<<a.E, 32, 0, st>>>(a);
+  else evac_warp_kernel<WMODE_GENERIC><<<a.E, 32, 0, st>>>(a);
   CK(cudaGetLastError());
   h->launches++;
   return EVAC_OK;
@@ -232,7 +213,7 @@ static int launch_warp(EvacHandle* h, const KArgs<float>& a, cudaStream_t st) {
 template <typename real>
 static int launch_step(EvacHandle* h, const KArgs<real>& a, cudaStream_t st) {
   if constexpr (std::is_same<real, float>::value) {
-    if (h->threads == 32 && h->warp_kernel) return launch_warp(h, a, st);
+    if (h->threads == 32) return launch_warp(h, a, st);
     switch (h->cluster) {
       case 2: return launch_cluster_t<2>(h, a, st);
       case 4: return launch_cluster_t<4>(h, a, st);
@@ -240,16 +221,14 @@ static int launch_step(EvacHandle* h, const KArgs<real>& a, cudaStream_t st) {
     }
   }
   switch (h->threads * 16 + h->ppt) {
-    case 32 * 16 + 2: return launch_step_t<real, 32, 2>(h, a, st);
-    case 64 * 16 + 1: return launch_step_t<real, 64, 1>(h, a, st);
+    case 32 * 16 + 2:
+      if constexpr (std::is_same<real, double>::value) return launch_step_t<real, 32, 2>(h, a, st);
+      break;  // float32: evac_warp_kernel
     case 128 * 16 + 1: return launch_step_t<real, 128, 1>(h, a, st);
     case 256 * 16 + 1: return launch_step_t<real, 256, 1>(h, a, st);
     case 256 * 16 + 2: return launch_step_t<real, 256, 2>(h, a, st);
     case 512 * 16 + 2: return launch_step_t<real, 512, 2>(h, a, st);
     case 512 * 16 + 4: return launch_step_t<real, 512, 4>(h, a, st);
-    case 512 * 16 + 8:
-      if constexpr (std::is_same<real, float>::value) return launch_step_t<real, 512, 8>(h, a, st);
-      break;
     case 1024 * 16 + 4: return launch_step_t<real, 1024, 4>(h, a, st);
     case 1024 * 16 + 8:
       if constexpr (std::is_same<real, float>::value) return launch_step_t<real, 1024, 8>(h, a, st);
@@ -340,11 +319,12 @@ int evac_create(const EvacConfig* cfg, int32_t num_envs, int32_t device, uint64_
   pick_shape(h->N, &h->threads, &h->ppt);
   if (h->N > 64 && h->prec == EVAC_PREC_F32 && cfg->neighbor_search != EVAC_SEARCH_BRUTE) {
     // above the 8192 pedestrians one SM's shared memory holds: a cluster of 4 / 8 CTAs (1024 threads x 4 pedestrians) per
-    // environment.  EVAC_CLUSTER = 1 | 2 | 4 | 8 overrides the choice where the crowd fits (A/B measurements, cluster-size
-    // invariance tests).  Measured on B200 (10 steps after 32): 128 x 8192 one 1024 x 8 CTA 226 us, cluster of 2 263 us;
-    // 256 x 4096 one CTA 161 us, cluster of 2 288 us -> clusters only where one CTA cannot hold the crowd.
+    // environment.  EVAC_CLUSTER = 1 | 2 | 4 | 8 overrides the choice where the crowd fits: a test hook, so that tests can
+    // check cluster-size invariance and compare clusters with the oracle.  Measured on B200 (10 steps after 32): 128 x 8192
+    // one 1024 x 8 CTA 226 us, cluster of 2 263 us; 256 x 4096 one CTA 161 us, cluster of 2 288 us -> clusters only where
+    // one CTA cannot hold the crowd.
     int want = h->N <= 8192 ? 1 : (h->N <= 16384 ? 4 : 8);
-    const char* cl = getenv("EVAC_CLUSTER");
+    const char* cl = getenv("EVAC_CLUSTER");  // test hook (see above)
     if (cl) {
       const int v = atoi(cl);
       if ((v == 2 || v == 4 || v == 8) && v * 4096 >= h->N) want = v;
@@ -353,15 +333,12 @@ int evac_create(const EvacConfig* cfg, int32_t num_envs, int32_t device, uint64_
     h->cluster = want;
     if (h->cluster > 1) { h->threads = 1024; h->ppt = 4; }
   }
-  { const char* wk = getenv("EVAC_WARP_KERNEL"); h->warp_kernel = !(wk && strcmp(wk, "generic") == 0); }
-  { const char* wp = getenv("EVAC_WARP_WPC"); if (wp) h->warps_per_cta = atoi(wp); }
   if (h->N > 64 && h->threads > 32 && h->prec == EVAC_PREC_F32 && cfg->neighbor_search != EVAC_SEARCH_BRUTE) {
     // cell edge >= (1 + 1e-4) x vision radius: two pedestrians closer than the radius always sit in the same or
     // in adjacent cells, float32 rounding of the cell index included; at most 64 x 64 cells
     // reach 2 (default when the grid fits): half-size cells, 5 x 5 block -> 1.44x fewer candidates in 5 row segments
-    // (measured 10-17 % faster than the 3 x 3 block of full-size cells at 256 x 4096); EVAC_CELL_REACH=1 forces the latter
-    const char* rs = getenv("EVAC_CELL_REACH");
-    int reach = (rs && atoi(rs) == 1) ? 1 : 2;
+    // (measured 10-17 % faster than the 3 x 3 block of full-size cells at 256 x 4096)
+    int reach = 2;
     double edge = cfg->to_pedestrian * (1.0 + 1e-4) / reach;
     if (2.0 * cfg->width / edge > 64.0 || 2.0 * cfg->height / edge > 64.0) { reach = 1; edge = cfg->to_pedestrian * (1.0 + 1e-4); }
     int gx = (int)fmin(64.0, floor(2.0 * cfg->width / edge)), gy = (int)fmin(64.0, floor(2.0 * cfg->height / edge));
@@ -377,18 +354,16 @@ int evac_create(const EvacConfig* cfg, int32_t num_envs, int32_t device, uint64_
     // Measured on B200, 20 steps after 0 / 64 / 300 warm-up steps: 256 x 4096 (2.7 per cell) 144 / 177 / 271 -> 129 / 167 / 265 us,
     // 1024 x 1000 109 -> 107 us, 2048 x 256 (0.17 per cell) 58 -> 63 us  => on from half a pedestrian per cell
     h->cell_pair_walk = 2 * h->N >= gx * gy;
+    // EVAC_CELL_PAIR_WALK=0 | 1 is a test hook: tests compare the paired walk with the one-slot walk bit for bit
     { const char* pw = getenv("EVAC_CELL_PAIR_WALK"); if (pw) h->cell_pair_walk = atoi(pw) != 0; }
-    // bit 1 (EVAC_CELL_DYNAMIC=1, A/B): the warps draw their chunks of the paired walk from a shared counter instead of taking
-    // equal static shares; results are bit-identical.  Measured on B200 (256 x 4096, 20 steps after 0 / 64 / 300 warm-up steps):
-    // 109.2 / 147.5 / 246.1 us static vs 111.7 / 146.3 / 247.3 us dynamic -- the flocked regime is bound by the total number of
-    // candidate pairs, not by the balance between the warps of a CTA, so the static shares stay.
-    { const char* dy = getenv("EVAC_CELL_DYNAMIC"); if (h->cell_pair_walk && dy && atoi(dy) == 1) h->cell_pair_walk |= 2; }
-    // bit 2 (EVAC_CELL_GROUP=1, A/B): grouped walk -- four lanes share one window of 8 consecutive sorted slots, a quarter of the
-    // shared-memory wavefronts for ~25 % more candidates; one-CTA kernels only; bit-identical results.  Measured on B200
-    // (256 x 4096, 20 steps after 0 / 64 / 300 warm-up steps): 109.8 / 147.8 / 246.1 us paired vs 118.1 / 153.4 / 247.9 us grouped
-    // (128 x 8192: 226.9 vs 234.6; 1024 x 1000: 85.1 vs 89.9) -- the walk is not bound by shared-memory bandwidth either: what it
-    // costs is the number of evaluated candidate pairs times the trip-count divergence inside a warp, so the paired walk stays.
-    { const char* gr = getenv("EVAC_CELL_GROUP"); if (h->cell_pair_walk && h->cluster == 1 && gr && atoi(gr) == 1) h->cell_pair_walk |= 4; }
+    // Walks measured on B200 and not kept (256 x 4096, 20 steps after 0 / 64 / 300 warm-up steps):
+    //  * chunks of the paired walk drawn from a shared counter instead of equal static shares: 109.2 / 147.5 / 246.1 us static vs
+    //    111.7 / 146.3 / 247.3 us dynamic -- the flocked regime is bound by the total number of candidate pairs, not by the
+    //    balance between the warps of a CTA;
+    //  * a grouped walk (four lanes share one window of 8 consecutive sorted slots, a quarter of the shared-memory wavefronts for
+    //    ~25 % more candidates): 109.8 / 147.8 / 246.1 us paired vs 118.1 / 153.4 / 247.9 us grouped (128 x 8192: 226.9 vs 234.6;
+    //    1024 x 1000: 85.1 vs 89.9) -- the walk is not bound by shared-memory bandwidth either: what it costs is the number of
+    //    evaluated candidate pairs times the trip-count divergence inside a warp.
   } else if (h->threads == 32 && h->prec == EVAC_PREC_F32 && cfg->neighbor_search == EVAC_SEARCH_CELLS) {
     // one-warp kernel, opt-in: vertical strips (a 1-D cell list, at most 32 strips), same edge rule.  Measured on
     // B200 (profiles/README.md): 15 % fewer instructions than the all-pairs tile but no wall-clock gain (the warp is
@@ -404,7 +379,7 @@ int evac_create(const EvacConfig* cfg, int32_t num_envs, int32_t device, uint64_
     if (_e != cudaSuccess) { evac_destroy(h); return fail(EVAC_ERR_CUDA, "cudaMalloc(%zu) failed: %s", (size_t)(bytes), cudaGetErrorString(_e)); } \
     cudaMemset((ptr), 0, (bytes));                                             \
   } while (0)
-  if (h->threads == 32 && h->warp_kernel && h->prec == EVAC_PREC_F32) {
+  if (h->threads == 32 && h->prec == EVAC_PREC_F32) {
     // the one-warp kernel family keeps the whole state of an environment in one packed 1152-byte block (EnvBlock)
     ALLOC(h->blocks, (size_t)h->E * BLK_BYTES);
   } else {
@@ -574,18 +549,16 @@ int evac_step_host(EvacHandle* h, const float* actions, const float* noise, floa
   for (int i = 0; i < 7; ++i)
     if (ptrs[i] != h->pin_key[i]) { h->pin_key[i] = ptrs[i]; h->pin_val[i] = is_pinned(ptrs[i]); }
   const bool pa = h->pin_val[0], pn = h->pin_val[1], po = h->pin_val[2], pr = h->pin_val[3], pt = h->pin_val[4], pu = h->pin_val[5], ps = h->pin_val[6];
-  // Small batches (the reference-shaped single environment above all; up to 1 MB of inputs + results = ~680 envs x 60): when every
-  // caller buffer is page-locked the kernel
-  // reads the actions / noise from and writes its results into HOST memory directly (unified addressing: a page-locked host
-  // pointer is a device pointer) -- one launch + one synchronise instead of copy, launch, copy, synchronise; a few KB over PCIe
-  // cost less than the latency of two copy operations.  EVAC_HOST_ZEROCOPY=0: off, EVAC_HOST_ZEROCOPY_BYTES: the limit (A/B).  Measured
-  // per step with / without (tools/host_face_sweep.py): 21 / 27 us (1 env), 24 / 28 (32), 27 / 32 (128), 40 / 45 (512); beyond, the copy
-  // engine wins (2048 envs: 124 / 95 us, 4096: 401 / 145 -- the strided observation stores over PCIe).
+  // Small batches (the reference-shaped single environment above all; up to kZeroCopyMaxBytes of inputs + results = ~680 envs x
+  // 60): when every caller buffer is page-locked the kernel reads the actions / noise from and writes its results into HOST memory
+  // directly (unified addressing: a page-locked host pointer is a device pointer) -- one launch + one synchronise instead of copy,
+  // launch, copy, synchronise; a few KB over PCIe cost less than the latency of two copy operations.  Measured per step with /
+  // without: 21 / 27 us (1 env), 24 / 28 (32), 27 / 32 (128), 40 / 45 (512); beyond, the copy engine wins (2048 envs: 124 / 95 us,
+  // 4096: 401 / 145 -- the strided observation stores over PCIe).
   {
-    static const bool zc_on = [] { const char* z = getenv("EVAC_HOST_ZEROCOPY"); return !(z && z[0] == '0'); }();
-    static const size_t zc_max = [] { const char* z = getenv("EVAC_HOST_ZEROCOPY_BYTES"); return z ? (size_t)atoll(z) : (size_t)1 << 20; }();
+    constexpr size_t kZeroCopyMaxBytes = (size_t)1 << 20;
     const size_t bytes = E * (D * 4 + 14 + N * 5);
-    if (zc_on && bytes <= zc_max && pa && (!noise || pn) && (!obs || po) && (!reward || pr) && (!terminated || pt) && (!truncated || pu) &&
+    if (bytes <= kZeroCopyMaxBytes && pa && (!noise || pn) && (!obs || po) && (!reward || pr) && (!terminated || pt) && (!truncated || pu) &&
         (!statuses || ps)) {
       if (int r = rollout_impl(h, 1, EVAC_AGENT_TABLE, actions, noise, obs, 0, reward ? reward : h->d_reward, terminated ? terminated : h->d_term,
                                truncated ? truncated : h->d_trunc, nullptr, statuses, st)) return r;
@@ -594,13 +567,13 @@ int evac_step_host(EvacHandle* h, const float* actions, const float* noise, floa
     }
   }
   // large batches: the results go through the copy engine; page-locked ACTIONS (8 bytes per environment) are still read by the kernel
-  // straight from host memory -- one copy operation less in front of the launch (EVAC_HOST_ACTIONS_ZEROCOPY=0: copy them, A/B)
-  static const bool act_zc = [] { const char* z = getenv("EVAC_HOST_ACTIONS_ZEROCOPY"); return !(z && z[0] == '0'); }();
-  const float* act_dev = h->d_actions;
-  if (pa && act_zc) act_dev = actions;
-  else {
-    if (!pa) memcpy(h->h_actions, actions, E * 8);
-    CK(cudaMemcpyAsync(h->d_actions, pa ? actions : h->h_actions, E * 8, cudaMemcpyHostToDevice, st));
+  // straight from host memory -- one copy operation less in front of the launch (measured 86.5 vs 91.1 us at 2048 envs, 142.8 vs
+  // 143.0 at 4096)
+  const float* act_dev = actions;
+  if (!pa) {
+    memcpy(h->h_actions, actions, E * 8);
+    CK(cudaMemcpyAsync(h->d_actions, h->h_actions, E * 8, cudaMemcpyHostToDevice, st));
+    act_dev = h->d_actions;
   }
   if (noise) {
     if (!pn) memcpy(h->h_noise, noise, E * N * 4);
@@ -746,10 +719,9 @@ __global__ void __launch_bounds__(256) probe_fma_kernel(float* out, int iters, f
   }
 }
 
-// Standalone launch of the SAME pairwise_pass device function the fused step kernel uses, on the same
-// warp shapes (one environment per warp, THREADS x PPT = 32x2, or one per 64-thread CTA as 64x1).  WPC = environments
-// (independent warps, each with its own tile) per CTA: one-warp CTAs cap an SM at 32 resident warps (the CTA limit);
-// WPC = 2 with 48 registers reaches 40.
+// Standalone launch of the SAME pairwise_pass device function the fused step kernel uses (one environment per warp,
+// THREADS x PPT = 32x2) and of narrower mappings: THREADS lanes per environment, WPC environments (each with its own tile) per
+// CTA, UNR slot pairs per unrolled iteration.
 template <int THREADS, int PPT, int UNR = 4, int WPC = 1, int MINB = 1>
 __global__ void __launch_bounds__(THREADS * WPC, MINB) probe_pairwise_kernel(const float2* __restrict__ pos, const float2* __restrict__ unit,
                                                                              float2* __restrict__ out, int N, int reps, float thr2, int E) {
@@ -925,29 +897,19 @@ int evac_probe_pairwise(int32_t device, int32_t num_envs, int32_t n, int32_t rep
   cudaEvent_t e0, e1;
   CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
   const float thr2 = round_up_f32(sq_boundary(0.1));
-  const char* shape = getenv("EVAC_SHAPE_64");
-  const bool shape_32x2 = !(shape && strcmp(shape, "64x1") == 0);
-  const char* unr_s = getenv("EVAC_PROBE_UNROLL");  // A/B: unroll factor of the slot-pair loop (2 | 4 | 8)
-  const int unr = unr_s ? atoi(unr_s) : 4;
-  const char* wpc_s = getenv("EVAC_PROBE_WPC");     // A/B: environments (warps) per CTA of the 32x2 shape: 1 (default) | 2 | 4
-  const int wpc = wpc_s ? atoi(wpc_s) : 1;
   const size_t tb = Tile<float>::bytes(64);
+  // EVAC_PROBE_HALFWARP selects the mapping: unset, one environment per warp (32 x 2, the step kernel's); 2, 16 lanes x 4
+  // pedestrians per environment, two environments per warp; 8, 8 lanes x 8 pedestrians, four environments per warp
+  const char* hw = getenv("EVAC_PROBE_HALFWARP");
+  const int mapping = hw ? atoi(hw) : 0;
   for (int rep = 0; rep < 2; ++rep) {
     CK(cudaEventRecord(e0));
-    const char* hw = getenv("EVAC_PROBE_HALFWARP");  // A/B: 16 lanes x 4 pedestrians per environment, two environments per warp (unroll 1 | 2 | 4); 8: 8 lanes x 8
-    if (hw && atoi(hw) == 1) probe_pairwise_kernel<16, 4, 1, 2, 16><<<(num_envs + 1) / 2, 32, 2 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else if (hw && atoi(hw) == 2) probe_pairwise_kernel<16, 4, 2, 2, 16><<<(num_envs + 1) / 2, 32, 2 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
+    if (mapping == 2) probe_pairwise_kernel<16, 4, 2, 2, 16><<<(num_envs + 1) / 2, 32, 2 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
     // quarter warp x 8 pedestrians per environment, four environments per warp: one broadcast LDS.128 pair per 64 packed math
     // instructions (32 x 2: per 16) -- measured 50.9 % of the FFMA2 peak at 65 536 x 60 (32 x 2: 46.2 %, 16 x 4: 48.1 %); unroll 1 / 4,
     // 12 resident warps or eight environments per CTA: 46.4 / 48.3 / 50.1 / 50.2 %
-    else if (hw && atoi(hw) == 8) probe_pairwise_kernel<8, 8, 2, 4, 16><<<(num_envs + 3) / 4, 32, 4 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else if (hw && atoi(hw) == 4) probe_pairwise_kernel<16, 4, 4, 2, 16><<<(num_envs + 1) / 2, 32, 2 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else if (shape_32x2 && wpc == 2) probe_pairwise_kernel<32, 2, 4, 2, 20><<<(num_envs + 1) / 2, 64, 2 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else if (shape_32x2 && wpc == 4) probe_pairwise_kernel<32, 2, 4, 4, 10><<<(num_envs + 3) / 4, 128, 4 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else if (shape_32x2 && unr == 8) probe_pairwise_kernel<32, 2, 8><<<num_envs, 32, tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else if (shape_32x2 && unr == 2) probe_pairwise_kernel<32, 2, 2><<<num_envs, 32, tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else if (shape_32x2) probe_pairwise_kernel<32, 2><<<num_envs, 32, tb>>>(pos, unit, out, n, reps, thr2, num_envs);
-    else probe_pairwise_kernel<64, 1><<<num_envs, 64, tb>>>(pos, unit, out, n, reps, thr2, num_envs);
+    else if (mapping == 8) probe_pairwise_kernel<8, 8, 2, 4, 16><<<(num_envs + 3) / 4, 32, 4 * tb>>>(pos, unit, out, n, reps, thr2, num_envs);
+    else probe_pairwise_kernel<32, 2><<<num_envs, 32, tb>>>(pos, unit, out, n, reps, thr2, num_envs);
     CK(cudaEventRecord(e1));
     CK(cudaEventSynchronize(e1));
   }

@@ -393,7 +393,7 @@ struct CellSmem {
   uint16_t* sorted_idx;  // [SLOTS]  original index | 0x8000 if VISCEK/FOLLOWER
   int* cell_start;       // [C + 1]
   int* warp_tot;         // [32]
-  int* row_pairs;        // [cells_y + 1 <= 65]  paired walk: number of slot pairs in the cell rows below (exclusive scan)
+  int* row_pairs;        // [cells_y + 1 <= 65, 68 reserved: 16-byte multiple]  paired walk: number of slot pairs in the cell rows below (exclusive scan)
   static __host__ __device__ constexpr size_t bytes(int slots, int cells) {
     return (size_t)slots * 8 + (size_t)slots * 2 + (((size_t)cells + 1 + 3) & ~(size_t)3) * 4 + (32 + 68) * 4;
   }
@@ -526,14 +526,12 @@ __device__ __forceinline__ void cell_list_pass(const Tile<float>& tile, const Ce
   }
   if (tid < 2) tile.put(n_src + tid, PARK, PARK, 0.f, 0.f);  // pad to an even count (the tile has 2 spare slots)
   if (a.cell_pair_walk && warp == 0) {
-    // walk units per cell row -- slot pairs, or groups of 8 slots for the grouped walk (cell_pair_walk & 4); a unit never
-    // straddles two rows -- exclusive scan over the <= 64 rows by one warp
-    const int ush = (a.cell_pair_walk & 4) ? 3 : 1;
+    // slot pairs per cell row (a pair never straddles two rows) -- exclusive scan over the <= 64 rows by one warp
     int cnt[2], inc = 0;
 #pragma unroll
     for (int k = 0; k < 2; ++k) {
       const int r = lane + 32 * k;
-      cnt[k] = r < a.cells_y ? (cs.cell_start[(r + 1) * a.cells_x] - cs.cell_start[r * a.cells_x] + (1 << ush) - 1) >> ush : 0;
+      cnt[k] = r < a.cells_y ? (cs.cell_start[(r + 1) * a.cells_x] - cs.cell_start[r * a.cells_x] + 1) >> 1 : 0;
     }
     int run = 0;
 #pragma unroll
@@ -546,110 +544,21 @@ __device__ __forceinline__ void cell_list_pass(const Tile<float>& tile, const Ce
       run += __shfl_sync(0xffffffffu, inc, 31);
     }
     if (lane == 0 && a.cells_y == 64) cs.row_pairs[64] = run;
-    if (lane == 0) cs.row_pairs[66] = 0;  // chunk counter of the dynamic walk
   }
   __syncthreads();  // list[] (aliased by res[]) is dead from here on
   // ---- 5. walk the sorted slots
   const float thr2 = a.thr2_ped;
-  if (a.cell_pair_walk & 4) {
-    // Grouped walk: FOUR lanes share one window.  A unit = up to 8 consecutive sorted slots of one cell row; lane q of the
-    // group owns slots 2q, 2q + 1 of it and all four lanes walk the union of the unit's windows in lock step, so their
-    // LDS.128 carry the same address: a warp instruction touches 8 distinct 16-byte words (one 128-byte wavefront) instead of
-    // 32 (four).  The per-thread walk is bound by shared-memory bandwidth, not by issue slots (1 KB per warp and slot-pair
-    // iteration against 16 packed instructions): a quarter of the wavefronts for ~25 % more candidates (the union of 8 slots
-    // spans a cell or two more than the union of 2).  A slot outside a pedestrian's own window fails the distance test and
-    // adds an exact zero, so the sums are bit-identical to the other walks.
-    const int reach = a.cell_reach;
-    const int n_units = cs.row_pairs[a.cells_y];
-#pragma unroll 1
-    for (int T = tid; T < 4 * n_units; T += THREADS) {
-      const int t = T >> 2, q = T & 3;
-      int row = 0;
-      {
-        int hi_r = a.cells_y;
-        while (hi_r - row > 1) { const int mid = (row + hi_r) >> 1; if (cs.row_pairs[mid] <= t) row = mid; else hi_r = mid; }
-      }
-      const int row_end = cs.cell_start[(row + 1) * a.cells_x];
-      const int s_first = cs.cell_start[row * a.cells_x] + 8 * (t - cs.row_pairs[row]);
-      const int s_last = min(s_first + 7, row_end - 1);
-      const int s0 = s_first + 2 * q;
-      const bool v0 = s0 <= s_last, v1 = s0 + 1 <= s_last;
-      const int id0 = v0 ? cs.sorted_idx[s0] : 0, id1 = v1 ? cs.sorted_idx[s0 + 1] : 0;
-      // (a lane without a VISCEK / FOLLOWER pedestrian leaves; the others of its group keep their common addresses)
-      if (!((id0 | id1) & 0x8000)) continue;
-      float xa, ya, xb, yb;  // first / last slot of the unit: the cells the union window spans
-      { const float4 p = tile.P2[s_first >> 1]; xa = (s_first & 1) ? p.y : p.x; ya = (s_first & 1) ? p.w : p.z; }
-      { const float4 p = tile.P2[s_last >> 1]; xb = (s_last & 1) ? p.y : p.x; yb = (s_last & 1) ? p.w : p.z; }
-      int cxa, cxb, cy_;
-      cell_of(xa, ya, a, cxa, cy_);
-      cell_of(xb, yb, a, cxb, cy_);
-      const int cx0 = max(min(cxa, cxb) - reach, 0), cx1 = min(max(cxa, cxb) + reach, a.cells_x - 1);
-      float x0 = PARK, y0 = PARK, x1 = PARK, y1 = PARK;
-      if (v0) { const float4 p = tile.P2[s0 >> 1]; x0 = (s0 & 1) ? p.y : p.x; y0 = (s0 & 1) ? p.w : p.z; }
-      if (v1) { const float4 p = tile.P2[(s0 + 1) >> 1]; x1 = ((s0 + 1) & 1) ? p.y : p.x; y1 = ((s0 + 1) & 1) ? p.w : p.z; }
-      const float2 nx0 = make_float2(-x0, -x0), ny0 = make_float2(-y0, -y0), nx1 = make_float2(-x1, -x1), ny1 = make_float2(-y1, -y1);
-      float2 ax0 = make_float2(0.f, 0.f), ay0 = ax0, ax1 = ax0, ay1 = ax0;
-      int done = 0;
-      for (int r = max(row - reach, 0); r <= min(row + reach, a.cells_y - 1); ++r) {
-        const int lo = max(cs.cell_start[r * a.cells_x + cx0] & ~1, done);
-        const int hi = (cs.cell_start[r * a.cells_x + cx1 + 1] + 1) & ~1;
-        int j = lo >> 1;
-        const int je = hi >> 1;
-        if (j < je) {
-          float4 p = tile.P2[j], u = tile.U2[j];
-#pragma unroll 2
-          for (; j < je; ++j) {
-            const float4 pn = tile.P2[j + 1], un = tile.U2[j + 1];
-            const float2 sxp = make_float2(p.x, p.y), syp = make_float2(p.z, p.w), sux = make_float2(u.x, u.y), suy = make_float2(u.z, u.w);
-            {
-              const float2 dx = __fadd2_rn(sxp, nx0), dy = __fadd2_rn(syp, ny0);
-              float2 d2 = __fmul2_rn(dx, dx);
-              d2 = __ffma2_rn(dy, dy, d2);
-              const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-              ax0 = __ffma2_rn(w, sux, ax0);
-              ay0 = __ffma2_rn(w, suy, ay0);
-            }
-            {
-              const float2 dx = __fadd2_rn(sxp, nx1), dy = __fadd2_rn(syp, ny1);
-              float2 d2 = __fmul2_rn(dx, dx);
-              d2 = __ffma2_rn(dy, dy, d2);
-              const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-              ax1 = __ffma2_rn(w, sux, ax1);
-              ay1 = __ffma2_rn(w, suy, ay1);
-            }
-            p = pn;
-            u = un;
-          }
-        }
-        done = max(done, hi);
-      }
-      if (id0 & 0x8000) cs.res[id0 & 0x7fff] = make_float2(ax0.x + ax0.y, ay0.x + ay0.y);
-      if (id1 & 0x8000) cs.res[id1 & 0x7fff] = make_float2(ax1.x + ax1.y, ay1.x + ay1.y);
-    }
-  } else if (a.cell_pair_walk) {
+  if (a.cell_pair_walk) {
     // Two adjacent sorted slots of ONE cell row per thread: they sit in the same or in neighbouring cells, so one walk over
     // the union of their windows serves both -- every loaded source pair is evaluated against two pedestrians (half the
     // LDS per evaluated pair, like the 2-pedestrians-per-lane all-pairs pass).  A slot outside a pedestrian's own window
     // fails the distance test and adds an exact zero, so the sums equal the one-slot walk bit for bit.
     const int reach = a.cell_reach;
     const int n_pairs = cs.row_pairs[a.cells_y];
-    // chunks of 32 slot pairs are handed to the warps either statically (warp w: chunks w, w + WARPS, ...) or, cell_pair_walk & 2,
-    // drawn from one shared counter: a walk costs as much as its cells are crowded, so in a flocked crowd equal shares of
-    // slot pairs leave most warps waiting at the barrier for the ones that drew the dense cells.  The result of a pair does
-    // not depend on who walks it (bit-identical either way).
-    const bool dynamic = (a.cell_pair_walk & 2) != 0;
-    int* const next_chunk = cs.row_pairs + 66;  // (row_pairs has 68 entries, 65 used; zeroed below the scan barrier)
-    int chunk = warp;
+    // chunks of 32 slot pairs are handed to the warps statically: warp w walks chunks w, w + WARPS, ...
 #pragma unroll 1
-    for (;;) {
-      if (dynamic) {
-        int c = 0;
-        if (lane == 0) c = atomicAdd(next_chunk, 1);
-        chunk = __shfl_sync(0xffffffffu, c, 0);
-      }
-      if (chunk * 32 >= n_pairs) break;
+    for (int chunk = warp; chunk * 32 < n_pairs; chunk += WARPS) {
       const int t = chunk * 32 + lane;
-      chunk += WARPS;
       if (t >= n_pairs) continue;
       int row = 0;
       {  // largest row with row_pairs[row] <= t
@@ -924,7 +833,7 @@ __device__ __forceinline__ void random_layout(uint64_t seed, uint32_t env, uint3
 // CL > 1: ONE environment per thread-block cluster of CL CTAs (evac_cluster.cuh) -- CTA r owns pedestrians
 // [r * SLOTS, (r + 1) * SLOTS); float32 + cell list only; per-environment scalars are written by CTA 0.
 template <typename real, int THREADS, int PPT, int CL = 1>  // @region load
-__global__ void __launch_bounds__(THREADS, (THREADS == 32 ? 32 : (THREADS == 64 ? 16 : (THREADS == 512 && PPT == 8 ? 2 : 1)))) evac_step_kernel(const __grid_constant__ KArgs<real> a) {
+__global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_kernel(const __grid_constant__ KArgs<real> a) {
   constexpr int WARPS = THREADS / 32;
   constexpr int SLOTS = THREADS * PPT;
   constexpr bool F64 = std::is_same<real, double>::value;

@@ -168,7 +168,8 @@ int evac_policy_create(const EvacPolicyConfig* cfg, int32_t device, EvacPolicy**
   alloc(&p->d_w1t, (size_t)p->K16 * HD_COLS); alloc(&p->d_b1, HD_COLS);
   alloc(&p->d_w2t, (size_t)HD_HS * HD_COLS); alloc(&p->d_b2, HD_COLS);
   alloc(&p->d_w3, (size_t)(1 + p->A) * HD_HS); alloc(&p->d_b3, 4); alloc(&p->d_logstd, 4);
-  // EVAC_POLICY_TC=0 keeps layer 1 of the heads on the CUDA cores (A/B switch); the tensor-core kernel reads float4 rows (K % 4 == 0)
+  // the tensor-core kernel reads float4 rows (K % 4 == 0); otherwise layer 1 of the heads runs on the CUDA cores.
+  // EVAC_POLICY_TC=0 is a test hook: it selects the CUDA-core heads so that tests can compare the two kernels bit for bit.
   const char* tc_env = getenv("EVAC_POLICY_TC");
   p->use_tc = (p->K % 4 == 0) && !(tc_env && tc_env[0] == '0');
   p->tc_chunks = (p->K + TC_KC - 1) / TC_KC;
@@ -348,7 +349,7 @@ int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream) {
     const int gx = (h.E + TC_M - 1) / TC_M;
     // shapes: 64 columns x 4 stages (critic and actor in separate CTAs) while 128-column tiles would not fill the SMs, 128 columns
     // x 3 stages beyond (X is read once).  Measured per 8192 / 20 000 / 65 536 envs: 20.3 / 49.3 / 121.5 us (64x4), 29.7 / 50.4 /
-    // 105.0 us (128x3); 64 columns x 2 stages with two CTAs per SM: 24.6 / 53.6 / 113.1 us.  EVAC_POLICY_TC_SHAPE=64x4 | 128x3: A/B.
+    // 105.0 us (128x3); 64 columns x 2 stages with two CTAs per SM: 24.6 / 53.6 / 113.1 us.
     auto k64 = evac_policy_heads_tc_kernel<64, 4, 2, 1>;
     auto k128 = evac_policy_heads_tc_kernel<128, 3, 2, 1>;
     using S64 = TCShape<64, 4, 2>; using S128 = TCShape<128, 3, 2>;
@@ -358,19 +359,9 @@ int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream) {
       PCK(cudaFuncSetAttribute(k128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S128::SMEM_BYTES));
       tc_attr[p->device & 15] = true;
     }
-    bool wide = gx >= 2 * 148;
-    if (const char* sh = getenv("EVAC_POLICY_TC_SHAPE")) wide = strcmp(sh, "128x3") == 0 ? true : strcmp(sh, "64x4") == 0 ? false : wide;
-    if (!wide) { t.w1tc = p->d_w1tc64; k64<<<dim3(gx, 2), TC_THREADS, S64::SMEM_BYTES, st>>>(t); }
+    if (gx < 2 * 148) { t.w1tc = p->d_w1tc64; k64<<<dim3(gx, 2), TC_THREADS, S64::SMEM_BYTES, st>>>(t); }
     else { t.w1tc = p->d_w1tc128; k128<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t); }
     PCK(cudaGetLastError());
-#ifdef EVAC_TC_TRACE
-    if (getenv("EVAC_TC_TRACE_PRINT")) {
-      unsigned long long tr[2][16];
-      cudaDeviceSynchronize();
-      cudaMemcpyFromSymbol(tr, tc_trace, sizeof(tr));
-      for (int w = 0; w < 2; ++w) { fprintf(stderr, "tc_trace %s:", w ? "mma" : "producer"); for (int i = 1; i < 10; ++i) fprintf(stderr, " %lld", tr[w][i] ? (long long)(tr[w][i] - tr[0][0]) : -1LL); fprintf(stderr, "\n"); }
-    }
-#endif
     p->launches++;
     return EVAC_OK;
   }

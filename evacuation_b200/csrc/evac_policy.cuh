@@ -31,13 +31,8 @@
 
 namespace evacp {
 
-#ifndef EVAC_PW_WARPS
-#define EVAC_PW_WARPS 4
-#endif
-#ifndef EVAC_PW_MINB
-#define EVAC_PW_MINB 4
-#endif
-constexpr int PW_WARPS = EVAC_PW_WARPS;   // environments (warps) per CTA of the embedding kernel
+constexpr int PW_WARPS = 4;  // environments (warps) per CTA of the embedding kernel
+constexpr int PW_MINB = 4;   // resident CTAs per SM the embedding kernel's register allocation is sized for
 constexpr int PW_MAX_S = 64;  // rows per environment handled by one warp
 
 __host__ __device__ constexpr int round_up(int a, int b) { return (a + b - 1) / b * b; }
@@ -86,11 +81,7 @@ __device__ __forceinline__ float2 hi(const float4& v) { return make_float2(v.z, 
 // NaN-propagating max / min (torch.relu / torch.clamp keep NaN; fmaxf / fminf would drop it)
 __device__ __forceinline__ float max_nan(float a, float b) { float r; asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
 __device__ __forceinline__ float min_nan(float a, float b) { float r; asm("min.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b)); return r; }
-#ifdef EVAC_PROBE_NOEXP  // measurement variant (never shipped): the attention loop without its MUFU.EX2
-__device__ __forceinline__ float ex2(float x) { return x * 0.001f + 1.f; }
-#else
 __device__ __forceinline__ float ex2(float x) { float r; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
-#endif
 
 __host__ __device__ __forceinline__ uint32_t fmix32(uint32_t h) {
   h ^= h >> 16; h *= 0x85EBCA6Bu; h ^= h >> 13; h *= 0xC2B2AE35u; h ^= h >> 16;
@@ -180,16 +171,8 @@ __device__ __forceinline__ void attn_group(const float* __restrict__ ks, const f
   float4 k4[H], v4[H];
 #pragma unroll
   for (int h = 0; h < H; ++h) {
-#ifdef EVAC_PROBE_NOLDS  // measurement variant (never shipped): opaque register moves instead of the six broadcast LDS.128
-    {
-      auto opq = [](float y) { float x; asm volatile("mov.f32 %0, %1;" : "=f"(x) : "f"(y)); return x; };
-      k4[h] = make_float4(opq(qa[h].x), opq(qb[h].x), opq(nma.x), opq(nmb.x));
-      v4[h] = make_float4(opq(qb[h].x), opq(qa[h].x), opq(nmb.x), opq(nma.x));
-    }
-#else
     k4[h] = *reinterpret_cast<const float4*>(ks + h * PW_MAX_S + j);
     v4[h] = *reinterpret_cast<const float4*>(vs + h * PW_MAX_S + j);
-#endif
   }
 #pragma unroll
   for (int half = 0; half < 2; ++half) {
@@ -207,19 +190,15 @@ __device__ __forceinline__ void attn_group(const float* __restrict__ ks, const f
     }
     l = __fadd2_rn(l, p0);
     l = __fadd2_rn(l, p1);
-#ifndef EVAC_PROBE_NOVAL  // (measurement variant, never shipped: the attention loop without its value FFMA2s)
 #pragma unroll
     for (int h = 0; h < H; ++h) acc[h] = __ffma2_rn(p0, splat(half ? v4[h].z : v4[h].x), acc[h]);
 #pragma unroll
     for (int h = 0; h < H; ++h) acc[h] = __ffma2_rn(p1, splat(half ? v4[h].w : v4[h].y), acc[h]);
-#else
-    acc[0] = __fadd2_rn(acc[0], lo(v4[half]));
-#endif
   }
 }
 
 template <int D, int H, bool TRAIN>
-__global__ void __launch_bounds__(PW_WARPS * 32, EVAC_PW_MINB) evac_policy_embed_kernel(const __grid_constant__ PArgs a) {
+__global__ void __launch_bounds__(PW_WARPS * 32, PW_MINB) evac_policy_embed_kernel(const __grid_constant__ PArgs a) {
   using L = EmbLayout<D, H>;
   extern __shared__ float4 smem4[];
   float* wsm = reinterpret_cast<float*>(smem4);

@@ -152,13 +152,6 @@ __device__ __forceinline__ void tc_tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) 
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-#ifdef EVAC_TC_TRACE  // measurement variant (never shipped): nanosecond stamps of CTA 0's phases
-#define TC_STAMP(i) do { if (blockIdx.x == 0 && blockIdx.y == 0 && (tid == 0 || tid == TC_ET)) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); tc_trace[tid == 0 ? 0 : 1][i] = t_; } } while (0)
-__device__ unsigned long long tc_trace[2][16];
-#else
-#define TC_STAMP(i)
-#endif
-
 template <int NT, int ST, int AH, int MINB>
 __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(const __grid_constant__ TCArgs a) {
   using SH = TCShape<NT, ST, AH>;
@@ -179,7 +172,6 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
   const int ny = TC_COLS / NT, y = blockIdx.y;   // NT = 64: y = 0 critic, y = 1 actor
   const HArgs& h = a.h;
 
-  TC_STAMP(0);
   if (tid == 0) {
     for (int s = 0; s < STAGES; ++s) { tc_mbar_init(&full[s], TC_ET); tc_mbar_init(&empty[s], 1); }
     tc_mbar_init(&accum[0], 1); tc_mbar_init(&accum[1], 1); tc_mbar_init(full2, TC_ET);
@@ -196,7 +188,6 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem = *tmem_slot;
-  TC_STAMP(1);
   uint8_t* a2 = smem;                       // H1 operand tiles: k-chunk j at j * 32 KB (hi | lo)
   uint8_t* w2 = smem + SH::A2_BYTES;        // layer-2 weight tiles of this CTA's head(s)
 
@@ -207,8 +198,6 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
     for (int c = 0; c < a.chunks; ++c) {
       const int s = c % STAGES;
       tc_mbar_wait(&full[s], (uint32_t)((c / STAGES) & 1));
-      if (c == 0) TC_STAMP(2);
-      if (c == a.chunks - 1) TC_STAMP(3);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       if (tc_elect()) {
         const uint32_t xh = tc_desc_lo(tc_smem_u32(smem + s * SH::STAGE_BYTES)), xl = xh + (TC_XTILE_BYTES >> 4);
@@ -229,7 +218,6 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
     }
     // ---- layer 2: per head [128 x 64] x [64 x 64], operands written by epilogue 1 / the second bulk copy
     tc_mbar_wait(full2, 0u);
-    TC_STAMP(4);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     if (tc_elect()) {
 #pragma unroll
@@ -277,7 +265,6 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
       if (c < a.chunks) request(c);
       cp_async_commit();
     }
-    TC_STAMP(2);
     for (int c = 0; c < a.chunks; ++c) {
       if (c + TC_AHEAD < a.chunks) request(c + TC_AHEAD);
       cp_async_commit();               // one group per iteration, empty or not: group index == chunk index
@@ -295,10 +282,8 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
       tc_mbar_arrive(&full[c % STAGES]);
     }
     // ---- epilogue 1: TMEM lane = environment (this thread's row), column = hidden unit -> H1 operand tiles of layer 2
-    TC_STAMP(3);
     tc_mbar_wait(&accum[0], 0u);           // every layer-1 MMA has completed: accumulators final, the ring is free
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    TC_STAMP(4);
     if (tid == 0) {
       tc_mbar_expect_tx(full2, SH::W2_BYTES);
       tc_bulk_load(w2, a.w2tc + (size_t)(NT == 64 ? y : 0) * (TC_W2_HEAD_BYTES / 4), SH::W2_BYTES, full2);
@@ -333,10 +318,8 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_mbar_arrive(full2);
-    TC_STAMP(5);
     // ---- epilogue 2: H2 = tanh(. + b2) and the output layer as dot products over the TMEM loads, then the sampling tail
     tc_mbar_wait(&accum[1], 0u);
-    TC_STAMP(6);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     float o[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll 1
@@ -359,7 +342,6 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
         }
       }
     }
-    TC_STAMP(7);
     const int e = e0 + row;
     if constexpr (NT == 128) {   // column half 0 = the critic's 64 columns, half 1 = the actor's: every thread finishes one head
 #pragma unroll
@@ -375,10 +357,8 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
       }
     }
   }
-  TC_STAMP(8);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  TC_STAMP(9);
   if (warp == TC_EW) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(TMEM_COLS) : "memory");

@@ -48,39 +48,24 @@ struct WPed {
   int st;       // status (ST_NONE for padding lanes)
 };
 
-#ifndef EVAC_WARP_MINB
 // resident warps per SM the register allocation is sized for.  28 -> 70 registers per thread, no spills in the step loop, and
 // still 29 warps per SM: the headline batch (4096 envs = 27.7 warps per SM) stays one wave.  Measured on B200 against 32
 // (64 registers, 8 bytes spilled per step): 9.23 -> 8.90 us per 4096-env step, 5.11 -> 4.92 us in-rollout; 24 (76 registers,
 // 26 warps per SM) pushes 4096 envs into a second wave: 9.81 us.
-#define EVAC_WARP_MINB 28
-#endif
-#ifndef EVAC_PAIR_UNROLL
-#define EVAC_PAIR_UNROLL 4  // slot pairs per unrolled iteration of the pairwise loop
-#endif
-// WPC = environments (independent warps) per CTA: fewer, fatter CTAs for the block scheduler; no block-level barrier anywhere.
-template <int MODE, int WPC>
-__global__ void __launch_bounds__(32 * WPC, EVAC_WARP_MINB / WPC) evac_warp_kernel(const __grid_constant__ KArgs<float> a) {  // @region wload
-  // Tile<float> of 64 slots (+ the look-ahead entries) per warp = 66 float4.  EVAC_OBS_STAGED (A/B variant): after the pairwise
-  // pass the same memory stages the observation row ((64 + 2) x 6 floats = 99 float4), see the observation section
-#if defined(EVAC_OBS_STAGED) || defined(EVAC_OBS_BULK)
-  __shared__ __align__(128) float4 tile_all[WPC][99];
-#else
-  __shared__ __align__(16) float4 tile_all[WPC][66];
-#endif
+constexpr int WARP_MINB = 28;
+constexpr int PAIR_UNROLL = 4;  // slot pairs per unrolled iteration of the pairwise loop
+// One environment per one-warp CTA (launch_warp in evac_abi.cu); no block-level barrier anywhere.
+template <int MODE>
+__global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_constant__ KArgs<float> a) {  // @region wload
+  // Tile<float> of 64 slots (+ the look-ahead entries) = 66 float4
+  __shared__ __align__(16) float4 tile_smem[66];
   // strip culling (a.cells_x > 0): the sources are sorted by vertical strip (edge >= vision radius) so that a
   // pedestrian only visits the slots of its own and the two adjacent strips
-  __shared__ uint2 strip_mask_all[WPC][32];   // per strip: which lanes' pedestrian 0 (.x) / pedestrian 1 (.y) sit in it
-  __shared__ int strip_start_all[WPC][33];    // first slot of every strip (+ total)
-  const int wic = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31, e = blockIdx.x * WPC + wic, N = a.N;
+  __shared__ uint2 strip_mask[32];   // per strip: which lanes' pedestrian 0 (.x) / pedestrian 1 (.y) sit in it
+  __shared__ int strip_start[33];    // first slot of every strip (+ total)
+  const int lane = threadIdx.x & 31, e = blockIdx.x, N = a.N;
   if (e >= a.E) return;
-#ifdef EVAC_PROBE_EMPTY  // measurement variant (never shipped): launch + CTA scheduling cost only
-  if (a.N >= 0) return;
-#endif
-  const Tile<float> tile(reinterpret_cast<unsigned char*>(tile_all[wic]), 64);
-  uint2* strip_mask = strip_mask_all[wic];
-  int* strip_start = strip_start_all[wic];
+  const Tile<float> tile(reinterpret_cast<unsigned char*>(tile_smem), 64);
   const int S = a.cells_x;
   const uint32_t lt_mask = (1u << lane) - 1u;
   const bool valid[2] = {lane < N, lane + 32 < N};
@@ -118,12 +103,6 @@ __global__ void __launch_bounds__(32 * WPC, EVAC_WARP_MINB / WPC) evac_warp_kern
   const float2 wall = make_float2(a.width, a.height);
 
   for (int s = 0; s < a.num_steps; ++s) {  // @region wrng
-#ifdef EVAC_PROBE_FLOOR  // measurement variant (never shipped): load -> observation -> write back, no dynamics
-    float2 act_tbl = make_float2(0.f, 0.f);
-    if (a.agent_kind == AGENT_TABLE) act_tbl = a.actions[(size_t)s * a.E + e];
-    ap.x += 1e-9f * act_tbl.x;
-    reward_sum += act_tbl.y;
-#else
     // ---------------- Time.step [area.py:53-59]
     const int now_prev = now;
     now += 1;
@@ -243,12 +222,8 @@ __global__ void __launch_bounds__(32 * WPC, EVAC_WARP_MINB / WPC) evac_warp_kern
       for (int k = 0; k < 2; ++k) windowed_pass(tile, win_lo[k], win_hi[k], q[k].p.x, q[k].p.y, a.thr2_ped, sx[k], sy[k]);
     } else {
       const float xi[2] = {q[0].p.x, q[1].p.x}, yi[2] = {q[0].p.y, q[1].p.y};
-#ifdef EVAC_PROBE_NOPAIR  // measurement variant (never shipped): the step without its pairwise pass
-      sx[0] = sx[1] = q[0].d.x; sy[0] = sy[1] = q[1].d.y;
-#else
-      if (__any_sync(0xffffffffu, fv[0] | fv[1])) pairwise_pass<2, false, EVAC_PAIR_UNROLL>(tile, n_src, xi, yi, a.thr2_ped, sx, sy, cnt);
+      if (__any_sync(0xffffffffu, fv[0] | fv[1])) pairwise_pass<2, false, PAIR_UNROLL>(tile, n_src, xi, yi, a.thr2_ped, sx, sy, cnt);
       else sx[0] = sx[1] = sy[0] = sy[1] = 0.f;
-#endif
     }
     // ---------------- new headings, enslaving, integration, reflection, statuses  // @region wupdate
     const float2 e_ad = make_float2(__fmul_rn(a.enslaving_f, ad.x), __fmul_rn(a.enslaving_f, ad.y));  // float32 like area.py:140
@@ -338,27 +313,19 @@ __global__ void __launch_bounds__(32 * WPC, EVAC_WARP_MINB / WPC) evac_warp_kern
         }
       }
     }
-#endif  // EVAC_PROBE_FLOOR
     // ---------------- observation [wrappers.py:8-96, gravity_encoding.py:8-81]  // @region wobs
-#if defined(EVAC_PROBE_NOOBS)
-    if (false) {
-#else
     if (obs_e != nullptr && (a.obs_every_step || s == a.num_steps - 1)) {
-#endif
       float* row = obs_e + (a.obs_every_step ? (size_t)s * a.E * a.obs_dim : (size_t)0);
       if constexpr (MODE == WMODE_REL_OHE_BOX) {
         // rows = [agent; exit; pedestrians], cols = [x, y, ohe(4)]; relative positions / sqrt(2) (float32 hypotenuse).
-        // Default: three float2 stores per pedestrian straight from registers (24-byte row stride: a warp's STG.64 touches 24
-        // sectors for 256 useful bytes, the sectors are completed in L2 by the neighbouring lanes' stores).
-        // EVAC_OBS_STAGED: the row is assembled in shared memory and copied out with one 16-byte (N even) or 8-byte store per
-        // lane and round -- 512 contiguous bytes per warp instruction.  Measured on B200, same box, 4096 x 60 per-step regime:
-        // the load -> observe -> write-back skeleton gets faster (5.23 -> 4.82 us) but the FULL step slower (8.42 -> 8.66 us:
-        // STS -> LDS -> STG adds a dependent shared-memory round trip to every warp's tail), so the direct stores stay.
-        // EVAC_OBS_BULK: the staged row leaves as ONE cp.async.bulk (shared -> global, the TMA engine's 1-D path; UBLKCP in the
-        // SASS) issued by lane 0, its wait deferred behind the state write-back: 8.76 vs 8.52 us, same box -- also slower.
+        // Three float2 stores per pedestrian straight from registers (24-byte row stride: a warp's STG.64 touches 24 sectors for
+        // 256 useful bytes, the sectors are completed in L2 by the neighbouring lanes' stores).  Measured on B200, same box,
+        // 4096 x 60 per-step regime, against a row staged in shared memory and copied out with one 16-byte store per lane and
+        // round: the load -> observe -> write-back skeleton gets faster (5.23 -> 4.82 us) but the FULL step slower (8.42 ->
+        // 8.66 us: STS -> LDS -> STG adds a dependent shared-memory round trip to every warp's tail); the staged row sent as ONE
+        // cp.async.bulk by lane 0: 8.76 vs 8.52 us -- also slower, so the direct stores stay.
         const float inv_hyp = (float)(1.0 / 1.41421353816986083984375);
         const float2 nap = make_float2(-ap.x, -ap.y);
-#if !defined(EVAC_OBS_STAGED) && !defined(EVAC_OBS_BULK)
         if (lane == 0) {
           const float2 ex = __fmul2_rn(__fadd2_rn(exit_p, nap), splat(inv_hyp));
           float2* r = reinterpret_cast<float2*>(row);
@@ -375,60 +342,6 @@ __global__ void __launch_bounds__(32 * WPC, EVAC_WARP_MINB / WPC) evac_warp_kern
             r[2] = make_float2(st == ST_FOLLOWER ? 1.f : 0.f, st == ST_VISCEK ? 1.f : 0.f);
           }
         }
-#else
-        float2* stage = reinterpret_cast<float2*>(tile_all[wic]);
-        if (lane == 0) {
-          const float2 ex = __fmul2_rn(__fadd2_rn(exit_p, nap), splat(inv_hyp));
-          stage[0] = ap; stage[1] = make_float2(0.f, 0.f); stage[2] = make_float2(0.f, 0.f);  // agent row, status [0,0,0,0]
-          stage[3] = ex; stage[4] = make_float2(1.f, 0.f); stage[5] = make_float2(0.f, 0.f);  // exit row,  status [1,0,0,0]
-        }
-#pragma unroll
-        for (int k = 0; k < 2; ++k) {
-          if (valid[k]) {
-            float2* r = stage + (lane + 32 * k + 2) * 3;
-            const int st = q[k].st;  // column 4 - status: ESCAPED -> 0, EXITING -> 1, FOLLOWER -> 2, VISCEK -> 3
-            r[0] = __fmul2_rn(__fadd2_rn(q[k].p, nap), splat(inv_hyp));
-            r[1] = make_float2(st == ST_ESCAPED ? 1.f : 0.f, st == ST_EXITING ? 1.f : 0.f);
-            r[2] = make_float2(st == ST_FOLLOWER ? 1.f : 0.f, st == ST_VISCEK ? 1.f : 0.f);
-          }
-        }
-#ifdef EVAC_OBS_BULK
-        // A/B variant: the staged row leaves the SM as ONE bulk asynchronous copy (cp.async.bulk shared -> global, the TMA
-        // engine's 1-D path) issued by lane 0, N even (24 (N + 2) bytes is then a multiple of 16)
-        if ((N & 1) == 0) {
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the async proxy
-          __syncwarp();
-          if (lane == 0) {
-            const uint32_t src = (uint32_t)__cvta_generic_to_shared(tile_all[wic]);
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(row), "r"(src), "r"((N + 2) * 24) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            // the tile may only be rewritten (next step) once the copy has read it; after the last step the wait moves behind
-            // the state write-back at the end of the kernel
-            if (s != a.num_steps - 1) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-          }
-        } else {
-          __syncwarp();
-          const int n8 = (N + 2) * 3;
-          float2* dst = reinterpret_cast<float2*>(row);
-#pragma unroll
-          for (int c = 0; c < 7; ++c) { const int j = lane + 32 * c; if (j < n8) dst[j] = stage[j]; }
-        }
-#else
-        __syncwarp();
-        if ((N & 1) == 0) {
-          const int n16 = (N + 2) * 3 / 2;  // float4 chunks of the row
-          const float4* src = tile_all[wic];
-          float4* dst = reinterpret_cast<float4*>(row);
-#pragma unroll
-          for (int c = 0; c < 4; ++c) { const int j = lane + 32 * c; if (j < n16) dst[j] = src[j]; }
-        } else {
-          const int n8 = (N + 2) * 3;
-          float2* dst = reinterpret_cast<float2*>(row);
-#pragma unroll
-          for (int c = 0; c < 7; ++c) { const int j = lane + 32 * c; if (j < n8) dst[j] = stage[j]; }
-        }
-#endif
-#endif
       } else if (MODE == WMODE_GRAV || a.positions == POS_GRAV) {
         // gravity encoding [gravity_encoding.py:8-38]: per VISCEK pedestrian -alpha / (|R| + eps)^(alpha + 2) * R, R = agent - p.
         // Straight-line and unconditional for both pedestrians of the lane (select, not branch); MUFU square root and
@@ -469,14 +382,9 @@ __global__ void __launch_bounds__(32 * WPC, EVAC_WARP_MINB / WPC) evac_warp_kern
   }  // steps
 
   // ---------------- write back  // @region wwriteback
-#if defined(EVAC_PROBE_NOSTATE)
-  if (q[0].p.x == 123.456f)
-#endif
-  {
-    ped_l[0] = make_float4(q[0].p.x, q[0].p.y, q[0].d.x, q[0].d.y);
-    ped_l[32] = make_float4(q[1].p.x, q[1].p.y, q[1].d.x, q[1].d.y);
-    *st_l = (unsigned short)(q[0].st | (q[1].st << 8));
-  }
+  ped_l[0] = make_float4(q[0].p.x, q[0].p.y, q[0].d.x, q[0].d.y);
+  ped_l[32] = make_float4(q[1].p.x, q[1].p.y, q[1].d.x, q[1].d.y);
+  *st_l = (unsigned short)(q[0].st | (q[1].st << 8));
   if (a.status_out != nullptr) {  // host face: dense [E,N] statuses travel in the result block
     uint8_t* so = a.status_out + (size_t)e * N + lane;
     if (valid[0]) so[0] = (uint8_t)q[0].st;
@@ -490,9 +398,6 @@ __global__ void __launch_bounds__(32 * WPC, EVAC_WARP_MINB / WPC) evac_warp_kern
     if (a.reward) a.reward[e] = reward_sum;
     if (a.terminated) a.terminated[e] = (uint8_t)any_term;
     if (a.truncated) a.truncated[e] = (uint8_t)any_trunc;
-#ifdef EVAC_OBS_BULK
-    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-#endif
   }
 }
 

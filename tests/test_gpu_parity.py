@@ -343,9 +343,8 @@ def test_cell_list_paired_walk_is_bit_identical_to_the_single_slot_walk(n, width
     dirs = np.stack([np.cos(ang), np.sin(ang)], axis=-1)
     actions = rs.uniform(-1, 1, (steps, E, 2)).astype(np.float32)
     out = {}
-    for walk in ("0", "1", "g"):  # one slot per thread / two adjacent slots per thread / four lanes sharing the window of 8 slots
-        monkeypatch.setenv("EVAC_CELL_PAIR_WALK", "0" if walk == "0" else "1")
-        monkeypatch.setenv("EVAC_CELL_GROUP", "1" if walk == "g" else "0")
+    for walk in ("0", "1"):  # one slot per thread / two adjacent slots per thread
+        monkeypatch.setenv("EVAC_CELL_PAIR_WALK", walk)
         env = _make_env(env_kw, wrap, E, neighbor_search="cells")
         u = env.unwrapped
         u.reset()
@@ -361,7 +360,6 @@ def test_cell_list_paired_walk_is_bit_identical_to_the_single_slot_walk(n, width
         u.close()
     for k in ("pos", "dir", "st", "rew", "obs"):
         assert np.array_equal(out["0"][k], out["1"][k], equal_nan=True), k
-        assert np.array_equal(out["0"][k], out["g"][k], equal_nan=True), ("grouped walk", k)
 
 
 def test_pedestrian_count_limits():

@@ -1,6 +1,6 @@
 """Standalone pairwise pass in the mappings of evac_probe_pairwise: EVAC_PROBE_HALFWARP unset = 32 lanes x 2 pedestrians (the fused
-step's), 1 | 2 | 4 = 16 x 4 (unroll), 8 = 8 x 8.  Prints one JSON line: TFLOP/s (8 flop per ordered pair) and fraction of the FFMA2 peak
-measured in the same process.  Usage: [EVAC_PROBE_HALFWARP=8] python tools/probe_pairwise_shapes.py"""
+step's), 2 = 16 x 4, 8 = 8 x 8.  Prints one JSON line: TFLOP/s (8 flop per ordered pair) and fraction of the FFMA2 peak
+measured in the same process.  Usage: [EVAC_PROBE_HALFWARP=2|8] python tools/probe_pairwise_shapes.py"""
 import ctypes as C, json, os, sys
 sys.path.insert(0, os.getcwd())
 from evacuation_b200 import _native as nat

@@ -1,6 +1,6 @@
 """Latency of the reference-shaped single environment through the drop-in API (`setup_env(EnvConfig(60), wrap).step(a)`, NumPy in /
 NumPy out, rng="numpy"): microseconds per step for the three wrapper sets of BASELINE.md section 3 item 1.
-EVAC_HOST_ZEROCOPY=0 selects the copy-engine path of evac_step_host for an A/B.  Usage: python tools/single_env_latency.py"""
+Usage: python tools/single_env_latency.py"""
 import json
 import os
 import sys
@@ -11,7 +11,7 @@ import numpy as np
 
 import evacuation_b200 as eb
 
-out = {"zerocopy": os.environ.get("EVAC_HOST_ZEROCOPY", "1")}
+out = {}
 for name, wrap in (("abs_no_dict", {}), ("rel_ohe_box", dict(positions="rel", statuses="ohe", type="Box")), ("grav_alpha3", dict(positions="grav", alpha=3))):
     env = eb.setup_env(eb.EnvConfig(number_of_pedestrians=60, wandb_enabled=False), eb.EnvWrappersConfig(**wrap), device="cuda:0")
     np.random.seed(0)

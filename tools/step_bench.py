@@ -1,5 +1,5 @@
 """Per-step timing in the bench's regime (R independent C2 batches stepped round-robin in one CUDA graph, inputs larger than
-L2) for the library selected by EVAC_B200_LIB -- used to A/B kernel variants in one gpurun call.
+L2) for the library selected by EVAC_B200_LIB (default: the in-tree build) -- compares two builds in one process per build.
 Usage: python tools/step_bench.py [E] [K] [R] [mode]   (mode: rel_ohe_box | grav)"""
 import json
 import os
