@@ -730,7 +730,7 @@ __global__ void __launch_bounds__(THREADS * WPC, MINB) probe_pairwise_kernel(con
   Tile<float> tile(smem_raw + (size_t)wic * Tile<float>::bytes(THREADS * PPT), THREADS * PPT);
   const int tid = threadIdx.x % THREADS, e = blockIdx.x * WPC + wic;
   if (e >= E) return;
-  float xi[PPT], yi[PPT], sx[PPT], sy[PPT], cnt[PPT], accx[PPT], accy[PPT];
+  float xi[PPT], yi[PPT], sx[PPT], sy[PPT], accx[PPT], accy[PPT];
 #pragma unroll
   for (int k = 0; k < PPT; ++k) {
     const int i = k * THREADS + tid;
@@ -741,7 +741,7 @@ __global__ void __launch_bounds__(THREADS * WPC, MINB) probe_pairwise_kernel(con
   }
   if (THREADS == 32) __syncwarp(); else __syncthreads();
   for (int r = 0; r < reps; ++r) {
-    pairwise_pass<PPT, false, UNR>(tile, N, xi, yi, thr2, sx, sy, cnt);
+    pairwise_pass<PPT, UNR>(tile, N, xi, yi, thr2, sx, sy);
 #pragma unroll
     for (int k = 0; k < PPT; ++k) {
       accx[k] += sx[k]; accy[k] += sy[k];

@@ -1,20 +1,21 @@
 // Crowds larger than one SM's shared memory: ONE environment per thread-block CLUSTER of CL CTAs (CL = 2, 4, 8;
 // 1024 threads x 4 pedestrians each -> up to 32 768 pedestrians), the cell-list neighbour search of
 // evac_kernels.cuh::cell_list_pass distributed over the cluster through distributed shared memory (DSMEM).
-// Included by evac_kernels.cuh (needs Tile, CellSmem, cell_of).  [area.py:105-119; SURVEY 8 row f3]
+// Included by evac_kernels.cuh (needs Tile, CellSmem and the phases shared with cell_list_pass).  [area.py:105-119; SURVEY 8 row f3]
 //
 //   CTA r owns pedestrians [r * SLOTS, (r + 1) * SLOTS) in registers (as in the one-CTA kernel) and the slice
 //   [r * SLOTS, (r + 1) * SLOTS) of the SORTED source tile in its shared memory.
-//   1. every CTA: histogram of its own moving pedestrians over the cells + rank inside (cell, CTA)      -> cluster barrier
-//   2. every CTA (redundantly): cell totals = sum of the CL histograms read through DSMEM, exclusive scan ->
-//      cell_start[] (global slot numbering), base[c] = cell_start[c] + pedestrians of lower-ranked CTAs in c.
-//      Global slot = base[c] + rank: the tile is sorted by (cell, pedestrian index) exactly like the one-CTA pass,
-//      so every float32 sum has the same value as there.
+//   1. every CTA: histogram of its own moving pedestrians over the cells + rank inside (cell, CTA) (rank_in_cells)
+//                                                                                                       -> cluster barrier
+//   2. every CTA (redundantly): cell totals = sum of the CL histograms read through DSMEM, exclusive scan (scan_cell_counts)
+//      -> cell_start[] (global slot numbering); below[c] = pedestrians of lower-ranked CTAs in c.
+//      Global slot = cell_start[c] + below[c] + rank: the tile is sorted by (cell, pedestrian index) exactly like the
+//      one-CTA pass, so every float32 sum has the same value as there.
 //   3. scatter of the source records into the tile slice of the CTA that owns the slot (DSMEM stores) -> cluster barrier
-//   4. paired walk (two adjacent sorted slots of one cell row per thread); the warps of the whole cluster draw chunks of
-//      slot pairs from one counter, so a crowd that has collapsed into one corner is still walked by all CTAs; tile reads
-//      go to whichever CTA owns the slot pair; the result goes to the CTA that owns the pedestrian     -> cluster barrier
-//   5. the owners read their results.
+//   4. paired walk (walk_slot_pair over ClusterSlots); the warps of the whole cluster draw chunks of slot pairs from one
+//      counter, so a crowd that has collapsed into one corner is still walked by all CTAs; tile reads go to whichever CTA
+//      owns the slot pair; the result goes to the CTA that owns the pedestrian                          -> cluster barrier
+//   5. the owners read their results (read_results).
 // (textually included inside namespace evac, after cell_list_pass; <cooperative_groups.h> comes from evac_kernels.cuh)
 #pragma once
 namespace cg = cooperative_groups;
@@ -22,13 +23,13 @@ namespace cg = cooperative_groups;
 // extra per-CTA arrays of the cluster pass, placed after CellSmem
 struct ClusterSmem {
   int* hist;    // [C + 1] own moving pedestrians per cell (read by the other CTAs)
-  int* base;    // [C + 1] first global slot of this CTA's pedestrians of each cell
+  int* below;   // [C + 1] moving pedestrians of the lower-ranked CTAs in each cell
   int* flags;   // [4]     [0] a source of this CTA has no direction (NaN poisoning)  [1] (CTA 0) next slot pair of the walk
   static __host__ __device__ constexpr size_t bytes(int cells) { return 2 * (((size_t)cells + 1 + 3) & ~(size_t)3) * 4 + 16; }
   __device__ __forceinline__ ClusterSmem(unsigned char* p, int cells) {
     hist = reinterpret_cast<int*>(p);
-    base = hist + ((cells + 1 + 3) & ~3);
-    flags = base + ((cells + 1 + 3) & ~3);
+    below = hist + ((cells + 1 + 3) & ~3);
+    flags = below + ((cells + 1 + 3) & ~3);
   }
 };
 
@@ -53,57 +54,57 @@ __device__ __forceinline__ float4 ld_cluster_f4(uint32_t addr) {
   return v;
 }
 
+// The sorted tile distributed over the cluster, with the interface of CtaSlots (evac_kernels.cuh): slot pair -> owning CTA by
+// owner_of_pair; a run is the part of [j, je) inside one CTA's slice, read with one MAPA and ld.shared::cluster; a result goes
+// to the shared memory of the CTA that owns the pedestrian.
+template <int SLOTS, int CL>
+struct ClusterSlots {
+  const Tile<float>& tile;
+  const CellSmem& cs;
+  struct Run {
+    uint32_t pa, ua;
+    __device__ __forceinline__ float4 p(int q) const { return ld_cluster_f4(pa + 16u * (uint32_t)q); }
+    __device__ __forceinline__ float4 u(int q) const { return ld_cluster_f4(ua + 16u * (uint32_t)q); }
+  };
+  __device__ __forceinline__ int sorted_idx(int s) const {
+    int owner, lp;
+    owner_of_pair<SLOTS, CL>(s >> 1, owner, lp);
+    return cg::this_cluster().map_shared_rank(cs.sorted_idx, owner)[s - owner * SLOTS];
+  }
+  __device__ __forceinline__ float4 p2(int pair) const {
+    int owner, lp;
+    owner_of_pair<SLOTS, CL>(pair, owner, lp);
+    return *cg::this_cluster().map_shared_rank(tile.P2 + lp, owner);
+  }
+  __device__ __forceinline__ Run run(int j, int je, int& end) const {
+    int owner, lp;
+    owner_of_pair<SLOTS, CL>(j, owner, lp);
+    end = owner == CL - 1 ? je : min(je, (owner + 1) * (SLOTS / 2));
+    const uint32_t pa = mapa_u32(smem_u32(tile.P2 + lp), owner);
+    return {pa, pa + (uint32_t)((SLOTS / 2 + 1) * sizeof(float4))};  // U2 = P2 + SLOTS / 2 + 1 in every CTA
+  }
+  __device__ __forceinline__ void put_res(int i, float2 r) const { cg::this_cluster().map_shared_rank(cs.res, i / SLOTS)[i % SLOTS] = r; }
+};
+
 template <int THREADS, int PPT, int CL, typename A>
 __device__ __forceinline__ void cell_list_pass_cluster(const Tile<float>& tile, const CellSmem& cs, const ClusterSmem& xs, const A& a,
                                                        const float (&px)[PPT], const float (&py)[PPT], const float (&ux)[PPT],
                                                        const float (&uy)[PPT], const bool (&efv)[PPT], const int (&st)[PPT],
                                                        float (&sx)[PPT], float (&sy)[PPT]) {
-  constexpr int WARPS = THREADS / 32, SLOTS = THREADS * PPT;
+  constexpr int SLOTS = THREADS * PPT;
   cg::cluster_group cluster = cg::this_cluster();
   const int rank_cta = (int)cluster.block_rank();
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int C = a.cells_x * a.cells_y;
-  // ---- 1. own histogram + rank inside (cell, CTA): lanes of one warp that share a cell find each other with MATCH.ANY,
-  // the leader records the group size in cnt[warp][cell] (uint8; aliases the tile slice, which is only written in step 3)
+  // ---- 1. own histogram + rank inside (cell, CTA); the [WARPS][C] byte table fits the tile slice (the host caps the grid at
+  // 2048 cells), and nobody writes the slice before the cluster barrier
   for (int c = tid; c <= C; c += THREADS) xs.hist[c] = 0;
   if (tid == 0) { xs.flags[0] = 0; xs.flags[1] = 0; }
   int cell[PPT], rank[PPT];
-  bool nan_src = false;
-  {
-    uint8_t* cnt = reinterpret_cast<uint8_t*>(tile.P2);  // [WARPS][C] <= the tile slice (the host caps the grid at 2048 cells)
-    const int n16 = (WARPS * C + 15) >> 4;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-#pragma unroll
-    for (int k = 0; k < PPT; ++k) {
-      for (int i = tid; i < n16; i += THREADS) reinterpret_cast<uint4*>(cnt)[i] = make_uint4(0u, 0u, 0u, 0u);
-      __syncthreads();
-      cell[k] = 0; rank[k] = 0;
-      int lrank = 0;
-      const uint32_t act = __ballot_sync(0xffffffffu, efv[k]);
-      if (efv[k]) {
-        int cx, cy;
-        cell[k] = cell_of(px[k], py[k], a, cx, cy);
-        nan_src |= (ux[k] != ux[k]) | (uy[k] != uy[k]);
-        const uint32_t peers = __match_any_sync(act, cell[k]);
-        lrank = __popc(peers & lt_mask);
-        if (lrank == 0) {
-          const int n = __popc(peers);
-          cnt[warp * C + cell[k]] = (uint8_t)n;
-          atomicAdd(&xs.hist[cell[k]], n);
-        }
-      }
-      __syncthreads();
-      if (efv[k]) {
-        int above = 0;
-        for (int w = warp; w < WARPS; ++w) above += cnt[w * C + cell[k]];
-        rank[k] = xs.hist[cell[k]] - above + lrank;
-      }
-      __syncthreads();
-    }
-  }
+  const bool nan_src = rank_in_cells<THREADS, PPT>(tile, xs.hist, a, px, py, ux, uy, efv, cell, rank);
   if (__syncthreads_or(nan_src) && tid == 0) xs.flags[0] = 1;
   cluster.sync();  // every histogram is final and nobody uses its tile slice as scratch any more
-  // ---- 2. cell totals over the cluster, exclusive scan, own base
+  // ---- 2. cell totals over the cluster, exclusive scan
   bool poisoned = false;
 #pragma unroll
   for (int r = 0; r < CL; ++r) poisoned |= cluster.map_shared_rank(xs.flags, r)[0] != 0;
@@ -118,31 +119,17 @@ __device__ __forceinline__ void cell_list_pass_cluster(const Tile<float>& tile, 
       }
     }
     cs.cell_start[c] = tot;
-    xs.base[c] = below;
+    xs.below[c] = below;
   }
   __syncthreads();
-  {
-    const int per = (C + THREADS) / THREADS;
-    const int lo = min(tid * per, C + 1), hi = min(lo + per, C + 1);
-    int sum = 0;
-    for (int c = lo; c < hi; ++c) sum += cs.cell_start[c];
-    int inc = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
-    if (lane == 31) cs.warp_tot[warp] = inc;
-    __syncthreads();
-    int off = inc - sum;
-    for (int w = 0; w < warp; ++w) off += cs.warp_tot[w];
-    for (int c = lo; c < hi; ++c) { const int v = cs.cell_start[c]; cs.cell_start[c] = off; xs.base[c] += off; off += v; }
-  }
-  __syncthreads();
-  const int n_src = cs.cell_start[C];
-  // ---- 3. scatter into the slice of the CTA that owns the slot
+  const int n_src = scan_cell_counts<THREADS>(cs, C);
+  // ---- 3. scatter into the slice of the CTA that owns the slot: global slot = cell start + pedestrians of the lower-ranked
+  // CTAs in the cell + rank inside (cell, CTA)
   const int base_i = rank_cta * SLOTS;
 #pragma unroll
   for (int k = 0; k < PPT; ++k) {
     if (efv[k]) {
-      const int g = xs.base[cell[k]] + rank[k];
+      const int g = cs.cell_start[cell[k]] + xs.below[cell[k]] + rank[k];
       int owner, lp;
       owner_of_pair<SLOTS, CL>(g >> 1, owner, lp);
       const bool fv = (unsigned)(st[k] - ST_VISCEK) <= (unsigned)(ST_FOLLOWER - ST_VISCEK);
@@ -159,31 +146,12 @@ __device__ __forceinline__ void cell_list_pass_cluster(const Tile<float>& tile, 
     owner_of_pair<SLOTS, CL>(g >> 1, owner, lp);
     if (owner == rank_cta) tile.put(2 * lp + (g & 1), PARK, PARK, 0.f, 0.f);
   }
-  if (warp == 0) {  // slot pairs per cell row, exclusive scan over the <= 64 rows
-    int cntp[2], inc = 0, run = 0;
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      const int r = lane + 32 * k;
-      cntp[k] = r < a.cells_y ? (cs.cell_start[(r + 1) * a.cells_x] - cs.cell_start[r * a.cells_x] + 1) >> 1 : 0;
-    }
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      inc = cntp[k];
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
-      const int r = lane + 32 * k;
-      if (r <= a.cells_y) cs.row_pairs[r] = run + inc - cntp[k];
-      run += __shfl_sync(0xffffffffu, inc, 31);
-    }
-    if (lane == 0 && a.cells_y == 64) cs.row_pairs[64] = run;
-  }
+  if (warp == 0) scan_row_pairs(cs, a);
   cluster.sync();  // the whole sorted tile is in place
   // ---- 4. paired walk.  The warps of the whole cluster draw chunks of 32 slot pairs from ONE counter (a DSMEM atomic on
   // CTA 0's shared memory): a walk costs as much as its cells are crowded, so equal shares of slot pairs would leave the
   // CTAs of a cluster waiting at the barrier for the one that drew the densest cells (ncu: `barrier` was the top stall).
   // The result of a pair does not depend on who walks it.
-  const float thr2 = a.thr2_ped;
-  const int reach = a.cell_reach;
   const int n_pairs = cs.row_pairs[a.cells_y];
   int* const next_pair = cluster.map_shared_rank(xs.flags, 0) + 1;
 #pragma unroll 1
@@ -193,93 +161,12 @@ __device__ __forceinline__ void cell_list_pass_cluster(const Tile<float>& tile, 
     tb = __shfl_sync(0xffffffffu, tb, 0);
     if (tb >= n_pairs) break;
     const int t = tb + lane;
-    if (t < n_pairs) do {  // (`continue` below leaves this one-trip loop)
-    int row = 0;
-    {
-      int hi_r = a.cells_y;
-      while (hi_r - row > 1) { const int mid = (row + hi_r) >> 1; if (cs.row_pairs[mid] <= t) row = mid; else hi_r = mid; }
-    }
-    const int row_end = cs.cell_start[(row + 1) * a.cells_x];
-    const int s0 = cs.cell_start[row * a.cells_x] + 2 * (t - cs.row_pairs[row]);
-    const bool two = s0 + 1 < row_end;
-    int o0, l0, o1 = 0, l1 = 0;
-    owner_of_pair<SLOTS, CL>(s0 >> 1, o0, l0);
-    if (two) owner_of_pair<SLOTS, CL>((s0 + 1) >> 1, o1, l1);
-    const int id0 = cluster.map_shared_rank(cs.sorted_idx, o0)[s0 - o0 * SLOTS];
-    const int id1 = two ? cluster.map_shared_rank(cs.sorted_idx, o1)[s0 + 1 - o1 * SLOTS] : 0;
-    if (!((id0 | id1) & 0x8000)) continue;
-    const float4 p0 = *cluster.map_shared_rank(tile.P2 + l0, o0);
-    const float x0 = (s0 & 1) ? p0.y : p0.x, y0 = (s0 & 1) ? p0.w : p0.z;
-    float x1 = x0, y1 = y0;
-    if (two) { const float4 p1 = *cluster.map_shared_rank(tile.P2 + l1, o1); x1 = ((s0 + 1) & 1) ? p1.y : p1.x; y1 = ((s0 + 1) & 1) ? p1.w : p1.z; }
-    int cxa, cxb, cy_;
-    cell_of(x0, y0, a, cxa, cy_);
-    cell_of(x1, y1, a, cxb, cy_);
-    const int cx0 = max(min(cxa, cxb) - reach, 0), cx1 = min(max(cxa, cxb) + reach, a.cells_x - 1);
-    const float2 nx0 = make_float2(-x0, -x0), ny0 = make_float2(-y0, -y0), nx1 = make_float2(-x1, -x1), ny1 = make_float2(-y1, -y1);
-    float2 ax0 = make_float2(0.f, 0.f), ay0 = ax0, ax1 = ax0, ay1 = ax0;
-    int done = 0;
-    for (int r = max(row - reach, 0); r <= min(row + reach, a.cells_y - 1); ++r) {
-      const int lo = max(cs.cell_start[r * a.cells_x + cx0] & ~1, done);
-      const int hi = (cs.cell_start[r * a.cells_x + cx1 + 1] + 1) & ~1;
-      int j = lo >> 1;
-      const int je = hi >> 1;
-      while (j < je) {
-        // one segment = the part of [j, je) inside one CTA's slice: plain pointer walk over that CTA's shared memory
-        int owner, lp;
-        owner_of_pair<SLOTS, CL>(j, owner, lp);
-        const int seg_end = owner == CL - 1 ? je : min(je, (owner + 1) * (SLOTS / 2));
-        const uint32_t pa = mapa_u32(smem_u32(tile.P2 + lp), owner);
-        const uint32_t ua = pa + (uint32_t)((SLOTS / 2 + 1) * sizeof(float4));  // U2 = P2 + SLOTS / 2 + 1 in every CTA
-        const int n = seg_end - j;
-        // software pipeline: the next slot pair is in flight while this one is evaluated (the look-ahead of the last
-        // iteration reads the spare entry behind the slice / the first U2 entry: allocated, never used)
-        float4 p = ld_cluster_f4(pa), u = ld_cluster_f4(ua);
-#pragma unroll 2
-        for (int q = 0; q < n; ++q) {
-          const float4 pn = ld_cluster_f4(pa + 16u * (uint32_t)(q + 1)), un = ld_cluster_f4(ua + 16u * (uint32_t)(q + 1));
-          const float2 sxp = make_float2(p.x, p.y), syp = make_float2(p.z, p.w), sux = make_float2(u.x, u.y), suy = make_float2(u.z, u.w);
-          {
-            const float2 dx = __fadd2_rn(sxp, nx0), dy = __fadd2_rn(syp, ny0);
-            float2 d2 = __fmul2_rn(dx, dx);
-            d2 = __ffma2_rn(dy, dy, d2);
-            const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-            ax0 = __ffma2_rn(w, sux, ax0);
-            ay0 = __ffma2_rn(w, suy, ay0);
-          }
-          {
-            const float2 dx = __fadd2_rn(sxp, nx1), dy = __fadd2_rn(syp, ny1);
-            float2 d2 = __fmul2_rn(dx, dx);
-            d2 = __ffma2_rn(dy, dy, d2);
-            const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-            ax1 = __ffma2_rn(w, sux, ax1);
-            ay1 = __ffma2_rn(w, suy, ay1);
-          }
-          p = pn;
-          u = un;
-        }
-        j = seg_end;
-      }
-      done = max(done, hi);
-    }
-    if (id0 & 0x8000) { const int i = id0 & 0x7fff; cluster.map_shared_rank(cs.res, i / SLOTS)[i % SLOTS] = make_float2(ax0.x + ax0.y, ay0.x + ay0.y); }
-    if (id1 & 0x8000) { const int i = id1 & 0x7fff; cluster.map_shared_rank(cs.res, i / SLOTS)[i % SLOTS] = make_float2(ax1.x + ax1.y, ay1.x + ay1.y); }
-    } while (0);
+    if (t < n_pairs) walk_slot_pair(ClusterSlots<SLOTS, CL>{tile, cs}, cs, a, t);
     __syncwarp();
   }
   cluster.sync();  // every result has reached its owner
   // ---- 5. back to the owners
-  const float qnan = __int_as_float(0x7fc00000);
-#pragma unroll
-  for (int k = 0; k < PPT; ++k) {
-    sx[k] = sy[k] = 0.f;
-    const bool fv = (unsigned)(st[k] - ST_VISCEK) <= (unsigned)(ST_FOLLOWER - ST_VISCEK);
-    if (fv) {
-      const float2 r = cs.res[k * THREADS + tid];
-      sx[k] = poisoned ? qnan : r.x;
-      sy[k] = poisoned ? qnan : r.y;
-    }
-  }
+  read_results<THREADS, PPT>(cs, poisoned, st, sx, sy);
 }
 
 // Sum of per-CTA partials over the cluster in rank order (every CTA gets the same bits).  `slot` is a [8]-double

@@ -288,6 +288,20 @@ struct Tile<float> {
   }
 };
 
+// THE pair evaluation of every float32 neighbour search: one slot pair of the tile (p = P2 entry, u = U2 entry) against one
+// pedestrian at (-nx, -ny) (splatted), adds the unit directions of the slots with d² < thr² to (ax, ay).  The host picks thr²
+// (sq_boundary, evac_abi.cu) so that this strict < on this float32 expression equals sqrt(d²) < radius.  w * u with w = 0 and
+// u = NaN gives NaN, like the reference's (intersection * efv_directions) product.
+__device__ __forceinline__ void accumulate_pair(float4 p, float4 u, float2 nx, float2 ny, float thr2, float2& ax, float2& ay) {
+  const float2 dx = __fadd2_rn(make_float2(p.x, p.y), nx);
+  const float2 dy = __fadd2_rn(make_float2(p.z, p.w), ny);
+  float2 d2 = __fmul2_rn(dx, dx);
+  d2 = __ffma2_rn(dy, dy, d2);
+  const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
+  ax = __ffma2_rn(w, make_float2(u.x, u.y), ax);
+  ay = __ffma2_rn(w, make_float2(u.z, u.w), ay);
+}
+
 template <>
 struct Tile<double> {
   double *X, *Y, *UX, *UY;
@@ -308,17 +322,15 @@ struct Tile<double> {
 
 // The pairwise neighbour-alignment pass [area.py:105-119]: for each of this thread's PPT pedestrians
 // i, sum the unit directions of all slots j with |p_i - p_j|^2 < thr2 (self included).
-// count[] (number of neighbours, area.py:108) is only produced when COUNT is set (fp64 parity mode).
-template <int PPT, bool COUNT, int UNR = 4>  // @region pairwise
+// The fp64 pass (parity mode) also returns cnt[], the number of neighbours (area.py:108).
+template <int PPT, int UNR = 4>  // @region pairwise
 __device__ __forceinline__ void pairwise_pass(const Tile<float>& t, int nslots, const float (&xi)[PPT],
-                                              const float (&yi)[PPT], float thr2, float (&sx)[PPT], float (&sy)[PPT],
-                                              float (&cnt)[PPT]) {
-  float2 ax[PPT], ay[PPT], ac[PPT], nx[PPT], ny[PPT];
+                                              const float (&yi)[PPT], float thr2, float (&sx)[PPT], float (&sy)[PPT]) {
+  float2 ax[PPT], ay[PPT], nx[PPT], ny[PPT];
 #pragma unroll
   for (int k = 0; k < PPT; ++k) {
     ax[k] = make_float2(0.f, 0.f);
     ay[k] = make_float2(0.f, 0.f);
-    ac[k] = make_float2(0.f, 0.f);
     nx[k] = make_float2(-xi[k], -xi[k]);
     ny[k] = make_float2(-yi[k], -yi[k]);
   }
@@ -332,16 +344,7 @@ __device__ __forceinline__ void pairwise_pass(const Tile<float>& t, int nslots, 
     const float4 pn = t.P2[j + 1];
     const float4 un = t.U2[j + 1];
 #pragma unroll
-    for (int k = 0; k < PPT; ++k) {
-      const float2 dx = __fadd2_rn(make_float2(p.x, p.y), nx[k]);
-      const float2 dy = __fadd2_rn(make_float2(p.z, p.w), ny[k]);
-      float2 d2 = __fmul2_rn(dx, dx);
-      d2 = __ffma2_rn(dy, dy, d2);
-      const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-      ax[k] = __ffma2_rn(w, make_float2(u.x, u.y), ax[k]);  // 0 * NaN = NaN, like the reference's
-      ay[k] = __ffma2_rn(w, make_float2(u.z, u.w), ay[k]);  // (intersection * efv_directions) product
-      if (COUNT) ac[k] = __fadd2_rn(ac[k], w);
-    }
+    for (int k = 0; k < PPT; ++k) accumulate_pair(p, u, nx[k], ny[k], thr2, ax[k], ay[k]);
     p = pn;
     u = un;
   }
@@ -349,11 +352,10 @@ __device__ __forceinline__ void pairwise_pass(const Tile<float>& t, int nslots, 
   for (int k = 0; k < PPT; ++k) {
     sx[k] = ax[k].x + ax[k].y;
     sy[k] = ay[k].x + ay[k].y;
-    cnt[k] = ac[k].x + ac[k].y;
   }
 }
 
-template <int PPT, bool COUNT>  // @region pairwise64
+template <int PPT>  // @region pairwise64
 __device__ __forceinline__ void pairwise_pass(const Tile<double>& t, int nslots, const double (&xi)[PPT],
                                               const double (&yi)[PPT], double thr2, double (&sx)[PPT],
                                               double (&sy)[PPT], double (&cnt)[PPT]) {
@@ -385,8 +387,9 @@ __device__ __forceinline__ void pairwise_pass(const Tile<double>& t, int nslots,
 //      order, hence every float32 result, is deterministic
 //   5. threads walk the SORTED slots (neighbouring lanes sit in the same / adjacent cells: shared-memory
 //      broadcasts, coherent trip counts), three contiguous slot ranges (one per cell row), packed f32x2
-//      pair evaluation like pairwise_pass; result scattered to res[original index]
+//      pair evaluation (accumulate_pair); result scattered to res[original index]
 //   6. the owner threads read res[] back.
+// Steps 1, 2, the paired walk of step 5 and step 6 are functions shared with the cluster pass (evac_cluster.cuh).
 struct CellSmem {
   float2* res;           // [SLOTS]  (aliases `list` until step 5)
   uint16_t* list;        // [SLOTS]  provisional cell lists
@@ -414,6 +417,196 @@ __device__ __forceinline__ int cell_of(float x, float y, const A& a, int& cx, in
   return cy * a.cells_x + cx;
 }
 
+// ---- Phases shared by cell_list_pass (one CTA) and cell_list_pass_cluster (evac_cluster.cuh).  Both sort the sources by
+// (cell, pedestrian index), so every float32 sum has the same value in either.
+
+// Step 1: the cell of every moving pedestrian and its rank among the moving pedestrians of that cell in pedestrian index
+// order (pass k, warp, lane); the cell totals are added to count[] (zeroed by the caller).
+//   * lanes of one warp that share a cell find each other with MATCH.ANY (rank among them = lower lanes),
+//   * the leader records the group size in cnt[warp][cell] (uint8, [WARPS][C] bytes that alias the tile: the caller writes
+//     the tile only afterwards) and adds it to the counter (integer atomics commute),
+//   * after the barrier a source's rank is counter-after-this-pass minus the groups of the warps at or above its own.
+// Returns whether one of this thread's sources has no direction.
+template <int THREADS, int PPT, typename A>
+__device__ __forceinline__ bool rank_in_cells(const Tile<float>& tile, int* count, const A& a, const float (&px)[PPT],
+                                              const float (&py)[PPT], const float (&ux)[PPT], const float (&uy)[PPT],
+                                              const bool (&efv)[PPT], int (&cell)[PPT], int (&rank)[PPT]) {
+  constexpr int WARPS = THREADS / 32;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int C = a.cells_x * a.cells_y;
+  uint8_t* cnt = reinterpret_cast<uint8_t*>(tile.P2);
+  const int n16 = (WARPS * C + 15) >> 4;
+  const uint32_t lt_mask = (1u << lane) - 1u;
+  bool nan_src = false;
+#pragma unroll
+  for (int k = 0; k < PPT; ++k) {
+    for (int i = tid; i < n16; i += THREADS) reinterpret_cast<uint4*>(cnt)[i] = make_uint4(0u, 0u, 0u, 0u);
+    __syncthreads();
+    cell[k] = 0; rank[k] = 0;
+    int lrank = 0;
+    const uint32_t act = __ballot_sync(0xffffffffu, efv[k]);
+    if (efv[k]) {
+      int cx, cy;
+      cell[k] = cell_of(px[k], py[k], a, cx, cy);
+      nan_src |= (ux[k] != ux[k]) | (uy[k] != uy[k]);
+      const uint32_t peers = __match_any_sync(act, cell[k]);
+      lrank = __popc(peers & lt_mask);
+      if (lrank == 0) {
+        const int n = __popc(peers);
+        cnt[warp * C + cell[k]] = (uint8_t)n;
+        atomicAdd(&count[cell[k]], n);
+      }
+    }
+    __syncthreads();
+    if (efv[k]) {
+      int above = 0;
+      for (int w = warp; w < WARPS; ++w) above += cnt[w * C + cell[k]];
+      rank[k] = count[cell[k]] - above + lrank;
+    }
+    __syncthreads();  // cnt is cleared and the counters move on in the next pass
+  }
+  return nan_src;
+}
+
+// Step 2: exclusive scan of the C + 1 counters cs.cell_start[] in place (entry C receives the total).  Returns the total,
+// after a barrier.
+template <int THREADS>
+__device__ __forceinline__ int scan_cell_counts(const CellSmem& cs, int C) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int per = (C + THREADS) / THREADS;  // ceil((C + 1) / THREADS)
+  const int lo = min(tid * per, C + 1), hi = min(lo + per, C + 1);
+  int sum = 0;
+  for (int c = lo; c < hi; ++c) sum += cs.cell_start[c];
+  int inc = sum;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
+  if (lane == 31) cs.warp_tot[warp] = inc;
+  __syncthreads();
+  int off = inc - sum;
+  for (int w = 0; w < warp; ++w) off += cs.warp_tot[w];
+  for (int c = lo; c < hi; ++c) { const int v = cs.cell_start[c]; cs.cell_start[c] = off; off += v; }
+  __syncthreads();
+  return cs.cell_start[C];
+}
+
+// Paired walk, by warp 0: slot pairs per cell row (a pair never straddles two rows), exclusive scan over the <= 64 rows ->
+// cs.row_pairs[].
+template <typename A>
+__device__ __forceinline__ void scan_row_pairs(const CellSmem& cs, const A& a) {
+  const int lane = threadIdx.x & 31;
+  int cnt[2], inc = 0, run = 0;
+#pragma unroll
+  for (int k = 0; k < 2; ++k) {
+    const int r = lane + 32 * k;
+    cnt[k] = r < a.cells_y ? (cs.cell_start[(r + 1) * a.cells_x] - cs.cell_start[r * a.cells_x] + 1) >> 1 : 0;
+  }
+#pragma unroll
+  for (int k = 0; k < 2; ++k) {
+    inc = cnt[k];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
+    const int r = lane + 32 * k;
+    if (r <= a.cells_y) cs.row_pairs[r] = run + inc - cnt[k];
+    run += __shfl_sync(0xffffffffu, inc, 31);
+  }
+  if (lane == 0 && a.cells_y == 64) cs.row_pairs[64] = run;
+}
+
+// The sorted slots as the paired walk sees them in one CTA: sorted_idx[], the tile and res[] in this CTA's shared memory.
+// run(j, je, end): the slot pairs [j, end) that p(q) / u(q) read from one base (here all of [j, je)).
+// (The cluster pass has the same interface over the tile distributed across the cluster: ClusterSlots, evac_cluster.cuh.)
+struct CtaSlots {
+  const Tile<float>& tile;
+  const CellSmem& cs;
+  struct Run {
+    const float4 *P, *U;
+    __device__ __forceinline__ float4 p(int q) const { return P[q]; }
+    __device__ __forceinline__ float4 u(int q) const { return U[q]; }
+  };
+  __device__ __forceinline__ int sorted_idx(int s) const { return cs.sorted_idx[s]; }
+  __device__ __forceinline__ float4 p2(int pair) const { return tile.P2[pair]; }
+  __device__ __forceinline__ Run run(int j, int je, int& end) const {
+    end = je;
+    return {tile.P2 + j, tile.U2 + j};
+  }
+  __device__ __forceinline__ void put_res(int i, float2 r) const { cs.res[i] = r; }
+};
+
+// Paired walk of slot pair t: the two adjacent sorted slots 2t', 2t' + 1 of ONE cell row (row_pairs[] numbering) sit in the
+// same or in neighbouring cells, so one walk over the union of their windows serves both -- every loaded source pair is
+// evaluated against two pedestrians (half the LDS per evaluated pair, like the 2-pedestrians-per-lane all-pairs pass).  A slot
+// outside a pedestrian's own window fails the distance test and adds an exact zero, so the sums equal the one-slot walk bit
+// for bit.  cs: this CTA's cell_start[] and row_pairs[]; Slots: where the sorted slots and the results live.
+template <typename Slots, typename A>
+__device__ __forceinline__ void walk_slot_pair(const Slots& slots, const CellSmem& cs, const A& a, int t) {
+  int row = 0;
+  {  // largest row with row_pairs[row] <= t
+    int hi_r = a.cells_y;
+    while (hi_r - row > 1) { const int mid = (row + hi_r) >> 1; if (cs.row_pairs[mid] <= t) row = mid; else hi_r = mid; }
+  }
+  const int row_end = cs.cell_start[(row + 1) * a.cells_x];
+  const int s0 = cs.cell_start[row * a.cells_x] + 2 * (t - cs.row_pairs[row]);
+  const bool two = s0 + 1 < row_end;
+  const int id0 = slots.sorted_idx(s0), id1 = two ? slots.sorted_idx(s0 + 1) : 0;
+  if (!((id0 | id1) & 0x8000)) return;
+  const float4 p0 = slots.p2(s0 >> 1);
+  const float x0 = (s0 & 1) ? p0.y : p0.x, y0 = (s0 & 1) ? p0.w : p0.z;
+  float x1 = x0, y1 = y0;
+  if (two) { const float4 p1 = slots.p2((s0 + 1) >> 1); x1 = ((s0 + 1) & 1) ? p1.y : p1.x; y1 = ((s0 + 1) & 1) ? p1.w : p1.z; }
+  const int reach = a.cell_reach;
+  int cxa, cxb, cy_;
+  cell_of(x0, y0, a, cxa, cy_);
+  cell_of(x1, y1, a, cxb, cy_);
+  const int cx0 = max(min(cxa, cxb) - reach, 0), cx1 = min(max(cxa, cxb) + reach, a.cells_x - 1);
+  const float2 nx0 = make_float2(-x0, -x0), ny0 = make_float2(-y0, -y0), nx1 = make_float2(-x1, -x1), ny1 = make_float2(-y1, -y1);
+  const float thr2 = a.thr2_ped;
+  float2 ax0 = make_float2(0.f, 0.f), ay0 = ax0, ax1 = ax0, ay1 = ax0;
+  int done = 0;  // even slot index below which everything has been evaluated already
+  for (int r = max(row - reach, 0); r <= min(row + reach, a.cells_y - 1); ++r) {
+    const int lo = max(cs.cell_start[r * a.cells_x + cx0] & ~1, done);
+    const int hi = (cs.cell_start[r * a.cells_x + cx1 + 1] + 1) & ~1;
+    int j = lo >> 1;
+    const int je = hi >> 1;
+    while (j < je) {
+      int end;
+      const typename Slots::Run run = slots.run(j, je, end);
+      // software pipeline: the next slot pair is in flight while this one is evaluated (the look-ahead of the last iteration
+      // reads one entry past the run: at most the spare entry behind the tile or slice, allocated and never used)
+      float4 p = run.p(0), u = run.u(0);
+#pragma unroll 2
+      for (int q = 0; q < end - j; ++q) {
+        const float4 pn = run.p(q + 1), un = run.u(q + 1);
+        accumulate_pair(p, u, nx0, ny0, thr2, ax0, ay0);
+        accumulate_pair(p, u, nx1, ny1, thr2, ax1, ay1);
+        p = pn;
+        u = un;
+      }
+      j = end;
+    }
+    done = max(done, hi);
+  }
+  if (id0 & 0x8000) slots.put_res(id0 & 0x7fff, make_float2(ax0.x + ax0.y, ay0.x + ay0.y));
+  if (id1 & 0x8000) slots.put_res(id1 & 0x7fff, make_float2(ax1.x + ax1.y, ay1.x + ay1.y));
+}
+
+// Last step: the owners read their results back from res[]; one source without a direction poisons EVERY sum in the
+// reference (0 * NaN = NaN, area.py:101,118).
+template <int THREADS, int PPT>
+__device__ __forceinline__ void read_results(const CellSmem& cs, bool poisoned, const int (&st)[PPT], float (&sx)[PPT],
+                                             float (&sy)[PPT]) {
+  const float qnan = __int_as_float(0x7fc00000);
+#pragma unroll
+  for (int k = 0; k < PPT; ++k) {
+    sx[k] = sy[k] = 0.f;
+    const bool fv = (unsigned)(st[k] - ST_VISCEK) <= (unsigned)(ST_FOLLOWER - ST_VISCEK);
+    if (fv) {
+      const float2 r = cs.res[k * THREADS + threadIdx.x];
+      sx[k] = poisoned ? qnan : r.x;
+      sy[k] = poisoned ? qnan : r.y;
+    }
+  }
+}
+
 template <int THREADS, int PPT, typename A>
 __device__ __forceinline__ void cell_list_pass(const Tile<float>& tile, const CellSmem& cs, const A& a, const float (&px)[PPT],
                                                const float (&py)[PPT], const float (&ux)[PPT], const float (&uy)[PPT],
@@ -421,49 +614,15 @@ __device__ __forceinline__ void cell_list_pass(const Tile<float>& tile, const Ce
   constexpr int WARPS = THREADS / 32;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int C = a.cells_x * a.cells_y;
-  // ---- 1. histogram + rank of every source inside its cell.  The tile must come out sorted by (cell, pedestrian
-  // index) so that every float32 sum is deterministic.  Pedestrian index order = (pass k, warp, lane):
-  //   * lanes of one warp that share a cell find each other with MATCH.ANY (rank among them = lower lanes),
-  //   * the leader records the group size in cnt[warp][cell] (uint8; aliases the tile, which is only written in step 4)
-  //     and adds it to the cell counter (integer atomics commute),
-  //   * after the barrier a source's rank is counter-after-this-pass minus the groups of the warps at or above its own.
-  // If the [WARPS][C] byte table does not fit in the tile (more than 2048 cells at 32 warps) the ranks come from the
-  // arrival order of the atomics and are made canonical by counting lower indices in the cell (step 4b).
+  // ---- 1. histogram + rank of every source inside its cell (rank_in_cells).  If its [WARPS][C] byte table does not fit in
+  // the tile (more than 2048 cells at 32 warps) the ranks come from the arrival order of the atomics and are made canonical
+  // by counting lower indices in the cell (step 4b).
   for (int c = tid; c <= C; c += THREADS) cs.cell_start[c] = 0;
   int cell[PPT], rank[PPT];
   bool nan_src = false;
   const bool fast_rank = (size_t)WARPS * C + 16 <= Tile<float>::bytes(THREADS * PPT);
   if (fast_rank) {
-    uint8_t* cnt = reinterpret_cast<uint8_t*>(tile.P2);
-    const int n16 = (WARPS * C + 15) >> 4;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-#pragma unroll
-    for (int k = 0; k < PPT; ++k) {
-      for (int i = tid; i < n16; i += THREADS) reinterpret_cast<uint4*>(cnt)[i] = make_uint4(0u, 0u, 0u, 0u);
-      __syncthreads();
-      cell[k] = 0; rank[k] = 0;
-      int lrank = 0;
-      const uint32_t act = __ballot_sync(0xffffffffu, efv[k]);
-      if (efv[k]) {
-        int cx, cy;
-        cell[k] = cell_of(px[k], py[k], a, cx, cy);
-        nan_src |= (ux[k] != ux[k]) | (uy[k] != uy[k]);
-        const uint32_t peers = __match_any_sync(act, cell[k]);
-        lrank = __popc(peers & lt_mask);
-        if (lrank == 0) {
-          const int n = __popc(peers);
-          cnt[warp * C + cell[k]] = (uint8_t)n;
-          atomicAdd(&cs.cell_start[cell[k]], n);
-        }
-      }
-      __syncthreads();
-      if (efv[k]) {
-        int above = 0;
-        for (int w = warp; w < WARPS; ++w) above += cnt[w * C + cell[k]];
-        rank[k] = cs.cell_start[cell[k]] - above + lrank;
-      }
-      __syncthreads();  // cnt is cleared and the counters move on in the next pass
-    }
+    nan_src = rank_in_cells<THREADS, PPT>(tile, cs.cell_start, a, px, py, ux, uy, efv, cell, rank);
   } else {
     __syncthreads();
 #pragma unroll
@@ -477,25 +636,9 @@ __device__ __forceinline__ void cell_list_pass(const Tile<float>& tile, const Ce
       }
     }
   }
-  // 0 * NaN = NaN: one source without a direction poisons EVERY sum in the reference (area.py:101,118)
   const bool poisoned = __syncthreads_or(nan_src);
-  // ---- 2. exclusive scan of the C + 1 counters (entry C receives the total)
-  {
-    const int per = (C + THREADS) / THREADS;  // ceil((C + 1) / THREADS)
-    const int lo = min(tid * per, C + 1), hi = min(lo + per, C + 1);
-    int sum = 0;
-    for (int c = lo; c < hi; ++c) sum += cs.cell_start[c];
-    int inc = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
-    if (lane == 31) cs.warp_tot[warp] = inc;
-    __syncthreads();
-    int off = inc - sum;
-    for (int w = 0; w < warp; ++w) off += cs.warp_tot[w];
-    for (int c = lo; c < hi; ++c) { const int v = cs.cell_start[c]; cs.cell_start[c] = off; off += v; }
-  }
-  __syncthreads();
-  const int n_src = cs.cell_start[C];
+  // ---- 2. exclusive scan of the C + 1 counters
+  const int n_src = scan_cell_counts<THREADS>(cs, C);
   // ---- 3. (arrival-order ranks only) provisional scatter, 4b. canonical rank = number of lower indices in the cell
   if (!fast_rank) {
 #pragma unroll
@@ -525,153 +668,56 @@ __device__ __forceinline__ void cell_list_pass(const Tile<float>& tile, const Ce
     }
   }
   if (tid < 2) tile.put(n_src + tid, PARK, PARK, 0.f, 0.f);  // pad to an even count (the tile has 2 spare slots)
-  if (a.cell_pair_walk && warp == 0) {
-    // slot pairs per cell row (a pair never straddles two rows) -- exclusive scan over the <= 64 rows by one warp
-    int cnt[2], inc = 0;
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      const int r = lane + 32 * k;
-      cnt[k] = r < a.cells_y ? (cs.cell_start[(r + 1) * a.cells_x] - cs.cell_start[r * a.cells_x] + 1) >> 1 : 0;
-    }
-    int run = 0;
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      inc = cnt[k];
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
-      const int r = lane + 32 * k;
-      if (r <= a.cells_y) cs.row_pairs[r] = run + inc - cnt[k];
-      run += __shfl_sync(0xffffffffu, inc, 31);
-    }
-    if (lane == 0 && a.cells_y == 64) cs.row_pairs[64] = run;
-  }
+  if (a.cell_pair_walk && warp == 0) scan_row_pairs(cs, a);
   __syncthreads();  // list[] (aliased by res[]) is dead from here on
   // ---- 5. walk the sorted slots
-  const float thr2 = a.thr2_ped;
   if (a.cell_pair_walk) {
-    // Two adjacent sorted slots of ONE cell row per thread: they sit in the same or in neighbouring cells, so one walk over
-    // the union of their windows serves both -- every loaded source pair is evaluated against two pedestrians (half the
-    // LDS per evaluated pair, like the 2-pedestrians-per-lane all-pairs pass).  A slot outside a pedestrian's own window
-    // fails the distance test and adds an exact zero, so the sums equal the one-slot walk bit for bit.
-    const int reach = a.cell_reach;
-    const int n_pairs = cs.row_pairs[a.cells_y];
     // chunks of 32 slot pairs are handed to the warps statically: warp w walks chunks w, w + WARPS, ...
+    const int n_pairs = cs.row_pairs[a.cells_y];
 #pragma unroll 1
     for (int chunk = warp; chunk * 32 < n_pairs; chunk += WARPS) {
       const int t = chunk * 32 + lane;
-      if (t >= n_pairs) continue;
-      int row = 0;
-      {  // largest row with row_pairs[row] <= t
-        int hi_r = a.cells_y;
-        while (hi_r - row > 1) { const int mid = (row + hi_r) >> 1; if (cs.row_pairs[mid] <= t) row = mid; else hi_r = mid; }
-      }
-      const int row_end = cs.cell_start[(row + 1) * a.cells_x];
-      const int s0 = cs.cell_start[row * a.cells_x] + 2 * (t - cs.row_pairs[row]);
-      const bool two = s0 + 1 < row_end;
-      const int id0 = cs.sorted_idx[s0], id1 = two ? cs.sorted_idx[s0 + 1] : 0;
-      if (!((id0 | id1) & 0x8000)) continue;
-      const float4 p0 = tile.P2[s0 >> 1];
-      const float x0 = (s0 & 1) ? p0.y : p0.x, y0 = (s0 & 1) ? p0.w : p0.z;
-      float x1 = x0, y1 = y0;
-      if (two) { const float4 p1 = tile.P2[(s0 + 1) >> 1]; x1 = ((s0 + 1) & 1) ? p1.y : p1.x; y1 = ((s0 + 1) & 1) ? p1.w : p1.z; }
-      int cxa, cxb, cy_;
-      cell_of(x0, y0, a, cxa, cy_);
-      cell_of(x1, y1, a, cxb, cy_);
-      const int cx0 = max(min(cxa, cxb) - reach, 0), cx1 = min(max(cxa, cxb) + reach, a.cells_x - 1);
-      const float2 nx0 = make_float2(-x0, -x0), ny0 = make_float2(-y0, -y0), nx1 = make_float2(-x1, -x1), ny1 = make_float2(-y1, -y1);
-      float2 ax0 = make_float2(0.f, 0.f), ay0 = ax0, ax1 = ax0, ay1 = ax0;
-      int done = 0;
-      for (int r = max(row - reach, 0); r <= min(row + reach, a.cells_y - 1); ++r) {
-        const int lo = max(cs.cell_start[r * a.cells_x + cx0] & ~1, done);
-        const int hi = (cs.cell_start[r * a.cells_x + cx1 + 1] + 1) & ~1;
+      if (t < n_pairs) walk_slot_pair(CtaSlots{tile, cs}, cs, a, t);
+    }
+  } else {
+    const float thr2 = a.thr2_ped;
+#pragma unroll 1
+    for (int s = tid; s < n_src; s += THREADS) {
+      const int id = cs.sorted_idx[s];
+      if (!(id & 0x8000)) continue;
+      const float4 pp = tile.P2[s >> 1];
+      const float x = (s & 1) ? pp.y : pp.x, y = (s & 1) ? pp.w : pp.z;
+      int cx, cy;
+      cell_of(x, y, a, cx, cy);
+      const int reach = a.cell_reach;
+      const int cx0 = max(cx - reach, 0), cx1 = min(cx + reach, a.cells_x - 1);
+      const float2 nx = make_float2(-x, -x), ny = make_float2(-y, -y);
+      float2 ax = make_float2(0.f, 0.f), ay = make_float2(0.f, 0.f);
+      int done = 0;  // even slot index below which everything has been evaluated already
+      for (int row = max(cy - reach, 0); row <= min(cy + reach, a.cells_y - 1); ++row) {
+        const int lo = max(cs.cell_start[row * a.cells_x + cx0] & ~1, done);
+        const int hi = (cs.cell_start[row * a.cells_x + cx1 + 1] + 1) & ~1;
         int j = lo >> 1;
         const int je = hi >> 1;
         if (j < je) {
+          // software pipeline as in walk_slot_pair
           float4 p = tile.P2[j], u = tile.U2[j];
 #pragma unroll 2
           for (; j < je; ++j) {
             const float4 pn = tile.P2[j + 1], un = tile.U2[j + 1];
-            const float2 sxp = make_float2(p.x, p.y), syp = make_float2(p.z, p.w), sux = make_float2(u.x, u.y), suy = make_float2(u.z, u.w);
-            {
-              const float2 dx = __fadd2_rn(sxp, nx0), dy = __fadd2_rn(syp, ny0);
-              float2 d2 = __fmul2_rn(dx, dx);
-              d2 = __ffma2_rn(dy, dy, d2);
-              const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-              ax0 = __ffma2_rn(w, sux, ax0);
-              ay0 = __ffma2_rn(w, suy, ay0);
-            }
-            {
-              const float2 dx = __fadd2_rn(sxp, nx1), dy = __fadd2_rn(syp, ny1);
-              float2 d2 = __fmul2_rn(dx, dx);
-              d2 = __ffma2_rn(dy, dy, d2);
-              const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-              ax1 = __ffma2_rn(w, sux, ax1);
-              ay1 = __ffma2_rn(w, suy, ay1);
-            }
+            accumulate_pair(p, u, nx, ny, thr2, ax, ay);
             p = pn;
             u = un;
           }
         }
         done = max(done, hi);
       }
-      if (id0 & 0x8000) cs.res[id0 & 0x7fff] = make_float2(ax0.x + ax0.y, ay0.x + ay0.y);
-      if (id1 & 0x8000) cs.res[id1 & 0x7fff] = make_float2(ax1.x + ax1.y, ay1.x + ay1.y);
+      cs.res[id & 0x7fff] = make_float2(ax.x + ax.y, ay.x + ay.y);
     }
-  } else {
-#pragma unroll 1
-  for (int s = tid; s < n_src; s += THREADS) {
-    const int id = cs.sorted_idx[s];
-    if (!(id & 0x8000)) continue;
-    const float4 pp = tile.P2[s >> 1];
-    const float x = (s & 1) ? pp.y : pp.x, y = (s & 1) ? pp.w : pp.z;
-    int cx, cy;
-    cell_of(x, y, a, cx, cy);
-    const int reach = a.cell_reach;
-    const int cx0 = max(cx - reach, 0), cx1 = min(cx + reach, a.cells_x - 1);
-    const float2 nx = make_float2(-x, -x), ny = make_float2(-y, -y);
-    float2 ax = make_float2(0.f, 0.f), ay = make_float2(0.f, 0.f);
-    int done = 0;  // even slot index below which everything has been evaluated already
-    for (int row = max(cy - reach, 0); row <= min(cy + reach, a.cells_y - 1); ++row) {
-      const int lo = max(cs.cell_start[row * a.cells_x + cx0] & ~1, done);
-      const int hi = (cs.cell_start[row * a.cells_x + cx1 + 1] + 1) & ~1;
-      int j = lo >> 1;
-      const int je = hi >> 1;
-      if (j < je) {
-        // software pipeline: the operands of the next slot pair are in flight while this one is evaluated
-        // (the look-ahead of the last iteration reads at most the tile's spare entry)
-        float4 p = tile.P2[j], u = tile.U2[j];
-#pragma unroll 2
-        for (; j < je; ++j) {
-          const float4 pn = tile.P2[j + 1], un = tile.U2[j + 1];
-          const float2 dx = __fadd2_rn(make_float2(p.x, p.y), nx);
-          const float2 dy = __fadd2_rn(make_float2(p.z, p.w), ny);
-          float2 d2 = __fmul2_rn(dx, dx);
-          d2 = __ffma2_rn(dy, dy, d2);
-          const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-          ax = __ffma2_rn(w, make_float2(u.x, u.y), ax);
-          ay = __ffma2_rn(w, make_float2(u.z, u.w), ay);
-          p = pn;
-          u = un;
-        }
-      }
-      done = max(done, hi);
-    }
-    cs.res[id & 0x7fff] = make_float2(ax.x + ax.y, ay.x + ay.y);
-  }
   }
   __syncthreads();
   // ---- 6. back to the owners
-  const float qnan = __int_as_float(0x7fc00000);
-#pragma unroll
-  for (int k = 0; k < PPT; ++k) {
-    sx[k] = sy[k] = 0.f;
-    const bool fv = (unsigned)(st[k] - ST_VISCEK) <= (unsigned)(ST_FOLLOWER - ST_VISCEK);
-    if (fv) {
-      const float2 r = cs.res[k * THREADS + tid];
-      sx[k] = poisoned ? qnan : r.x;
-      sy[k] = poisoned ? qnan : r.y;
-    }
-  }
+  read_results<THREADS, PPT>(cs, poisoned, st, sx, sy);
 }
 
 // A one-warp CTA only needs warp-level convergence + memory ordering, not a hardware barrier.  // @region helpers
@@ -825,9 +871,10 @@ __device__ __forceinline__ void random_layout(uint64_t seed, uint32_t env, uint3
 
 // ------------------------------------------------------------------------------------------
 // THE fused step kernel.  grid = one CTA per environment (grid-stride), THREADS threads,
-// PPT pedestrians per thread (pedestrian i = k*THREADS + tid).  N <= 64 runs as ONE WARP per
-// environment (THREADS = 32, PPT = 2): no block barrier, reductions are pure REDUX / shuffles, and
-// the moving pedestrians are compacted (ballot + popc) so the pairwise pass only visits them.
+// PPT pedestrians per thread (pedestrian i = k*THREADS + tid).  float32 N <= 64 runs evac_warp_kernel
+// (evac_warp.cuh) instead; fp64 N <= 64 runs here as ONE WARP per environment (THREADS = 32, PPT = 2):
+// no block barrier, reductions are pure REDUX / shuffles, and the moving pedestrians are compacted
+// (ballot + popc) so the pairwise pass only visits them.
 #include "evac_cluster.cuh"
 
 // CL > 1: ONE environment per thread-block cluster of CL CTAs (evac_cluster.cuh) -- CTA r owns pedestrians
@@ -879,7 +926,6 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
     int now = a.now[e];
     int episode = a.episode[e];
     const long long overall_start = a.overall[e];
-    const int now_start = now;
     int steps_total = 0;
     double acc_r = 0, acc_i = 0, acc_s = 0;
     const uint32_t env_g = (uint32_t)(a.env_offset + e);
@@ -971,7 +1017,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
         else { r_agent = -5.f; term_agent = a.term_wall != 0; }
       }
       // ---------------- pairwise alignment [area.py:105-119]  // @region pairwise
-      real sx[PPT], sy[PPT], cnt[PPT];
+      real sx[PPT], sy[PPT], cnt[PPT];  // cnt: number of neighbours, used by the fp64 update only
       if constexpr (!COMPACT && !F64) {
         if (use_cells) {
           const CellSmem cs(smem_raw + Tile<real>::bytes(SLOTS), SLOTS, a.cells_x * a.cells_y);
@@ -983,14 +1029,14 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
           }
         }
       }
-      if (use_cells) {
+      if (!use_cells) {
+        if (__any_sync(0xffffffffu, any_fv)) {
+          if constexpr (F64) pairwise_pass<PPT>(tile, n_src, px, py, a.thr2_ped, sx, sy, cnt);
+          else pairwise_pass<PPT>(tile, n_src, px, py, a.thr2_ped, sx, sy);
+        } else {
 #pragma unroll
-        for (int k = 0; k < PPT; ++k) cnt[k] = (real)0;
-      } else if (__any_sync(0xffffffffu, any_fv)) {
-        pairwise_pass<PPT, F64>(tile, n_src, px, py, a.thr2_ped, sx, sy, cnt);
-      } else {
-#pragma unroll
-        for (int k = 0; k < PPT; ++k) sx[k] = sy[k] = cnt[k] = (real)0;
+          for (int k = 0; k < PPT; ++k) sx[k] = sy[k] = cnt[k] = (real)0;
+        }
       }
       // ---------------- new directions, enslaving, integration, reflection, statuses  // @region update
       int k_exit = 0, k_fol = 0, n_esc = 0, n_exi = 0, n_fol = 0;
@@ -1173,7 +1219,6 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
       if (a.terminated) a.terminated[e] = (uint8_t)any_term;
       if (a.truncated) a.truncated[e] = (uint8_t)any_trunc;
     }
-    (void)now_start;
     cta_sync<WARPS>();  // smem tile / scratch reuse by the next environment of this CTA
   }
 }

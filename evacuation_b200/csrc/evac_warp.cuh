@@ -17,7 +17,7 @@ enum { WMODE_GENERIC = 0, WMODE_REL_OHE_BOX = 1, WMODE_GRAV = 2 };
 
 __device__ __forceinline__ float2 splat(float v) { return make_float2(v, v); }
 
-// Neighbour sums of ONE pedestrian over the slot pairs [j0, j1) of the strip-sorted tile (same packed evaluation as
+// Neighbour sums of ONE pedestrian over the slot pairs [j0, j1) of the strip-sorted tile (accumulate_pair like
 // pairwise_pass; trip counts differ per lane, finished lanes idle).
 __device__ __forceinline__ void windowed_pass(const Tile<float>& t, int j0, int j1, float x, float y, float thr2, float& sx, float& sy) {
   const float2 nx = splat(-x), ny = splat(-y);
@@ -27,13 +27,7 @@ __device__ __forceinline__ void windowed_pass(const Tile<float>& t, int j0, int 
 #pragma unroll 2
     for (int j = j0; j < j1; ++j) {
       const float4 pn = t.P2[j + 1], un = t.U2[j + 1];  // look-ahead (at most the tile's spare entry)
-      const float2 dx = __fadd2_rn(make_float2(p.x, p.y), nx);
-      const float2 dy = __fadd2_rn(make_float2(p.z, p.w), ny);
-      float2 d2 = __fmul2_rn(dx, dx);
-      d2 = __ffma2_rn(dy, dy, d2);
-      const float2 w = make_float2(d2.x < thr2 ? 1.f : 0.f, d2.y < thr2 ? 1.f : 0.f);
-      ax = __ffma2_rn(w, make_float2(u.x, u.y), ax);
-      ay = __ffma2_rn(w, make_float2(u.z, u.w), ay);
+      accumulate_pair(p, u, nx, ny, thr2, ax, ay);
       p = pn;
       u = un;
     }
@@ -216,13 +210,13 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
       else { r_agent = -5.f; term_agent = a.term_wall != 0; }
     }
     // ---------------- pairwise alignment [area.py:105-119]  // @region wpairwise
-    float sx[2], sy[2], cnt[2];
+    float sx[2], sy[2];
     if (culled) {
 #pragma unroll
       for (int k = 0; k < 2; ++k) windowed_pass(tile, win_lo[k], win_hi[k], q[k].p.x, q[k].p.y, a.thr2_ped, sx[k], sy[k]);
     } else {
       const float xi[2] = {q[0].p.x, q[1].p.x}, yi[2] = {q[0].p.y, q[1].p.y};
-      if (__any_sync(0xffffffffu, fv[0] | fv[1])) pairwise_pass<2, false, PAIR_UNROLL>(tile, n_src, xi, yi, a.thr2_ped, sx, sy, cnt);
+      if (__any_sync(0xffffffffu, fv[0] | fv[1])) pairwise_pass<2, PAIR_UNROLL>(tile, n_src, xi, yi, a.thr2_ped, sx, sy);
       else sx[0] = sx[1] = sy[0] = sy[1] = 0.f;
     }
     // ---------------- new headings, enslaving, integration, reflection, statuses  // @region wupdate
