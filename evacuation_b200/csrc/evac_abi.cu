@@ -237,13 +237,17 @@ static int launch_step(EvacHandle* h, const KArgs<real>& a, cudaStream_t st) {
   return fail(EVAC_ERR_INVALID, "no kernel shape for N=%d", h->N);
 }
 
-template <typename real>
+// f(make_args<real>(h)) with real = the handle's precision
+template <typename F>
+static int with_args(const EvacHandle* h, F&& f) { return h->prec == EVAC_PREC_F64 ? f(make_args<double>(h)) : f(make_args<float>(h)); }
+
 static int launch_aux(EvacHandle* h, int flags, const uint8_t* mask, float* obs, cudaStream_t st) {
-  KArgs<real> a = make_args<real>(h);
-  evac_aux_kernel<real><<<h->E, 128, 0, st>>>(a, flags, mask, obs);
-  CK(cudaGetLastError());
-  h->launches++;
-  return EVAC_OK;
+  return with_args(h, [&](const auto& a) -> int {
+    evac_aux_kernel<<<h->E, 128, 0, st>>>(a, flags, mask, obs);
+    CK(cudaGetLastError());
+    h->launches++;
+    return EVAC_OK;
+  });
 }
 
 static int set_device(const EvacHandle* h) {
@@ -423,14 +427,14 @@ int evac_reset(EvacHandle* h, const uint8_t* reset_mask, float* obs, void* strea
   if (int r = set_device(h)) return r;
   cudaStream_t st = (cudaStream_t)stream;
   const int flags = AUX_RESET | (obs ? AUX_OBS : 0);
-  return h->prec == EVAC_PREC_F64 ? launch_aux<double>(h, flags, reset_mask, obs, st) : launch_aux<float>(h, flags, reset_mask, obs, st);
+  return launch_aux(h, flags, reset_mask, obs, st);
 }
 
 int evac_observe(EvacHandle* h, float* obs, void* stream) {
   if (!h || !obs) return fail(EVAC_ERR_INVALID, "NULL argument");
   if (int r = set_device(h)) return r;
   cudaStream_t st = (cudaStream_t)stream;
-  return h->prec == EVAC_PREC_F64 ? launch_aux<double>(h, AUX_OBS, nullptr, obs, st) : launch_aux<float>(h, AUX_OBS, nullptr, obs, st);
+  return launch_aux(h, AUX_OBS, nullptr, obs, st);
 }
 
 int evac_set_state(EvacHandle* h, const void* positions, const void* directions, const uint8_t* statuses,
@@ -444,7 +448,7 @@ int evac_set_state(EvacHandle* h, const void* positions, const void* directions,
     evac_block_io_kernel<true><<<h->E, 64, 0, st>>>(h->blocks, h->E, h->N, io);
     CK(cudaGetLastError());
     h->launches++;
-    if (!statuses && (positions || agent_position)) return launch_aux<float>(h, AUX_STATUS, nullptr, nullptr, st);
+    if (!statuses && (positions || agent_position)) return launch_aux(h, AUX_STATUS, nullptr, nullptr, st);
     return EVAC_OK;
   }
   if (positions) CK(cudaMemcpyAsync(h->pos, positions, en * es, cudaMemcpyDeviceToDevice, st));
@@ -456,7 +460,7 @@ int evac_set_state(EvacHandle* h, const void* positions, const void* directions,
   if (statuses) {
     CK(cudaMemcpyAsync(h->status, statuses, en, cudaMemcpyDeviceToDevice, st));
   } else if (positions || agent_position) {  // pedestrians.py:21-26: statuses follow from the positions
-    return h->prec == EVAC_PREC_F64 ? launch_aux<double>(h, AUX_STATUS, nullptr, nullptr, st) : launch_aux<float>(h, AUX_STATUS, nullptr, nullptr, st);
+    return launch_aux(h, AUX_STATUS, nullptr, nullptr, st);
   }
   return EVAC_OK;
 }
@@ -492,18 +496,12 @@ static int rollout_impl(EvacHandle* h, int32_t num_steps, int32_t agent_kind, co
   if (agent_kind == EVAC_AGENT_TABLE && !actions) return fail(EVAC_ERR_INVALID, "actions is NULL");
   if (int r = set_device(h)) return r;
   cudaStream_t st = (cudaStream_t)stream;
-  if (h->prec == EVAC_PREC_F64) {
-    KArgs<double> a = make_args<double>(h);
+  return with_args(h, [&](auto a) -> int {
     a.actions = (const float2*)actions; a.noise = noise; a.obs = obs; a.obs_every_step = obs_every_step;
     a.reward = reward_sum; a.terminated = terminated; a.truncated = truncated; a.num_steps = num_steps; a.agent_kind = agent_kind;
     a.status_counts = status_counts; a.status_out = status_out;
-    return launch_step<double>(h, a, st);
-  }
-  KArgs<float> a = make_args<float>(h);
-  a.actions = (const float2*)actions; a.noise = noise; a.obs = obs; a.obs_every_step = obs_every_step;
-  a.reward = reward_sum; a.terminated = terminated; a.truncated = truncated; a.num_steps = num_steps; a.agent_kind = agent_kind;
-  a.status_counts = status_counts; a.status_out = status_out;
-  return launch_step<float>(h, a, st);
+    return launch_step(h, a, st);
+  });
 }
 
 int evac_rollout(EvacHandle* h, int32_t num_steps, int32_t agent_kind, const float* actions, const float* noise, float* obs,

@@ -870,6 +870,82 @@ __device__ __forceinline__ void random_layout(uint64_t seed, uint32_t env, uint3
 }
 
 // ------------------------------------------------------------------------------------------
+// The per-environment part of a step, shared by evac_warp_kernel and evac_step_kernel.  Each kernel keeps its own loads
+// (placed where their latency hides) and reductions, and passes the loaded values and reduced counts in.
+
+// RandomAgent: action_space.sample() ~ U[-1,1)^2 [random_agent.py:8-9]
+__device__ __forceinline__ float2 random_action(uint64_t seed, uint32_t env, uint32_t episode, uint32_t now_prev) {
+  const uint2 r = evac_agent_block(seed, env, episode, now_prev);
+  return make_float2(2.f * u01(r.x) - 1.f, 2.f * u01(r.y) - 1.f);
+}
+
+// WacuumCleaner / RotatingAgent action; calls = the RotatingAgent's act() count including this call, which never restarts
+// with an episode [rotating_agent.py:8-16].  (Table and random actions are selected by the caller, next to their loads.)
+template <typename A>
+__device__ __forceinline__ float2 scripted_action(const A& a, long long calls, float2 ap, int& wac_state) {
+  if (a.agent_kind == AGENT_WACUUM) { float2 act; wacuum_act(ap.x, ap.y, wac_state, a, act.x, act.y); return act; }
+  const double ph = 0.05 * (double)calls;  // float64 like the reference
+  return make_float2((float)sin(ph), (float)cos(ph));
+}
+
+// Area.agent_step [area.py:182-210], IEEE float32 like the reference
+template <typename A>
+__device__ __forceinline__ void agent_step(const A& a, float2 act, float2& ap, float2& ad, float& r_agent, bool& term_agent) {
+  const float nrm = __fadd_rn(__fsqrt_rn(__fadd_rn(__fmul_rn(act.x, act.x), __fmul_rn(act.y, act.y))), a.eps_f);
+  const float ax = __fdiv_rn(act.x, nrm), ay = __fdiv_rn(act.y, nrm);
+  ad.x = __fmul_rn(a.step_size_f, ax); ad.y = __fmul_rn(a.step_size_f, ay);
+  const float ptx = __fadd_rn(ap.x, ad.x), pty = __fadd_rn(ap.y, ad.y);
+  const bool collide = (ptx < -a.width_f) | (ptx > a.width_f) | (pty < -a.height_f) | (pty > a.height_f);
+  r_agent = 0.f; term_agent = false;
+  if (!collide) { ap.x = ptx; ap.y = pty; }
+  else { r_agent = -5.f; term_agent = a.term_wall != 0; }
+}
+
+// rewards + termination [reward.py:19-46, area.py:174-180, env.py:158-171]; sd = sum of the distances to the exit
+template <typename real>
+__device__ __forceinline__ void step_reward(const KArgs<real>& a, int N, int now, real sd, int K_exit, int K_fol, int N_esc, float r_agent,
+                                            bool term_agent, real& intrinsic, real& r_status, real& reward, bool& terminated) {
+  real tf;
+  if constexpr (std::is_same<real, double>::value) { tf = (real)1 - (real)now / (real)(200 * N); intrinsic = (real)0 - sd / (real)N; }
+  else { tf = (real)1 - (real)now * a.inv_200n; intrinsic = (real)0 - sd * a.inv_n; }
+  real r_ped = a.init_reward;
+  if (a.exit_reward) r_ped += ((real)15 + (real)10 * tf) * (real)K_exit;
+  if (a.follow_reward) r_ped += ((real)10 + (real)5 * tf) * (real)K_fol;
+  r_status = (real)r_agent + r_ped;
+  reward = r_status + a.intrinsic_coef * intrinsic;
+  terminated = term_agent || (N_esc == N);
+}
+
+// pedestrians.status_stats after step s, before a same-step reset [pedestrians.py:37-44]
+template <typename real>
+__device__ __forceinline__ void store_status_counts(const KArgs<real>& a, int s, int e, int N, int N_esc, int N_exi, int N_fol) {
+  reinterpret_cast<ushort4*>(a.status_counts)[(size_t)s * a.E + e] =
+      make_ushort4((unsigned short)N_esc, (unsigned short)N_exi, (unsigned short)N_fol, (unsigned short)(N - N_esc - N_exi - N_fol));
+}
+
+// a finished episode: the logging dict of env.py:115-125 from its final accumulators and overall_timesteps
+template <typename real>
+__device__ __forceinline__ void record_episode(const KArgs<real>& a, int e, double acc_i, double acc_s, double acc_r, int now, int N,
+                                               int N_esc, int N_exi, int N_fol, long long overall) {
+  float* es = a.ep_stats + (size_t)e * NUM_EPISODE_STATS;
+  const float v[NUM_EPISODE_STATS] = {(float)acc_i, (float)acc_s, (float)acc_r, (float)now, (float)N_esc, (float)N_exi,
+                                      (float)N_fol, (float)(N - N_esc - N_exi - N_fol), (float)overall};
+#pragma unroll
+  for (int t = 0; t < NUM_EPISODE_STATS; ++t) { es[t] = v[t]; atomicAdd(a.totals + 1 + t, (double)v[t]); }
+  atomicAdd(a.totals, 1.0);
+  a.ep_finished[e] = 1;
+}
+
+// pedestrian i of a new episode: random layout and its status with the agent at the origin; returns the status
+template <typename real>
+__device__ __forceinline__ int reset_pedestrian(const KArgs<real>& a, uint32_t env, uint32_t episode, uint32_t i, real& px, real& py,
+                                                real& dx, real& dy) {
+  random_layout<real>(a.seed, env, episode, i, px, py, dx, dy);
+  real d2e;
+  return status_of<real>(px, py, (real)0, (real)0, a, d2e);
+}
+
+// ------------------------------------------------------------------------------------------
 // THE fused step kernel.  grid = one CTA per environment (grid-stride), THREADS threads,
 // PPT pedestrians per thread (pedestrian i = k*THREADS + tid).  float32 N <= 64 runs evac_warp_kernel
 // (evac_warp.cuh) instead; fp64 N <= 64 runs here as ONE WARP per environment (THREADS = 32, PPT = 2):
@@ -940,13 +1016,10 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
       const int now_prev = now;
       now += 1; steps_total += 1;
       const bool truncated = now >= a.max_timesteps;
-      // ---------------- random streams of this step (Philox2x32-10, philox.cuh): the RandomAgent action
-      // (action_space.sample() ~ U[-1,1)^2) is computed redundantly by every thread; the noise words are drawn where used
+      // ---------------- random streams of this step (Philox2x32-10, philox.cuh): the RandomAgent action is computed
+      // redundantly by every thread; the noise words are drawn where used
       float2 action_r = make_float2(0.f, 0.f);
-      if (a.agent_kind == AGENT_RANDOM) {
-        const uint2 r = evac_agent_block(a.seed, env_g, (uint32_t)episode, (uint32_t)now_prev);
-        action_r = make_float2(2.f * u01(r.x) - 1.f, 2.f * u01(r.y) - 1.f);
-      }
+      if (a.agent_kind == AGENT_RANDOM) action_r = random_action(a.seed, env_g, (uint32_t)episode, (uint32_t)now_prev);
       // ---------------- escaped / exiting preparation + source records [area.py:79-101]  // @region prep
       bool any_fv = false;
       bool efv[PPT];
@@ -992,30 +1065,13 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
         }
       }
       cta_sync<WARPS>();
-      // ---------------- action source + Area.agent_step [area.py:182-210], float32 like the reference  // @region agent
-      float r_agent = 0.f;
-      bool term_agent = false;
-      {
-        float ax, ay;
-        if (a.agent_kind == AGENT_TABLE) {
-          const float2 av = a.actions[(size_t)s * a.E + e];
-          ax = av.x; ay = av.y;
-        } else if (a.agent_kind == AGENT_RANDOM) {
-          ax = action_r.x; ay = action_r.y;
-        } else if (a.agent_kind == AGENT_WACUUM) {
-          wacuum_act(ap.x, ap.y, wac_state, a, ax, ay);
-        } else {  // RotatingAgent [rotating_agent.py:8-16]: i counts the agent's act() calls and never restarts with an episode
-          const double ph = 0.05 * (double)(overall_start + steps_total);  // float64 like the reference
-          ax = (float)sin(ph); ay = (float)cos(ph);
-        }
-        const float nrm = __fadd_rn(__fsqrt_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay))), a.eps_f);
-        ax = __fdiv_rn(ax, nrm); ay = __fdiv_rn(ay, nrm);
-        ad.x = __fmul_rn(a.step_size_f, ax); ad.y = __fmul_rn(a.step_size_f, ay);
-        const float ptx = __fadd_rn(ap.x, ad.x), pty = __fadd_rn(ap.y, ad.y);
-        const bool collide = (ptx < -a.width_f) | (ptx > a.width_f) | (pty < -a.height_f) | (pty > a.height_f);
-        if (!collide) { ap.x = ptx; ap.y = pty; }
-        else { r_agent = -5.f; term_agent = a.term_wall != 0; }
-      }
+      // ---------------- action source + Area.agent_step [area.py:182-210]  // @region agent
+      float2 act;
+      if (a.agent_kind == AGENT_TABLE) act = a.actions[(size_t)s * a.E + e];
+      else if (a.agent_kind == AGENT_RANDOM) act = action_r;
+      else act = scripted_action(a, overall_start + steps_total, ap, wac_state);
+      float r_agent; bool term_agent;
+      agent_step(a, act, ap, ad, r_agent, term_agent);
       // ---------------- pairwise alignment [area.py:105-119]  // @region pairwise
       real sx[PPT], sy[PPT], cnt[PPT];  // cnt: number of neighbours, used by the fp64 update only
       if constexpr (!COMPACT && !F64) {
@@ -1117,34 +1173,17 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
         cluster_sum<CL, 6>(cl_slot, v);
         K_exit = (int)v[0]; K_fol = (int)v[1]; N_esc = (int)v[2]; N_exi = (int)v[3]; N_fol = (int)v[4]; sd = v[5];
       }
-      if (a.status_counts != nullptr && lead) {
-        const ushort4 c4 = make_ushort4((unsigned short)N_esc, (unsigned short)N_exi, (unsigned short)N_fol, (unsigned short)(N - N_esc - N_exi - N_fol));
-        reinterpret_cast<ushort4*>(a.status_counts)[(size_t)s * a.E + e] = c4;
-      }
-      // ---------------- rewards + termination [reward.py:19-46, area.py:174-180, env.py:158-171]
-      real tf, intrinsic;
-      if constexpr (F64) { tf = (real)1 - (real)now / (real)(200 * N); intrinsic = (real)0 - (real)sd / (real)N; }
-      else { tf = (real)1 - (real)now * a.inv_200n; intrinsic = (real)0 - (real)sd * a.inv_n; }
-      real r_ped = a.init_reward;
-      if (a.exit_reward) r_ped += ((real)15 + (real)10 * tf) * (real)K_exit;
-      if (a.follow_reward) r_ped += ((real)10 + (real)5 * tf) * (real)K_fol;
-      const real r_status = (real)r_agent + r_ped;
-      const real reward = r_status + a.intrinsic_coef * intrinsic;
-      const bool terminated = term_agent || (N_esc == N);
+      if (a.status_counts != nullptr && lead) store_status_counts(a, s, e, N, N_esc, N_exi, N_fol);
+      real intrinsic, r_status, reward; bool terminated;
+      step_reward(a, N, now, (real)sd, K_exit, K_fol, N_esc, r_agent, term_agent, intrinsic, r_status, reward, terminated);
       reward_sum += (float)reward;
       any_term |= terminated; any_trunc |= truncated;
       acc_r += (double)reward; acc_i += (double)intrinsic; acc_s += (double)r_status;
       // ---------------- same-step auto-reset  // @region reset
       if (a.auto_reset && (terminated || truncated)) {
-        if (lead) {  // the logging dict of env.py:115-125
+        if (lead) {
           if (!acc_reset) { acc_r += a.acc[3 * (size_t)e]; acc_i += a.acc[3 * (size_t)e + 1]; acc_s += a.acc[3 * (size_t)e + 2]; }
-          float* es = a.ep_stats + (size_t)e * NUM_EPISODE_STATS;
-          const float v[NUM_EPISODE_STATS] = {(float)acc_i, (float)acc_s, (float)acc_r, (float)now, (float)N_esc, (float)N_exi,
-                                              (float)N_fol, (float)(N - N_esc - N_exi - N_fol), (float)(a.overall[e] + steps_total)};
-#pragma unroll
-          for (int q = 0; q < NUM_EPISODE_STATS; ++q) { es[q] = v[q]; atomicAdd(a.totals + 1 + q, (double)v[q]); }
-          atomicAdd(a.totals, 1.0);
-          a.ep_finished[e] = 1;
+          record_episode(a, e, acc_i, acc_s, acc_r, now, N, N_esc, N_exi, N_fol, a.overall[e] + steps_total);
         }
         acc_r = acc_i = acc_s = 0; acc_reset = true;
         now = 0; episode += 1; wac_state = 0;
@@ -1152,11 +1191,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
 #pragma unroll
         for (int k = 0; k < PPT; ++k) {
           const int i = base_i + k * THREADS + tid;
-          if (i < N) {
-            random_layout<real>(a.seed, env_g, (uint32_t)episode, (uint32_t)i, px[k], py[k], dx[k], dy[k]);
-            real d2e;
-            st[k] = status_of<real>(px[k], py[k], (real)0, (real)0, a, d2e);
-          }
+          if (i < N) st[k] = reset_pedestrian<real>(a, env_g, (uint32_t)episode, (uint32_t)i, px[k], py[k], dx[k], dy[k]);
         }
       }
       // ---------------- observation  // @region obs

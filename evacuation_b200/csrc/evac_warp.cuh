@@ -1,6 +1,8 @@
 // One-warp-per-environment fused step kernel for N <= 64 pedestrians, float32 (the BASELINE headline
-// shapes: 60 pedestrians).  Same semantics as evac_step_kernel (evac_kernels.cuh; reference file:line
-// citations there and inline below) but written as straight-line warp code:
+// shapes: 60 pedestrians).  Same semantics as evac_step_kernel (evac_kernels.cuh; reference file:line citations there and
+// inline below), and the same code for the agent, rewards, episode record and reset (random_action, scripted_action,
+// agent_step, step_reward, store_status_counts, record_episode, reset_pedestrian), but the pedestrian work is
+// written as straight-line warp code:
 //   * lane L owns pedestrians L and L + 32; every per-pedestrian quantity is kept as an (x, y) float2 so the
 //     epilogue arithmetic runs on Blackwell's packed FP32 instructions (FADD2 / FMUL2 / FFMA2) exactly like the
 //     pairwise pass -- one instruction per pedestrian instead of one per component;
@@ -185,30 +187,13 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     }
     if (lane < 2) tile.put(n_src + lane, PARK, PARK, 0.f, 0.f);  // pad to an even count
     __syncwarp();
-    // ---------------- action source + Area.agent_step [area.py:182-210], IEEE float32 like the reference  // @region wagent
-    float r_agent = 0.f;
-    bool term_agent = false;
-    {
-      float ax, ay;
-      if (a.agent_kind == AGENT_TABLE) {
-        ax = act_tbl.x; ay = act_tbl.y;
-      } else if (a.agent_kind == AGENT_RANDOM) {  // RandomAgent: action_space.sample() ~ U[-1,1)^2 [random_agent.py:8-9]
-        const uint2 r = evac_agent_block(a.seed, env_g, (uint32_t)episode, (uint32_t)now_prev);
-        ax = 2.f * u01(r.x) - 1.f; ay = 2.f * u01(r.y) - 1.f;
-      } else if (a.agent_kind == AGENT_WACUUM) {
-        wacuum_act(ap.x, ap.y, wac_state, a, ax, ay);
-      } else {  // RotatingAgent [rotating_agent.py:8-16]: i counts the agent's act() calls and never restarts with an episode
-        const double ph = 0.05 * (double)(overall + 1);  // float64 like the reference
-        ax = (float)sin(ph); ay = (float)cos(ph);
-      }
-      const float nrm = __fadd_rn(__fsqrt_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay))), a.eps_f);
-      ax = __fdiv_rn(ax, nrm); ay = __fdiv_rn(ay, nrm);
-      ad.x = __fmul_rn(a.step_size_f, ax); ad.y = __fmul_rn(a.step_size_f, ay);
-      const float ptx = __fadd_rn(ap.x, ad.x), pty = __fadd_rn(ap.y, ad.y);
-      const bool collide = (ptx < -a.width_f) | (ptx > a.width_f) | (pty < -a.height_f) | (pty > a.height_f);
-      if (!collide) { ap.x = ptx; ap.y = pty; }
-      else { r_agent = -5.f; term_agent = a.term_wall != 0; }
-    }
+    // ---------------- action source + Area.agent_step [area.py:182-210]  // @region wagent
+    float2 act;
+    if (a.agent_kind == AGENT_TABLE) act = act_tbl;
+    else if (a.agent_kind == AGENT_RANDOM) act = random_action(a.seed, env_g, (uint32_t)episode, (uint32_t)now_prev);
+    else act = scripted_action(a, overall + 1, ap, wac_state);
+    float r_agent; bool term_agent;
+    agent_step(a, act, ap, ad, r_agent, term_agent);
     // ---------------- pairwise alignment [area.py:105-119]  // @region wpairwise
     float sx[2], sy[2];
     if (culled) {
@@ -266,19 +251,12 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     counts = __reduce_add_sync(0xffffffffu, counts);
     const float sd = warp_sum(sum_dexit);
     const int K_exit = counts & 0xff, K_fol = (counts >> 8) & 0xff, N_esc = (counts >> 16) & 0xff, N_exi = (counts >> 24) & 0xff;
-    if (a.status_counts != nullptr) {  // pedestrians.status_stats after this step (before a same-step reset)
+    if (a.status_counts != nullptr) {
       const int n_fol = __popc(__ballot_sync(0xffffffffu, q[0].st == ST_FOLLOWER)) + __popc(__ballot_sync(0xffffffffu, q[1].st == ST_FOLLOWER));
-      if (lane == 0)
-        reinterpret_cast<ushort4*>(a.status_counts)[(size_t)s * a.E + e] =
-            make_ushort4((unsigned short)N_esc, (unsigned short)N_exi, (unsigned short)n_fol, (unsigned short)(N - N_esc - N_exi - n_fol));
+      if (lane == 0) store_status_counts(a, s, e, N, N_esc, N_exi, n_fol);
     }
-    const float tf = 1.f - (float)now * a.inv_200n, intrinsic = 0.f - sd * a.inv_n;
-    float r_ped = a.init_reward;
-    if (a.exit_reward) r_ped += (15.f + 10.f * tf) * (float)K_exit;
-    if (a.follow_reward) r_ped += (10.f + 5.f * tf) * (float)K_fol;
-    const float r_status = r_agent + r_ped;
-    const float reward = r_status + a.intrinsic_coef * intrinsic;
-    const bool terminated = term_agent || (N_esc == N);
+    float intrinsic, r_status, reward; bool terminated;
+    step_reward(a, N, now, sd, K_exit, K_fol, N_esc, r_agent, term_agent, intrinsic, r_status, reward, terminated);
     reward_sum += reward;
     any_term |= terminated; any_trunc |= truncated;
     acc_r += (double)reward; acc_i += (double)intrinsic; acc_s += (double)r_status;
@@ -286,26 +264,13 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     // ---------------- same-step auto-reset (gymnasium vector-env semantics)  // @region wreset
     if (a.auto_reset && (terminated || truncated)) {
       const int N_fol = __popc(__ballot_sync(0xffffffffu, q[0].st == ST_FOLLOWER)) + __popc(__ballot_sync(0xffffffffu, q[1].st == ST_FOLLOWER));
-      if (lane == 0) {  // the logging dict of env.py:115-125
-        float* es = a.ep_stats + (size_t)e * NUM_EPISODE_STATS;
-        const float v[NUM_EPISODE_STATS] = {(float)acc_i, (float)acc_s, (float)acc_r, (float)now, (float)N_esc, (float)N_exi,
-                                            (float)N_fol, (float)(N - N_esc - N_exi - N_fol), (float)overall};
-#pragma unroll
-        for (int t = 0; t < NUM_EPISODE_STATS; ++t) { es[t] = v[t]; atomicAdd(a.totals + 1 + t, (double)v[t]); }
-        atomicAdd(a.totals, 1.0);
-        a.ep_finished[e] = 1;
-      }
+      if (lane == 0) record_episode(a, e, acc_i, acc_s, acc_r, now, N, N_esc, N_exi, N_fol, overall);
       acc_r = acc_i = acc_s = 0;
       now = 0; episode += 1; wac_state = 0;
       ap = make_float2(0.f, 0.f); ad = make_float2(0.f, 0.f);
 #pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        if (valid[k]) {
-          float dummy;
-          random_layout<float>(a.seed, env_g, (uint32_t)episode, (uint32_t)(lane + 32 * k), q[k].p.x, q[k].p.y, q[k].d.x, q[k].d.y);
-          q[k].st = status_of<float>(q[k].p.x, q[k].p.y, 0.f, 0.f, a, dummy);
-        }
-      }
+      for (int k = 0; k < 2; ++k)
+        if (valid[k]) q[k].st = reset_pedestrian<float>(a, env_g, (uint32_t)episode, (uint32_t)(lane + 32 * k), q[k].p.x, q[k].p.y, q[k].d.x, q[k].d.y);
     }
     // ---------------- observation [wrappers.py:8-96, gravity_encoding.py:8-81]  // @region wobs
     if (obs_e != nullptr && (a.obs_every_step || s == a.num_steps - 1)) {
