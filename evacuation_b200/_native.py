@@ -93,6 +93,7 @@ SIGNATURES = {
     "evac_save_state": (C.c_int, [_P, _P, _P]),
     "evac_load_state": (C.c_int, [_P, _P, _P]),
     "evac_policy_default_config": (C.c_int, [C.POINTER(EvacPolicyConfig), C.c_int32, C.c_int32]),
+    "evac_policy_default_linear_config": (C.c_int, [C.POINTER(EvacPolicyConfig), C.c_int32]),
     "evac_policy_create": (C.c_int, [C.POINTER(EvacPolicyConfig), C.c_int32, C.POINTER(_P)]),
     "evac_policy_destroy": (C.c_int, [_P]),
     "evac_policy_num_weights": (C.c_int64, [_P]),

@@ -1,5 +1,5 @@
-// C ABI of the fused RPO transformer-embedding policy forward and the reward normaliser (include/evac_b200.h,
-// "rollout-loop glue").  Host side: weight repacking + launch plumbing; the arithmetic lives in evac_policy.cuh.
+// C ABI of the fused RPO policy forward (the transformer embedding + heads, or, with num_blocks = 0, the linear network on the
+// observation) and the reward normaliser (include/evac_b200.h, "rollout-loop glue").  Host side: weight repacking + launch plumbing; the arithmetic lives in evac_policy.cuh.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdarg.h>
@@ -33,6 +33,10 @@ static int pfail(int code, const char* fmt, ...) {
     cudaError_t _e = (call);                                                                       \
     if (_e != cudaSuccess) return pfail(EVAC_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__); \
   } while (0)
+
+// widest observation the linear policy (num_blocks = 0) takes: every flattened observation at N <= 64 (Dict rel + ohe: 388) fits
+// with room; the heads' K loops have no structural limit, the cap bounds the weight upload and the per-CTA K loop
+constexpr int PL_MAX_K = 4096;
 
 struct EvacPolicy {
   EvacPolicyConfig cfg;
@@ -118,6 +122,58 @@ static int launch_embed(EvacPolicy* p, const PArgs& a, bool train, cudaStream_t 
   return EVAC_OK;
 }
 
+// the heads kernel on X = the embedding, or the observation of the linear policy (+ its fused normaliser when n.mean is set)
+static int launch_heads(EvacPolicy* p, const EvacPolicyIO* io, const float* x, const NArgs& n, cudaStream_t st) {
+  const bool norm = n.mean != nullptr;
+  HArgs h;
+  memset(&h, 0, sizeof(h));
+  h.E = io->num_envs; h.K = p->K; h.K16 = p->K16; h.NH = p->NH; h.A = p->A;
+  h.emb = x; h.w1t = p->d_w1t; h.b1 = p->d_b1; h.w2t = p->d_w2t; h.b2 = p->d_b2; h.w3 = p->d_w3; h.b3 = p->d_b3; h.logstd = p->d_logstd;
+  h.given_action = io->given_action;
+  h.mean = io->mean; h.value = io->value; h.action = io->action; h.action_clipped = io->action_clipped; h.logprob = io->logprob; h.entropy = io->entropy;
+  h.sample = io->sample;
+  h.seed_lo = (uint32_t)io->seed; h.seed_hi = (uint32_t)(io->seed >> 32);
+  h.offset = io->offset; h.offset_dev = reinterpret_cast<const unsigned long long*>(io->offset_device); h.env_offset = io->env_index_offset;
+  if (p->use_tc) {
+    // the heads on the tensor cores; 64-column tiles (critic and actor in separate CTAs) while 128-column tiles would not fill the SMs
+    TCArgs t;
+    t.h = h; t.chunks = p->tc_chunks; t.w2tc = p->d_w2tc;
+    const int gx = (h.E + TC_M - 1) / TC_M;
+    // shapes: 64 columns x 4 stages (critic and actor in separate CTAs) while 128-column tiles would not fill the SMs, 128 columns
+    // x 3 stages beyond (X is read once).  Measured per 8192 / 20 000 / 65 536 envs: 20.3 / 49.3 / 121.5 us (64x4), 29.7 / 50.4 /
+    // 105.0 us (128x3); 64 columns x 2 stages with two CTAs per SM: 24.6 / 53.6 / 113.1 us.
+    // The fused normaliser always takes the 128-column tiles: one CTA per row tile updates the statistics (DESIGN.md section 7).
+    auto k64 = evac_policy_heads_tc_kernel<64, 4, 2, 1>;
+    auto k128 = evac_policy_heads_tc_kernel<128, 3, 2, 1>;
+    auto k128n = evac_policy_heads_tc_kernel<128, 3, 2, 1, true>;
+    using S64 = TCShape<64, 4, 2>; using S128 = TCShape<128, 3, 2>;
+    static thread_local bool tc_attr[16] = {false};
+    if (!tc_attr[p->device & 15]) {
+      PCK(cudaFuncSetAttribute(k64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S64::SMEM_BYTES));
+      PCK(cudaFuncSetAttribute(k128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S128::SMEM_BYTES));
+      PCK(cudaFuncSetAttribute(k128n, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S128::SMEM_BYTES));
+      tc_attr[p->device & 15] = true;
+    }
+    if (norm) { t.w1tc = p->d_w1tc128; k128n<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t, n); }
+    else if (gx < 2 * 148) { t.w1tc = p->d_w1tc64; k64<<<dim3(gx, 2), TC_THREADS, S64::SMEM_BYTES, st>>>(t, n); }
+    else { t.w1tc = p->d_w1tc128; k128<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t, n); }
+    PCK(cudaGetLastError());
+    p->launches++;
+    return EVAC_OK;
+  }
+  static thread_local size_t hattr[16] = {0};
+  if (p->heads_smem > 48 * 1024 && hattr[p->device & 15] < p->heads_smem) {
+    PCK(cudaFuncSetAttribute(evac_policy_heads_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->heads_smem));
+    PCK(cudaFuncSetAttribute(evac_policy_heads_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->heads_smem));
+    hattr[p->device & 15] = p->heads_smem;
+  }
+  if (norm) evac_policy_heads_kernel<true><<<(h.E + HD_TM - 1) / HD_TM, HD_THREADS, p->heads_smem, st>>>(h, n);
+  else evac_policy_heads_kernel<false><<<(h.E + HD_TM - 1) / HD_TM, HD_THREADS, p->heads_smem, st>>>(h, n);
+  PCK(cudaGetLastError());
+  p->launches++;
+  return EVAC_OK;
+}
+
 extern "C" {
 
 int evac_policy_default_config(EvacPolicyConfig* cfg, int32_t number_of_pedestrians, int32_t d_model) {
@@ -137,17 +193,34 @@ int evac_policy_default_config(EvacPolicyConfig* cfg, int32_t number_of_pedestri
   return EVAC_OK;
 }
 
+int evac_policy_default_linear_config(EvacPolicyConfig* cfg, int32_t obs_dim) {
+  if (!cfg) return pfail(EVAC_ERR_INVALID, "cfg is NULL");
+  memset(cfg, 0, sizeof(*cfg));
+  cfg->abi_version = EVAC_ABI_VERSION;
+  cfg->seq_len = 1;            // K = seq_len * d_model = obs_dim
+  cfg->d_model = obs_dim;
+  cfg->num_blocks = 0;         // RPOLinearNetwork directly on the observation
+  cfg->num_hidden = 64;        // rpo_linear_agent_network.py:12
+  cfg->action_dim = 2;
+  return EVAC_OK;
+}
+
 int evac_policy_create(const EvacPolicyConfig* cfg, int32_t device, EvacPolicy** out) {
   if (!cfg || !out) return pfail(EVAC_ERR_INVALID, "cfg / out is NULL");
   if (cfg->abi_version != EVAC_ABI_VERSION) return pfail(EVAC_ERR_INVALID, "EvacPolicyConfig.abi_version %d != %d", cfg->abi_version, EVAC_ABI_VERSION);
-  if (cfg->seq_len < 1 || cfg->seq_len > PW_MAX_S)
+  const bool linear = cfg->num_blocks == 0;
+  if (!linear && (cfg->seq_len < 1 || cfg->seq_len > PW_MAX_S))
     return pfail(EVAC_ERR_UNSUPPORTED, "fused policy: seq_len (number_of_pedestrians + 2) must be 1..%d, got %d", PW_MAX_S, cfg->seq_len);
-  if (cfg->dim_feedforward < 1 || cfg->num_blocks < 1 || cfg->num_blocks > 8) return pfail(EVAC_ERR_INVALID, "bad dim_feedforward / num_blocks");
+  if (cfg->num_blocks < 0 || cfg->num_blocks > 8 || (!linear && cfg->dim_feedforward < 1)) return pfail(EVAC_ERR_INVALID, "bad dim_feedforward / num_blocks");
+  // the linear network's K: from 1 (rows that are not a multiple of 4 floats take the heads' scalar loads) to PL_MAX_K
+  const int64_t K_lin = (int64_t)cfg->seq_len * cfg->d_model;
+  if (linear && (cfg->seq_len < 1 || cfg->d_model < 1 || K_lin > PL_MAX_K))
+    return pfail(EVAC_ERR_UNSUPPORTED, "fused linear policy: seq_len * d_model (the observation width) must be 1..%d, got %lld", PL_MAX_K, (long long)K_lin);
   if (cfg->num_hidden < 4 || cfg->num_hidden > 64 || cfg->num_hidden % 4) return pfail(EVAC_ERR_UNSUPPORTED, "fused policy: num_hidden must be a multiple of 4 in 4..64, got %d", cfg->num_hidden);
   if (cfg->action_dim < 1 || cfg->action_dim > 3) return pfail(EVAC_ERR_UNSUPPORTED, "fused policy: action_dim must be 1..3");
   if (!(cfg->dropout >= 0.f && cfg->dropout < 1.f)) return pfail(EVAC_ERR_INVALID, "dropout must be in [0, 1)");
   const int F4 = round_up(cfg->dim_feedforward, 4);
-  const int ws = block_stride(cfg->d_model, cfg->num_heads, F4);
+  const int ws = linear ? 0 : block_stride(cfg->d_model, cfg->num_heads, F4);
   if (ws < 0) return pfail(EVAC_ERR_UNSUPPORTED, "fused policy: (d_model, num_heads) = (%d, %d) is not instantiated", cfg->d_model, cfg->num_heads);
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return pfail(EVAC_ERR_NO_DEVICE, "no CUDA device (evacuation_b200 has no CPU fallback)");
@@ -159,12 +232,12 @@ int evac_policy_create(const EvacPolicyConfig* cfg, int32_t device, EvacPolicy**
   p->S = cfg->seq_len; p->D = cfg->d_model; p->H = cfg->num_heads; p->F = cfg->dim_feedforward; p->F4 = F4; p->NB = cfg->num_blocks;
   p->NH = cfg->num_hidden; p->A = cfg->action_dim; p->K = p->S * p->D; p->K16 = round_up(p->K, HD_KC);
   p->wstride = ws;
-  p->embed_smem = ((size_t)p->NB * ws + (size_t)PW_WARPS * 2 * p->H * PW_MAX_S) * sizeof(float);
+  p->embed_smem = linear ? 0 : ((size_t)p->NB * ws + (size_t)PW_WARPS * 2 * p->H * PW_MAX_S) * sizeof(float);
   p->heads_smem = HD_SMEM_FLOATS * sizeof(float);
   if (p->embed_smem > 200 * 1024 || p->heads_smem > 200 * 1024) { delete p; return pfail(EVAC_ERR_UNSUPPORTED, "fused policy: shape needs too much shared memory"); }
   cudaError_t e = cudaSuccess;
   auto alloc = [&](float** q, size_t n) { if (e == cudaSuccess) { e = cudaMalloc(q, n * sizeof(float)); if (e == cudaSuccess) e = cudaMemset(*q, 0, n * sizeof(float)); } };
-  alloc(&p->d_emb_w, (size_t)p->NB * ws);
+  if (!linear) alloc(&p->d_emb_w, (size_t)p->NB * ws);
   alloc(&p->d_w1t, (size_t)p->K16 * HD_COLS); alloc(&p->d_b1, HD_COLS);
   alloc(&p->d_w2t, (size_t)HD_HS * HD_COLS); alloc(&p->d_b2, HD_COLS);
   alloc(&p->d_w3, (size_t)(1 + p->A) * HD_HS); alloc(&p->d_b3, 4); alloc(&p->d_logstd, 4);
@@ -233,7 +306,7 @@ int evac_policy_load_weights(EvacPolicy* p, const float* w, int64_t count) {
   b3[0] = c4b[0];
   for (int r = 0; r < A; ++r) { b3[1 + r] = a4b[r]; ls[r] = lsd[r]; }
   PCK(cudaDeviceSynchronize());
-  PCK(cudaMemcpy(p->d_emb_w, emb.data(), emb.size() * sizeof(float), cudaMemcpyHostToDevice));
+  if (!emb.empty()) PCK(cudaMemcpy(p->d_emb_w, emb.data(), emb.size() * sizeof(float), cudaMemcpyHostToDevice));
   PCK(cudaMemcpy(p->d_w1t, w1t.data(), w1t.size() * sizeof(float), cudaMemcpyHostToDevice));
   PCK(cudaMemcpy(p->d_b1, b1.data(), b1.size() * sizeof(float), cudaMemcpyHostToDevice));
   PCK(cudaMemcpy(p->d_w2t, w2t.data(), w2t.size() * sizeof(float), cudaMemcpyHostToDevice));
@@ -285,7 +358,7 @@ int evac_policy_load_weights(EvacPolicy* p, const float* w, int64_t count) {
 
 int evac_policy_reserve(EvacPolicy* p, int32_t max_envs) {
   if (!p || max_envs < 1) return pfail(EVAC_ERR_INVALID, "bad arguments");
-  if (max_envs <= p->scratch_envs) return EVAC_OK;
+  if (max_envs <= p->scratch_envs || p->NB == 0) return EVAC_OK;   // the linear policy has no embedding scratch
   PCK(cudaSetDevice(p->device));
   if (p->d_scratch) { PCK(cudaDeviceSynchronize()); PCK(cudaFree(p->d_scratch)); p->d_scratch = nullptr; p->scratch_envs = 0; }
   PCK(cudaMalloc(&p->d_scratch, (size_t)max_envs * p->K * sizeof(float)));
@@ -301,6 +374,16 @@ int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream) {
     return pfail(EVAC_ERR_INVALID, "norm_mean, norm_var and norm_count must be given together");
   cudaStream_t st = (cudaStream_t)stream;
   PCK(cudaSetDevice(p->device));
+  if (p->NB == 0) {
+    // the linear policy: no embedding kernel; the heads read the observation, with the NormalizeObservation update fused into
+    // their X load, and always run (so that the normaliser does even without head outputs)
+    if (io->embedding) return pfail(EVAC_ERR_INVALID, "the linear policy (num_blocks = 0) has no embedding output");
+    if ((p->K & 3) == 0 && ((reinterpret_cast<uintptr_t>(io->obs) | reinterpret_cast<uintptr_t>(io->norm_mean) | reinterpret_cast<uintptr_t>(io->norm_var) |
+                             reinterpret_cast<uintptr_t>(io->obs_norm)) & 15u) != 0)
+      return pfail(EVAC_ERR_INVALID, "obs, norm_mean, norm_var and obs_norm must be 16-byte aligned");
+    NArgs n{io->norm_mean, io->norm_var, io->norm_count, io->obs_norm, io->norm_eps, io->norm_clip};
+    return launch_heads(p, io, io->obs, n, st);
+  }
   const bool heads = io->mean || io->value || io->action || io->action_clipped || io->logprob || io->entropy;
   float* emb = io->embedding;
   if (!emb && p->scratch_envs < io->num_envs) {
@@ -334,46 +417,7 @@ int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream) {
 #undef X
   if (rc) return rc;
   if (!heads) return EVAC_OK;
-  HArgs h;
-  memset(&h, 0, sizeof(h));
-  h.E = io->num_envs; h.K = p->K; h.K16 = p->K16; h.NH = p->NH; h.A = p->A;
-  h.emb = emb; h.w1t = p->d_w1t; h.b1 = p->d_b1; h.w2t = p->d_w2t; h.b2 = p->d_b2; h.w3 = p->d_w3; h.b3 = p->d_b3; h.logstd = p->d_logstd;
-  h.given_action = io->given_action;
-  h.mean = io->mean; h.value = io->value; h.action = io->action; h.action_clipped = io->action_clipped; h.logprob = io->logprob; h.entropy = io->entropy;
-  h.sample = io->sample;
-  h.seed_lo = a.seed_lo; h.seed_hi = a.seed_hi; h.offset = a.offset; h.offset_dev = a.offset_dev; h.env_offset = io->env_index_offset;
-  if (p->use_tc) {
-    // the heads on the tensor cores; 64-column tiles (critic and actor in separate CTAs) while 128-column tiles would not fill the SMs
-    TCArgs t;
-    t.h = h; t.chunks = p->tc_chunks; t.w2tc = p->d_w2tc;
-    const int gx = (h.E + TC_M - 1) / TC_M;
-    // shapes: 64 columns x 4 stages (critic and actor in separate CTAs) while 128-column tiles would not fill the SMs, 128 columns
-    // x 3 stages beyond (X is read once).  Measured per 8192 / 20 000 / 65 536 envs: 20.3 / 49.3 / 121.5 us (64x4), 29.7 / 50.4 /
-    // 105.0 us (128x3); 64 columns x 2 stages with two CTAs per SM: 24.6 / 53.6 / 113.1 us.
-    auto k64 = evac_policy_heads_tc_kernel<64, 4, 2, 1>;
-    auto k128 = evac_policy_heads_tc_kernel<128, 3, 2, 1>;
-    using S64 = TCShape<64, 4, 2>; using S128 = TCShape<128, 3, 2>;
-    static thread_local bool tc_attr[16] = {false};
-    if (!tc_attr[p->device & 15]) {
-      PCK(cudaFuncSetAttribute(k64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S64::SMEM_BYTES));
-      PCK(cudaFuncSetAttribute(k128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S128::SMEM_BYTES));
-      tc_attr[p->device & 15] = true;
-    }
-    if (gx < 2 * 148) { t.w1tc = p->d_w1tc64; k64<<<dim3(gx, 2), TC_THREADS, S64::SMEM_BYTES, st>>>(t); }
-    else { t.w1tc = p->d_w1tc128; k128<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t); }
-    PCK(cudaGetLastError());
-    p->launches++;
-    return EVAC_OK;
-  }
-  static thread_local size_t hattr[16] = {0};
-  if (p->heads_smem > 48 * 1024 && hattr[p->device & 15] < p->heads_smem) {
-    PCK(cudaFuncSetAttribute(evac_policy_heads_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->heads_smem));
-    hattr[p->device & 15] = p->heads_smem;
-  }
-  evac_policy_heads_kernel<<<(h.E + HD_TM - 1) / HD_TM, HD_THREADS, p->heads_smem, st>>>(h);
-  PCK(cudaGetLastError());
-  p->launches++;
-  return EVAC_OK;
+  return launch_heads(p, io, emb, NArgs{}, st);
 }
 
 int64_t evac_policy_launch_count(const EvacPolicy* p) { return p ? p->launches : -1; }

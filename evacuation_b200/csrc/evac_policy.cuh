@@ -506,6 +506,36 @@ __device__ __forceinline__ void heads_finish(const HArgs& a, int e, const float*
   if (a.entropy) a.entropy[e] = ent;
 }
 
+// NormalizeObservation + clip of the linear policy (num_blocks = 0), fused into the heads' load of X; with blocks it runs in the
+// embedding kernel's prologue instead.  Same fields and meaning as the PArgs norm_* fields.
+struct NArgs {
+  float* mean;                   // [E, K] running mean / variance (in place)
+  float* var;
+  const double* count;           // device scalar: samples seen so far (the caller advances it)
+  float* obs_norm;               // optional [E, K] out
+  float eps, clip;
+};
+
+// The per-call weights of one RunningMeanStd sample (gymnasium; op for op VectorNormalizer._update).
+struct NormWeights {
+  float w_new, w_old, w_mix;
+};
+__device__ __forceinline__ NormWeights norm_weights(const NArgs& n) {
+  const double cnt = *n.count, tot = cnt + 1.0;
+  NormWeights w;
+  w.w_new = (float)(1.0 / tot); w.w_old = (float)(cnt / tot);
+  w.w_mix = __fmul_rn(w.w_old, w.w_new);
+  return w;
+}
+// one (env, k) element: update its statistics in place, return the normalised, clipped value
+__device__ __forceinline__ float norm_update(float x, float& mean, float& var, const NormWeights& w, const NArgs& n) {
+  const float delta = __fsub_rn(x, mean);
+  mean = __fadd_rn(mean, __fmul_rn(delta, w.w_new));
+  var = __fadd_rn(__fmul_rn(var, w.w_old), __fmul_rn(__fmul_rn(delta, delta), w.w_mix));
+  const float z = __fmul_rn(__fsub_rn(x, mean), rsqrtf(__fadd_rn(var, n.eps)));
+  return min_nan(max_nan(z, -n.clip), n.clip);
+}
+
 __device__ __forceinline__ void cp_async16(float* dst_smem, const float* src, int src_bytes) {
   const unsigned d = (unsigned)__cvta_generic_to_shared(dst_smem);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d), "l"(src), "r"(src_bytes) : "memory");
@@ -531,7 +561,11 @@ __device__ __forceinline__ void heads_tile_fma(float (&acc)[8][8], const float4 
   }
 }
 
-__global__ void __launch_bounds__(HD_THREADS, 2) evac_policy_heads_kernel(const __grid_constant__ HArgs a) {
+// NORM: the linear policy's NormalizeObservation (NArgs) on every X element as it is loaded.  One CTA owns its 32 rows and every
+// column, and each k-chunk is loaded once, so each (env, k) statistic is read and written by exactly one thread of the grid.  The
+// X chunks then travel through registers (load, update, normalise, st.shared) instead of cp.async; the weight chunks keep the ring.
+template <bool NORM>
+__global__ void __launch_bounds__(HD_THREADS, 2) evac_policy_heads_kernel(const __grid_constant__ HArgs a, const __grid_constant__ NArgs n) {
   extern __shared__ float4 smem4[];
   float* wc = reinterpret_cast<float*>(smem4);        // [HD_STAGES][HD_KC][HD_COLS]
   float* xc = wc + HD_STAGES * HD_KC * HD_COLS;       // [HD_STAGES][HD_TM][HD_XS]
@@ -579,7 +613,21 @@ __global__ void __launch_bounds__(HD_THREADS, 2) evac_policy_heads_kernel(const 
       cp_async16(wd + 4 * v, ws + 4 * v, 16);
     }
     float* xd = xc + buf * HD_TM * HD_XS;
-    if (x_vec) {
+    if constexpr (NORM) {
+      const NormWeights nw = norm_weights(n);
+      for (int v = tid; v < HD_TM * HD_KC; v += HD_THREADS) {
+        const int r = v / HD_KC, kk = v - r * HD_KC, k = k0 + kk;
+        float z = 0.f;
+        if (r < ne && k < a.K) {
+          const size_t i = (size_t)(e0 + r) * a.K + k;
+          float mean = n.mean[i], var = n.var[i];
+          z = norm_update(a.emb[i], mean, var, nw, n);
+          n.mean[i] = mean; n.var[i] = var;
+          if (n.obs_norm != nullptr) n.obs_norm[i] = z;
+        }
+        xd[r * HD_XS + kk] = z;
+      }
+    } else if (x_vec) {
       for (int v = tid; v < HD_TM * HD_KC / 4; v += HD_THREADS) {
         const int r = v >> 2, kq = (v & 3) * 4;
         const int k = k0 + kq;

@@ -152,8 +152,12 @@ __device__ __forceinline__ void tc_tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) 
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-template <int NT, int ST, int AH, int MINB>
-__global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(const __grid_constant__ TCArgs a) {
+// NORM: the linear policy's NormalizeObservation (NArgs) on X as the producers load it.  Only with NT = 128: one CTA then owns its
+// rows and every column, so each (env, k) statistic is read and written by exactly one thread of the grid (with NT = 64 the critic
+// and the actor CTA of a row tile would both read the statistics while one of them updates them).
+template <int NT, int ST, int AH, int MINB, bool NORM = false>
+__global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(const __grid_constant__ TCArgs a, const __grid_constant__ NArgs n) {
+  static_assert(!NORM || NT == TC_COLS, "the fused normaliser needs one CTA per row tile");
   using SH = TCShape<NT, ST, AH>;
   constexpr int STAGES = SH::STAGES, HEADS = SH::HEADS, TC_AHEAD = SH::AHEAD;
   // TMEM columns: layer 1 [0, NT) = xh wh + xl wh, [NT, 2 NT) = xh wl (summed by epilogue 1); layer 2 from 2 NT; power of two
@@ -248,12 +252,14 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
       const int s = c % STAGES, use = c / STAGES;
       if (use > 0) tc_mbar_wait(&empty[s], (uint32_t)((use - 1) & 1));  // the MMAs that read this stage have completed
       uint8_t* st = smem + s * SH::STAGE_BYTES;
+      if constexpr (!NORM) {   // with NORM the X tiles of chunk c are written when chunk c is finished (below)
 #pragma unroll
-      for (int i = 0; i < 1024 / TC_ET; ++i) {
-        const int idx = i * TC_ET + tid, r = idx >> 3, c4 = idx & 7;
-        const int e = e0 + r, q = c * 8 + c4;
-        const bool in = e < h.E && q < kq;
-        cp_async16(reinterpret_cast<float*>(st + tc_swizzle(r, c4)), h.emb + (in ? (size_t)e * h.K + 4 * q : (size_t)0), in ? 16 : 0);
+        for (int i = 0; i < 1024 / TC_ET; ++i) {
+          const int idx = i * TC_ET + tid, r = idx >> 3, c4 = idx & 7;
+          const int e = e0 + r, q = c * 8 + c4;
+          const bool in = e < h.E && q < kq;
+          cp_async16(reinterpret_cast<float*>(st + tc_swizzle(r, c4)), h.emb + (in ? (size_t)e * h.K + 4 * q : (size_t)0), in ? 16 : 0);
+        }
       }
       if (tid == 0) {
         tc_mbar_expect_tx(&full[s], 2 * SH::WTILE_BYTES);
@@ -270,13 +276,52 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
       cp_async_commit();               // one group per iteration, empty or not: group index == chunk index
       cp_async_wait<TC_AHEAD>();       // this thread's requests of chunk c have landed
       uint8_t* st = smem + (c % STAGES) * SH::STAGE_BYTES;
+      if constexpr (NORM) {
+        // X through registers: the raw rows and their statistics in (all loads of the chunk issued before the first use),
+        // update + normalise + clip, statistics and obs_norm out, then the normalised value as the hi tile (the tensor core
+        // truncates it itself, as it does the cp.async'd raw value above) and its remainder as the lo tile
+        const NormWeights nw = norm_weights(n);
+        float4 x[1024 / TC_ET], m[1024 / TC_ET], v[1024 / TC_ET];
+        const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
-      for (int i = 0; i < 1024 / TC_ET; ++i) {
-        const int idx = i * TC_ET + tid, r = idx >> 3, c4 = idx & 7;
-        const uint32_t off = tc_swizzle(r, c4);
-        const float4 x = *reinterpret_cast<const float4*>(st + off);
-        *reinterpret_cast<float4*>(st + TC_XTILE_BYTES + off) =
-            make_float4(x.x - tc_trunc(x.x), x.y - tc_trunc(x.y), x.z - tc_trunc(x.z), x.w - tc_trunc(x.w));
+        for (int i = 0; i < 1024 / TC_ET; ++i) {
+          const int idx = i * TC_ET + tid, r = idx >> 3, c4 = idx & 7;
+          const int e = e0 + r, q = c * 8 + c4;
+          x[i] = m[i] = v[i] = zero;
+          if (e < h.E && q < kq) {
+            const size_t g = (size_t)e * h.K + 4 * q;
+            x[i] = *reinterpret_cast<const float4*>(h.emb + g);
+            m[i] = *reinterpret_cast<const float4*>(n.mean + g);
+            v[i] = *reinterpret_cast<const float4*>(n.var + g);
+          }
+        }
+#pragma unroll
+        for (int i = 0; i < 1024 / TC_ET; ++i) {
+          const int idx = i * TC_ET + tid, r = idx >> 3, c4 = idx & 7;
+          const int e = e0 + r, q = c * 8 + c4;
+          float4 z = zero;
+          if (e < h.E && q < kq) {
+            const size_t g = (size_t)e * h.K + 4 * q;
+            z.x = norm_update(x[i].x, m[i].x, v[i].x, nw, n); z.y = norm_update(x[i].y, m[i].y, v[i].y, nw, n);
+            z.z = norm_update(x[i].z, m[i].z, v[i].z, nw, n); z.w = norm_update(x[i].w, m[i].w, v[i].w, nw, n);
+            *reinterpret_cast<float4*>(n.mean + g) = m[i];
+            *reinterpret_cast<float4*>(n.var + g) = v[i];
+            if (n.obs_norm != nullptr) *reinterpret_cast<float4*>(n.obs_norm + g) = z;
+          }
+          const uint32_t off = tc_swizzle(r, c4);
+          *reinterpret_cast<float4*>(st + off) = z;
+          *reinterpret_cast<float4*>(st + TC_XTILE_BYTES + off) =
+              make_float4(z.x - tc_trunc(z.x), z.y - tc_trunc(z.y), z.z - tc_trunc(z.z), z.w - tc_trunc(z.w));
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < 1024 / TC_ET; ++i) {
+          const int idx = i * TC_ET + tid, r = idx >> 3, c4 = idx & 7;
+          const uint32_t off = tc_swizzle(r, c4);
+          const float4 x = *reinterpret_cast<const float4*>(st + off);
+          *reinterpret_cast<float4*>(st + TC_XTILE_BYTES + off) =
+              make_float4(x.x - tc_trunc(x.x), x.y - tc_trunc(x.y), x.z - tc_trunc(x.z), x.w - tc_trunc(x.w));
+        }
       }
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // cp.async / generic-proxy stores -> visible to the tensor core (async proxy)
       tc_mbar_arrive(&full[c % STAGES]);

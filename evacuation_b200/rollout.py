@@ -12,6 +12,9 @@ batched equivalent of that glue so that the loop never leaves the GPU:
   (`src/agents/networks/rpo_transformer_agent_network.py:36-163`,
   `rpo_linear_agent_network.py:19-61`) restated in plain PyTorch (library GEMMs / SDPA: this is
   the consumer of the step kernel, not a kernel target of this tier);
+* `RPOLinearPolicy`    -- the bare `RPOLinearNetwork` on the flattened observation (the gravity-encoding
+  and flat-observation configs), restated the same way;
+* `FusedRPOTransformerPolicy` / `FusedRPOLinearPolicy` -- their forward passes as the library's kernels;
 * `PolicyRollout`      -- policy -> step -> normalise, one iteration captured in a CUDA graph
   and replayed (the tiny-GEMM policy is otherwise launch-bound).
 
@@ -150,6 +153,45 @@ class _Block(nn.Module):
         return x.view(shape)
 
 
+def _rpo_heads(module: nn.Module, obs_dim: int, action_dim: int, num_hidden: int) -> None:
+    """RPOLinearNetwork's parameters (rpo_linear_agent_network.py:23-42) as `critic`, `actor_mean`, `actor_logstd` of `module`."""
+    module.critic = nn.Sequential(_ortho(nn.Linear(obs_dim, num_hidden)), nn.Tanh(), _ortho(nn.Linear(num_hidden, num_hidden)), nn.Tanh(),
+                                  _ortho(nn.Linear(num_hidden, 1), std=1.0))
+    module.actor_mean = nn.Sequential(_ortho(nn.Linear(obs_dim, num_hidden)), nn.Tanh(), _ortho(nn.Linear(num_hidden, num_hidden)), nn.Tanh(),
+                                      _ortho(nn.Linear(num_hidden, action_dim), std=0.01))
+    module.actor_logstd = nn.Parameter(torch.zeros(1, action_dim))
+
+
+def _rpo_action_and_value(module: nn.Module, x, action: Optional[torch.Tensor]):
+    """rpo_linear_agent_network.py:47-61 on the heads' input x: (action, logprob, entropy, value)."""
+    mean = module.actor_mean(x)
+    std = torch.exp(module.actor_logstd.expand_as(mean))
+    if action is None:
+        action = mean + std * torch.randn_like(mean)  # Normal(mean, std).sample()
+    else:  # RPO: perturb the mean when re-evaluating stored actions
+        mean = mean + torch.empty_like(mean).uniform_(-module.rpo_alpha, module.rpo_alpha)
+    var = std * std
+    logprob = (-((action - mean) ** 2) / (2 * var) - torch.log(std) - 0.5 * math.log(2 * math.pi)).sum(1)
+    entropy = (0.5 + 0.5 * math.log(2 * math.pi) + torch.log(std)).sum(1)
+    return action, logprob, entropy, module.critic(x)
+
+
+class RPOLinearPolicy(nn.Module):
+    """RPOLinearNetwork (rpo_linear_agent_network.py:19-61) directly on the flattened observation: the policy of the reference's
+    gravity-encoding (6 floats) and flat rel / ohe observation configs.  Parameter names are the reference's."""
+
+    def __init__(self, obs_dim: int, action_dim: int = 2, num_hidden: int = 64, rpo_alpha: float = 0.5):
+        super().__init__()
+        self.rpo_alpha = rpo_alpha
+        _rpo_heads(self, obs_dim, action_dim, num_hidden)
+
+    def get_value(self, x):
+        return self.critic(x)
+
+    def get_action_and_value(self, x, action: Optional[torch.Tensor] = None):
+        return _rpo_action_and_value(self, x, action)
+
+
 class RPOTransformerPolicy(nn.Module):
     """RPOTransformerEmbedding (rpo_transformer_agent_network.py:133-163) over RPOLinearNetwork
     (rpo_linear_agent_network.py:19-61).  `obs_dim` = (N + 2) * d_model flattened MatrixObs row."""
@@ -161,11 +203,7 @@ class RPOTransformerPolicy(nn.Module):
         d_model = obs_dim // (number_of_pedestrians + 2)
         self.rpo_alpha, self.chunk = rpo_alpha, chunk
         self.embedding = nn.Sequential(*[_Block(d_model, num_heads, dim_feedforward, dropout, use_resid) for _ in range(num_blocks)])
-        self.critic = nn.Sequential(_ortho(nn.Linear(obs_dim, num_hidden)), nn.Tanh(), _ortho(nn.Linear(num_hidden, num_hidden)), nn.Tanh(),
-                                    _ortho(nn.Linear(num_hidden, 1), std=1.0))
-        self.actor_mean = nn.Sequential(_ortho(nn.Linear(obs_dim, num_hidden)), nn.Tanh(), _ortho(nn.Linear(num_hidden, num_hidden)), nn.Tanh(),
-                                        _ortho(nn.Linear(num_hidden, action_dim), std=0.01))
-        self.actor_logstd = nn.Parameter(torch.zeros(1, action_dim))
+        _rpo_heads(self, obs_dim, action_dim, num_hidden)
 
     def embed(self, x):
         if x.shape[0] <= self.chunk:
@@ -176,17 +214,7 @@ class RPOTransformerPolicy(nn.Module):
         return self.critic(self.embed(x))
 
     def get_action_and_value(self, x, action: Optional[torch.Tensor] = None):
-        x = self.embed(x)
-        mean = self.actor_mean(x)
-        std = torch.exp(self.actor_logstd.expand_as(mean))
-        if action is None:
-            action = mean + std * torch.randn_like(mean)  # Normal(mean, std).sample()
-        else:  # RPO: perturb the mean when re-evaluating stored actions
-            mean = mean + torch.empty_like(mean).uniform_(-self.rpo_alpha, self.rpo_alpha)
-        var = std * std
-        logprob = (-((action - mean) ** 2) / (2 * var) - torch.log(std) - 0.5 * math.log(2 * math.pi)).sum(1)
-        entropy = (0.5 + 0.5 * math.log(2 * math.pi) + torch.log(std)).sum(1)
-        return action, logprob, entropy, self.critic(x)
+        return _rpo_action_and_value(self, self.embed(x), action)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -200,24 +228,18 @@ _FLAT_HEAD_KEYS = ("critic.0.weight", "critic.0.bias", "critic.2.weight", "criti
 
 def flatten_policy_weights(state_dict, num_blocks: int):
     """The reference module's `state_dict()` -> the flat float32 vector `evac_policy_load_weights` documents
-    (include/evac_b200.h).  Works on the unmodified reference `RPOTransformerEmbedding` and on `RPOTransformerPolicy`."""
+    (include/evac_b200.h).  Works on the unmodified reference `RPOTransformerEmbedding` and on `RPOTransformerPolicy`; with
+    num_blocks = 0 on `RPOLinearPolicy` (the heads only)."""
     parts = [state_dict[f"embedding.{b}.{k}"] for b in range(num_blocks) for k in _FLAT_BLOCK_KEYS]
     parts += [state_dict[k] for k in _FLAT_HEAD_KEYS]
     return torch.cat([p.detach().to(torch.float32).reshape(-1).cpu() for p in parts]).contiguous()
 
 
-class FusedRPOTransformerPolicy:
-    """Forward-only CUDA implementation of `RPOTransformerPolicy` (= the reference's `RPOTransformerEmbedding`):
-    two hand-written kernels behind `evac_policy_forward` (csrc/evac_policy.cuh) instead of ~60 library launches --
-    the transformer blocks run one warp per environment out of registers, the actor / critic heads 32 environments
-    per CTA, Normal sampling, log-probability and ClipAction included.  Optionally fuses the per-env
-    NormalizeObservation + clip of `VectorNormalizer` into its prologue (`normalizer=`).
+class _FusedRPOPolicy:
+    """What the fused policies share: the `evac_policy` handle, weight snapshots, the device call counter and `forward`.
+    There is no CPU fallback: construction fails without the CUDA library / a device."""
 
-    Weights are snapshotted from a torch module (`load_from`); call it again after an optimiser step.  There is no
-    CPU fallback: construction fails without the CUDA library / a device."""
-
-    def __init__(self, module: "RPOTransformerPolicy", number_of_pedestrians: int, device="cuda", seed: int = 0,
-                 env_index_offset: int = 0, max_envs: int = 0):
+    def __init__(self, cfg, module, obs_dim: int, device, seed: int, env_index_offset: int):
         import ctypes as C
 
         from . import _native as nat
@@ -225,17 +247,8 @@ class FusedRPOTransformerPolicy:
         self._C, self._nat, self._lib = C, nat, nat.load()
         self.device = torch.device(device)
         if self.device.type != "cuda":
-            raise nat.EvacNativeError("FusedRPOTransformerPolicy needs a CUDA device (no CPU fallback)")
-        blk = module.embedding[0]
-        self.S, self.D = number_of_pedestrians + 2, blk.d_model
-        self.A = module.actor_mean[4].out_features
-        cfg = nat.EvacPolicyConfig()
-        nat.check(self._lib.evac_policy_default_config(C.byref(cfg), number_of_pedestrians, self.D))
-        cfg.num_heads, cfg.dim_feedforward = blk.attention.num_heads, blk.ff[0].out_features
-        cfg.num_blocks, cfg.use_resid = len(module.embedding), int(blk.use_resid)
-        cfg.dropout, cfg.layer_norm_eps = float(blk.dropout.p), float(blk.norm1.eps)
-        cfg.num_hidden, cfg.action_dim = module.critic[0].out_features, self.A
-        self.cfg, self.num_blocks = cfg, cfg.num_blocks
+            raise nat.EvacNativeError(f"{type(self).__name__} needs a CUDA device (no CPU fallback)")
+        self.cfg, self.num_blocks, self.obs_dim, self.A = cfg, cfg.num_blocks, int(obs_dim), cfg.action_dim
         self.seed, self.env_index_offset = int(seed), int(env_index_offset)
         self._h = C.c_void_p()
         idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
@@ -243,8 +256,6 @@ class FusedRPOTransformerPolicy:
         self.calls = torch.zeros((), dtype=torch.int64, device=self.device)  # device-side stream offset (graph-replay safe)
         self.training = True  # like the reference's rollouts (the module is never put in eval mode)
         self.load_from(module)
-        if max_envs:
-            nat.check(self._lib.evac_policy_reserve(self._h, int(max_envs)))
 
     def load_from(self, module) -> None:
         flat = flatten_policy_weights(module.state_dict(), self.num_blocks)
@@ -278,8 +289,8 @@ class FusedRPOTransformerPolicy:
                 given_action=None, sample=True, normalizer: Optional["VectorNormalizer"] = None, obs_norm=None, advance=True):
         """One fused forward on the current stream; every output is an optional preallocated tensor."""
         E = obs.shape[0]
-        if obs.numel() != E * self.S * self.D:
-            raise ValueError(f"obs must hold [E, {self.S * self.D}] values, got {tuple(obs.shape)}")
+        if obs.numel() != E * self.obs_dim:
+            raise ValueError(f"obs must hold [E, {self.obs_dim}] values, got {tuple(obs.shape)}")
         io = self._nat.EvacPolicyIO()
         io.num_envs, io.obs = E, self._ptr(obs)
         if normalizer is not None:
@@ -299,12 +310,7 @@ class FusedRPOTransformerPolicy:
         if advance:
             self.calls.add_(1)
 
-    # ---- the reference module's surface (rpo_transformer_agent_network.py:155-163)
-    def embed(self, x):
-        out = torch.empty((x.shape[0], self.S * self.D), device=self.device)
-        self.forward(x.contiguous(), embedding=out)
-        return out
-
+    # ---- the reference module's surface (rpo_linear_agent_network.py:44-61)
     def get_value(self, x):
         v = torch.empty(x.shape[0], device=self.device)
         self.forward(x.contiguous(), value=v, sample=False)
@@ -325,6 +331,55 @@ class FusedRPOTransformerPolicy:
                 self._h = None
         except Exception:
             pass
+
+
+class FusedRPOTransformerPolicy(_FusedRPOPolicy):
+    """Forward-only CUDA implementation of `RPOTransformerPolicy` (= the reference's `RPOTransformerEmbedding`):
+    two hand-written kernels behind `evac_policy_forward` (csrc/evac_policy.cuh) instead of ~60 library launches --
+    the transformer blocks run one warp per environment out of registers, the actor / critic heads 32 environments
+    per CTA, Normal sampling, log-probability and ClipAction included.  Optionally fuses the per-env
+    NormalizeObservation + clip of `VectorNormalizer` into its prologue (`normalizer=`).
+
+    Weights are snapshotted from a torch module (`load_from`); call it again after an optimiser step.  There is no
+    CPU fallback: construction fails without the CUDA library / a device."""
+
+    def __init__(self, module: "RPOTransformerPolicy", number_of_pedestrians: int, device="cuda", seed: int = 0,
+                 env_index_offset: int = 0, max_envs: int = 0):
+        from . import _native as nat
+
+        blk = module.embedding[0]
+        self.S, self.D = number_of_pedestrians + 2, blk.d_model
+        cfg = nat.EvacPolicyConfig()
+        nat.check(nat.load().evac_policy_default_config(cfg, number_of_pedestrians, self.D))
+        cfg.num_heads, cfg.dim_feedforward = blk.attention.num_heads, blk.ff[0].out_features
+        cfg.num_blocks, cfg.use_resid = len(module.embedding), int(blk.use_resid)
+        cfg.dropout, cfg.layer_norm_eps = float(blk.dropout.p), float(blk.norm1.eps)
+        cfg.num_hidden, cfg.action_dim = module.critic[0].out_features, module.actor_mean[4].out_features
+        super().__init__(cfg, module, self.S * self.D, device, seed, env_index_offset)
+        if max_envs:
+            self.reserve(max_envs)
+
+    # ---- the reference module's surface (rpo_transformer_agent_network.py:155-163)
+    def embed(self, x):
+        out = torch.empty((x.shape[0], self.S * self.D), device=self.device)
+        self.forward(x.contiguous(), embedding=out)
+        return out
+
+
+class FusedRPOLinearPolicy(_FusedRPOPolicy):
+    """Forward-only CUDA implementation of `RPOLinearPolicy` (the reference's RPOLinearNetwork on the flattened observation):
+    ONE kernel per forward -- the critic / actor MLPs on the tensor cores when `obs_dim` is a multiple of 4, else on the CUDA
+    cores, with Normal sampling, log-probability and ClipAction -- and with `normalizer=` the per-env NormalizeObservation + clip
+    of `VectorNormalizer` fused into the kernel's load of the observation.  `forward` takes the transformer class's keywords;
+    `embedding=` is rejected (ValueError): this network has none.  `train()` / `eval()` are accepted (there is no dropout)."""
+
+    def __init__(self, module: "RPOLinearPolicy", obs_dim: int, device="cuda", seed: int = 0, env_index_offset: int = 0):
+        from . import _native as nat
+
+        cfg = nat.EvacPolicyConfig()
+        nat.check(nat.load().evac_policy_default_linear_config(cfg, int(obs_dim)))
+        cfg.num_hidden, cfg.action_dim = module.critic[0].out_features, module.actor_mean[4].out_features
+        super().__init__(cfg, module, obs_dim, device, seed, env_index_offset)
 
 
 def normalize_reward_fused(norm: "VectorNormalizer", reward: torch.Tensor, terminated: torch.Tensor, out: torch.Tensor,
@@ -353,7 +408,7 @@ class PolicyRollout:
     One iteration is captured in a CUDA graph (`use_graph=True`) and replayed; storage tensors follow
     rpo_agent.py:160-163 (obs, actions, logprobs, rewards, dones, values)."""
 
-    def __init__(self, env, policy: RPOTransformerPolicy, gamma: float = 0.99, use_graph: bool = True, store: bool = True):
+    def __init__(self, env, policy, gamma: float = 0.99, use_graph: bool = True, store: bool = True):
         self.env, self.policy, self.store, self.use_graph = env, policy, store, use_graph
         u = env.unwrapped
         self.E, self.D, self.device = u.num_envs, u.obs_dim, u.device
@@ -364,36 +419,39 @@ class PolicyRollout:
                     (("action", (self.E, 2)), ("logprob", (self.E,)), ("value", (self.E,)), ("reward", (self.E,)))}
         self._graph = None
         self.launches_per_iteration = None
-        # fused policy: NormalizeObservation runs in the prologue of the policy kernel on the env's raw observation buffer,
-        # so `next_obs` (the normalised observation the policy saw) is produced INSIDE the iteration
-        self.fused = isinstance(policy, FusedRPOTransformerPolicy)
+        # fused policy: NormalizeObservation runs in the policy's first kernel on the env's raw observation buffer, so `next_obs`
+        # (the normalised observation the policy saw) is produced INSIDE the iteration
+        self.fused = isinstance(policy, _FusedRPOPolicy)
         self._raw_obs = None
         self._act_clipped = torch.zeros((self.E, 2), device=self.device)
         if self.fused:
             policy.reserve(self.E)
 
     def reset(self):
-        obs, _ = self.env.reset()
+        self.env.reset()
+        obs = self.env.unwrapped.flat_observation  # Box or Dict: the env's persistent [E, D] buffer (step() rewrites it)
         if self.fused:
-            self._raw_obs = obs.reshape(self.E, self.D)  # the env's persistent observation buffer (step() rewrites it)
+            self._raw_obs = obs
         else:
-            self.next_obs.copy_(self.norm.observation(obs.reshape(self.E, self.D)))
+            self.next_obs.copy_(self.norm.observation(obs))
         self.next_done.zero_()
 
     @torch.no_grad()
     def _iteration(self):
-        if self.fused:  # 4 launches: policy embedding, policy heads (+ sampling, ClipAction), env step, reward normaliser
+        if self.fused:
+            # transformer: 4 launches (policy embedding, policy heads (+ sampling, ClipAction), env step, reward normaliser);
+            # linear: 3 (the heads with the normaliser fused into their load of the observation, env step, reward normaliser)
             self.policy.forward(self._raw_obs, normalizer=self.norm, obs_norm=self.next_obs, action=self.out["action"],
                                 action_clipped=self._act_clipped, logprob=self.out["logprob"], value=self.out["value"])
-            obs, reward, term, trunc, _ = self.env.step(self._act_clipped)
-            assert obs.data_ptr() == self._raw_obs.data_ptr()
+            _, reward, term, trunc, _ = self.env.step(self._act_clipped)
+            assert self.env.unwrapped.flat_observation.data_ptr() == self._raw_obs.data_ptr()
             normalize_reward_fused(self.norm, reward, term, self.out["reward"], truncated=trunc, done_out=self.next_done)
             return
         action, logprob, _, value = self.policy.get_action_and_value(self.next_obs)
-        obs, reward, term, trunc, _ = self.env.step(action.clamp(-1.0, 1.0).contiguous())  # ClipAction
+        _, reward, term, trunc, _ = self.env.step(action.clamp(-1.0, 1.0).contiguous())  # ClipAction
         self.out["action"].copy_(action); self.out["logprob"].copy_(logprob); self.out["value"].copy_(value.flatten())
         self.out["reward"].copy_(self.norm.reward(reward, term))
-        self.next_obs.copy_(self.norm.observation(obs.reshape(self.E, self.D)))
+        self.next_obs.copy_(self.norm.observation(self.env.unwrapped.flat_observation))
         self.next_done.copy_(torch.logical_or(term, trunc).to(self.next_done.dtype))
 
     def _snapshot(self):
@@ -463,4 +521,5 @@ class PolicyRollout:
         return buf
 
 
-__all__ = ["VectorNormalizer", "RPOTransformerPolicy", "FusedRPOTransformerPolicy", "PolicyRollout", "flatten_policy_weights", "normalize_reward_fused"]
+__all__ = ["VectorNormalizer", "RPOTransformerPolicy", "RPOLinearPolicy", "FusedRPOTransformerPolicy", "FusedRPOLinearPolicy", "PolicyRollout",
+           "flatten_policy_weights", "normalize_reward_fused"]

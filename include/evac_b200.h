@@ -227,19 +227,26 @@ int32_t evac_abi_version(void);
  *   evac_policy_*            RPOTransformerEmbedding.get_action_and_value / get_value, forward only
  *                                                                  src/agents/networks/rpo_transformer_agent_network.py:36-163
  *                                                                  src/agents/networks/rpo_linear_agent_network.py:19-61
+ *                            or, with num_blocks = 0, RPOLinearNetwork on the flattened observation (the gravity-encoding
+ *                            and flat-observation configs): no embedding kernel, the heads read the observation
  *                            + (optional, fused) gymnasium NormalizeObservation + clip(-1, 1), ClipAction
  *                                                                  src/agents/rpo_agent.py:24-33,186-193
  *   evac_normalize_reward    gymnasium NormalizeReward(gamma) + clip(-100, 100)      src/agents/rpo_agent.py:31-32
  *
  * The policy reads the [E, (N+2)*d_model] MatrixObs rows evac_step writes and produces the [E,2] actions evac_step
- * consumes, so policy -> step -> normalise stays on the device (two launches for the policy, one for the step). */
+ * consumes, so policy -> step -> normalise stays on the device (two launches for the policy, one for the step; one for the
+ * linear policy).
+ *
+ * num_blocks = 0 means "RPOLinearNetwork directly on the observation": K = seq_len * d_model is the observation width
+ * (evac_policy_default_linear_config: seq_len 1, d_model = obs_dim), 1 <= K <= 4096, num_heads / dim_feedforward / use_resid /
+ * dropout / layer_norm_eps are unused, and the weights are the heads part of the layout below only. */
 typedef struct EvacPolicyConfig {
   int32_t abi_version;      /* must be EVAC_ABI_VERSION */
-  int32_t seq_len;          /* S = number_of_pedestrians + 2 rows of the observation, 1 .. 64 */
-  int32_t d_model;          /* values per row: 6 (ohe), 3 (cat) or 2 (no statuses) */
+  int32_t seq_len;          /* S = number_of_pedestrians + 2 rows of the observation, 1 .. 64 (num_blocks = 0: 1) */
+  int32_t d_model;          /* values per row: 6 (ohe), 3 (cat) or 2 (no statuses) (num_blocks = 0: the observation width) */
   int32_t num_heads;        /* RPOTransformerEmbeddingConfig.num_heads (3); 1 .. 4 (every (d_model, num_heads) pair is instantiated) */
   int32_t dim_feedforward;  /* .dim_feedforward (96) */
-  int32_t num_blocks;       /* .num_blocks (2) */
+  int32_t num_blocks;       /* .num_blocks (2); 0 .. 8, 0 = the linear policy without embedding */
   int32_t use_resid;        /* .use_resid (0) */
   float dropout;            /* .dropout (0.1); applied only when EvacPolicyIO.training != 0 */
   float layer_norm_eps;     /* nn.LayerNorm default 1e-5 */
@@ -250,6 +257,9 @@ typedef struct EvacPolicyConfig {
 typedef struct EvacPolicy EvacPolicy;
 
 int evac_policy_default_config(EvacPolicyConfig* cfg, int32_t number_of_pedestrians, int32_t d_model);
+/* RPOLinearNetwork defaults (num_hidden 64, action_dim 2) on an observation of obs_dim floats: num_blocks 0, seq_len 1,
+ * d_model obs_dim. */
+int evac_policy_default_linear_config(EvacPolicyConfig* cfg, int32_t obs_dim);
 int evac_policy_create(const EvacPolicyConfig* cfg, int32_t device, EvacPolicy** out);
 int evac_policy_destroy(EvacPolicy* p);
 /* Number of floats evac_policy_load_weights expects, in this order (PyTorch parameter layouts, row-major):
@@ -263,7 +273,7 @@ int64_t evac_policy_num_weights(const EvacPolicy* p);
 /* `weights` is a HOST pointer; the library repacks it for the kernels and uploads it (synchronous). */
 int evac_policy_load_weights(EvacPolicy* p, const float* weights, int64_t count);
 /* Pre-allocate the internal embedding scratch for up to `max_envs` environments (needed before a forward call is
- * captured in a CUDA graph without an `embedding` output buffer). */
+ * captured in a CUDA graph without an `embedding` output buffer).  No-op for the linear policy. */
 int evac_policy_reserve(EvacPolicy* p, int32_t max_envs);
 
 typedef struct EvacPolicyIO {
@@ -278,7 +288,7 @@ typedef struct EvacPolicyIO {
   float* obs_norm;
   float norm_eps, norm_clip;
   /* outputs (device), any may be NULL */
-  float* embedding;          /* [E, S*D] output of the transformer blocks */
+  float* embedding;          /* [E, S*D] output of the transformer blocks; must be NULL for the linear policy */
   float* mean;               /* [E, A] actor mean */
   float* value;              /* [E] critic */
   float* action;             /* [E, A] Normal(mean, exp(logstd)).sample() (or `given_action`, or the mean if !sample) */
@@ -297,7 +307,10 @@ typedef struct EvacPolicyIO {
 /* embedding kernel (+ heads kernel if any head output is requested), asynchronous on `stream`.  The heads -- the 372 x 128 and
  * 64 x 64 dense layers of rpo_linear_agent_network.py:23-42, the one dense contraction on this path -- run as 3xTF32 tcgen05.mma with
  * the accumulators in tensor memory (csrc/evac_policy_tc.cuh) whenever S * D is a multiple of 4; otherwise, or with EVAC_POLICY_TC=0 in
- * the environment at evac_policy_create, on the CUDA cores.  Both agree with a float64 evaluation to 3e-6. */
+ * the environment at evac_policy_create, on the CUDA cores.  Both agree with a float64 evaluation to 3e-6.
+ * Linear policy (num_blocks = 0): ONE launch, the heads kernel on `obs` (always, so that the normaliser runs even without head
+ * outputs); the NormalizeObservation update + clip runs in the heads' load of X, and `obs` (plus norm_mean / norm_var / obs_norm
+ * when K is a multiple of 4) must be 16-byte aligned. */
 int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream);
 int64_t evac_policy_launch_count(const EvacPolicy* p);
 
