@@ -70,7 +70,7 @@ struct EvacHandle {
   int64_t launches = 0;
   int threads = 0, ppt = 0;
   int num_sms = 0;
-  int cells_x = 0, cells_y = 0, cell_reach = 1;  // > 0: cell-list neighbour search (multi-warp fp32 shapes)
+  int cells_x = 0, cells_y = 0, cell_reach = 1;  // > 0: cell-list neighbour search (fp32; N <= 64: the sparse pass's cell masks)
   int cell_pair_walk = 1;        // paired walk of the sorted slots (0: one slot per thread)
   int cluster = 1;               // > 1: one environment per thread-block cluster of this many 1024 x 4 CTAs (N > 4096, evac_cluster.cuh)
 };
@@ -99,6 +99,14 @@ static int compute_obs_dim(const EvacConfig& c) {
   return 4 + 2 * n + sc * n;
 }
 
+// Cell grid of the one-warp kernel's sparse pass: edge >= (1 + 1e-4) x vision radius (two pedestrians closer than the radius
+// sit in the same or in adjacent cells, float32 rounding of the cell index included), 1 .. WCELLS cells per axis.
+static void warp_cell_grid(const EvacConfig& c, int* gx, int* gy) {
+  const double edge = c.to_pedestrian * (1.0 + 1e-4);
+  *gx = (int)fmax(1.0, fmin((double)WCELLS, floor(2.0 * c.width / edge)));
+  *gy = (int)fmax(1.0, fmin((double)WCELLS, floor(2.0 * c.height / edge)));
+}
+
 template <typename real>
 static KArgs<real> make_args(const EvacHandle* h) {
   const EvacConfig& c = h->cfg;
@@ -112,8 +120,9 @@ static KArgs<real> make_args(const EvacHandle* h) {
   a.thr2_ped = thr2_of<real>(c.to_pedestrian); a.thr2_leader = thr2_of<real>(c.to_leader);
   a.thr2_exit = thr2_of<real>(c.to_exit); a.thr2_escape = thr2_of<real>(c.to_escape);
   a.cells_x = h->cells_x; a.cells_y = h->cells_y; a.cell_reach = h->cell_reach; a.cell_pair_walk = h->cell_pair_walk;
-  a.cell_inv_x = h->cells_x > 0 ? (float)(h->cells_x / (2.0 * c.width)) : 0.f;
-  a.cell_inv_y = h->cells_y > 0 ? (float)(h->cells_y / (2.0 * c.height)) : 0.f;
+  a.cell_force = h->blocks != nullptr && c.neighbor_search == EVAC_SEARCH_CELLS;  // one-warp kernel, "cells"
+  a.cell_inv_x = a.cells_x > 0 ? (float)(a.cells_x / (2.0 * c.width)) : 0.f;
+  a.cell_inv_y = a.cells_y > 0 ? (float)(a.cells_y / (2.0 * c.height)) : 0.f;
   a.exit_reward = c.is_new_exiting_reward; a.follow_reward = c.is_new_followers_reward;
   a.term_wall = c.is_termination_agent_wall_collision;
   a.init_reward = (real)c.init_reward_each_step; a.intrinsic_coef = (real)c.intrinsic_reward_coef;
@@ -368,13 +377,10 @@ int evac_create(const EvacConfig* cfg, int32_t num_envs, int32_t device, uint64_
     //    ~25 % more candidates): 109.8 / 147.8 / 246.1 us paired vs 118.1 / 153.4 / 247.9 us grouped (128 x 8192: 226.9 vs 234.6;
     //    1024 x 1000: 85.1 vs 89.9) -- the walk is not bound by shared-memory bandwidth either: what it costs is the number of
     //    evaluated candidate pairs times the trip-count divergence inside a warp.
-  } else if (h->threads == 32 && h->prec == EVAC_PREC_F32 && cfg->neighbor_search == EVAC_SEARCH_CELLS) {
-    // one-warp kernel, opt-in: vertical strips (a 1-D cell list, at most 32 strips), same edge rule.  Measured on
-    // B200 (profiles/README.md): 15 % fewer instructions than the all-pairs tile but no wall-clock gain (the warp is
-    // latency-bound and the per-lane windows turn the broadcast LDS.128 into conflicting ones), and the all-pairs
-    // tile sums in pedestrian-index order like the reference -> AUTO keeps all pairs for N <= 64.
-    const int gx = (int)fmin(32.0, floor(2.0 * cfg->width / (cfg->to_pedestrian * (1.0 + 1e-4))));
-    if (gx >= 1) { h->cells_x = gx; h->cells_y = 1; }
+  } else if (h->threads == 32 && h->prec == EVAC_PREC_F32 && cfg->neighbor_search != EVAC_SEARCH_BRUTE) {
+    // one-warp kernel: the cell masks of the sparse pass.  "cells" pins the kernel to it (whenever exact), "auto" chooses per
+    // warp and step (KArgs::cell_force); evac_num_cells reports the grid only where it is pinned
+    warp_cell_grid(*cfg, &h->cells_x, &h->cells_y);
   }
   const size_t en = (size_t)h->E * h->N, es = h->prec == EVAC_PREC_F64 ? 16 : 8;
 #define ALLOC(ptr, bytes)                                                      \
@@ -417,7 +423,10 @@ int evac_destroy(EvacHandle* h) {
 }
 
 int32_t evac_obs_dim(const EvacHandle* h) { return h ? h->obs_dim : -1; }
-int32_t evac_num_cells(const EvacHandle* h) { return h ? h->cells_x * h->cells_y : -1; }
+int32_t evac_num_cells(const EvacHandle* h) {
+  if (!h) return -1;
+  return h->threads == 32 && h->cfg.neighbor_search == EVAC_SEARCH_AUTO ? 0 : h->cells_x * h->cells_y;
+}
 int32_t evac_num_envs(const EvacHandle* h) { return h ? h->E : -1; }
 int32_t evac_state_elem_size(const EvacHandle* h) { return h ? (h->prec == EVAC_PREC_F64 ? 8 : 4) : -1; }
 int64_t evac_launch_count(const EvacHandle* h) { return h ? h->launches : -1; }

@@ -56,10 +56,12 @@ struct KArgs {
   float width_f, height_f, step_size_f, eps_f, enslaving_f;  // the agent's arithmetic is float32 in the reference
   // thresholds on SQUARED distances, chosen on the host so that (d2 < thr2) == (sqrt(d2) < thr) exactly
   real thr2_ped, thr2_leader, thr2_exit, thr2_escape;
-  // uniform cell grid of the neighbour search (multi-warp shapes, float32): cells_x * cells_y cells of edge
-  // >= vision radius over [-width,width] x [-height,height]; cells_x == 0 -> brute-force tiled pass
+  // uniform cell grid of the neighbour search (float32): cells_x * cells_y cells of edge >= vision radius over
+  // [-width,width] x [-height,height]; cells_x == 0 -> brute-force tiled pass.  N <= 64: the cell masks of the one-warp
+  // kernel's sparse pass (evac_warp.cuh), taken per warp and step unless the all-pairs loop is cheaper or cell_force is set
   int cells_x, cells_y, cell_reach;  // neighbours within `cell_reach` cells (cell edge >= radius / cell_reach)
   int cell_pair_walk;                // cell_list_pass step 5: two adjacent sorted slots of one cell row per thread (shared window)
+  int cell_force;                    // N <= 64: the sparse pass whenever it is exact (no cost comparison)
   float cell_inv_x, cell_inv_y;      // cells per unit length
   int exit_reward, follow_reward, term_wall;
   real init_reward, intrinsic_coef;

@@ -19,24 +19,61 @@ enum { WMODE_GENERIC = 0, WMODE_REL_OHE_BOX = 1, WMODE_GRAV = 2 };
 
 __device__ __forceinline__ float2 splat(float v) { return make_float2(v, v); }
 
-// Neighbour sums of ONE pedestrian over the slot pairs [j0, j1) of the strip-sorted tile (accumulate_pair like
-// pairwise_pass; trip counts differ per lane, finished lanes idle).
-__device__ __forceinline__ void windowed_pass(const Tile<float>& t, int j0, int j1, float x, float y, float thr2, float& sx, float& sy) {
-  const float2 nx = splat(-x), ny = splat(-y);
+// ---- Sparse neighbour pass from 2-D cell masks (N <= 64, a.cells_x > 0).
+// A uniform grid of cells_x x cells_y cells (edge >= 1.0001 x vision radius, at most 32 per axis) over the area: every pair
+// with d² < thr² sits in the 3 x 3 block of cells around the target, float32 rounding of the cell index included.  Per row
+// and per column of the grid one 64-bit set of TILE SLOTS (.x = slots 0-31, .y = 32-63) of the moving sources in it; the
+// candidates of a target in cell (r, c) are (rows r-1..r+1) & (columns c-1..c+1).  Entry 0 and entry cells + 1 of both
+// arrays stay empty, so the three neighbouring entries of any cell are read without bounds tests.
+constexpr int WCELLS = 32;
+constexpr int WREC_PARK = 64;  // per-slot record of a parked source: what a lane with no candidate left reads
+
+__device__ __forceinline__ uint2 or3(const uint2* m, int c) {
+  const uint2 a = m[c], b = m[c + 1], d = m[c + 2];
+  return make_uint2(a.x | b.x | d.x, a.y | b.y | d.y);
+}
+
+// Neighbour sums of ONE pedestrian at (x, y) over the slots of the candidate set m, walked in increasing slot order, T times
+// (the warp's maximum: a lane whose set is empty reads the parked record, which fails the distance test and adds 0 * 0).
+// Bit-identical to pairwise_pass<2, ..> (the all-pairs loop) when no source direction is NaN:
+//   * the pair test is the same float32 expression as accumulate_pair, written with explicit round-to-nearest intrinsics so
+//     that no contraction can differ from the packed form: dx = x_j + (-x), dy likewise, d² = fma(dy, dy, dx * dx) < thr²;
+//   * the all-pairs loop keeps two chains per component, even slots in .x and odd slots in .y, each in increasing slot
+//     order, and returns .x + .y: here the candidate goes into the chain of its slot's parity (w = 0 in the other one),
+//     in increasing slot order too;
+//   * the all-pairs loop also adds fma(0, u_j, acc) for every slot that fails the test, which is what the sparse walk skips.
+//     That is an exact no-op: u_j is finite (no NaN source; a unit vector is finite or NaN), so 0 * u_j = ±0, and
+//     acc + ±0 == acc unless acc is -0 -- which it never is: acc starts at +0, and a round-to-nearest sum is -0 only when
+//     both terms are -0.  Slots outside the 3 x 3 block fail the test (the superset property above), so skipping them
+//     and skipping the failing candidates both leave every chain's bits unchanged.
+__device__ __forceinline__ void sparse_pass(const float4* rec, uint2 m, int T, float x, float y, float thr2, float& sx, float& sy) {
+  const float nx = -x, ny = -y;
   float2 ax = make_float2(0.f, 0.f), ay = make_float2(0.f, 0.f);
-  if (j0 < j1) {
-    float4 p = t.P2[j0], u = t.U2[j0];
-#pragma unroll 2
-    for (int j = j0; j < j1; ++j) {
-      const float4 pn = t.P2[j + 1], un = t.U2[j + 1];  // look-ahead (at most the tile's spare entry)
-      accumulate_pair(p, u, nx, ny, thr2, ax, ay);
-      p = pn;
-      u = un;
-    }
+  for (int t = 0; t < T; ++t) {
+    // next slot, written as selects (no branch): the lowest bit of .x, else 32 + the lowest bit of .y, else the parked record
+    const unsigned jy = 32u + min((unsigned)(__ffs(m.y) - 1), 32u);
+    const unsigned j = m.x ? (unsigned)(__ffs(m.x) - 1) : jy;
+    const unsigned y1 = m.y & (m.y - 1u);
+    m.y = m.x ? m.y : y1;
+    m.x &= m.x - 1u;
+    const float4 r = rec[j];
+    const float dx = __fadd_rn(r.x, nx), dy = __fadd_rn(r.y, ny);
+    const float d2 = __fmaf_rn(dy, dy, __fmul_rn(dx, dx));
+    const float w = d2 < thr2 ? 1.f : 0.f;
+    const float2 w2 = (j & 1) ? make_float2(0.f, w) : make_float2(w, 0.f);
+    ax = __ffma2_rn(w2, splat(r.z), ax);
+    ay = __ffma2_rn(w2, splat(r.w), ay);
   }
   sx = ax.x + ax.y;
   sy = ay.x + ay.y;
 }
+
+// Warp-maximum walk lengths against the all-pairs loop: the sparse pass is taken when
+// SPARSE_COST_NUM * (T0 + T1) <= SPARSE_COST_DEN * (slot pairs of the all-pairs loop).  1 : 1 is an estimate from the SASS,
+// NOT a measurement: one walk step (bit extraction, LDS.128, pair test, two FFMA2) is ~24 instructions in a two-step unrolled
+// body, one slot pair of the all-pairs loop (two LDS.128, four pair evaluations) ~20; the walk step also waits on its own
+// LDS.128 where the all-pairs loop loads one iteration ahead, so the true break-even may lie below 1 : 1.
+constexpr int SPARSE_COST_NUM = 1, SPARSE_COST_DEN = 1;
 
 // per-pedestrian working set of the warp kernel
 struct WPed {
@@ -55,14 +92,14 @@ template <int MODE>
 __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_constant__ KArgs<float> a) {  // @region wload
   // Tile<float> of 64 slots (+ the look-ahead entries) = 66 float4
   __shared__ __align__(16) float4 tile_smem[66];
-  // strip culling (a.cells_x > 0): the sources are sorted by vertical strip (edge >= vision radius) so that a
-  // pedestrian only visits the slots of its own and the two adjacent strips
-  __shared__ uint2 strip_mask[32];   // per strip: which lanes' pedestrian 0 (.x) / pedestrian 1 (.y) sit in it
-  __shared__ int strip_start[33];    // first slot of every strip (+ total)
+  // sparse pass (a.cells_x > 0): {x, y, ux, uy} of every slot (+ the parked record) and the row / column slot masks
+  __shared__ float4 rec[WREC_PARK + 1];
+  __shared__ uint2 row_mask[WCELLS + 2], col_mask[WCELLS + 2];
   const int lane = threadIdx.x & 31, e = blockIdx.x, N = a.N;
   if (e >= a.E) return;
   const Tile<float> tile(reinterpret_cast<unsigned char*>(tile_smem), 64);
-  const int S = a.cells_x;
+  const bool cells = a.cells_x > 0;
+  if (lane == 0) rec[WREC_PARK] = make_float4(PARK, PARK, 0.f, 0.f);
   const uint32_t lt_mask = (1u << lane) - 1u;
   const bool valid[2] = {lane < N, lane + 32 < N};
   const uint32_t env_g = (uint32_t)(a.env_offset + e);
@@ -136,56 +173,57 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
       if (so == ST_EXITING) q[k].d = __fmul2_rn(v, splat(fminf(n2 * inv, a.step_size) * inv));  // dir = u * min(|v|, step)
     }
     // ---------------- compact the moving pedestrians into the shared tile  // @region wcompact
-    int n_src;
-    int win_lo[2] = {0, 0}, win_hi[2] = {0, 0};  // slot window of this lane's pedestrians (strip culling)
-    bool culled = false;
-    if (S > 0) {
-      // deterministic counting sort by strip: atomicOr of lane bits (commutative, so the result does not depend on
-      // the order the atomics retire), rank = number of lower (pedestrian, lane) pairs of the same strip
-      int c[2];
+    const uint32_t m0 = __ballot_sync(0xffffffffu, efv[0]), m1 = __ballot_sync(0xffffffffu, efv[1]);
+    const int c0 = __popc(m0), slot[2] = {__popc(m0 & lt_mask), c0 + __popc(m1 & lt_mask)};
+    const int n_src = c0 + __popc(m1);
 #pragma unroll
-      for (int k = 0; k < 2; ++k) c[k] = min(max((int)((q[k].p.x + a.width_f) * a.cell_inv_x), 0), S - 1);  // (int)NaN == 0
-      strip_mask[lane] = make_uint2(0u, 0u);
-      __syncwarp();
-      if (efv[0]) atomicOr(&strip_mask[c[0]].x, 1u << lane);
-      if (efv[1]) atomicOr(&strip_mask[c[1]].y, 1u << lane);
-      __syncwarp();
-      {
-        const uint2 m = strip_mask[lane];
-        const int cnt = (lane < S) ? __popc(m.x) + __popc(m.y) : 0;
-        int inc = cnt;
+    for (int k = 0; k < 2; ++k)
+      if (efv[k]) tile.put(slot[k], q[k].p.x, q[k].p.y, u[k].x, u[k].y);
+    if (lane < 2) tile.put(n_src + lane, PARK, PARK, 0.f, 0.f);  // pad to an even count
+    // sparse pass: per-slot records and the row / column slot masks (atomicOr of slot bits: commutative, so the masks do
+    // not depend on the order the atomics retire).  A source without a direction (NaN) poisons every sum in the reference
+    // (0 * NaN in the all-pairs product), which only the all-pairs loop reproduces.  Each moving source is stored twice, in
+    // the pair-packed tile above and in its per-slot record below, because which pass runs is known only after the masks
+    // are built; a single layout serving both passes was not built or measured.
+    bool sparse = false;
+    uint2 cand[2] = {make_uint2(0u, 0u), make_uint2(0u, 0u)};
+    int T[2] = {0, 0};
+    if (cells) {
+      row_mask[lane] = col_mask[lane] = make_uint2(0u, 0u);
+      if (lane < 2) row_mask[WCELLS + lane] = col_mask[WCELLS + lane] = make_uint2(0u, 0u);
+      int cx[2], cy[2];
 #pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
-        strip_start[lane] = inc - cnt;
-        if (lane == 31) strip_start[32] = inc;
-        n_src = __shfl_sync(0xffffffffu, inc, 31);
+      for (int k = 0; k < 2; ++k) {  // entry 1 + cell index; (int)NaN == 0
+        cx[k] = 1 + min(max((int)((q[k].p.x + a.width_f) * a.cell_inv_x), 0), a.cells_x - 1);
+        cy[k] = 1 + min(max((int)((q[k].p.y + a.height_f) * a.cell_inv_y), 0), a.cells_y - 1);
+        if (efv[k]) rec[slot[k]] = make_float4(q[k].p.x, q[k].p.y, u[k].x, u[k].y);
       }
       __syncwarp();
 #pragma unroll
       for (int k = 0; k < 2; ++k) {
         if (efv[k]) {
-          const uint2 m = strip_mask[c[k]];
-          const int slot = strip_start[c[k]] + (k == 0 ? __popc(m.x & lt_mask) : __popc(m.x) + __popc(m.y & lt_mask));
-          tile.put(slot, q[k].p.x, q[k].p.y, u[k].x, u[k].y);
-        }
-        if (fv[k]) {
-          win_lo[k] = strip_start[max(c[k] - 1, 0)] >> 1;                      // in slot PAIRS: a neighbouring slot that
-          win_hi[k] = (strip_start[min(c[k] + 1, S - 1) + 1] + 1) >> 1;        // rides along fails the distance test
+          unsigned* r = slot[k] < 32 ? &row_mask[cy[k]].x : &row_mask[cy[k]].y;
+          unsigned* c = slot[k] < 32 ? &col_mask[cx[k]].x : &col_mask[cx[k]].y;
+          atomicOr(r, 1u << (slot[k] & 31));
+          atomicOr(c, 1u << (slot[k] & 31));
         }
       }
-      // cost model: two windowed loops (one pedestrian each) against one all-pairs loop shared by both pedestrians;
-      // a source without a direction (NaN) poisons every sum in the reference -> all-pairs path reproduces that
-      const int wmax0 = __reduce_max_sync(0xffffffffu, win_hi[0] - win_lo[0]), wmax1 = __reduce_max_sync(0xffffffffu, win_hi[1] - win_lo[1]);
+      __syncwarp();
+      int walk[2];
+#pragma unroll
+      for (int k = 0; k < 2; ++k) {
+        if (fv[k]) {
+          const uint2 rm = or3(row_mask, cy[k] - 1), cm = or3(col_mask, cx[k] - 1);
+          cand[k] = make_uint2(rm.x & cm.x, rm.y & cm.y);
+        }
+        walk[k] = __popc(cand[k].x) + __popc(cand[k].y);
+      }
+      T[0] = __reduce_max_sync(0xffffffffu, walk[0]);
+      T[1] = __reduce_max_sync(0xffffffffu, walk[1]);
       const bool nan_src = (efv[0] && (u[0].x != u[0].x || u[0].y != u[0].y)) || (efv[1] && (u[1].x != u[1].x || u[1].y != u[1].y));
-      culled = (wmax0 + wmax1) * 5 < ((n_src + 1) >> 1) * 8 && !__any_sync(0xffffffffu, nan_src);
-    } else {
-      const uint32_t m0 = __ballot_sync(0xffffffffu, efv[0]), m1 = __ballot_sync(0xffffffffu, efv[1]);
-      const int c0 = __popc(m0);
-      if (efv[0]) tile.put(__popc(m0 & lt_mask), q[0].p.x, q[0].p.y, u[0].x, u[0].y);
-      if (efv[1]) tile.put(c0 + __popc(m1 & lt_mask), q[1].p.x, q[1].p.y, u[1].x, u[1].y);
-      n_src = c0 + __popc(m1);
+      sparse = !__any_sync(0xffffffffu, nan_src) &&
+               (a.cell_force || SPARSE_COST_NUM * (T[0] + T[1]) <= SPARSE_COST_DEN * ((n_src + 1) >> 1));
     }
-    if (lane < 2) tile.put(n_src + lane, PARK, PARK, 0.f, 0.f);  // pad to an even count
     __syncwarp();
     // ---------------- action source + Area.agent_step [area.py:182-210]  // @region wagent
     float2 act;
@@ -196,9 +234,9 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     agent_step(a, act, ap, ad, r_agent, term_agent);
     // ---------------- pairwise alignment [area.py:105-119]  // @region wpairwise
     float sx[2], sy[2];
-    if (culled) {
+    if (sparse) {
 #pragma unroll
-      for (int k = 0; k < 2; ++k) windowed_pass(tile, win_lo[k], win_hi[k], q[k].p.x, q[k].p.y, a.thr2_ped, sx[k], sy[k]);
+      for (int k = 0; k < 2; ++k) sparse_pass(rec, cand[k], T[k], q[k].p.x, q[k].p.y, a.thr2_ped, sx[k], sy[k]);
     } else {
       const float xi[2] = {q[0].p.x, q[1].p.x}, yi[2] = {q[0].p.y, q[1].p.y};
       if (__any_sync(0xffffffffu, fv[0] | fv[1])) pairwise_pass<2, PAIR_UNROLL>(tile, n_src, xi, yi, a.thr2_ped, sx, sy);

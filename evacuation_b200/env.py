@@ -295,7 +295,9 @@ class EvacuationEnv:
 
     @property
     def num_cells(self) -> int:
-        """Cells of the neighbour-search grid (0 = all-pairs tiles)."""
+        """Cells of the neighbour-search grid the handle is pinned to (0 = all-pairs tiles).  N <= 64 under
+        neighbor_search="auto" also reports 0: every warp chooses per step between the all-pairs loop and the cell masks
+        of the sparse pass; "cells" pins it to the sparse pass (whenever exact), "brute" to the all-pairs loop."""
         return int(nat.load().evac_num_cells(self._handle()))
 
     @property
