@@ -87,11 +87,32 @@ __host__ __device__ __forceinline__ uint32_t fmix32(uint32_t h) {
   h ^= h >> 16; h *= 0x85EBCA6Bu; h ^= h >> 13; h *= 0xC2B2AE35u; h ^= h >> 16;
   return h;
 }
-// dropout stream: 16-bit word k of the (env, block, row) stream
-__device__ __forceinline__ uint32_t drop_word(uint32_t row_key, uint32_t k) {
+// Dropout stream (host-callable, so that the tests can pin their restatement of it to this code).  An element is dropped when
+// its 16-bit word is below round(p * 65536).
+// base key of one forward call: (seed, stream offset, global env index)
+__host__ __device__ __forceinline__ uint32_t drop_base_key(uint32_t seed_lo, uint32_t seed_hi, unsigned long long off, uint32_t env_g) {
+  return fmix32(seed_lo ^ fmix32(env_g * 0x9E3779B1u + (uint32_t)off) ^ (seed_hi * 0x85EBCA77u) ^ ((uint32_t)(off >> 32) * 0xC2B2AE3Du));
+}
+// key of the (block, row) stream
+__host__ __device__ __forceinline__ uint32_t drop_row_key(uint32_t base, int blk, int row) {
+  return fmix32(base ^ ((uint32_t)(blk * PW_MAX_S + row) * 0x27D4EB2Fu));
+}
+// 16-bit word k of the (env, block, row) stream: k = c for the attention output, k = 8 + c for the block output
+__host__ __device__ __forceinline__ uint32_t drop_word(uint32_t row_key, uint32_t k) {
   const uint32_t t = fmix32(row_key + (k >> 1) * 0x9E3779B9u);
   return (k & 1u) ? (t >> 16) : (t & 0xFFFFu);
 }
+// feed-forward group g (hidden features 4g .. 4g + 3): feature 4g + 2i + j reads 16-bit half j of word i, word 0 = drop_ff_word and
+// word 1 = drop_ff_mix of it (a cheap second mix: multiply + xor-shift)
+__host__ __device__ __forceinline__ uint32_t drop_ff_word(uint32_t row_key, uint32_t g) { return fmix32(row_key + (8u + g) * 0x9E3779B9u); }
+// the second mix of the words of a lane's two rows at once: one call keeps the kernel's instruction order and register allocation
+__host__ __device__ __forceinline__ uint2 drop_ff_mix(uint32_t ta, uint32_t tb) {
+  uint32_t a = ta * 0x9E3779B1u, b = tb * 0x9E3779B1u;
+  a ^= a >> 15; b ^= b >> 15;
+  return make_uint2(a, b);
+}
+// half j of word w dropped, compared in place against th16 = threshold << 16 (the lower half shifted up, the upper half as it is)
+__host__ __device__ __forceinline__ bool drop_ff_dropped(uint32_t w, int j, uint32_t th16) { return (j ? w : w << 16) < th16; }
 __device__ __forceinline__ float drop_mask(uint32_t row_key, uint32_t k, const PArgs& a) {
   return drop_word(row_key, k) < a.drop_thresh ? 0.f : a.drop_scale;
 }
@@ -265,14 +286,14 @@ __global__ void __launch_bounds__(PW_WARPS * 32, PW_MINB) evac_policy_embed_kern
   uint32_t drop_base = 0;
   if (TRAIN) {
     const unsigned long long off = a.offset + (a.offset_dev ? *a.offset_dev : 0ull);
-    drop_base = fmix32(a.seed_lo ^ fmix32(env_g * 0x9E3779B1u + (uint32_t)off) ^ (a.seed_hi * 0x85EBCA77u) ^ ((uint32_t)(off >> 32) * 0xC2B2AE3Du));
+    drop_base = drop_base_key(a.seed_lo, a.seed_hi, off, env_g);
   }
   for (int blk = 0; blk < a.NB; ++blk) {
     const float* __restrict__ W = wsm + blk * a.wstride;
     uint32_t key_a = 0, key_b = 0;
     if (TRAIN) {
-      key_a = fmix32(drop_base ^ ((uint32_t)(blk * PW_MAX_S + ra) * 0x27D4EB2Fu));
-      key_b = fmix32(drop_base ^ ((uint32_t)(blk * PW_MAX_S + rb) * 0x27D4EB2Fu));
+      key_a = drop_row_key(drop_base, blk, ra);
+      key_b = drop_row_key(drop_base, blk, rb);
     }
     // ---------------- set attention [rpo_transformer_agent_network.py:57-75]
     float ya[D], yb[D];
@@ -382,21 +403,20 @@ __global__ void __launch_bounds__(PW_WARPS * 32, PW_MINB) evac_policy_embed_kern
         h01b = __ffma2_rn(xsb[c], lo(w), h01b); h23b = __ffma2_rn(xsb[c], hi(w), h23b);
       }
       if (TRAIN) {
-        // four 16-bit words per row: the two halves of one fmix32 word and of a cheap second mix of it (multiply + xor-shift);
-        // a word below the threshold drops the element (the 1 / (1 - p) scale sits in the staged W2, see above).  The upper
-        // halves are compared in place against the threshold shifted up.
-        const uint32_t ta = fmix32(key_a + (8u + g) * 0x9E3779B9u), tb = fmix32(key_b + (8u + g) * 0x9E3779B9u);
-        uint32_t ta2 = ta * 0x9E3779B1u, tb2 = tb * 0x9E3779B1u;
-        ta2 ^= ta2 >> 15; tb2 ^= tb2 >> 15;
+        // four 16-bit words per row (drop_ff_word, drop_ff_mix); a dropped element is zeroed (the 1 / (1 - p) scale sits in the
+        // staged W2, see above)
+        const uint32_t ta = drop_ff_word(key_a, g), tb = drop_ff_word(key_b, g);
+        const uint2 t2 = drop_ff_mix(ta, tb);
+        const uint32_t ta2 = t2.x, tb2 = t2.y;
         const uint32_t th = a.drop_thresh << 16;
-        if ((ta << 16) < th) h01a.x = 0.f;
-        if (ta < th) h01a.y = 0.f;
-        if ((ta2 << 16) < th) h23a.x = 0.f;
-        if (ta2 < th) h23a.y = 0.f;
-        if ((tb << 16) < th) h01b.x = 0.f;
-        if (tb < th) h01b.y = 0.f;
-        if ((tb2 << 16) < th) h23b.x = 0.f;
-        if (tb2 < th) h23b.y = 0.f;
+        if (drop_ff_dropped(ta, 0, th)) h01a.x = 0.f;
+        if (drop_ff_dropped(ta, 1, th)) h01a.y = 0.f;
+        if (drop_ff_dropped(ta2, 0, th)) h23a.x = 0.f;
+        if (drop_ff_dropped(ta2, 1, th)) h23a.y = 0.f;
+        if (drop_ff_dropped(tb, 0, th)) h01b.x = 0.f;
+        if (drop_ff_dropped(tb, 1, th)) h01b.y = 0.f;
+        if (drop_ff_dropped(tb2, 0, th)) h23b.x = 0.f;
+        if (drop_ff_dropped(tb2, 1, th)) h23b.y = 0.f;
       }
       h01a.x = max_nan(h01a.x, 0.f); h01a.y = max_nan(h01a.y, 0.f); h23a.x = max_nan(h23a.x, 0.f); h23a.y = max_nan(h23a.y, 0.f);
       h01b.x = max_nan(h01b.x, 0.f); h01b.y = max_nan(h01b.y, 0.f); h23b.x = max_nan(h23b.x, 0.f); h23b.y = max_nan(h23b.y, 0.f);
@@ -469,6 +489,22 @@ struct HArgs {
   long long env_offset;
 };
 
+// Normal draws of the heads (host-callable, like the dropout stream): the Philox4x32-10 words of (seed, stream offset, global env)
+__host__ __device__ __forceinline__ evac::Philox4 normal_words(uint32_t seed_lo, uint32_t seed_hi, unsigned long long off, uint32_t env_g) {
+  return evac::philox4x32_10(env_g, (uint32_t)off, (uint32_t)(off >> 32), 0x504F4C49u, seed_lo, seed_hi);
+}
+// component c (< 3) of the standard Normal draw: Box-Muller on two 24-bit uniforms in (0, 1); words (0, 1) -> components 0 (cos)
+// and 1 (sin), words (2, 3) -> component 2 (cos)
+__host__ __device__ __forceinline__ float normal_draw(const uint32_t (&words)[4], int c) {
+  const int p = (c >> 1) * 2;
+  const float u1 = ((float)(words[p] >> 8) + 0.5f) * 5.9604644775390625e-08f;
+  const float u2 = ((float)(words[p + 1] >> 8) + 0.5f) * 5.9604644775390625e-08f;
+  const float rad = sqrtf(-2.f * logf(u1));
+  float sn, cs;
+  sincosf(6.28318530717958647692f * u2, &sn, &cs);
+  return rad * ((c & 1) ? sn : cs);
+}
+
 // value + Normal(mean, exp(logstd)): sample / log-probability / entropy of environment e [rpo_linear_agent_network.py:47-61];
 // o = {value, mean[0], mean[1], mean[2]}.  `critic` / `actor` select which half is written (the tensor-core kernel splits the
 // two heads over two CTAs for small batches).
@@ -478,23 +514,14 @@ __device__ __forceinline__ void heads_finish(const HArgs& a, int e, const float*
   const uint32_t env_g = (uint32_t)(a.env_offset + e);
   float lp = 0.f, ent = 0.f;
   const unsigned long long off = a.offset + (a.offset_dev ? *a.offset_dev : 0ull);
-  const evac::Philox4 r = evac::philox4x32_10(env_g, (uint32_t)off, (uint32_t)(off >> 32), 0x504F4C49u, a.seed_lo, a.seed_hi);
+  const evac::Philox4 r = normal_words(a.seed_lo, a.seed_hi, off, env_g);
   const uint32_t words[4] = {r.x, r.y, r.z, r.w};
   for (int c = 0; c < a.A; ++c) {
     const float mu = o[1 + c];
     const float ls = a.logstd[c], sd = expf(ls);
     float act = mu;
     if (a.given_action != nullptr) act = a.given_action[(size_t)e * a.A + c];
-    else if (a.sample) {
-      // Box-Muller on two 24-bit uniforms in (0, 1): pair (0, 1) -> components 0 and 1, pair (2, 3) -> component 2
-      const int p = (c >> 1) * 2;
-      const float u1 = ((float)(words[p] >> 8) + 0.5f) * 5.9604644775390625e-08f;
-      const float u2 = ((float)(words[p + 1] >> 8) + 0.5f) * 5.9604644775390625e-08f;
-      const float rad = sqrtf(-2.f * logf(u1));
-      float sn, cs;
-      sincosf(6.28318530717958647692f * u2, &sn, &cs);
-      act = fmaf(sd, rad * ((c & 1) ? sn : cs), mu);
-    }
+    else if (a.sample) act = fmaf(sd, normal_draw(words, c), mu);
     const float z = (act - mu) / sd;
     lp += -0.5f * z * z - ls - 0.918938533204672741780f;
     ent += 0.5f + 0.918938533204672741780f + ls;

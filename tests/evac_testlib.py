@@ -118,6 +118,101 @@ def philox_action(seed, env, episode, now):
     return np.array([np.float32(2) * u01(r[0]) - np.float32(1), np.float32(2) * u01(r[1]) - np.float32(1)], dtype=np.float32).reshape(2)
 
 
+# ---------------------------------------------------------------------------------------------
+# NumPy restatement of the fused policy's two streams (csrc/evac_policy.cuh): the dropout masks of the embedding kernel in
+# training mode and the Normal draws of the heads.  Seeds and stream offsets are 64-bit, env_g is the global env index
+# (env_index_offset + e, taken mod 2^32).
+_U32 = np.uint64(0xFFFFFFFF)
+PW_MAX_S = 64
+
+
+def _u32(x):
+    return np.asarray(x, dtype=np.uint64) & _U32
+
+
+def fmix32(h):
+    h = _u32(h)
+    h = h ^ (h >> np.uint64(16))
+    h = (h * np.uint64(0x85EBCA6B)) & _U32
+    h = h ^ (h >> np.uint64(13))
+    h = (h * np.uint64(0xC2B2AE35)) & _U32
+    return h ^ (h >> np.uint64(16))
+
+
+def drop_base_key(seed, offset, env_g):
+    seed_lo, seed_hi, off_lo, off_hi = (np.uint64(v) for v in (seed & 0xFFFFFFFF, seed >> 32, offset & 0xFFFFFFFF, offset >> 32))
+    inner = fmix32((_u32(env_g) * np.uint64(0x9E3779B1) + off_lo) & _U32)
+    return fmix32(seed_lo ^ inner ^ ((seed_hi * np.uint64(0x85EBCA77)) & _U32) ^ ((off_hi * np.uint64(0xC2B2AE3D)) & _U32))
+
+
+def drop_row_key(base, blk, row):
+    return fmix32(_u32(base) ^ ((_u32(np.asarray(blk) * PW_MAX_S + np.asarray(row)) * np.uint64(0x27D4EB2F)) & _U32))
+
+
+def drop_word(row_key, k):
+    """16-bit word k of a row's stream: k = c is the attention output's feature c, k = 8 + c the block output's."""
+    k = _u32(k)
+    t = fmix32(_u32(row_key) + (k >> np.uint64(1)) * np.uint64(0x9E3779B9))
+    return np.where((k & np.uint64(1)) == 1, t >> np.uint64(16), t & np.uint64(0xFFFF))
+
+
+def drop_ff_word(row_key, g):
+    return fmix32(_u32(row_key) + (np.uint64(8) + _u32(g)) * np.uint64(0x9E3779B9))
+
+
+def drop_ff_mix(t):
+    t = (_u32(t) * np.uint64(0x9E3779B1)) & _U32
+    return t ^ (t >> np.uint64(15))
+
+
+def drop_hidden_words(row_key, F):
+    """16-bit words of hidden features 0 .. F - 1: feature 4g + 2i + j is half j of word i of group g, word 0 = drop_ff_word,
+    word 1 = drop_ff_mix of it."""
+    f = np.arange(F, dtype=np.uint64)
+    w = drop_ff_word(np.asarray(row_key)[..., None], f >> np.uint64(2))
+    w = np.where(((f >> np.uint64(1)) & np.uint64(1)) == 1, drop_ff_mix(w), w)
+    return np.where((f & np.uint64(1)) == 1, w >> np.uint64(16), w & np.uint64(0xFFFF))
+
+
+def drop_site_words(seed, offset, env_g, blk, row, D, F):
+    """The 16-bit words of the three dropout sites of block `blk`, row `row` (broadcastable): attention output [.., D],
+    feed-forward hidden layer [.., F], block output [.., D]."""
+    key = drop_row_key(drop_base_key(seed, offset, env_g), blk, row)[..., None]
+    c = np.arange(D)
+    return drop_word(key, c), drop_hidden_words(key[..., 0], F), drop_word(key, 8 + c)
+
+
+def drop_threshold(p):
+    """lrint(p * 65536) of the float32 dropout probability: a word below it drops its element."""
+    return int(np.rint(np.float64(np.float32(p)) * 65536.0))
+
+
+def dropout_masks(seed, offset, env_index_offset, E, num_blocks, S, D, F, p):
+    """Per block, the float32 masks (attention [E, S, D], hidden [E, S, F], output [E, S, D]) of one forward call with stream
+    offset `offset`: 0 where dropped, float32(1 / (1 - p)) where kept."""
+    thr = np.uint64(drop_threshold(p))
+    keep = np.float32(1) / (np.float32(1) - np.float32(p))
+    env_g = (env_index_offset + np.arange(E, dtype=np.int64)) & 0xFFFFFFFF
+    rows = np.arange(S)
+    out = []
+    for b in range(num_blocks):
+        words = drop_site_words(seed, offset, env_g[:, None], b, rows[None, :], D, F)
+        out.append(tuple(np.where(w < thr, np.float32(0), keep).astype(np.float32) for w in words))
+    return out
+
+
+def policy_normal(seed, offset, env_g, A):
+    """[.., A] standard Normal draws of the heads: Philox4x32-10 counter (env_g, offset lo, offset hi, 'POLI'), key = seed;
+    24-bit uniforms u = ((w >> 8) + 0.5) * 2^-24 and the angle 2 pi u formed in float32 as the kernel forms them, Box-Muller
+    in float64: words (0, 1) give components 0 (cos) and 1 (sin), words (2, 3) component 2 (cos).  Returns (z, radius)."""
+    r = philox4x32_10(_u32(env_g), offset & 0xFFFFFFFF, offset >> 32, 0x504F4C49, seed & 0xFFFFFFFF, seed >> 32)
+    u = [((w >> np.uint32(8)).astype(np.float32) + np.float32(0.5)) * np.float32(2.0 ** -24) for w in r]
+    rad = [np.sqrt(-2.0 * np.log(u[p].astype(np.float64))) for p in (0, 2)]
+    ang = [(np.float32(2 * np.pi) * u[p]).astype(np.float64) for p in (1, 3)]
+    z = np.stack([rad[0] * np.cos(ang[0]), rad[0] * np.sin(ang[0]), rad[1] * np.cos(ang[1])], axis=-1)
+    return z[..., :A], np.stack([rad[0], rad[0], rad[1]], axis=-1)[..., :A]
+
+
 def philox_layout(seed, env, episode, n, dtype=np.float32):
     """(positions [n,2], directions [n,2]) of a kernel-side reset (csrc/evac_kernels.cuh::random_layout)."""
     r = evac_random(seed, STREAM_RESET, env, episode, 0, np.arange(n))

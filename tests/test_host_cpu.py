@@ -196,6 +196,105 @@ def test_noise_streams_do_not_alias_for_large_crowds(tmp_path):
         assert np.float32(v) == want[int(now)][int(i)], (now, i)
 
 
+_POLICY_STREAM_PROGRAM = r"""
+#include <cstdio>
+#include "evac_policy.cuh"
+using namespace evacp;
+// record per (seed, offset, env, block, row): the words of every dropout site for d_model 2, 3, 6 ([attention | output] each)
+// and F = 96 (hidden), then each word's dropped flag as the kernel decides it, at thresholds 6554 (p = 0.1) and 32768 (p = 0.5)
+int main(int argc, char** argv) {
+  FILE* f = fopen(argv[1], "wb");
+  FILE* g = fopen(argv[2], "w");
+  const unsigned long long seeds[2] = {0x2468ACE1ull, 0x13579BDF2468ACE1ull}, offs[3] = {0ull, 1ull, (1ull << 32) + 3ull};
+  const uint32_t envs[4] = {0u, 5u, 65535u, (1u << 31) + 7u}, thr[2] = {6554u, 32768u};
+  const int Ds[3] = {2, 3, 6};
+  for (int s = 0; s < 2; ++s) for (int o = 0; o < 3; ++o) for (int e = 0; e < 4; ++e) {
+    const uint32_t base = drop_base_key((uint32_t)seeds[s], (uint32_t)(seeds[s] >> 32), offs[o], envs[e]);
+    for (int blk = 0; blk < 8; ++blk) for (int row = 0; row < 64; row += 2) {
+      const uint32_t ka = drop_row_key(base, blk, row), kb = drop_row_key(base, blk, row + 1);  // a lane's two rows
+      for (int r = 0; r < 2; ++r) {
+        const uint32_t key = r ? kb : ka;
+        uint16_t w[118];
+        uint8_t m[2][118];
+        int n = 0;
+        for (int di = 0; di < 3; ++di)
+          for (int site = 0; site < 2; ++site)
+            for (int c = 0; c < Ds[di]; ++c, ++n) {
+              w[n] = (uint16_t)drop_word(key, (uint32_t)(8 * site + c));
+              for (int t = 0; t < 2; ++t) m[t][n] = w[n] < thr[t];
+            }
+        for (int fe = 0; fe < 96; ++fe, ++n) {
+          const uint32_t t0a = drop_ff_word(ka, (uint32_t)(fe >> 2)), t0b = drop_ff_word(kb, (uint32_t)(fe >> 2));
+          const uint2 t1 = drop_ff_mix(t0a, t0b);
+          const uint32_t word = (fe & 2) ? (r ? t1.y : t1.x) : (r ? t0b : t0a);
+          w[n] = (uint16_t)((fe & 1) ? word >> 16 : word & 0xFFFFu);
+          for (int t = 0; t < 2; ++t) m[t][n] = drop_ff_dropped(word, fe & 1, thr[t] << 16);
+        }
+        fwrite(w, 2, 118, f);
+        fwrite(m, 1, 236, f);
+      }
+    }
+    // Normal draws of the heads (host libm: equal to float32 rounding, not bit for bit)
+    const evac::Philox4 q = normal_words((uint32_t)seeds[s], (uint32_t)(seeds[s] >> 32), offs[o], envs[e]);
+    const uint32_t words[4] = {q.x, q.y, q.z, q.w};
+    fprintf(g, "%.9g %.9g %.9g\n", (double)normal_draw(words, 0), (double)normal_draw(words, 1), (double)normal_draw(words, 2));
+  }
+  fclose(f);
+  fclose(g);
+  return 0;
+}
+"""
+
+
+def test_policy_streams_match_their_numpy_restatement(tmp_path):
+    """The fused policy's dropout masks and Normal draws (csrc/evac_policy.cuh, compiled for the host) against the NumPy
+    restatement in evac_testlib that the GPU tests of training mode build their float64 references from: every word of the
+    attention, hidden (F = 96) and block-output sites for d_model 2 / 3 / 6, blocks 0..7, rows 0..63, seeds below and above 2^32,
+    stream offsets 0, 1, 2^32 + 3 (the upper half enters the key) and global env indices 0, 5, 65535, 2^31 + 7, bit for bit,
+    with the dropped flags at p = 0.1 and 0.5; and the three Box-Muller components of each (seed, offset, env)."""
+    import shutil
+
+    from evacuation_b200 import build as b
+
+    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
+    if not os.path.exists(nvcc):
+        pytest.skip("nvcc not available")
+    src, exe = tmp_path / "streams.cu", tmp_path / "streams"
+    src.write_text(_POLICY_STREAM_PROGRAM)
+    res = subprocess.run([nvcc, "-std=c++17", "-O1", "-gencode", "arch=compute_100a,code=sm_100a", "-I", b.CSRC, str(src), "-o", str(exe)],
+                         capture_output=True, text=True)
+    assert res.returncode == 0, res.stderr
+    words_path, normal_path = tmp_path / "words.bin", tmp_path / "normal.txt"
+    subprocess.run([str(exe), str(words_path), str(normal_path)], check=True)
+    raw = np.fromfile(words_path, dtype=np.uint8).reshape(2, 3, 4, 8, 64, 118 * 2 + 236)
+    got_words = raw[..., :236].copy().view(np.uint16)
+    got_flags = raw[..., 236:].reshape(raw.shape[:-1] + (2, 118))
+    got_z = np.loadtxt(normal_path).reshape(2, 3, 4, 3)
+
+    seeds, offs, envs = (0x2468ACE1, 0x13579BDF2468ACE1), (0, 1, 2 ** 32 + 3), (0, 5, 65535, 2 ** 31 + 7)
+    blk, row = np.arange(8)[:, None], np.arange(64)[None, :]
+    checked = 0
+    for s, seed in enumerate(seeds):
+        for o, off in enumerate(offs):
+            for e, env in enumerate(envs):
+                parts = []
+                for D in (2, 3, 6):
+                    attn, _, out = T.drop_site_words(seed, off, env, blk, row, D, 96)
+                    parts += [attn, out]
+                parts.append(T.drop_site_words(seed, off, env, blk, row, 6, 96)[1])
+                want = np.concatenate(parts, axis=-1).astype(np.uint16)
+                assert np.array_equal(got_words[s, o, e], want), (seed, off, env)
+                for t, p in enumerate((0.1, 0.5)):
+                    assert np.array_equal(got_flags[s, o, e, :, :, t], want < T.drop_threshold(p)), (seed, off, env, p)
+                z, rad = T.policy_normal(seed, off, np.array([env]), 3)
+                np.testing.assert_allclose(got_z[s, o, e], z[0], rtol=0, atol=2e-6 * (1 + rad[0].max()), err_msg=str((seed, off, env)))
+                checked += 1
+    assert checked == 24 and T.drop_threshold(0.1) == 6554 and T.drop_threshold(0.5) == 32768
+    # the streams do move with every input: seeds, offsets (both halves), env index, block and row
+    assert len({got_words[s, o, e, 0, 0].tobytes() for s in range(2) for o in range(3) for e in range(4)}) == 24
+    assert len({got_words[0, 0, 0, b_, r].tobytes() for b_ in range(8) for r in range(64)}) == 512
+
+
 def test_shard_partition():
     from evacuation_b200.distributed import shard_counts, shard_offset
 

@@ -186,29 +186,16 @@ def test_policy_restatement_matches_reference_network_variants():
 def test_hidden_dropout_words_are_unbiased_and_uncorrelated():
     """The fused policy's hidden-layer dropout (csrc/evac_policy.cuh, feed-forward loop) takes four 16-bit words per row and
     group of four features from ONE fmix32 word and a cheap second mix of it (multiply + xor-shift); an element is dropped
-    when its word is below round(p * 65536).  NumPy restatement of that word schedule: every word drops at rate p, the
-    indicators of different words are uncorrelated, and the number of dropped features per row is binomial
+    when its word is below round(p * 65536).  The word schedule is evac_testlib's restatement, which
+    tests/test_host_cpu.py::test_policy_streams_match_their_numpy_restatement pins to the kernel's code: every word drops at
+    rate p, the indicators of different words are uncorrelated, and the number of dropped features per row is binomial
     [torch.nn.Dropout(0.1) of rpo_transformer_agent_network.py:98]."""
-    def fmix32(h):
-        h = h.astype(np.uint64)
-        h ^= h >> 16
-        h = (h * 0x85EBCA6B) & 0xFFFFFFFF
-        h ^= h >> 13
-        h = (h * 0xC2B2AE35) & 0xFFFFFFFF
-        h ^= h >> 16
-        return h
+    import evac_testlib as T
 
     rng = np.random.default_rng(0)
     keys = rng.integers(0, 2 ** 32, size=200000, dtype=np.uint64)
     p = 0.1
-    thr = round(p * 65536)
-    words = []
-    for g in range(24):  # dim_feedforward 96 = 24 groups
-        t = fmix32((keys + (8 + g) * 0x9E3779B9) & 0xFFFFFFFF)
-        t2 = (t * 0x9E3779B1) & 0xFFFFFFFF
-        t2 ^= t2 >> 15
-        words += [t & 0xFFFF, t >> 16, t2 & 0xFFFF, t2 >> 16]
-    drop = np.stack(words, 1) < thr
+    drop = T.drop_hidden_words(keys, 96) < T.drop_threshold(p)  # dim_feedforward 96 = 24 groups
     rates = drop.mean(0)
     assert abs(drop.mean() - p) < 5e-4 and np.abs(rates - p).max() < 4e-3
     c = np.corrcoef(drop[:, :16].T.astype(np.float64))
