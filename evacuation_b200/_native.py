@@ -46,6 +46,15 @@ class EvacConfig(C.Structure):
     ]
 
 
+class EvacEnvParams(C.Structure):
+    _fields_ = [
+        ("noise_coef", C.c_double), ("enslaving_degree", C.c_double), ("alpha", C.c_double),
+        ("intrinsic_reward_coef", C.c_double), ("init_reward_each_step", C.c_double),
+        ("is_new_exiting_reward", C.c_int32), ("is_new_followers_reward", C.c_int32),
+        ("is_termination_agent_wall_collision", C.c_int32), ("max_timesteps", C.c_int32),
+    ]
+
+
 class EvacPolicyConfig(C.Structure):
     _fields_ = [
         ("abi_version", C.c_int32), ("seq_len", C.c_int32), ("d_model", C.c_int32), ("num_heads", C.c_int32),
@@ -92,6 +101,8 @@ SIGNATURES = {
     "evac_state_bytes": (C.c_int64, [_P]),
     "evac_save_state": (C.c_int, [_P, _P, _P]),
     "evac_load_state": (C.c_int, [_P, _P, _P]),
+    "evac_set_env_params": (C.c_int, [_P, _P, _P]),
+    "evac_get_env_params": (C.c_int, [_P, _P]),
     "evac_policy_default_config": (C.c_int, [C.POINTER(EvacPolicyConfig), C.c_int32, C.c_int32]),
     "evac_policy_default_linear_config": (C.c_int, [C.POINTER(EvacPolicyConfig), C.c_int32]),
     "evac_policy_create": (C.c_int, [C.POINTER(EvacPolicyConfig), C.c_int32, C.POINTER(_P)]),

@@ -73,6 +73,11 @@ struct EvacHandle {
   int cells_x = 0, cells_y = 0, cell_reach = 1;  // > 0: cell-list neighbour search (fp32; N <= 64: the sparse pass's cell masks)
   int cell_pair_walk = 1;        // paired walk of the sorted slots (0: one slot per thread)
   int cluster = 1;               // > 1: one environment per thread-block cluster of this many 1024 x 4 CTAs (N > 4096, evac_cluster.cuh)
+  // per-environment parameters (evac_set_env_params): the caller's records and their device conversion ([E] EnvParamRec<real>,
+  // allocated by the first call and kept); per_env selects the PE kernel instances
+  EvacEnvParams* env_params = nullptr;
+  void* d_params = nullptr;
+  bool per_env = false;
 };
 
 // smallest double b such that sqrt(v) >= t for every v >= b  <=>  (v < b) == (sqrt(v) < t)
@@ -107,6 +112,29 @@ static void warp_cell_grid(const EvacConfig& c, int* gx, int* gy) {
   *gy = (int)fmax(1.0, fmin((double)WCELLS, floor(2.0 * c.height / edge)));
 }
 
+// GravityEncoding: alpha + 2 when it is a small integer (ipow by squaring in the kernels), else 0 (pow)
+static int alpha_plus2_int_of(double alpha) {
+  const double ap2 = alpha + 2.0;
+  return (ap2 == floor(ap2) && ap2 >= 1.0 && ap2 <= 64.0) ? (int)ap2 : 0;
+}
+
+// one EvacEnvParams record as the kernels read it: the same conversions make_args applies to the EvacConfig fields
+template <typename real>
+static EnvParamRec<real> env_param_rec(const EvacEnvParams& p) {
+  EnvParamRec<real> r;
+  memset(&r, 0, sizeof(r));
+  r.one_minus_enslaving = (real)(1.0 - p.enslaving_degree);
+  r.alpha = (real)p.alpha;
+  r.init_reward = (real)p.init_reward_each_step;
+  r.intrinsic_coef = (real)p.intrinsic_reward_coef;
+  r.noise_coef = (float)(real)p.noise_coef;
+  r.enslaving_f = (float)p.enslaving_degree;
+  r.max_timesteps = p.max_timesteps;
+  r.bits = alpha_plus2_int_of(p.alpha) | (p.is_new_exiting_reward != 0) << 8 | (p.is_new_followers_reward != 0) << 9 |
+           (p.is_termination_agent_wall_collision != 0) << 10;
+  return r;
+}
+
 template <typename real>
 static KArgs<real> make_args(const EvacHandle* h) {
   const EvacConfig& c = h->cfg;
@@ -130,8 +158,7 @@ static KArgs<real> make_args(const EvacHandle* h) {
   a.inv_200n = (real)(1.0 / (200.0 * h->N)); a.inv_n = (real)(1.0 / h->N);
   a.positions = c.positions; a.statuses = c.statuses; a.obs_type = c.obs_type;
   a.alpha = (real)c.alpha; a.eps = (real)c.eps;
-  const double ap2 = c.alpha + 2.0;
-  a.alpha_plus2_int = (ap2 == floor(ap2) && ap2 >= 1.0 && ap2 <= 64.0) ? (int)ap2 : 0;
+  a.alpha_plus2_int = alpha_plus2_int_of(c.alpha);
   a.auto_reset = c.auto_reset;
   a.pos = reinterpret_cast<typename vec2<real>::type*>(h->pos);
   a.dir = reinterpret_cast<typename vec2<real>::type*>(h->dir);
@@ -150,34 +177,44 @@ static KArgs<real> make_args(const EvacHandle* h) {
   return a;
 }
 
+// the kernels' last argument: the handle's per-env records (read by the PE instances only)
+template <typename real>
+static const EnvParamRec<real>* params_of(const EvacHandle* h) {
+  return h->per_env ? static_cast<const EnvParamRec<real>*>(h->d_params) : nullptr;
+}
+
 // ------------------------------------------------------------------------------------------
-template <typename real, int THREADS, int PPT>
-static int launch_step_t(EvacHandle* h, const KArgs<real>& a, cudaStream_t st) {
+template <typename real, int THREADS, int PPT, bool PE>
+static int launch_step_pe(EvacHandle* h, const KArgs<real>& a, cudaStream_t st) {
   size_t smem = Tile<real>::bytes(THREADS * PPT);                                           // source tile
   if (a.cells_x > 0) smem += CellSmem::bytes(THREADS * PPT, a.cells_x * a.cells_y);         // + cell list
   static thread_local size_t attr_set[16] = {0};
-  auto kern = evac_step_kernel<real, THREADS, PPT>;
+  auto kern = evac_step_kernel<real, THREADS, PPT, 1, PE>;
   if (smem > 48 * 1024 && attr_set[h->device & 15] < smem) {
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // the whole unified L1 / shared-memory array as shared memory
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     attr_set[h->device & 15] = smem;
   }
-  kern<<<a.E, THREADS, smem, st>>>(a);
+  kern<<<a.E, THREADS, smem, st>>>(a, params_of<real>(h));
   CK(cudaGetLastError());
   h->launches++;
   return EVAC_OK;
 }
+template <typename real, int THREADS, int PPT>
+static int launch_step_t(EvacHandle* h, const KArgs<real>& a, cudaStream_t st) {
+  return h->per_env ? launch_step_pe<real, THREADS, PPT, true>(h, a, st) : launch_step_pe<real, THREADS, PPT, false>(h, a, st);
+}
 
 // One environment per cluster of CL CTAs (crowds above one SM's shared memory): grid = E x CL, cluster dimension as a
 // launch attribute.
-template <int CL>
-static int launch_cluster_t(EvacHandle* h, const KArgs<float>& a, cudaStream_t st) {
+template <int CL, bool PE>
+static int launch_cluster_pe(EvacHandle* h, const KArgs<float>& a, cudaStream_t st) {
   constexpr int THREADS = 1024, PPT = 4;
   const int C = a.cells_x * a.cells_y;
   const size_t smem = Tile<float>::bytes(THREADS * PPT) + CellSmem::bytes(THREADS * PPT, C) + ClusterSmem::bytes(C);
   static thread_local size_t attr_set[16] = {0};
-  auto kern = evac_step_kernel<float, THREADS, PPT, CL>;
+  auto kern = evac_step_kernel<float, THREADS, PPT, CL, PE>;
   if (attr_set[h->device & 15] < smem) {
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_set[h->device & 15] = smem;
@@ -192,9 +229,13 @@ static int launch_cluster_t(EvacHandle* h, const KArgs<float>& a, cudaStream_t s
   at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  CK(cudaLaunchKernelEx(&cfg, kern, a));
+  CK(cudaLaunchKernelEx(&cfg, kern, a, params_of<float>(h)));
   h->launches++;
   return EVAC_OK;
+}
+template <int CL>
+static int launch_cluster_t(EvacHandle* h, const KArgs<float>& a, cudaStream_t st) {
+  return h->per_env ? launch_cluster_pe<CL, true>(h, a, st) : launch_cluster_pe<CL, false>(h, a, st);
 }
 
 static void pick_shape(int n, int* threads, int* ppt) {
@@ -210,10 +251,15 @@ static void pick_shape(int n, int* threads, int* ppt) {
 
 // N <= 64, float32: the dedicated one-warp kernel (evac_warp.cuh), observation encoding resolved at compile time.  One
 // environment per CTA: measured on B200 at 4096 envs with 1 / 2 / 4 / 8 environments per CTA, 14.0 / 14.4 / 14.4 / 14.9 us.
+template <bool PE>
+static void launch_warp_pe(const KArgs<float>& a, const EnvParamRec<float>* params, cudaStream_t st) {
+  if (a.positions == POS_REL && a.statuses == STAT_OHE && a.obs_type == OBS_BOX) evac_warp_kernel<WMODE_REL_OHE_BOX, PE><<<a.E, 32, 0, st>>>(a, params);
+  else if (a.positions == POS_GRAV) evac_warp_kernel<WMODE_GRAV, PE><<<a.E, 32, 0, st>>>(a, params);
+  else evac_warp_kernel<WMODE_GENERIC, PE><<<a.E, 32, 0, st>>>(a, params);
+}
 static int launch_warp(EvacHandle* h, const KArgs<float>& a, cudaStream_t st) {
-  if (a.positions == POS_REL && a.statuses == STAT_OHE && a.obs_type == OBS_BOX) evac_warp_kernel<WMODE_REL_OHE_BOX><<<a.E, 32, 0, st>>>(a);
-  else if (a.positions == POS_GRAV) evac_warp_kernel<WMODE_GRAV><<<a.E, 32, 0, st>>>(a);
-  else evac_warp_kernel<WMODE_GENERIC><<<a.E, 32, 0, st>>>(a);
+  if (h->per_env) launch_warp_pe<true>(a, params_of<float>(h), st);
+  else launch_warp_pe<false>(a, nullptr, st);
   CK(cudaGetLastError());
   h->launches++;
   return EVAC_OK;
@@ -252,7 +298,9 @@ static int with_args(const EvacHandle* h, F&& f) { return h->prec == EVAC_PREC_F
 
 static int launch_aux(EvacHandle* h, int flags, const uint8_t* mask, float* obs, cudaStream_t st) {
   return with_args(h, [&](const auto& a) -> int {
-    evac_aux_kernel<<<h->E, 128, 0, st>>>(a, flags, mask, obs);
+    using real = decltype(a.width);  // the handle's precision
+    if (h->per_env) evac_aux_kernel<real, true><<<h->E, 128, 0, st>>>(a, flags, mask, obs, params_of<real>(h));
+    else evac_aux_kernel<real, false><<<h->E, 128, 0, st>>>(a, flags, mask, obs, nullptr);
     CK(cudaGetLastError());
     h->launches++;
     return EVAC_OK;
@@ -413,11 +461,13 @@ int evac_destroy(EvacHandle* h) {
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
   void* dptrs[] = {h->pos, h->dir, h->status, h->agent_pos, h->agent_dir, h->now, h->episode, h->overall, h->acc,
-                   h->ep_stats, h->ep_finished, h->totals, h->agent_state, h->blocks, h->d_actions, h->d_noise, h->d_obs /* one block: obs | reward | flags */};
+                   h->ep_stats, h->ep_finished, h->totals, h->agent_state, h->blocks, h->d_actions, h->d_noise, h->d_obs /* one block: obs | reward | flags */,
+                   h->d_params};
   for (void* p : dptrs) if (p) cudaFree(p);
   void* hptrs[] = {h->h_actions, h->h_noise, h->h_obs /* one block */};
   for (void* p : hptrs) if (p) cudaFreeHost(p);
   if (h->stream) cudaStreamDestroy(h->stream);
+  free(h->env_params);
   delete h;
   return EVAC_OK;
 }
@@ -675,6 +725,49 @@ int evac_load_state(EvacHandle* h, const void* image, void* stream) {
   if (!h || !image) return fail(EVAC_ERR_INVALID, "NULL argument");
   if (int r = set_device(h)) return r;
   return state_copy(h, (unsigned char*)image, false, (cudaStream_t)stream);
+}
+
+int evac_set_env_params(EvacHandle* h, const EvacEnvParams* params, void* stream) {
+  if (!h) return fail(EVAC_ERR_INVALID, "NULL handle");
+  if (!params) { h->per_env = false; return EVAC_OK; }
+  for (int e = 0; e < h->E; ++e)
+    if (params[e].max_timesteps < 1 || params[e].max_timesteps > (1 << 21))
+      return fail(EVAC_ERR_INVALID, "env %d: max_timesteps must be in 1 .. 2^21 (the step index is a 21-bit field of the Philox counter)", e);
+  if (int r = set_device(h)) return r;
+  const bool f64 = h->prec == EVAC_PREC_F64;
+  const size_t rec = f64 ? sizeof(EnvParamRec<double>) : sizeof(EnvParamRec<float>), bytes = (size_t)h->E * rec;
+  if (!h->env_params) {
+    h->env_params = (EvacEnvParams*)malloc((size_t)h->E * sizeof(EvacEnvParams));
+    if (!h->env_params) return fail(EVAC_ERR_INVALID, "out of host memory");
+    CK(cudaMalloc(&h->d_params, bytes));
+  }
+  unsigned char* conv = (unsigned char*)malloc(bytes);
+  if (!conv) return fail(EVAC_ERR_INVALID, "out of host memory");
+  for (int e = 0; e < h->E; ++e) {
+    if (f64) { const EnvParamRec<double> r = env_param_rec<double>(params[e]); memcpy(conv + e * rec, &r, rec); }
+    else { const EnvParamRec<float> r = env_param_rec<float>(params[e]); memcpy(conv + e * rec, &r, rec); }
+  }
+  // pageable source: the copy is staged before cudaMemcpyAsync returns, so `conv` may be freed right after it
+  const cudaError_t err = cudaMemcpyAsync(h->d_params, conv, bytes, cudaMemcpyHostToDevice, (cudaStream_t)stream);
+  free(conv);
+  if (err != cudaSuccess) return fail(EVAC_ERR_CUDA, "cudaMemcpyAsync(env params) failed: %s", cudaGetErrorString(err));
+  memcpy(h->env_params, params, (size_t)h->E * sizeof(EvacEnvParams));
+  h->per_env = true;
+  return EVAC_OK;
+}
+
+int evac_get_env_params(const EvacHandle* h, EvacEnvParams* out) {
+  if (!h || !out) return fail(EVAC_ERR_INVALID, "NULL argument");
+  if (h->per_env) { memcpy(out, h->env_params, (size_t)h->E * sizeof(EvacEnvParams)); return EVAC_OK; }
+  const EvacConfig& c = h->cfg;
+  for (int e = 0; e < h->E; ++e) {
+    EvacEnvParams& p = out[e];
+    p.noise_coef = c.noise_coef; p.enslaving_degree = c.enslaving_degree; p.alpha = c.alpha;
+    p.intrinsic_reward_coef = c.intrinsic_reward_coef; p.init_reward_each_step = c.init_reward_each_step;
+    p.is_new_exiting_reward = c.is_new_exiting_reward; p.is_new_followers_reward = c.is_new_followers_reward;
+    p.is_termination_agent_wall_collision = c.is_termination_agent_wall_collision; p.max_timesteps = c.max_timesteps;
+  }
+  return EVAC_OK;
 }
 
 int evac_episode_stats(EvacHandle* h, float* stats, uint8_t* finished, double* totals, void* stream) {

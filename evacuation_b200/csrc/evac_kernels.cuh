@@ -107,6 +107,51 @@ struct KArgs {
 };
 
 // ------------------------------------------------------------------------------------------
+// Per-environment parameters.  The host converts every EvacEnvParams record exactly as make_args converts the EvacConfig
+// fields of the same name, so an environment of a per-env launch computes what a uniform handle built with its record's values
+// computes, bit for bit.  One packed, 16-byte aligned record per environment: 32 bytes (float32: two LDG.128), 48 bytes
+// (float64: three), loaded once per environment and launch.  The [E] records reach the kernels as their LAST argument, after
+// KArgs and the aux kernel's own arguments, so that no argument of the uniform instances moves.
+template <typename real>
+struct __align__(16) EnvParamRec {
+  real one_minus_enslaving, alpha, init_reward, intrinsic_coef;
+  float noise_coef, enslaving_f;  // (float)(real)noise_coef, (float)enslaving_degree
+  int max_timesteps;
+  int bits;  // alpha_plus2_int | exit_reward << 8 | follow_reward << 9 | term_wall << 10
+};
+static_assert(sizeof(EnvParamRec<float>) == 32 && sizeof(EnvParamRec<double>) == 48, "EnvParamRec is packed");
+
+// The view the step functions read their per-environment parameters from: the fields of KArgs with the same names.  The
+// uniform instances pass KArgs itself (env_params<false>), so their code is the code without per-env parameters.
+template <typename real>
+struct EnvParams {
+  real one_minus_enslaving, alpha, init_reward, intrinsic_coef;
+  float noise_coef, enslaving_f;
+  int max_timesteps, alpha_plus2_int, exit_reward, follow_reward, term_wall;
+};
+
+template <bool PE, typename real>
+__device__ __forceinline__ std::conditional_t<PE, EnvParams<real>, const KArgs<real>&> env_params(const KArgs<real>& a,
+                                                                                                 const EnvParamRec<real>* params, int e) {
+  if constexpr (PE) {
+    constexpr int V = sizeof(EnvParamRec<real>) / 16;
+    union { uint4 v[V]; EnvParamRec<real> r; } u;
+    const uint4* src = reinterpret_cast<const uint4*>(params + e);
+#pragma unroll
+    for (int k = 0; k < V; ++k) u.v[k] = __ldg(src + k);
+    EnvParams<real> p;
+    p.one_minus_enslaving = u.r.one_minus_enslaving; p.alpha = u.r.alpha;
+    p.init_reward = u.r.init_reward; p.intrinsic_coef = u.r.intrinsic_coef;
+    p.noise_coef = u.r.noise_coef; p.enslaving_f = u.r.enslaving_f; p.max_timesteps = u.r.max_timesteps;
+    p.alpha_plus2_int = u.r.bits & 0xff;
+    p.exit_reward = (u.r.bits >> 8) & 1; p.follow_reward = (u.r.bits >> 9) & 1; p.term_wall = (u.r.bits >> 10) & 1;
+    return p;
+  } else {
+    return a;
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // EnvBlock: packed per-environment state of the one-warp kernel family (N <= 64, float32).  Everything a step reads and
 // writes sits in ONE 1152-byte, 128-byte-aligned block, so the kernel forms one address per environment and every access
 // is that address + an immediate (+ 16 * lane): two broadcast LDG.128 for the record, one LDG.128 per pedestrian
@@ -806,25 +851,25 @@ __device__ __forceinline__ void store_head_obs(float* __restrict__ row, float ap
   }
 }
 
-// per-pedestrian term of grad_potential_pedestrians [gravity_encoding.py:8-25]
-template <typename real>
-__device__ __forceinline__ void grav_term(real px, real py, float apx, float apy, const KArgs<real>& a, real& gx, real& gy) {
+// per-pedestrian term of grad_potential_pedestrians [gravity_encoding.py:8-25]; pp: the environment's parameters (env_params)
+template <typename real, typename P>
+__device__ __forceinline__ void grav_term(real px, real py, float apx, float apy, const KArgs<real>& a, const P& pp, real& gx, real& gy) {
   const real rx = (real)apx - px, ry = (real)apy - py;
   const real norm = sqrt_(rx * rx + ry * ry) + a.eps;
-  const real p = a.alpha_plus2_int ? ipow(norm, a.alpha_plus2_int) : (real)pow((double)norm, (double)a.alpha + 2.0);
-  const real c = div_(-a.alpha, p);
+  const real p = pp.alpha_plus2_int ? ipow(norm, pp.alpha_plus2_int) : (real)pow((double)norm, (double)pp.alpha + 2.0);
+  const real c = div_(-pp.alpha, p);
   gx = c * rx;
   gy = c * ry;
 }
 
-template <typename real>
+template <typename real, typename P>
 __device__ __forceinline__ void store_grav_obs(float* __restrict__ row, float apx, float apy, real gpx, real gpy,
-                                               int n_followers, const KArgs<real>& a) {
+                                               int n_followers, const KArgs<real>& a, const P& pp) {
   // grad_potential_exit [gravity_encoding.py:28-38], float32 like the reference (agent, exit are float32)
   const float rx = apx - 0.f, ry = apy + 1.f;
   const float norm = __fsqrt_rn(rx * rx + ry * ry) + (float)a.eps;
-  const float alpha = (float)a.alpha;
-  const float p = a.alpha_plus2_int ? ipow(norm, a.alpha_plus2_int) : powf(norm, alpha + 2.f);
+  const float alpha = (float)pp.alpha;
+  const float p = pp.alpha_plus2_int ? ipow(norm, pp.alpha_plus2_int) : powf(norm, alpha + 2.f);
   const float c = __fdiv_rn(-alpha, p);
   row[0] = apx;
   row[1] = apy;
@@ -890,9 +935,9 @@ __device__ __forceinline__ float2 scripted_action(const A& a, long long calls, f
   return make_float2((float)sin(ph), (float)cos(ph));
 }
 
-// Area.agent_step [area.py:182-210], IEEE float32 like the reference
-template <typename A>
-__device__ __forceinline__ void agent_step(const A& a, float2 act, float2& ap, float2& ad, float& r_agent, bool& term_agent) {
+// Area.agent_step [area.py:182-210], IEEE float32 like the reference; p: the environment's parameters (env_params)
+template <typename A, typename P>
+__device__ __forceinline__ void agent_step(const A& a, const P& p, float2 act, float2& ap, float2& ad, float& r_agent, bool& term_agent) {
   const float nrm = __fadd_rn(__fsqrt_rn(__fadd_rn(__fmul_rn(act.x, act.x), __fmul_rn(act.y, act.y))), a.eps_f);
   const float ax = __fdiv_rn(act.x, nrm), ay = __fdiv_rn(act.y, nrm);
   ad.x = __fmul_rn(a.step_size_f, ax); ad.y = __fmul_rn(a.step_size_f, ay);
@@ -900,21 +945,21 @@ __device__ __forceinline__ void agent_step(const A& a, float2 act, float2& ap, f
   const bool collide = (ptx < -a.width_f) | (ptx > a.width_f) | (pty < -a.height_f) | (pty > a.height_f);
   r_agent = 0.f; term_agent = false;
   if (!collide) { ap.x = ptx; ap.y = pty; }
-  else { r_agent = -5.f; term_agent = a.term_wall != 0; }
+  else { r_agent = -5.f; term_agent = p.term_wall != 0; }
 }
 
 // rewards + termination [reward.py:19-46, area.py:174-180, env.py:158-171]; sd = sum of the distances to the exit
-template <typename real>
-__device__ __forceinline__ void step_reward(const KArgs<real>& a, int N, int now, real sd, int K_exit, int K_fol, int N_esc, float r_agent,
-                                            bool term_agent, real& intrinsic, real& r_status, real& reward, bool& terminated) {
+template <typename real, typename P>
+__device__ __forceinline__ void step_reward(const KArgs<real>& a, const P& p, int N, int now, real sd, int K_exit, int K_fol, int N_esc,
+                                            float r_agent, bool term_agent, real& intrinsic, real& r_status, real& reward, bool& terminated) {
   real tf;
   if constexpr (std::is_same<real, double>::value) { tf = (real)1 - (real)now / (real)(200 * N); intrinsic = (real)0 - sd / (real)N; }
   else { tf = (real)1 - (real)now * a.inv_200n; intrinsic = (real)0 - sd * a.inv_n; }
-  real r_ped = a.init_reward;
-  if (a.exit_reward) r_ped += ((real)15 + (real)10 * tf) * (real)K_exit;
-  if (a.follow_reward) r_ped += ((real)10 + (real)5 * tf) * (real)K_fol;
+  real r_ped = p.init_reward;
+  if (p.exit_reward) r_ped += ((real)15 + (real)10 * tf) * (real)K_exit;
+  if (p.follow_reward) r_ped += ((real)10 + (real)5 * tf) * (real)K_fol;
   r_status = (real)r_agent + r_ped;
-  reward = r_status + a.intrinsic_coef * intrinsic;
+  reward = r_status + p.intrinsic_coef * intrinsic;
   terminated = term_agent || (N_esc == N);
 }
 
@@ -957,8 +1002,10 @@ __device__ __forceinline__ int reset_pedestrian(const KArgs<real>& a, uint32_t e
 
 // CL > 1: ONE environment per thread-block cluster of CL CTAs (evac_cluster.cuh) -- CTA r owns pedestrians
 // [r * SLOTS, (r + 1) * SLOTS); float32 + cell list only; per-environment scalars are written by CTA 0.
-template <typename real, int THREADS, int PPT, int CL = 1>  // @region load
-__global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_kernel(const __grid_constant__ KArgs<real> a) {
+// PE: per-environment parameters (every CTA loads its environment's EnvParamRec; env_params).
+template <typename real, int THREADS, int PPT, int CL = 1, bool PE = false>  // @region load
+__global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_kernel(const __grid_constant__ KArgs<real> a,
+                                                                                      const EnvParamRec<real>* __restrict__ params) {
   constexpr int WARPS = THREADS / 32;
   constexpr int SLOTS = THREADS * PPT;
   constexpr bool F64 = std::is_same<real, double>::value;
@@ -978,9 +1025,11 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
   const bool lead = tid == 0 && rank_cta == 0;  // writes the per-environment scalars
   const int N = a.N;
   const uint32_t lt_mask = (1u << lane) - 1u;
-  const float noise_c = (float)a.noise_coef;
+  const float noise_c_cfg = (float)a.noise_coef;  // uniform instances: read here as before (in the loop it schedules differently)
 
   for (int e = blockIdx.x / CL; e < a.E; e += gridDim.x / CL) {
+    decltype(auto) p = env_params<PE>(a, params, e);
+    const float noise_c = PE ? (float)p.noise_coef : noise_c_cfg;
     // ---------------- load state (coalesced real2 per thread)
     real2* __restrict__ pos_e = a.pos + (size_t)e * N;
     real2* __restrict__ dir_e = a.dir + (size_t)e * N;
@@ -1017,7 +1066,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
       // ---------------- Time.step [area.py:53-59]
       const int now_prev = now;
       now += 1; steps_total += 1;
-      const bool truncated = now >= a.max_timesteps;
+      const bool truncated = now >= p.max_timesteps;
       // ---------------- random streams of this step (Philox2x32-10, philox.cuh): the RandomAgent action is computed
       // redundantly by every thread; the noise words are drawn where used
       float2 action_r = make_float2(0.f, 0.f);
@@ -1073,7 +1122,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
       else if (a.agent_kind == AGENT_RANDOM) act = action_r;
       else act = scripted_action(a, overall_start + steps_total, ap, wac_state);
       float r_agent; bool term_agent;
-      agent_step(a, act, ap, ad, r_agent, term_agent);
+      agent_step(a, p, act, ap, ad, r_agent, term_agent);
       // ---------------- pairwise alignment [area.py:105-119]  // @region pairwise
       real sx[PPT], sy[PPT], cnt[PPT];  // cnt: number of neighbours, used by the fp64 update only
       if constexpr (!COMPACT && !F64) {
@@ -1099,7 +1148,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
       // ---------------- new directions, enslaving, integration, reflection, statuses  // @region update
       int k_exit = 0, k_fol = 0, n_esc = 0, n_exi = 0, n_fol = 0;
       real sum_dexit = (real)0;
-      const real e_adx = (real)__fmul_rn(a.enslaving_f, ad.x), e_ady = (real)__fmul_rn(a.enslaving_f, ad.y);
+      const real e_adx = (real)__fmul_rn(p.enslaving_f, ad.x), e_ady = (real)__fmul_rn(p.enslaving_f, ad.y);
 #pragma unroll
       for (int k = 0; k < PPT; ++k) {
         const int i = base_i + k * THREADS + tid;
@@ -1128,8 +1177,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
             dy[k] = a.step_size * (cx * sn + cy * cn);
           }
           if (so == ST_FOLLOWER) {  // area.py:138-142; e * agent.direction is float32 in the reference
-            dx[k] = e_adx + a.one_minus_enslaving * dx[k];
-            dy[k] = e_ady + a.one_minus_enslaving * dy[k];
+            dx[k] = e_adx + p.one_minus_enslaving * dx[k];
+            dy[k] = e_ady + p.one_minus_enslaving * dy[k];
           }
         }
         if (efv[k]) { px[k] += dx[k]; py[k] += dy[k]; }
@@ -1177,7 +1226,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
       }
       if (a.status_counts != nullptr && lead) store_status_counts(a, s, e, N, N_esc, N_exi, N_fol);
       real intrinsic, r_status, reward; bool terminated;
-      step_reward(a, N, now, (real)sd, K_exit, K_fol, N_esc, r_agent, term_agent, intrinsic, r_status, reward, terminated);
+      step_reward(a, p, N, now, (real)sd, K_exit, K_fol, N_esc, r_agent, term_agent, intrinsic, r_status, reward, terminated);
       reward_sum += (float)reward;
       any_term |= terminated; any_trunc |= truncated;
       acc_r += (double)reward; acc_i += (double)intrinsic; acc_s += (double)r_status;
@@ -1204,7 +1253,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
           int nf = 0;
 #pragma unroll
           for (int k = 0; k < PPT; ++k) {
-            if (st[k] == ST_VISCEK) { real tx, ty; grav_term<real>(px[k], py[k], ap.x, ap.y, a, tx, ty); gx += tx; gy += ty; }
+            if (st[k] == ST_VISCEK) { real tx, ty; grav_term<real>(px[k], py[k], ap.x, ap.y, a, p, tx, ty); gx += tx; gy += ty; }
             nf += (st[k] == ST_FOLLOWER);
           }
           nf = __reduce_add_sync(0xffffffffu, nf);
@@ -1221,7 +1270,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
             cluster_sum<CL, 3>(cl_slot, v);
             nf = (int)v[0]; wx = v[1]; wy = v[2];
           }
-          if (lead) store_grav_obs<real>(row, ap.x, ap.y, (real)wx, (real)wy, nf, a);
+          if (lead) store_grav_obs<real>(row, ap.x, ap.y, (real)wx, (real)wy, nf, a, p);
         } else {
           if (lead) store_head_obs<real>(row, ap.x, ap.y, a);
 #pragma unroll
@@ -1265,9 +1314,11 @@ __global__ void __launch_bounds__(THREADS, THREADS == 32 ? 32 : 1) evac_step_ker
 // One 128-thread CTA per environment, pedestrians strided over the threads.
 enum { AUX_RESET = 1, AUX_STATUS = 2, AUX_OBS = 4 };
 
-template <typename real>
+// PE: per-environment parameters (the gravity encoding's alpha).
+template <typename real, bool PE = false>
 __global__ void __launch_bounds__(128) evac_aux_kernel(const __grid_constant__ KArgs<real> a, int flags,
-                                                       const uint8_t* __restrict__ mask, float* __restrict__ obs) {
+                                                       const uint8_t* __restrict__ mask, float* __restrict__ obs,
+                                                       const EnvParamRec<real>* __restrict__ params) {
   __shared__ RedScratch<4> red;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int N = a.N;
@@ -1301,13 +1352,14 @@ __global__ void __launch_bounds__(128) evac_aux_kernel(const __grid_constant__ K
       if ((flags & AUX_RESET) && sel) ap = make_float2(0.f, 0.f);
       float* row = obs + (size_t)e * a.obs_dim;
       if (a.positions == POS_GRAV) {
+        decltype(auto) p = env_params<PE>(a, params, e);
         real gx = (real)0, gy = (real)0;
         int nf = 0;
         for (int i = tid; i < N; i += 128) {
           real px, py, dx, dy;
           int s;
           state_load_ped<real>(a, e, i, px, py, dx, dy, s);
-          if (s == ST_VISCEK) { real tx, ty; grav_term<real>(px, py, ap.x, ap.y, a, tx, ty); gx += tx; gy += ty; }
+          if (s == ST_VISCEK) { real tx, ty; grav_term<real>(px, py, ap.x, ap.y, a, p, tx, ty); gx += tx; gy += ty; }
           nf += (s == ST_FOLLOWER);
         }
         nf = __reduce_add_sync(0xffffffffu, nf);
@@ -1317,7 +1369,7 @@ __global__ void __launch_bounds__(128) evac_aux_kernel(const __grid_constant__ K
         if (tid == 0) {
           int t = 0; double tx = 0, ty = 0;
           for (int w = 0; w < 4; ++w) { t += red.i[w][0]; tx += red.f[w][0]; ty += red.f[w][1]; }
-          store_grav_obs<real>(row, ap.x, ap.y, (real)tx, (real)ty, t, a);
+          store_grav_obs<real>(row, ap.x, ap.y, (real)tx, (real)ty, t, a, p);
         }
       } else {
         if (tid == 0) store_head_obs<real>(row, ap.x, ap.y, a);

@@ -87,9 +87,11 @@ struct WPed {
 // 26 warps per SM) pushes 4096 envs into a second wave: 9.81 us.
 constexpr int WARP_MINB = 28;
 constexpr int PAIR_UNROLL = 4;  // slot pairs per unrolled iteration of the pairwise loop
-// One environment per one-warp CTA (launch_warp in evac_abi.cu); no block-level barrier anywhere.
-template <int MODE>
-__global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_constant__ KArgs<float> a) {  // @region wload
+// One environment per one-warp CTA (launch_warp in evac_abi.cu); no block-level barrier anywhere.  PE: per-environment
+// parameters (the environment's EnvParamRec, loaded with the state; env_params).
+template <int MODE, bool PE = false>
+__global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_constant__ KArgs<float> a,
+                                                                  const EnvParamRec<float>* __restrict__ params) {  // @region wload
   // Tile<float> of 64 slots (+ the look-ahead entries) = 66 float4
   __shared__ __align__(16) float4 tile_smem[66];
   // sparse pass (a.cells_x > 0): {x, y, ux, uy} of every slot (+ the parked record) and the row / column slot masks
@@ -130,7 +132,8 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
   int now = rec1.x, episode = rec1.y, wac_state = rec1.z;
   float reward_sum = 0.f;
   int any_term = 0, any_trunc = 0;
-  const float noise_c = a.noise_coef;
+  decltype(auto) p = env_params<PE>(a, params, e);
+  const float noise_c = p.noise_coef;
   const float* noise_e = a.noise ? a.noise + (size_t)e * N : nullptr;
   float* obs_e = a.obs ? a.obs + (size_t)e * a.obs_dim : nullptr;
   const float2 wall = make_float2(a.width, a.height);
@@ -139,7 +142,7 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     // ---------------- Time.step [area.py:53-59]
     const int now_prev = now;
     now += 1;
-    const bool truncated = now >= a.max_timesteps;
+    const bool truncated = now >= p.max_timesteps;
     // the action is requested first so that its (cold) latency overlaps the preparation below
     float2 act_tbl = make_float2(0.f, 0.f);
     if (a.agent_kind == AGENT_TABLE) act_tbl = a.actions[(size_t)s * a.E + e];
@@ -231,7 +234,7 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     else if (a.agent_kind == AGENT_RANDOM) act = random_action(a.seed, env_g, (uint32_t)episode, (uint32_t)now_prev);
     else act = scripted_action(a, overall + 1, ap, wac_state);
     float r_agent; bool term_agent;
-    agent_step(a, act, ap, ad, r_agent, term_agent);
+    agent_step(a, p, act, ap, ad, r_agent, term_agent);
     // ---------------- pairwise alignment [area.py:105-119]  // @region wpairwise
     float sx[2], sy[2];
     if (sparse) {
@@ -243,7 +246,7 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
       else sx[0] = sx[1] = sy[0] = sy[1] = 0.f;
     }
     // ---------------- new headings, enslaving, integration, reflection, statuses  // @region wupdate
-    const float2 e_ad = make_float2(__fmul_rn(a.enslaving_f, ad.x), __fmul_rn(a.enslaving_f, ad.y));  // float32 like area.py:140
+    const float2 e_ad = make_float2(__fmul_rn(p.enslaving_f, ad.x), __fmul_rn(p.enslaving_f, ad.y));  // float32 like area.py:140
     int counts = 0;  // k_exit | k_fol << 8 | n_esc << 16 | n_exi << 24   (each <= 64)
     float sum_dexit = 0.f;
 #pragma unroll
@@ -259,7 +262,7 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
         float2 nd = __fmul2_rn(splat(c.x), make_float2(cn, sn));
         nd = __ffma2_rn(make_float2(-c.y, c.y), make_float2(sn, cn), nd);
         nd = __fmul2_rn(nd, splat(a.step_size));
-        if (so == ST_FOLLOWER) nd = __ffma2_rn(splat(a.one_minus_enslaving), nd, e_ad);  // area.py:138-142
+        if (so == ST_FOLLOWER) nd = __ffma2_rn(splat(p.one_minus_enslaving), nd, e_ad);  // area.py:138-142
         q[k].d = nd;
       }
       if (efv[k]) q[k].p = __fadd2_rn(q[k].p, q[k].d);
@@ -294,7 +297,7 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
       if (lane == 0) store_status_counts(a, s, e, N, N_esc, N_exi, n_fol);
     }
     float intrinsic, r_status, reward; bool terminated;
-    step_reward(a, N, now, sd, K_exit, K_fol, N_esc, r_agent, term_agent, intrinsic, r_status, reward, terminated);
+    step_reward(a, p, N, now, sd, K_exit, K_fol, N_esc, r_agent, term_agent, intrinsic, r_status, reward, terminated);
     reward_sum += reward;
     any_term |= terminated; any_trunc |= truncated;
     acc_r += (double)reward; acc_i += (double)intrinsic; acc_s += (double)r_status;
@@ -345,19 +348,19 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
         // reciprocal (~2 ulp each against the parity bar of 2e-5 of the largest term); the two sums over the warp in double.
         float gx = 0.f, gy = 0.f;
         int nf = 0;
-        const float alpha = (float)a.alpha, eps = (float)a.eps;
+        const float alpha = (float)p.alpha, eps = (float)a.eps;
 #pragma unroll
         for (int k = 0; k < 2; ++k) {
           const float2 R = __fadd2_rn(ap, make_float2(-q[k].p.x, -q[k].p.y));
           const float norm = sqrt_fast(fmaf(R.x, R.x, R.y * R.y)) + eps;
           const float n2 = norm * norm;
           float pw;
-          switch (a.alpha_plus2_int) {  // alpha = 2 .. 5 (BASELINE config 3) without a loop
+          switch (p.alpha_plus2_int) {  // alpha = 2 .. 5 (BASELINE config 3) without a loop
             case 4: pw = n2 * n2; break;
             case 5: pw = n2 * n2 * norm; break;
             case 6: pw = n2 * n2 * n2; break;
             case 7: pw = n2 * n2 * n2 * norm; break;
-            default: pw = a.alpha_plus2_int ? ipow(norm, a.alpha_plus2_int) : powf(norm, alpha + 2.f);
+            default: pw = p.alpha_plus2_int ? ipow(norm, p.alpha_plus2_int) : powf(norm, alpha + 2.f);
           }
           const float c = __fdividef(-alpha, pw);
           const bool vk = q[k].st == ST_VISCEK;
@@ -367,7 +370,7 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
         }
         nf = __reduce_add_sync(0xffffffffu, nf);
         const double wx = warp_sum((double)gx), wy = warp_sum((double)gy);
-        if (lane == 0) store_grav_obs<float>(row, ap.x, ap.y, (float)wx, (float)wy, nf, a);
+        if (lane == 0) store_grav_obs<float>(row, ap.x, ap.y, (float)wx, (float)wy, nf, a, p);
       } else {
         if (lane == 0) store_head_obs<float>(row, ap.x, ap.y, a);
 #pragma unroll

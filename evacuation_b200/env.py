@@ -41,6 +41,42 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+# Per-environment dynamics and reward parameters (EvacuationEnv.set_env_params; EvacEnvParams in include/evac_b200.h):
+# the EnvConfig / EnvWrappersConfig fields that enter one environment's own arithmetic.
+ENV_PARAM_FIELDS = tuple(name for name, _ in nat.EvacEnvParams._fields_)
+_ENV_PARAM_DTYPE = np.dtype(nat.EvacEnvParams)  # the C record, field for field
+# fields that stay uniform over a batch, and why
+_ENV_PARAM_EXCLUDED = {
+    **dict.fromkeys(("width", "height", "to_pedestrian"), "it sizes the neighbour-search grid"),
+    **dict.fromkeys(("to_leader", "step_size"), "it places the WacuumCleaner's lanes"),
+    **dict.fromkeys(("eps", "to_exit", "to_escape"), "the reference's parameter sweeps do not vary it"),
+    **dict.fromkeys(("number_of_pedestrians", "positions", "statuses", "type"), "it is a shape"),
+}
+
+
+def merge_env_params(current: dict, num_envs: int, fields: dict) -> dict:
+    """`current` (field -> [E] array, every field of ENV_PARAM_FIELDS) updated with `fields`: each value is a scalar
+    (broadcast to every environment) or a length-E sequence, NumPy array or tensor.  Returns new [E] arrays (float64 for the
+    reals, int32 for the flags and max_timesteps).  ValueError for an unknown or excluded field name, a wrong length or a
+    non-integer value of an integer field.  The value ranges are checked by the library (evac_set_env_params)."""
+    out = {k: np.array(current[k], dtype=_ENV_PARAM_DTYPE[k], copy=True) for k in ENV_PARAM_FIELDS}
+    for name, value in fields.items():
+        if name in _ENV_PARAM_EXCLUDED:
+            raise ValueError(f"`{name}` cannot be set per environment: {_ENV_PARAM_EXCLUDED[name]}")
+        if name not in out:
+            raise ValueError(f"unknown per-environment parameter `{name}`; the fields are {', '.join(ENV_PARAM_FIELDS)}")
+        v = np.asarray(value.detach().cpu().numpy() if torch.is_tensor(value) else value)
+        if v.ndim != 0 and v.shape != (num_envs,):
+            raise ValueError(f"`{name}`: expected a scalar or {num_envs} values, got shape {v.shape}")
+        dt = _ENV_PARAM_DTYPE[name]
+        if dt.kind == "i":
+            vf = v.astype(np.float64)
+            if not np.all(np.isfinite(vf) & (vf == np.round(vf)) & (np.abs(vf) < 2**31)):
+                raise ValueError(f"`{name}` takes integer values")
+        out[name][...] = v.astype(dt)
+    return out
+
+
 class _Pedestrians:
     """`env.unwrapped.pedestrians` (src/env/env/pedestrians.py): live views of the device state."""
 
@@ -181,6 +217,11 @@ class EvacuationEnv:
         self._positions, self._statuses, self._obs_type, self._alpha = "abs", "no", "Dict", 3.0
         self._h = None
         self._host_statuses = None  # numpy-rng face: statuses after the last step (for the |fv| draw)
+        # per-environment parameters (set_env_params): [E] arrays of every field, or None (uniform: the construction config);
+        # _env_params_mode counts the switches between the two, which select different kernel instances (PolicyRollout
+        # re-captures its graph after one)
+        self._env_params = None
+        self._env_params_mode = 0
 
         n = cfg.number_of_pedestrians
         self.pedestrians = _Pedestrians(self)
@@ -221,6 +262,8 @@ class EvacuationEnv:
         state = self.get_state() if self._h is not None else None
         for k, v in kw.items():
             setattr(self, "_" + k, v)
+        if "alpha" in kw and self._env_params is not None:  # a wrapper's alpha applies to every environment
+            self._env_params["alpha"][:] = float(kw["alpha"])
         if self._h is not None:
             self.close()
             self._handle()
@@ -255,6 +298,8 @@ class EvacuationEnv:
         nat.check(lib.evac_create(C.byref(c), self.num_envs, self.device.index, C.c_uint64(self.seed_value),
                                   C.c_int64(self.env_index_offset), C.byref(h)))
         self._h = h
+        if self._env_params is not None:  # a re-created handle (observation wrappers, reset(seed=...)) keeps them
+            self._upload_env_params(self._env_params)
         self._obs_dim = lib.evac_obs_dim(h)
         E, dev = self.num_envs, self.device
         self._obs = torch.empty((E, self._obs_dim), dtype=torch.float32, device=dev)
@@ -359,6 +404,42 @@ class EvacuationEnv:
             raise ValueError(f"state image has {image.numel()} bytes, this environment needs {int(lib.evac_state_bytes(h))}")
         nat.check(lib.evac_load_state(h, _ptr(image), self._stream()))
         self._host_statuses = None
+
+    def set_env_params(self, *uniform, **fields):
+        """Per-environment dynamics and reward parameters: one batch runs a whole parameter grid, or a policy trains over a
+        range of them (domain randomisation).  `fields` are EnvConfig / EnvWrappersConfig names (ENV_PARAM_FIELDS: noise_coef,
+        enslaving_degree, alpha, intrinsic_reward_coef, init_reward_each_step, is_new_exiting_reward, is_new_followers_reward,
+        is_termination_agent_wall_collision, max_timesteps); each value is a scalar or a length-E sequence / array / tensor.
+        Fields not named keep their current per-environment values.  `set_env_params(None)` returns to the construction
+        config.  Stream-ordered like step(): steps already enqueued use the old values.  Environment e then computes, bit for
+        bit, what environment e of an env constructed with e's values (same num_envs, seed, env_index_offset) computes.
+        The parameters are configuration: save_state() / load_state() do not carry them.  An observation wrapper applied
+        afterwards that sets alpha (GravityEncoding(alpha=...)) sets it for every environment."""
+        if uniform:
+            if len(uniform) != 1 or uniform[0] is not None or fields:
+                raise TypeError("set_env_params takes keyword fields, or the single positional argument None")
+            params = None
+        else:
+            params = merge_env_params(self.env_params(), self.num_envs, fields)
+        self._handle()
+        self._upload_env_params(params)
+        if (params is None) != (self._env_params is None):
+            self._env_params_mode += 1
+        self._env_params = params
+
+    def _upload_env_params(self, params):
+        rec = None
+        if params is not None:
+            rec = np.zeros(self.num_envs, dtype=_ENV_PARAM_DTYPE)
+            for k in ENV_PARAM_FIELDS:
+                rec[k] = params[k]
+        nat.check(nat.load().evac_set_env_params(self._h, None if rec is None else C.c_void_p(rec.ctypes.data), self._stream()))
+
+    def env_params(self) -> dict:
+        """field -> [E] NumPy array of the per-environment parameters (the construction config's values when uniform)."""
+        rec = np.zeros(self.num_envs, dtype=_ENV_PARAM_DTYPE)
+        nat.check(nat.load().evac_get_env_params(self._handle(), C.c_void_p(rec.ctypes.data)))
+        return {k: rec[k].copy() for k in ENV_PARAM_FIELDS}
 
     def accumulators(self):
         """(acc [E,3] float64: episode_reward, episode_intrinsic_reward, episode_status_reward; overall_timesteps [E] int64)
@@ -479,7 +560,11 @@ class EvacuationEnv:
         # ONE draw for the whole batch, environment-major then ascending pedestrian index: MT19937 hands out the same values as one
         # call per environment would (a double costs two words wherever the call boundary falls)
         fv = self._host_statuses.reshape(E, N) <= 2  # VISCEK = 1, FOLLOWER = 2 (statuses are 1..4)
-        noise[fv] = np.random.uniform(low=-c / 2, high=c / 2, size=int(np.count_nonzero(fv)))
+        if self._env_params is not None:  # per-env noise_coef: the same draws, each scaled by its environment's coefficient
+            c = np.repeat(self._env_params["noise_coef"], np.count_nonzero(fv, axis=1))
+            noise[fv] = np.random.uniform(low=-c / 2, high=c / 2)
+        else:
+            noise[fv] = np.random.uniform(low=-c / 2, high=c / 2, size=int(np.count_nonzero(fv)))
         return noise
 
     def step(self, action, noise=None):

@@ -418,6 +418,7 @@ class PolicyRollout:
         self.out = {k: torch.zeros(s, device=self.device) for k, s in
                     (("action", (self.E, 2)), ("logprob", (self.E,)), ("value", (self.E,)), ("reward", (self.E,)))}
         self._graph = None
+        self._graph_params_mode = None  # env's _env_params_mode at capture: uniform and per-env steps are different kernels
         self.launches_per_iteration = None
         # fused policy: NormalizeObservation runs in the policy's first kernel on the env's raw observation buffer, so `next_obs`
         # (the normalised observation the policy saw) is produced INSIDE the iteration
@@ -491,12 +492,15 @@ class PolicyRollout:
         # kernels of THIS library recorded into one graph replay: the handles count launches at capture time; the fused loop's
         # evac_normalize_reward is a handle-less entry point (+1)
         self.launches_per_iteration = count() - before + (1 if self.fused else 0)
+        self._graph_params_mode = self.env.unwrapped._env_params_mode
         self._restore(snap)
         torch.cuda.set_rng_state(rng_state, self.device)
         torch.cuda.synchronize(self.device)
 
     def run(self, num_steps: int):
         """Returns the storage dict ([T, E, ...]) when `store`, else None."""
+        if self._graph is not None and self._graph_params_mode != self.env.unwrapped._env_params_mode:
+            self._graph = None  # set_env_params switched between the uniform and the per-env step kernel: capture again
         if self.use_graph and self._graph is None:
             self._capture()
         buf = None

@@ -30,6 +30,9 @@
  *   evac_get_state/evac_set_state  env.unwrapped.{pedestrians,agent,time} attribute access
  *                                                                  (wrappers.py:35,48; gravity_encoding.py:50,64-65)
  *   evac_episode_stats           the per-episode logging dict      src/env/env/env.py:114-127
+ *   evac_set_env_params /        one EnvConfig per environment     the reference's parameter sweeps (noise x enslaving
+ *   evac_get_env_params          (gymnasium SyncVectorEnv over      x alpha grids) as one batch
+ *                                differently configured envs)
  *
  * Conventions
  *   - plain C, no torch / C++ types; all array arguments are raw pointers.
@@ -183,7 +186,8 @@ int evac_step_host(EvacHandle* h, const float* actions, const float* noise, floa
  * key word), running-episode accumulators, scripted-agent state, finished-episode statistics -- as one flat byte image in
  * DEVICE memory of evac_state_bytes(h) bytes.  The image is only meaningful for a handle created with the same
  * configuration, number of environments and library build; together with (seed, env_index_offset) it resumes a run
- * bit-identically (the random streams are counter-based: nothing else carries state).
+ * bit-identically (the random streams are counter-based: nothing else carries state).  Per-environment parameters
+ * (evac_set_env_params) are configuration and are not part of the image.
  * [the reference has no checkpointing of the environment; SURVEY.md section 5] */
 int64_t evac_state_bytes(EvacHandle* h);
 int evac_save_state(EvacHandle* h, void* image, void* stream);
@@ -215,6 +219,39 @@ int evac_episode_stats(EvacHandle* h, float* stats, uint8_t* finished, double* t
  * (area.py:42-59): acc [E,3] float64 = episode_reward, episode_intrinsic_reward, episode_status_reward;
  * overall_timesteps [E] int64.  Device pointers; either may be NULL. */
 int evac_get_accumulators(EvacHandle* h, double* acc, int64_t* overall_timesteps, void* stream);
+
+/* ---- per-environment dynamics and reward parameters: one handle runs a whole parameter grid (or domain randomisation)
+ * in one launch per step, where a uniform handle needs one handle per configuration.
+ *
+ * The fields are the EvacConfig fields that enter one environment's own arithmetic.  Left out, and uniform over the handle:
+ *   - width, height, to_pedestrian: they size the neighbour-search grid (cell list, cell masks, cluster grid);
+ *   - to_leader, width, height, step_size: they place the WacuumCleaner's lanes;
+ *   - eps, to_exit, to_escape: the reference's parameter sweeps do not vary them;
+ *   - number_of_pedestrians and the observation modes: they are shapes.
+ * Each record is converted exactly as evac_create converts the same EvacConfig fields, and the random streams are keyed by
+ * (seed, global env index, episode, step), not by these values: environment e of a handle with per-env parameters computes
+ * bit for bit what environment e of a uniform handle created with e's values (same E, seed and env_index_offset) computes. */
+typedef struct EvacEnvParams {
+  double noise_coef;
+  double enslaving_degree;
+  double alpha;                                /* GravityEncoding alpha (observation and reset / evac_observe) */
+  double intrinsic_reward_coef;
+  double init_reward_each_step;
+  int32_t is_new_exiting_reward;
+  int32_t is_new_followers_reward;
+  int32_t is_termination_agent_wall_collision;
+  int32_t max_timesteps;                       /* 1 .. 2^21, like EvacConfig */
+} EvacEnvParams;
+
+/* `params`: HOST array of E records, or NULL to return to the handle's uniform EvacConfig values.  Stream-ordered on
+ * `stream`: steps enqueued before the call use the old values, steps after it the new ones (the host array may be reused as
+ * soon as the call returns).  The device copy is allocated once per handle, so a CUDA graph captured while per-env parameters
+ * are set reads the values of later calls.  Setting or clearing them switches the step / observe kernels between their uniform
+ * and per-environment instances: a graph captured before the switch still runs the other instance and must be re-captured.
+ * The parameters are configuration, not state: evac_state_bytes / evac_save_state / evac_load_state do not include them. */
+int evac_set_env_params(EvacHandle* h, const EvacEnvParams* params, void* stream);
+/* out: HOST array of E records -- the per-env values, or the EvacConfig values of every env of a uniform handle. */
+int evac_get_env_params(const EvacHandle* h, EvacEnvParams* out);
 
 /* Number of kernels this library launched since the handle was created. */
 int64_t evac_launch_count(const EvacHandle* h);
