@@ -75,6 +75,21 @@ class EvacPolicyIO(C.Structure):
     ]
 
 
+class EvacPolicyRolloutIO(C.Structure):
+    _fields_ = [
+        ("obs", C.c_void_p), ("next_done", C.c_void_p),
+        ("norm_mean", C.c_void_p), ("norm_var", C.c_void_p), ("norm_count", C.c_void_p),
+        ("norm_eps", C.c_float), ("norm_clip", C.c_float), ("norm_update", C.c_int32),
+        ("returns", C.c_void_p), ("ret_mean", C.c_void_p), ("ret_var", C.c_void_p), ("ret_count", C.c_void_p),
+        ("gamma", C.c_float), ("eps", C.c_float), ("clip", C.c_float),
+        ("sample", C.c_int32), ("seed", C.c_uint64), ("offset", C.c_uint64), ("offset_device", C.c_void_p),
+        ("env_index_offset", C.c_int64),
+        ("obs_norm", C.c_void_p), ("action", C.c_void_p), ("logprob", C.c_void_p), ("value", C.c_void_p),
+        ("reward_norm", C.c_void_p), ("dones", C.c_void_p), ("status_counts", C.c_void_p),
+        ("reward_sum", C.c_void_p), ("terminated", C.c_void_p), ("truncated", C.c_void_p),
+    ]
+
+
 # every symbol include/evac_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 SIGNATURES = {
@@ -113,6 +128,7 @@ SIGNATURES = {
     "evac_policy_forward": (C.c_int, [_P, C.POINTER(EvacPolicyIO), _P]),
     "evac_policy_launch_count": (C.c_int64, [_P]),
     "evac_normalize_reward": (C.c_int, [C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_float, C.c_float, C.c_float, _P]),
+    "evac_rollout_policy": (C.c_int, [_P, _P, C.c_int32, C.POINTER(EvacPolicyRolloutIO), _P]),
     "evac_probe_fma": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
     "evac_probe_pairwise": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
 }

@@ -575,6 +575,62 @@ int evac_step(EvacHandle* h, const float* actions, const float* noise, float* ob
   return evac_rollout(h, 1, EVAC_AGENT_TABLE, actions, noise, obs, 0, reward, terminated, truncated, nullptr, stream);
 }
 
+int evac_rollout_policy(EvacHandle* h, const EvacPolicy* p, int32_t num_steps, const EvacPolicyRolloutIO* io, void* stream) {
+  if (!h || !p || !io) return fail(EVAC_ERR_INVALID, "evac_rollout_policy: handle / policy / io is NULL");
+  if (num_steps < 1) return fail(EVAC_ERR_INVALID, "num_steps must be >= 1");
+  if (h->blocks == nullptr)
+    return fail(EVAC_ERR_UNSUPPORTED, "evac_rollout_policy runs in the one-warp step kernel: float32 and N <= 64 (N = %d, %s)", h->N,
+                h->prec == EVAC_PREC_F64 ? "float64" : "float32");
+  if (h->cfg.positions != EVAC_POS_GRAV) return fail(EVAC_ERR_UNSUPPORTED, "evac_rollout_policy needs positions = grav (obs_dim 6)");
+  evacp::HArgs ha;
+  int nb = 0, pdev = 0;
+  if (int r = evac_policy_heads_view_(p, &ha, &nb, &pdev)) return r;
+  if (nb != 0 || ha.K != 6 || ha.A != 2)
+    return fail(EVAC_ERR_UNSUPPORTED, "evac_rollout_policy takes the linear policy (num_blocks = 0) with K = 6 and action_dim 2, got "
+                "num_blocks %d, K %d, action_dim %d", nb, ha.K, ha.A);
+  if (pdev != h->device) return fail(EVAC_ERR_INVALID, "policy on device %d, environments on device %d", pdev, h->device);
+  if (!io->obs || !io->next_done) return fail(EVAC_ERR_INVALID, "obs and next_done are required");
+  if ((io->norm_mean != nullptr) != (io->norm_var != nullptr) || (io->norm_mean && !io->norm_count))
+    return fail(EVAC_ERR_INVALID, "norm_mean, norm_var and norm_count must be given together");
+  const bool rn = io->returns != nullptr;
+  if (rn != (io->ret_mean != nullptr) || rn != (io->ret_var != nullptr) || rn != (io->ret_count != nullptr))
+    return fail(EVAC_ERR_INVALID, "returns, ret_mean, ret_var and ret_count must be given together");
+  if (io->reward_norm && !rn) return fail(EVAC_ERR_INVALID, "reward_norm needs the reward normaliser (returns, ret_mean, ret_var, ret_count)");
+  if (int r = set_device(h)) return r;
+  cudaStream_t st = (cudaStream_t)stream;
+  KArgs<float> a = make_args<float>(h);
+  a.obs = io->obs; a.obs_every_step = 0; a.num_steps = num_steps;
+  a.reward = io->reward_sum; a.terminated = io->terminated; a.truncated = io->truncated; a.status_counts = io->status_counts;
+  WPolArgs w;
+  memset(&w, 0, sizeof(w));
+  w.h = ha;
+  w.h.E = h->E;
+  w.h.value = io->value; w.h.action = io->action; w.h.logprob = io->logprob;
+  w.h.sample = io->sample;
+  w.h.seed_lo = (uint32_t)io->seed; w.h.seed_hi = (uint32_t)(io->seed >> 32);
+  w.h.offset = io->offset; w.h.offset_dev = reinterpret_cast<const unsigned long long*>(io->offset_device);
+  w.h.env_offset = io->env_index_offset;
+  w.n.mean = io->norm_mean; w.n.var = io->norm_var; w.n.count = io->norm_count; w.n.obs_norm = io->obs_norm;
+  w.n.eps = io->norm_eps; w.n.clip = io->norm_clip;
+  w.norm_update = io->norm_update != 0;
+  w.next_done = io->next_done; w.dones = io->dones;
+  w.returns = io->returns; w.ret_mean = io->ret_mean; w.ret_var = io->ret_var; w.ret_count = io->ret_count;
+  w.reward_norm = io->reward_norm;
+  w.gamma = io->gamma; w.ret_eps = io->eps; w.ret_clip = io->clip;
+  if (h->per_env) evac_warp_policy_kernel<true><<<a.E, 32, 0, st>>>(a, params_of<float>(h), w);
+  else evac_warp_policy_kernel<false><<<a.E, 32, 0, st>>>(a, nullptr, w);
+  CK(cudaGetLastError());
+  h->launches++;
+  double* oc = io->norm_mean && io->norm_update ? io->norm_count : nullptr;
+  unsigned long long* off = reinterpret_cast<unsigned long long*>(io->offset_device);
+  if (oc || io->ret_count || off) {
+    evac_policy_counters_kernel<<<1, 1, 0, st>>>(oc, io->ret_count, off, num_steps);
+    CK(cudaGetLastError());
+    h->launches++;
+  }
+  return EVAC_OK;
+}
+
 static bool is_pinned(const void* p) {
   if (!p) return false;
   cudaPointerAttributes attr;

@@ -174,6 +174,17 @@ static int launch_heads(EvacPolicy* p, const EvacPolicyIO* io, const float* x, c
   return EVAC_OK;
 }
 
+int evac_policy_heads_view_(const EvacPolicy* p, HArgs* h, int* num_blocks, int* device) {
+  if (!p) return pfail(EVAC_ERR_INVALID, "policy is NULL");
+  if (!p->loaded) return pfail(EVAC_ERR_INVALID, "evac_policy_load_weights has not been called");
+  memset(h, 0, sizeof(*h));
+  h->K = p->K; h->K16 = p->K16; h->NH = p->NH; h->A = p->A;
+  h->w1t = p->d_w1t; h->b1 = p->d_b1; h->w2t = p->d_w2t; h->b2 = p->d_b2; h->w3 = p->d_w3; h->b3 = p->d_b3; h->logstd = p->d_logstd;
+  *num_blocks = p->NB;
+  *device = p->device;
+  return EVAC_OK;
+}
+
 extern "C" {
 
 int evac_policy_default_config(EvacPolicyConfig* cfg, int32_t number_of_pedestrians, int32_t d_model) {

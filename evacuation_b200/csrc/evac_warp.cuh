@@ -12,6 +12,7 @@
 //     shared-memory staging; no block barrier anywhere (one warp: __syncwarp only).
 #pragma once
 #include "evac_kernels.cuh"
+#include "evac_policy_ops.cuh"
 
 namespace evac {
 
@@ -87,17 +88,166 @@ struct WPed {
 // 26 warps per SM) pushes 4096 envs into a second wave: 9.81 us.
 constexpr int WARP_MINB = 28;
 constexpr int PAIR_UNROLL = 4;  // slot pairs per unrolled iteration of the pairwise loop
-// One environment per one-warp CTA (launch_warp in evac_abi.cu); no block-level barrier anywhere.  PE: per-environment
-// parameters (the environment's EnvParamRec, loaded with the state; env_params).
-template <int MODE, bool PE = false>
-__global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_constant__ KArgs<float> a,
-                                                                  const EnvParamRec<float>* __restrict__ params) {  // @region wload
+// ---- The linear RPO policy as the agent of the grav kernel (evac_rollout_policy): each step runs rpo_agent.py:180-203 --
+// NormalizeObservation, the heads, Normal sampling, ClipAction, the step, NormalizeReward and next_done -- inside the step loop.
+// The heads are the CUDA-core heads kernel's sums for K = 6 (evac_policy_heads_kernel<NORM>, the kernel K = 6 takes), in the same
+// order: lane L owns hidden columns L and L + 32 of each head, the layer-1 and layer-2 outputs are exchanged through shared memory.
+struct WPolArgs {
+  evacp::HArgs h;      // weights (CUDA-core layout), NH, A = 2, sample, seed, offset, offset_dev, env_offset; value / action / logprob
+                       // are the per-step bases [T, E, ..] (each may be NULL; value NULL skips the critic columns)
+  evacp::NArgs n;      // NormalizeObservation (n.mean NULL: none); *n.count is read once per launch; n.obs_norm [T, E, 6] or NULL
+  int norm_update;     // 0: the statistics are used frozen (evaluation)
+  float* next_done;    // [E] in / out
+  float* dones;        // [T, E]: next_done before each step (or NULL)
+  float *returns, *ret_mean, *ret_var;  // NormalizeReward state [E] (returns NULL: no reward normaliser)
+  const double* ret_count;
+  float* reward_norm;  // [T, E] or NULL
+  float gamma, ret_eps, ret_clip;
+};
+constexpr int WPOL_H1 = 16, WPOL_H2 = WPOL_H1 + 128, WPOL_SMEM = WPOL_H2 + 128;  // pol_sm layout (floats)
+// resident warps per SM the policy instance is sized for (DESIGN.md section 7.2)
+constexpr int WARP_POL_MINB = 16;
+
+// Policy part of step s of environment e: returns the clipped action every lane applies.  sm[0..5] holds the raw observation.
+// Lane k < 6 updates (or, frozen, reads) the statistics of value k; `cnt` is the normaliser's sample count before this step.
+__device__ __forceinline__ float2 warp_policy_act(const WPolArgs& P, int E, int s, int e, int lane, float& mean, float& var, double cnt,
+                                                  float done, float* sm) {
+  const size_t se = (size_t)s * E + e;
+  if (lane == 0 && P.dones != nullptr) P.dones[se] = done;
+  // ---- NormalizeObservation + clip (op for op the heads kernel's NORM load)
+  const float x = lane < 6 ? sm[lane] : 0.f;
+  float z = x;
+  if (P.n.mean != nullptr) {
+    if (P.norm_update) {
+      evacp::NArgs n = P.n;
+      n.count = &cnt;
+      z = evacp::norm_update(x, mean, var, evacp::norm_weights(n), n);
+    } else {
+      z = evacp::min_nan(evacp::max_nan(__fmul_rn(__fsub_rn(x, mean), rsqrtf(__fadd_rn(var, P.n.eps))), -P.n.clip), P.n.clip);
+    }
+  }
+  if (lane < 6) {
+    sm[8 + lane] = z;
+    if (P.n.obs_norm != nullptr) P.n.obs_norm[se * 6 + lane] = z;
+  }
+  __syncwarp();
+  const evacp::HArgs& h = P.h;
+  const bool critic = h.value != nullptr;
+  const float4 x03 = *reinterpret_cast<const float4*>(sm + 8);
+  const float2 x45 = *reinterpret_cast<const float2*>(sm + 12);
+  // ---- layer 1, column o = 32 j + lane (j = 0, 1 critic, 2, 3 actor).  The heads kernel sums four split-K chains over k = 4g .. 4g + 3
+  // of the 16-wide chunk: chain 0 from b1 over k = 0..3, chain 1 from +0 over k = 4..7, chains 2 and 3 from +0 over k >= 8.  Every
+  // term with k >= 6 is fma(+0, +0, acc) (the observation is zero-filled, the weight rows are zero padding) = acc + 0.f, and chains 2
+  // and 3 are exactly +0, so they are written as the additions of +0 they are (acc + 0.f is not acc when acc is -0).
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    if (j < 2 && !critic) continue;
+    const int o = 32 * j + lane;
+    const float* w = h.w1t + o;
+    float g0 = h.b1[o];
+    g0 = fmaf(x03.x, w[0], g0); g0 = fmaf(x03.y, w[128], g0); g0 = fmaf(x03.z, w[256], g0); g0 = fmaf(x03.w, w[384], g0);
+    float g1 = fmaf(x45.x, w[512], 0.f);
+    g1 = fmaf(x45.y, w[640], g1);
+    g1 = __fadd_rn(__fadd_rn(g1, 0.f), 0.f);                                   // k = 6, 7
+    sm[WPOL_H1 + o] = tanhf(__fadd_rn(__fadd_rn(__fadd_rn(g0, g1), 0.f), 0.f));  // + chain 2 + chain 3
+  }
+  __syncwarp();
+  // ---- layer 2: four chains over k in [16 g, 16 g + 16), chain 0 from b2, summed in order (the heads kernel's split-K groups)
+  float c[4][4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+#pragma unroll
+    for (int g = 0; g < 4; ++g) c[j][g] = (g == 0 && (j >= 2 || critic)) ? h.b2[32 * j + lane] : 0.f;
+  const float* hc = sm + WPOL_H1;
+  const float* ha = sm + WPOL_H1 + 64;
+#pragma unroll 1
+  for (int kk = 0; kk < 16; kk += 4) {
+#pragma unroll
+    for (int g = 0; g < 4; ++g) {
+      const int k = 16 * g + kk;
+      const float4 va = *reinterpret_cast<const float4*>(ha + k);
+      const float av[4] = {va.x, va.y, va.z, va.w};
+      const float* wr = h.w2t + (size_t)k * 128 + lane;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        c[2][g] = fmaf(av[q], wr[q * 128 + 64], c[2][g]);
+        c[3][g] = fmaf(av[q], wr[q * 128 + 96], c[3][g]);
+      }
+      if (critic) {
+        const float4 vc = *reinterpret_cast<const float4*>(hc + k);
+        const float cv[4] = {vc.x, vc.y, vc.z, vc.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          c[0][g] = fmaf(cv[q], wr[q * 128], c[0][g]);
+          c[1][g] = fmaf(cv[q], wr[q * 128 + 32], c[1][g]);
+        }
+      }
+    }
+  }
+  __syncwarp();  // h1 is read by every lane before h2 (its neighbour in sm) is written
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+    if (j >= 2 || critic) sm[WPOL_H2 + 32 * j + lane] = tanhf(((c[j][0] + c[j][1]) + c[j][2]) + c[j][3]);
+  __syncwarp();
+  // ---- layer 3: row r = lane (0 value, 1..2 the action mean), one chain from b3[r] over k < NH
+  float o3 = 0.f;
+  if (lane < 3 && (lane > 0 || critic)) {
+    const float* hp = sm + WPOL_H2 + (lane == 0 ? 0 : 64);
+    const float* w = h.w3 + lane * 64;
+    o3 = h.b3[lane];
+    for (int k = 0; k < h.NH; ++k) o3 = fmaf(hp[k], w[k], o3);
+  }
+  const float m0 = __shfl_sync(0xffffffffu, o3, 1), m1 = __shfl_sync(0xffffffffu, o3, 2);
+  // ---- Normal(mean, exp(logstd)) sample, log-probability, ClipAction: heads_finish of environment e, with the step's stream offset
+  if (lane == 0) {
+    evacp::HArgs f = h;
+    f.A = 2;
+    f.given_action = nullptr; f.mean = nullptr; f.entropy = nullptr;
+    f.value = h.value ? h.value + se : nullptr;
+    f.action = h.action ? h.action + se * 2 : nullptr;
+    f.logprob = h.logprob ? h.logprob + se : nullptr;
+    f.action_clipped = sm + 14;
+    f.offset = h.offset + (unsigned long long)s;
+    f.env_offset = h.env_offset + e;
+    const float o[4] = {o3, m0, m1, 0.f};
+    evacp::heads_finish(f, 0, o, true, true);
+  }
+  __syncwarp();
+  return make_float2(sm[14], sm[15]);
+}
+
+// NormalizeReward + clip and next_done of one step (lane 0), op for op evac_normalize_reward_kernel on what evac_step writes: the
+// reward 0.f + reward (its one-step sum), terminated and truncated.  Returns next_done.
+__device__ __forceinline__ float warp_policy_reward(const WPolArgs& P, size_t se, float reward, bool terminated, bool truncated, float& ret,
+                                                   float& mean, float& var, double cnt) {
+  if (P.returns != nullptr) {
+    evacp::NArgs n{};
+    n.count = &cnt;
+    const evacp::NormWeights w = evacp::norm_weights(n);  // the same weights the reward kernel forms from *count
+    const float r = __fadd_rn(0.f, reward);
+    const float keep = terminated ? 0.f : 1.f;
+    ret = __fadd_rn(__fmul_rn(ret, __fmul_rn(P.gamma, keep)), r);
+    const float delta = __fsub_rn(ret, mean);
+    mean = __fadd_rn(mean, __fmul_rn(delta, w.w_new));
+    var = __fadd_rn(__fmul_rn(var, w.w_old), __fmul_rn(__fmul_rn(delta, delta), w.w_mix));
+    const float z = __fmul_rn(r, rsqrtf(__fadd_rn(var, P.ret_eps)));
+    if (P.reward_norm != nullptr) P.reward_norm[se] = evacp::min_nan(evacp::max_nan(z, -P.ret_clip), P.ret_clip);
+  }
+  return (terminated || truncated) ? 1.f : 0.f;
+}
+// The step loop of one environment (one warp).  PE: per-environment parameters (the environment's EnvParamRec, loaded with the
+// state; env_params).  POL: the action of every step comes from the linear policy (warp_policy_act, evac_rollout_policy).
+template <int MODE, bool PE, bool POL>
+__device__ __forceinline__ void warp_env_loop(const KArgs<float>& a, const EnvParamRec<float>* __restrict__ params,
+                                              const WPolArgs* pol, const int lane) {  // @region wload
   // Tile<float> of 64 slots (+ the look-ahead entries) = 66 float4
   __shared__ __align__(16) float4 tile_smem[66];
   // sparse pass (a.cells_x > 0): {x, y, ux, uy} of every slot (+ the parked record) and the row / column slot masks
   __shared__ float4 rec[WREC_PARK + 1];
   __shared__ uint2 row_mask[WCELLS + 2], col_mask[WCELLS + 2];
-  const int lane = threadIdx.x & 31, e = blockIdx.x, N = a.N;
+  // POL: [raw observation (6) + 2 | normalised observation (6) + clipped action (2) | h1 (128) | h2 (128)]
+  __shared__ __align__(16) float pol_sm[POL ? WPOL_SMEM : 1];
+  const int e = blockIdx.x, N = a.N;
   if (e >= a.E) return;
   const Tile<float> tile(reinterpret_cast<unsigned char*>(tile_smem), 64);
   const bool cells = a.cells_x > 0;
@@ -137,6 +287,21 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
   const float* noise_e = a.noise ? a.noise + (size_t)e * N : nullptr;
   float* obs_e = a.obs ? a.obs + (size_t)e * a.obs_dim : nullptr;
   const float2 wall = make_float2(a.width, a.height);
+  // POL: lane k < 6 keeps the running mean / variance of observation value k, lane 0 next_done and the NormalizeReward state
+  [[maybe_unused]] float o_mean = 0.f, o_var = 0.f, done = 0.f, ret = 0.f, r_mean = 0.f, r_var = 0.f;
+  [[maybe_unused]] double o_cnt = 0.0, r_cnt = 0.0;
+  if constexpr (POL) {
+    if (lane < 6) {
+      pol_sm[lane] = obs_e[lane];
+      if (pol->n.mean != nullptr) { o_mean = pol->n.mean[(size_t)e * 6 + lane]; o_var = pol->n.var[(size_t)e * 6 + lane]; }
+    }
+    if (pol->n.mean != nullptr) o_cnt = *pol->n.count;
+    if (lane == 0) {
+      done = pol->next_done[e];
+      if (pol->returns != nullptr) { ret = pol->returns[e]; r_mean = pol->ret_mean[e]; r_var = pol->ret_var[e]; r_cnt = *pol->ret_count; }
+    }
+    __syncwarp();
+  }
 
   for (int s = 0; s < a.num_steps; ++s) {  // @region wrng
     // ---------------- Time.step [area.py:53-59]
@@ -145,7 +310,8 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     const bool truncated = now >= p.max_timesteps;
     // the action is requested first so that its (cold) latency overlaps the preparation below
     float2 act_tbl = make_float2(0.f, 0.f);
-    if (a.agent_kind == AGENT_TABLE) act_tbl = a.actions[(size_t)s * a.E + e];
+    if constexpr (POL) act_tbl = warp_policy_act(*pol, a.E, s, e, lane, o_mean, o_var, o_cnt, done, pol_sm);
+    else if (a.agent_kind == AGENT_TABLE) act_tbl = a.actions[(size_t)s * a.E + e];
     // ---------------- angular noise of this lane's two pedestrians [area.py:124]
     float nz[2];
     if (noise_e != nullptr) {
@@ -230,7 +396,7 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     __syncwarp();
     // ---------------- action source + Area.agent_step [area.py:182-210]  // @region wagent
     float2 act;
-    if (a.agent_kind == AGENT_TABLE) act = act_tbl;
+    if (POL || a.agent_kind == AGENT_TABLE) act = act_tbl;
     else if (a.agent_kind == AGENT_RANDOM) act = random_action(a.seed, env_g, (uint32_t)episode, (uint32_t)now_prev);
     else act = scripted_action(a, overall + 1, ap, wac_state);
     float r_agent; bool term_agent;
@@ -302,6 +468,10 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     any_term |= terminated; any_trunc |= truncated;
     acc_r += (double)reward; acc_i += (double)intrinsic; acc_s += (double)r_status;
     overall += 1;
+    if constexpr (POL) {
+      if (lane == 0) done = warp_policy_reward(*pol, (size_t)s * a.E + e, reward, terminated, truncated, ret, r_mean, r_var, r_cnt);
+      o_cnt += 1.0; r_cnt += 1.0;  // the caller's per-step `count += 1.0`, in the same order
+    }
     // ---------------- same-step auto-reset (gymnasium vector-env semantics)  // @region wreset
     if (a.auto_reset && (terminated || truncated)) {
       const int N_fol = __popc(__ballot_sync(0xffffffffu, q[0].st == ST_FOLLOWER)) + __popc(__ballot_sync(0xffffffffu, q[1].st == ST_FOLLOWER));
@@ -314,8 +484,9 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
         if (valid[k]) q[k].st = reset_pedestrian<float>(a, env_g, (uint32_t)episode, (uint32_t)(lane + 32 * k), q[k].p.x, q[k].p.y, q[k].d.x, q[k].d.y);
     }
     // ---------------- observation [wrappers.py:8-96, gravity_encoding.py:8-81]  // @region wobs
-    if (obs_e != nullptr && (a.obs_every_step || s == a.num_steps - 1)) {
+    if (obs_e != nullptr && (a.obs_every_step || s == a.num_steps - 1 || POL)) {
       float* row = obs_e + (a.obs_every_step ? (size_t)s * a.E * a.obs_dim : (size_t)0);
+      if constexpr (POL) row = pol_sm;  // the next step's policy reads the 6 values from shared memory; obs gets the last step's
       if constexpr (MODE == WMODE_REL_OHE_BOX) {
         // rows = [agent; exit; pedestrians], cols = [x, y, ohe(4)]; relative positions / sqrt(2) (float32 hypotenuse).
         // Three float2 stores per pedestrian straight from registers (24-byte row stride: a warp's STG.64 touches 24 sectors for
@@ -399,6 +570,41 @@ __global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_c
     if (a.terminated) a.terminated[e] = (uint8_t)any_term;
     if (a.truncated) a.truncated[e] = (uint8_t)any_trunc;
   }
+  if constexpr (POL) {
+    if (lane < 6) {
+      obs_e[lane] = pol_sm[lane];
+      if (pol->n.mean != nullptr && pol->norm_update) { pol->n.mean[(size_t)e * 6 + lane] = o_mean; pol->n.var[(size_t)e * 6 + lane] = o_var; }
+    }
+    if (lane == 0) {
+      pol->next_done[e] = done;
+      if (pol->returns != nullptr) { pol->returns[e] = ret; pol->ret_mean[e] = r_mean; pol->ret_var[e] = r_var; }
+    }
+  }
+}
+
+// One environment per one-warp CTA (launch_warp in evac_abi.cu); no block-level barrier anywhere.
+template <int MODE, bool PE = false>
+__global__ void __launch_bounds__(32, WARP_MINB) evac_warp_kernel(const __grid_constant__ KArgs<float> a,
+                                                                  const EnvParamRec<float>* __restrict__ params) {
+  // lane is read here: the kernel's launch bounds (32 threads) make threadIdx.x & 31 free only at the kernel's own level
+  warp_env_loop<MODE, PE, false>(a, params, nullptr, threadIdx.x & 31);
+}
+
+// evac_rollout_policy: the gravity-encoding step loop with the linear policy as its agent (DESIGN.md section 7.2).
+template <bool PE>
+__global__ void __launch_bounds__(32, WARP_POL_MINB) evac_warp_policy_kernel(const __grid_constant__ KArgs<float> a,
+                                                                             const EnvParamRec<float>* __restrict__ params,
+                                                                             const __grid_constant__ WPolArgs pol) {
+  warp_env_loop<WMODE_GRAV, PE, true>(a, params, &pol, threadIdx.x & 31);
+}
+
+// The counters the caller advances once per step (NormalizeObservation's and NormalizeReward's sample counts, the policy's stream
+// offset), advanced by n steps AFTER the step kernel: every CTA of that kernel reads them at its start.  Sequential += 1.0, so the
+// counts equal what n per-step `count += 1.0` give (1e-4 + n is not always that).
+__global__ void evac_policy_counters_kernel(double* obs_count, double* ret_count, unsigned long long* offset, int n) {
+  if (obs_count != nullptr) { double c = *obs_count; for (int i = 0; i < n; ++i) c += 1.0; *obs_count = c; }
+  if (ret_count != nullptr) { double c = *ret_count; for (int i = 0; i < n; ++i) c += 1.0; *ret_count = c; }
+  if (offset != nullptr) *offset += (unsigned long long)n;
 }
 
 }  // namespace evac

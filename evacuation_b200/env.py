@@ -672,18 +672,33 @@ class EvacuationEnv:
         self.last_status_counts = trace
         return self._structure(obs), self._reward, self._terminated_b, self._truncated_b
 
-    def efficiency_curve(self, num_steps: int, agent: str = "random", chunk: int = 250):
+    def efficiency_curve(self, num_steps: int, agent="random", chunk: int = 250, normalizer=None):
         """The "quantification of evacuation efficiency" statistic of src/plotting_old/plot.py:165-201: the number of
         escaped pedestrians after every step, mean and standard deviation over the environments (one episode each,
         from a fresh reset) -> (mean[num_steps], std[num_steps]) float64 tensors; `1 - mean / N` is the plotted
         "% NOT evacuated".  Everything runs on the device (`evac_rollout` with the scripted `agent`); create the env
-        with auto_reset=False so that finished episodes stay at N escaped."""
+        with auto_reset=False so that finished episodes stay at N escaped.
+
+        `agent` may also be a trained `FusedRPOLinearPolicy` (gravity encoding): it acts with the clipped actor mean, on the
+        observation normalised by `normalizer` (a `VectorNormalizer`, used frozen; None = the raw observation), in
+        `evac_rollout_policy` launches of `chunk` steps that record the status counts."""
         self.reset()
+        fused = not isinstance(agent, str)
+        if fused:
+            from .rollout import fused_policy_rollout
+            next_done = torch.zeros(self.num_envs, dtype=torch.float32, device=self.device)
         means, stds = [], []
         done = 0
         while done < num_steps:
             k = min(chunk, num_steps - done)
-            self.rollout(k, agent=agent, status_counts=True)
+            if fused:
+                trace = torch.empty((k, self.num_envs, 4), dtype=torch.int16, device=self.device)
+                fused_policy_rollout(self, agent, k, next_done, normalizer=normalizer, norm_update=False, normalize_reward=False,
+                                     sample=False, status_counts=trace)
+                self._host_statuses = None
+                self.last_status_counts = trace
+            else:
+                self.rollout(k, agent=agent, status_counts=True)
             esc = self.last_status_counts[:, :, 0].to(torch.float64)
             means.append(esc.mean(dim=1)); stds.append(esc.std(dim=1, unbiased=False))
             done += k

@@ -401,6 +401,88 @@ def normalize_reward_fused(norm: "VectorNormalizer", reward: torch.Tensor, termi
     return out
 
 
+def policy_launch_sizes(num_steps: int, steps_per_launch: int) -> list:
+    """Iterations of each `evac_rollout_policy` launch: `steps_per_launch` each, the last launch the remainder."""
+    if int(num_steps) < 1 or int(steps_per_launch) < 1:
+        raise ValueError(f"num_steps and steps_per_launch must be >= 1, got {num_steps}, {steps_per_launch}")
+    n, k = int(num_steps), int(steps_per_launch)
+    return [k] * (n // k) + ([n % k] if n % k else [])
+
+
+def check_policy_rollout_tensors(num_envs: int, obs_dim: int, normalizer: Optional["VectorNormalizer"] = None, next_done=None,
+                                 **outputs) -> None:
+    """The shapes and dtypes `fused_policy_rollout` needs (ValueError otherwise): the normaliser's [E, obs_dim] / [E] float32 statistics
+    and float64 scalar counts, next_done [E] float32, and every given per-step output as [T, E, ...] of its dtype.  Device-free."""
+    E, D = int(num_envs), int(obs_dim)
+
+    def want(name, t, shape, dtype):
+        if t is None:
+            return
+        if tuple(t.shape) != tuple(shape) or t.dtype != dtype or not t.is_contiguous():
+            raise ValueError(f"{name}: expected a contiguous {dtype} tensor of shape {tuple(shape)}, got {t.dtype} {tuple(t.shape)}")
+
+    want("next_done", next_done, (E,), torch.float32)
+    if normalizer is not None:
+        n = normalizer
+        want("obs_mean", n.obs_mean, (E, D), torch.float32); want("obs_var", n.obs_var, (E, D), torch.float32)
+        for k in ("returns", "ret_mean", "ret_var"):
+            want(k, getattr(n, k), (E,), torch.float32)
+        want("obs_count", n.obs_count, (), torch.float64); want("ret_count", n.ret_count, (), torch.float64)
+    T = None
+    for k, t in outputs.items():
+        if t is None:
+            continue
+        T = t.shape[0] if T is None else T
+        tail, dtype = {"obs_norm": ((D,), torch.float32), "action": ((2,), torch.float32), "status_counts": ((4,), torch.int16)}.get(k, ((), torch.float32))
+        want(k, t, (T, E, *tail), dtype)
+
+
+def fused_policy_rollout(env, policy: "FusedRPOLinearPolicy", num_steps: int, next_done: torch.Tensor, *, normalizer: Optional["VectorNormalizer"] = None,
+                         norm_update: bool = True, normalize_reward: bool = True, sample: bool = True, obs_norm=None, action=None, logprob=None, value=None, reward_norm=None,
+                         dones=None, status_counts=None) -> None:
+    """`num_steps` iterations of the gravity-encoding rollout loop (rpo_agent.py:180-203) in ONE step-kernel launch
+    (`evac_rollout_policy`): the fused linear policy (with `normalizer`'s NormalizeObservation, updated or, `norm_update=False`,
+    frozen), ClipAction, the env step with same-step auto-reset and (`normalize_reward`) its NormalizeReward, for every environment
+    of `env`.  Reads the raw
+    observation from, and leaves the last one in, `env.unwrapped.flat_observation`; advances the normaliser's counts and
+    `policy.calls` by `num_steps`.  The per-step outputs are optional [num_steps, E, ...] tensors.  Supported: a handle of the
+    one-warp kernel (float32, N <= 64) with positions = grav and a `FusedRPOLinearPolicy` on its 6 values with action_dim 2;
+    anything else raises NotImplementedError."""
+    import ctypes as C
+
+    from . import _native as nat
+
+    if not isinstance(policy, _FusedRPOPolicy):
+        raise NotImplementedError(f"the one-launch rollout runs the fused linear policy, not {type(policy).__name__}")
+    u = env.unwrapped
+    E = u.num_envs
+    if int(num_steps) < 1:
+        raise ValueError(f"num_steps must be >= 1, got {num_steps}")
+    check_policy_rollout_tensors(E, u.obs_dim, normalizer, next_done, obs_norm=obs_norm, action=action, logprob=logprob, value=value,
+                                 reward_norm=reward_norm, dones=dones, status_counts=status_counts)
+    for k, t in (("obs_norm", obs_norm), ("action", action), ("logprob", logprob), ("value", value), ("reward_norm", reward_norm),
+                 ("dones", dones), ("status_counts", status_counts)):
+        if t is not None and t.shape[0] != num_steps:
+            raise ValueError(f"{k}: expected {num_steps} steps, got {t.shape[0]}")
+    p = lambda t: None if t is None else t.data_ptr()
+    io = nat.EvacPolicyRolloutIO()
+    io.obs, io.next_done = p(u.flat_observation), p(next_done)
+    if normalizer is not None:
+        n = normalizer
+        io.norm_mean, io.norm_var, io.norm_count = p(n.obs_mean), p(n.obs_var), p(n.obs_count)
+        io.norm_eps, io.norm_clip, io.norm_update = n.epsilon, n.obs_clip, int(bool(norm_update))
+        if normalize_reward:
+            io.returns, io.ret_mean, io.ret_var, io.ret_count = p(n.returns), p(n.ret_mean), p(n.ret_var), p(n.ret_count)
+            io.gamma, io.eps, io.clip = n.gamma, n.epsilon, n.reward_clip
+    io.sample, io.seed, io.offset, io.offset_device = int(bool(sample)), policy.seed, 0, p(policy.calls)
+    io.env_index_offset = policy.env_index_offset
+    io.obs_norm, io.action, io.logprob, io.value = p(obs_norm), p(action), p(logprob), p(value)
+    io.reward_norm, io.dones, io.status_counts = p(reward_norm), p(dones), p(status_counts)
+    io.reward_sum, io.terminated, io.truncated = p(u._reward), p(u._terminated), p(u._truncated)
+    st = torch.cuda.current_stream(u.device).cuda_stream
+    nat.check(nat.load().evac_rollout_policy(u._handle(), policy._h, int(num_steps), C.byref(io), C.c_void_p(st)))
+
+
 # ---------------------------------------------------------------------------------------------
 class PolicyRollout:
     """policy forward -> ClipAction -> fused env step (same-step auto-reset) -> normalise, `num_steps` times.
@@ -497,8 +579,15 @@ class PolicyRollout:
         torch.cuda.set_rng_state(rng_state, self.device)
         torch.cuda.synchronize(self.device)
 
-    def run(self, num_steps: int):
-        """Returns the storage dict ([T, E, ...]) when `store`, else None."""
+    def run(self, num_steps: int, steps_per_launch: int = 1):
+        """Returns the storage dict ([T, E, ...]) when `store`, else None.
+
+        `steps_per_launch` > 1 (the gravity-encoding config with a `FusedRPOLinearPolicy`): each launch of `evac_rollout_policy` runs
+        that many iterations in the step kernel (the last launch the remainder), bit-identical to the per-step loop and writing the
+        storage in place; `self.out` and `self.next_obs` are not updated on this path.  Switching between the two paths mid-run
+        continues the same trajectory.  Anything else raises NotImplementedError; 1 is the CUDA-graph loop."""
+        if steps_per_launch != 1:
+            return self._run_fused(num_steps, steps_per_launch)
         if self._graph is not None and self._graph_params_mode != self.env.unwrapped._env_params_mode:
             self._graph = None  # set_env_params switched between the uniform and the per-env step kernel: capture again
         if self.use_graph and self._graph is None:
@@ -524,6 +613,26 @@ class PolicyRollout:
                 buf["values"][t].copy_(self.out["value"]); buf["rewards"][t].copy_(self.out["reward"])
         return buf
 
+    def _new_storage(self, num_steps):
+        return dict(obs=torch.empty((num_steps, self.E, self.D), device=self.device), actions=torch.empty((num_steps, self.E, 2), device=self.device),
+                    logprobs=torch.empty((num_steps, self.E), device=self.device), rewards=torch.empty((num_steps, self.E), device=self.device),
+                    dones=torch.empty((num_steps, self.E), device=self.device), values=torch.empty((num_steps, self.E), device=self.device))
+
+    def _run_fused(self, num_steps, steps_per_launch):
+        sizes = policy_launch_sizes(num_steps, steps_per_launch)
+        if not isinstance(self.policy, FusedRPOLinearPolicy):
+            raise NotImplementedError(f"steps_per_launch > 1 runs the fused linear policy, not {type(self.policy).__name__}")
+        if self._raw_obs is None:
+            raise ValueError("call reset() first")
+        buf = self._new_storage(num_steps) if self.store else None
+        t = 0
+        for k in sizes:
+            o = {} if buf is None else dict(obs_norm=buf["obs"][t:t + k], action=buf["actions"][t:t + k], logprob=buf["logprobs"][t:t + k],
+                                            value=buf["values"][t:t + k], reward_norm=buf["rewards"][t:t + k], dones=buf["dones"][t:t + k])
+            fused_policy_rollout(self.env, self.policy, k, self.next_done, normalizer=self.norm, **o)
+            t += k
+        return buf
+
 
 __all__ = ["VectorNormalizer", "RPOTransformerPolicy", "RPOLinearPolicy", "FusedRPOTransformerPolicy", "FusedRPOLinearPolicy", "PolicyRollout",
-           "flatten_policy_weights", "normalize_reward_fused"]
+           "flatten_policy_weights", "normalize_reward_fused", "fused_policy_rollout"]

@@ -272,7 +272,8 @@ int32_t evac_abi_version(void);
  *
  * The policy reads the [E, (N+2)*d_model] MatrixObs rows evac_step writes and produces the [E,2] actions evac_step
  * consumes, so policy -> step -> normalise stays on the device (two launches for the policy, one for the step; one for the
- * linear policy).
+ * linear policy).  For the gravity encoding (K = 6) evac_rollout_policy (below) runs the whole loop, num_steps iterations per
+ * step-kernel launch.
  *
  * num_blocks = 0 means "RPOLinearNetwork directly on the observation": K = seq_len * d_model is the observation width
  * (evac_policy_default_linear_config: seq_len 1, d_model = obs_dim), 1 <= K <= 4096, num_heads / dim_feedforward / use_resid /
@@ -357,6 +358,63 @@ int64_t evac_policy_launch_count(const EvacPolicy* p);
 int evac_normalize_reward(int32_t num_envs, const float* reward, const uint8_t* terminated, const uint8_t* truncated, float* returns,
                           float* ret_mean, float* ret_var, const double* count, float* out, float* done_out, float gamma, float eps,
                           float clip, void* stream);
+
+/* ---- the gravity-encoding rollout loop in ONE step-kernel launch per num_steps iterations ------------------------------
+ *
+ *   evac_rollout_policy      num_steps iterations of rpo_agent.py:180-203 for every environment, with the linear policy
+ *                            (num_blocks = 0) as the agent of the one-warp step kernel: NormalizeObservation + clip, the heads,
+ *                            Normal sampling (or the mean), ClipAction, the step with same-step auto-reset, NormalizeReward +
+ *                            clip and next_done.  The state, both normalisers' per-env statistics and the loop's next_done stay
+ *                            on chip for the whole launch.
+ *
+ * Every value is bit-identical to num_steps iterations of the per-step loop (evac_policy_forward with the fused normaliser on
+ * obs, evac_step on the clipped action, evac_normalize_reward with done_out, and `count += 1.0` / `offset += 1` after each):
+ * the heads are the CUDA-core heads kernel's sums (the kernel K = 6 takes) in the same order.
+ *
+ * Supported, anything else fails with EVAC_ERR_UNSUPPORTED: a handle that runs the one-warp kernel (float32, N <= 64) with
+ * positions = grav (obs_dim 6), uniform or per-environment parameters; a policy with num_blocks = 0, K = 6 and action_dim 2, any
+ * num_hidden it accepts.  The flat-observation linear policy is not taken: at K = 364 layer 1 of the two heads alone is 47 k FMAs
+ * and 186 KB of weights per environment and step -- work for the tensor-core heads kernel, not for one warp.
+ * Noise is always the in-kernel stream.  Sampling draws of iteration s use stream offset offset + *offset_device + s and the
+ * policy's env_index_offset (in the io struct); the environment streams use the handle's.
+ *
+ * Launches (counted on the handle, evac_launch_count): the step kernel, plus one single-thread kernel that advances norm_count
+ * (when norm_update != 0), ret_count and *offset_device by num_steps when any of them is given.  They are advanced after the
+ * step kernel because every CTA of it reads them at its start. */
+typedef struct EvacPolicyRolloutIO {
+  /* inputs and carried state (device) */
+  float* obs;                /* [E, 6] raw observation: read before the first iteration, overwritten with the one after the last */
+  float* next_done;          /* [E] in / out */
+  float* norm_mean;          /* [E, 6] NormalizeObservation running mean / variance (in place), or NULL: no normaliser */
+  float* norm_var;
+  double* norm_count;        /* device scalar: samples seen before the call */
+  float norm_eps, norm_clip;
+  int32_t norm_update;       /* 1: update the statistics (evac_policy_forward's fused normaliser), 0: use them frozen (evaluation) */
+  float* returns;            /* [E] NormalizeReward state (in place), or NULL: no reward normaliser */
+  float* ret_mean;
+  float* ret_var;
+  double* ret_count;         /* device scalar: samples seen before the call */
+  float gamma, eps, clip;
+  int32_t sample;            /* 0: the action is the actor mean */
+  uint64_t seed, offset;     /* as in EvacPolicyIO */
+  uint64_t* offset_device;   /* NULL or a DEVICE counter added to offset; advanced by num_steps */
+  int64_t env_index_offset;  /* global index of env 0 in the POLICY's Normal draws (EvacPolicyIO.env_index_offset); the
+                                environment streams are keyed by the handle's own env_index_offset */
+  /* per-step outputs [num_steps, E, ...] (device), any may be NULL */
+  float* obs_norm;           /* [T, E, 6] the normalised observation the policy saw */
+  float* action;             /* [T, E, 2] the action before ClipAction */
+  float* logprob;            /* [T, E] */
+  float* value;              /* [T, E]; NULL skips the critic */
+  float* reward_norm;        /* [T, E] the normalised, clipped reward (needs the reward normaliser) */
+  float* dones;              /* [T, E] next_done BEFORE the step */
+  uint16_t* status_counts;   /* [T, E, 4] as evac_rollout writes them */
+  /* per-launch outputs [E] (device), any may be NULL: as in evac_rollout */
+  float* reward_sum;
+  uint8_t* terminated;
+  uint8_t* truncated;
+} EvacPolicyRolloutIO;
+
+int evac_rollout_policy(EvacHandle* h, const EvacPolicy* p, int32_t num_steps, const EvacPolicyRolloutIO* io, void* stream);
 
 /* ---- measurement helpers (used by bench.py; not part of the reference surface) ---- */
 /* FP32 FMA-pipe peak probe: every thread runs `iters` x 8 independent FMA chains; packed != 0 uses
