@@ -11,7 +11,7 @@ import os
 from . import build as _build
 from .build import LIB_PATH
 
-EVAC_ABI_VERSION = 5
+EVAC_ABI_VERSION = 6
 NUM_EPISODE_STATS = 9
 EPISODE_STAT_KEYS = (  # env.py:115-125
     "episode_intrinsic_reward", "episode_status_reward", "episode_reward", "episode_length",
@@ -71,7 +71,7 @@ class EvacPolicyIO(C.Structure):
         ("embedding", C.c_void_p), ("mean", C.c_void_p), ("value", C.c_void_p), ("action", C.c_void_p),
         ("action_clipped", C.c_void_p), ("logprob", C.c_void_p), ("entropy", C.c_void_p), ("given_action", C.c_void_p),
         ("sample", C.c_int32), ("training", C.c_int32), ("seed", C.c_uint64), ("offset", C.c_uint64),
-        ("offset_device", C.c_void_p), ("env_index_offset", C.c_int64),
+        ("offset_device", C.c_void_p), ("env_index_offset", C.c_int64), ("norm_frozen", C.c_int32),
     ]
 
 

@@ -51,6 +51,7 @@ struct EvacPolicy {
   float *d_w1tc64 = nullptr, *d_w1tc128 = nullptr, *d_w2tc = nullptr;
   int tc_chunks = 0;
   bool use_tc = false;
+  bool tc_cols128 = false;  // EVAC_POLICY_TC=128: 128-column tiles at every batch size (measurement hook)
   bool loaded = false;
   int64_t launches = 0;
   size_t embed_smem = 0, heads_smem = 0;
@@ -104,26 +105,31 @@ static void pack_block(const float* src, float* dst, int F, int F4) {
   (void)F4;
 }
 
+// frozen: evaluation with the normaliser's statistics read-only (never together with train)
 template <int D, int H>
-static int launch_embed(EvacPolicy* p, const PArgs& a, bool train, cudaStream_t st) {
+static int launch_embed(EvacPolicy* p, const PArgs& a, bool train, bool frozen, cudaStream_t st) {
   auto k_eval = evac_policy_embed_kernel<D, H, false>;
   auto k_train = evac_policy_embed_kernel<D, H, true>;
+  auto k_frozen = evac_policy_embed_kernel<D, H, false, true>;
   static thread_local size_t attr_set[16] = {0};
   if (p->embed_smem > 48 * 1024 && attr_set[p->device & 15] < p->embed_smem) {
     PCK(cudaFuncSetAttribute(k_eval, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->embed_smem));
     PCK(cudaFuncSetAttribute(k_train, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->embed_smem));
+    PCK(cudaFuncSetAttribute(k_frozen, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->embed_smem));
     attr_set[p->device & 15] = p->embed_smem;
   }
   const int grid = (a.E + PW_WARPS - 1) / PW_WARPS;
   if (train) k_train<<<grid, PW_WARPS * 32, p->embed_smem, st>>>(a);
+  else if (frozen) k_frozen<<<grid, PW_WARPS * 32, p->embed_smem, st>>>(a);
   else k_eval<<<grid, PW_WARPS * 32, p->embed_smem, st>>>(a);
   PCK(cudaGetLastError());
   p->launches++;
   return EVAC_OK;
 }
 
-// the heads kernel on X = the embedding, or the observation of the linear policy (+ its fused normaliser when n.mean is set)
-static int launch_heads(EvacPolicy* p, const EvacPolicyIO* io, const float* x, const NArgs& n, cudaStream_t st) {
+// the heads kernel on X = the embedding, or the observation of the linear policy (+ its fused normaliser when n.mean is set: updated,
+// or read-only when frozen)
+static int launch_heads(EvacPolicy* p, const EvacPolicyIO* io, const float* x, const NArgs& n, bool frozen, cudaStream_t st) {
   const bool norm = n.mean != nullptr;
   HArgs h;
   memset(&h, 0, sizeof(h));
@@ -142,21 +148,33 @@ static int launch_heads(EvacPolicy* p, const EvacPolicyIO* io, const float* x, c
     // shapes: 64 columns x 4 stages (critic and actor in separate CTAs) while 128-column tiles would not fill the SMs, 128 columns
     // x 3 stages beyond (X is read once).  Measured per 8192 / 20 000 / 65 536 envs: 20.3 / 49.3 / 121.5 us (64x4), 29.7 / 50.4 /
     // 105.0 us (128x3); 64 columns x 2 stages with two CTAs per SM: 24.6 / 53.6 / 113.1 us.
-    // The fused normaliser always takes the 128-column tiles: one CTA per row tile updates the statistics (DESIGN.md section 7).
+    // The fused normaliser's update always takes the 128-column tiles: one CTA per row tile updates the statistics (DESIGN.md
+    // section 7).  Frozen, it writes nothing two CTAs share and takes the normaliser-free rule (DESIGN.md section 7.3).
     auto k64 = evac_policy_heads_tc_kernel<64, 4, 2, 1>;
     auto k128 = evac_policy_heads_tc_kernel<128, 3, 2, 1>;
     auto k128n = evac_policy_heads_tc_kernel<128, 3, 2, 1, true>;
+    auto k64f = evac_policy_heads_tc_kernel<64, 4, 2, 1, true, true>;
+    auto k128f = evac_policy_heads_tc_kernel<128, 3, 2, 1, true, true>;
     using S64 = TCShape<64, 4, 2>; using S128 = TCShape<128, 3, 2>;
     static thread_local bool tc_attr[16] = {false};
     if (!tc_attr[p->device & 15]) {
       PCK(cudaFuncSetAttribute(k64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S64::SMEM_BYTES));
       PCK(cudaFuncSetAttribute(k128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S128::SMEM_BYTES));
       PCK(cudaFuncSetAttribute(k128n, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S128::SMEM_BYTES));
+      PCK(cudaFuncSetAttribute(k64f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S64::SMEM_BYTES));
+      PCK(cudaFuncSetAttribute(k128f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S128::SMEM_BYTES));
       tc_attr[p->device & 15] = true;
     }
-    if (norm) { t.w1tc = p->d_w1tc128; k128n<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t, n); }
-    else if (gx < 2 * 148) { t.w1tc = p->d_w1tc64; k64<<<dim3(gx, 2), TC_THREADS, S64::SMEM_BYTES, st>>>(t, n); }
-    else { t.w1tc = p->d_w1tc128; k128<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t, n); }
+    if (norm && !frozen) { t.w1tc = p->d_w1tc128; k128n<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t, n); }
+    else if (gx < 2 * 148 && !p->tc_cols128) {
+      t.w1tc = p->d_w1tc64;
+      if (norm) k64f<<<dim3(gx, 2), TC_THREADS, S64::SMEM_BYTES, st>>>(t, n);
+      else k64<<<dim3(gx, 2), TC_THREADS, S64::SMEM_BYTES, st>>>(t, n);
+    } else {
+      t.w1tc = p->d_w1tc128;
+      if (norm) k128f<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t, n);
+      else k128<<<dim3(gx, 1), TC_THREADS, S128::SMEM_BYTES, st>>>(t, n);
+    }
     PCK(cudaGetLastError());
     p->launches++;
     return EVAC_OK;
@@ -165,9 +183,11 @@ static int launch_heads(EvacPolicy* p, const EvacPolicyIO* io, const float* x, c
   if (p->heads_smem > 48 * 1024 && hattr[p->device & 15] < p->heads_smem) {
     PCK(cudaFuncSetAttribute(evac_policy_heads_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->heads_smem));
     PCK(cudaFuncSetAttribute(evac_policy_heads_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->heads_smem));
+    PCK(cudaFuncSetAttribute(evac_policy_heads_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->heads_smem));
     hattr[p->device & 15] = p->heads_smem;
   }
-  if (norm) evac_policy_heads_kernel<true><<<(h.E + HD_TM - 1) / HD_TM, HD_THREADS, p->heads_smem, st>>>(h, n);
+  if (norm && frozen) evac_policy_heads_kernel<true, true><<<(h.E + HD_TM - 1) / HD_TM, HD_THREADS, p->heads_smem, st>>>(h, n);
+  else if (norm) evac_policy_heads_kernel<true><<<(h.E + HD_TM - 1) / HD_TM, HD_THREADS, p->heads_smem, st>>>(h, n);
   else evac_policy_heads_kernel<false><<<(h.E + HD_TM - 1) / HD_TM, HD_THREADS, p->heads_smem, st>>>(h, n);
   PCK(cudaGetLastError());
   p->launches++;
@@ -256,6 +276,9 @@ int evac_policy_create(const EvacPolicyConfig* cfg, int32_t device, EvacPolicy**
   // EVAC_POLICY_TC=0 is a test hook: it selects the CUDA-core heads so that tests can compare the two kernels bit for bit.
   const char* tc_env = getenv("EVAC_POLICY_TC");
   p->use_tc = (p->K % 4 == 0) && !(tc_env && tc_env[0] == '0');
+  // EVAC_POLICY_TC=128 is a measurement hook: the tensor-core heads take the 128-column tiles at every batch size, so that the
+  // two tilings can be timed at the same size (tools/policy_eval.py)
+  p->tc_cols128 = tc_env && strcmp(tc_env, "128") == 0;
   p->tc_chunks = (p->K + TC_KC - 1) / TC_KC;
   if (p->use_tc) {
     alloc(&p->d_w1tc64, (size_t)p->tc_chunks * 2 * TC_COLS * TC_KC);
@@ -383,6 +406,9 @@ int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream) {
   if (io->num_envs < 1 || !io->obs) return pfail(EVAC_ERR_INVALID, "num_envs < 1 or obs is NULL");
   if ((io->norm_mean != nullptr) != (io->norm_var != nullptr) || (io->norm_mean && !io->norm_count))
     return pfail(EVAC_ERR_INVALID, "norm_mean, norm_var and norm_count must be given together");
+  if (io->norm_frozen && io->training && p->NB > 0)
+    return pfail(EVAC_ERR_UNSUPPORTED, "norm_frozen (evaluation) runs the transformer without dropout: set training = 0");
+  const bool frozen = io->norm_frozen != 0 && io->norm_mean != nullptr;
   cudaStream_t st = (cudaStream_t)stream;
   PCK(cudaSetDevice(p->device));
   if (p->NB == 0) {
@@ -393,7 +419,7 @@ int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream) {
                              reinterpret_cast<uintptr_t>(io->obs_norm)) & 15u) != 0)
       return pfail(EVAC_ERR_INVALID, "obs, norm_mean, norm_var and obs_norm must be 16-byte aligned");
     NArgs n{io->norm_mean, io->norm_var, io->norm_count, io->obs_norm, io->norm_eps, io->norm_clip};
-    return launch_heads(p, io, io->obs, n, st);
+    return launch_heads(p, io, io->obs, n, frozen, st);
   }
   const bool heads = io->mean || io->value || io->action || io->action_clipped || io->logprob || io->entropy;
   float* emb = io->embedding;
@@ -423,12 +449,12 @@ int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream) {
   a.norm_eps = io->norm_eps; a.norm_clip = io->norm_clip;
   a.w = p->d_emb_w; a.wstride = p->wstride;
   int rc = EVAC_ERR_UNSUPPORTED;
-#define X(d, h) if (p->D == d && p->H == h) rc = launch_embed<d, h>(p, a, train, st);
+#define X(d, h) if (p->D == d && p->H == h) rc = launch_embed<d, h>(p, a, train, frozen, st);
   EVAC_POLICY_SHAPES(X)
 #undef X
   if (rc) return rc;
   if (!heads) return EVAC_OK;
-  return launch_heads(p, io, emb, NArgs{}, st);
+  return launch_heads(p, io, emb, NArgs{}, false, st);
 }
 
 int64_t evac_policy_launch_count(const EvacPolicy* p) { return p ? p->launches : -1; }

@@ -216,8 +216,10 @@ __device__ __forceinline__ void attn_group(const float* __restrict__ ks, const f
   }
 }
 
-template <int D, int H, bool TRAIN>
+// FROZEN: evaluation with the normaliser's statistics read-only (EvacPolicyIO.norm_frozen); instantiated with TRAIN = false only
+template <int D, int H, bool TRAIN, bool FROZEN = false>
 __global__ void __launch_bounds__(PW_WARPS * 32, PW_MINB) evac_policy_embed_kernel(const __grid_constant__ PArgs a) {
+  static_assert(!(TRAIN && FROZEN), "evaluation runs without dropout");
   using L = EmbLayout<D, H>;
   extern __shared__ float4 smem4[];
   float* wsm = reinterpret_cast<float*>(smem4);
@@ -253,7 +255,21 @@ __global__ void __launch_bounds__(PW_WARPS * 32, PW_MINB) evac_policy_embed_kern
   for (int c = 0; c < D; ++c) xa[c] = xb[c] = 0.f;
   if (va) load_row<D>(a.obs + row0 + ra * D, xa);
   if (vb) load_row<D>(a.obs + row0 + rb * D, xb);
-  if (a.norm_mean != nullptr) {
+  if (FROZEN && a.norm_mean != nullptr) {
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      if (k == 0 ? va : vb) {
+        float (&x)[D] = k == 0 ? xa : xb;
+        const size_t off = row0 + (k == 0 ? ra : rb) * D;
+        float mean[D], var[D];
+        load_row<D>(a.norm_mean + off, mean);
+        load_row<D>(a.norm_var + off, var);
+#pragma unroll
+        for (int c = 0; c < D; ++c) x[c] = norm_frozen(x[c], mean[c], var[c], a.norm_eps, a.norm_clip);
+        if (a.obs_norm != nullptr) store_row<D>(a.obs_norm + off, x);
+      }
+    }
+  } else if (a.norm_mean != nullptr) {
     const double cnt = *a.norm_count, tot = cnt + 1.0;
     const float w_new = (float)(1.0 / tot), w_old = (float)(cnt / tot);
     const float w_mix = __fmul_rn(w_old, w_new);
@@ -491,8 +507,10 @@ __device__ __forceinline__ void heads_tile_fma(float (&acc)[8][8], const float4 
 // NORM: the linear policy's NormalizeObservation (NArgs) on every X element as it is loaded.  One CTA owns its 32 rows and every
 // column, and each k-chunk is loaded once, so each (env, k) statistic is read and written by exactly one thread of the grid.  The
 // X chunks then travel through registers (load, update, normalise, st.shared) instead of cp.async; the weight chunks keep the ring.
-template <bool NORM>
+// FROZEN (with NORM): the statistics are only read (evaluation, EvacPolicyIO.norm_frozen); obs_norm is the one store.
+template <bool NORM, bool FROZEN = false>
 __global__ void __launch_bounds__(HD_THREADS, 2) evac_policy_heads_kernel(const __grid_constant__ HArgs a, const __grid_constant__ NArgs n) {
+  static_assert(NORM || !FROZEN, "FROZEN is a mode of the fused normaliser");
   extern __shared__ float4 smem4[];
   float* wc = reinterpret_cast<float*>(smem4);        // [HD_STAGES][HD_KC][HD_COLS]
   float* xc = wc + HD_STAGES * HD_KC * HD_COLS;       // [HD_STAGES][HD_TM][HD_XS]
@@ -540,7 +558,18 @@ __global__ void __launch_bounds__(HD_THREADS, 2) evac_policy_heads_kernel(const 
       cp_async16(wd + 4 * v, ws + 4 * v, 16);
     }
     float* xd = xc + buf * HD_TM * HD_XS;
-    if constexpr (NORM) {
+    if constexpr (FROZEN) {
+      for (int v = tid; v < HD_TM * HD_KC; v += HD_THREADS) {
+        const int r = v / HD_KC, kk = v - r * HD_KC, k = k0 + kk;
+        float z = 0.f;
+        if (r < ne && k < a.K) {
+          const size_t i = (size_t)(e0 + r) * a.K + k;
+          z = norm_frozen(a.emb[i], n.mean[i], n.var[i], n.eps, n.clip);
+          if (n.obs_norm != nullptr) n.obs_norm[i] = z;
+        }
+        xd[r * HD_XS + kk] = z;
+      }
+    } else if constexpr (NORM) {
       const NormWeights nw = norm_weights(n);
       for (int v = tid; v < HD_TM * HD_KC; v += HD_THREADS) {
         const int r = v / HD_KC, kk = v - r * HD_KC, k = k0 + kk;

@@ -110,6 +110,12 @@ __device__ __forceinline__ float norm_update(float x, float& mean, float& var, c
   const float z = __fmul_rn(__fsub_rn(x, mean), rsqrtf(__fadd_rn(var, n.eps)));
   return min_nan(max_nan(z, -n.clip), n.clip);
 }
+// one (env, k) element against frozen statistics (evaluation, EvacPolicyIO.norm_frozen): the normalised, clipped value, op for
+// op norm_update's last two lines; nothing is written
+__device__ __forceinline__ float norm_frozen(float x, float mean, float var, float eps, float clip) {
+  const float z = __fmul_rn(__fsub_rn(x, mean), rsqrtf(__fadd_rn(var, eps)));
+  return min_nan(max_nan(z, -clip), clip);
+}
 
 }  // namespace evacp
 

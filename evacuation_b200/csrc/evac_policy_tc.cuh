@@ -155,9 +155,12 @@ __device__ __forceinline__ void tc_tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) 
 // NORM: the linear policy's NormalizeObservation (NArgs) on X as the producers load it.  Only with NT = 128: one CTA then owns its
 // rows and every column, so each (env, k) statistic is read and written by exactly one thread of the grid (with NT = 64 the critic
 // and the actor CTA of a row tile would both read the statistics while one of them updates them).
-template <int NT, int ST, int AH, int MINB, bool NORM = false>
+// FROZEN (with NORM): the statistics are only read (evaluation, EvacPolicyIO.norm_frozen), so nothing is shared that a CTA writes
+// and both tilings are valid; with NT = 64 the critic CTA (blockIdx.y = 0) alone stores obs_norm.
+template <int NT, int ST, int AH, int MINB, bool NORM = false, bool FROZEN = false>
 __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(const __grid_constant__ TCArgs a, const __grid_constant__ NArgs n) {
-  static_assert(!NORM || NT == TC_COLS, "the fused normaliser needs one CTA per row tile");
+  static_assert(NORM || !FROZEN, "FROZEN is a mode of the fused normaliser");
+  static_assert(!NORM || FROZEN || NT == TC_COLS, "the fused normaliser's update needs one CTA per row tile");
   using SH = TCShape<NT, ST, AH>;
   constexpr int STAGES = SH::STAGES, HEADS = SH::HEADS, TC_AHEAD = SH::AHEAD;
   // TMEM columns: layer 1 [0, NT) = xh wh + xl wh, [NT, 2 NT) = xh wl (summed by epilogue 1); layer 2 from 2 NT; power of two
@@ -279,8 +282,10 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
       if constexpr (NORM) {
         // X through registers: the raw rows and their statistics in (all loads of the chunk issued before the first use),
         // update + normalise + clip, statistics and obs_norm out, then the normalised value as the hi tile (the tensor core
-        // truncates it itself, as it does the cp.async'd raw value above) and its remainder as the lo tile
-        const NormWeights nw = norm_weights(n);
+        // truncates it itself, as it does the cp.async'd raw value above) and its remainder as the lo tile.  FROZEN: no update, the
+        // statistics are not stored
+        NormWeights nw;
+        if constexpr (!FROZEN) nw = norm_weights(n);
         float4 x[1024 / TC_ET], m[1024 / TC_ET], v[1024 / TC_ET];
         const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
@@ -302,11 +307,17 @@ __global__ void __launch_bounds__(TC_THREADS, MINB) evac_policy_heads_tc_kernel(
           float4 z = zero;
           if (e < h.E && q < kq) {
             const size_t g = (size_t)e * h.K + 4 * q;
-            z.x = norm_update(x[i].x, m[i].x, v[i].x, nw, n); z.y = norm_update(x[i].y, m[i].y, v[i].y, nw, n);
-            z.z = norm_update(x[i].z, m[i].z, v[i].z, nw, n); z.w = norm_update(x[i].w, m[i].w, v[i].w, nw, n);
-            *reinterpret_cast<float4*>(n.mean + g) = m[i];
-            *reinterpret_cast<float4*>(n.var + g) = v[i];
-            if (n.obs_norm != nullptr) *reinterpret_cast<float4*>(n.obs_norm + g) = z;
+            if constexpr (FROZEN) {
+              z.x = norm_frozen(x[i].x, m[i].x, v[i].x, n.eps, n.clip); z.y = norm_frozen(x[i].y, m[i].y, v[i].y, n.eps, n.clip);
+              z.z = norm_frozen(x[i].z, m[i].z, v[i].z, n.eps, n.clip); z.w = norm_frozen(x[i].w, m[i].w, v[i].w, n.eps, n.clip);
+              if (n.obs_norm != nullptr && y == 0) *reinterpret_cast<float4*>(n.obs_norm + g) = z;
+            } else {
+              z.x = norm_update(x[i].x, m[i].x, v[i].x, nw, n); z.y = norm_update(x[i].y, m[i].y, v[i].y, nw, n);
+              z.z = norm_update(x[i].z, m[i].z, v[i].z, nw, n); z.w = norm_update(x[i].w, m[i].w, v[i].w, nw, n);
+              *reinterpret_cast<float4*>(n.mean + g) = m[i];
+              *reinterpret_cast<float4*>(n.var + g) = v[i];
+              if (n.obs_norm != nullptr) *reinterpret_cast<float4*>(n.obs_norm + g) = z;
+            }
           }
           const uint32_t off = tc_swizzle(r, c4);
           *reinterpret_cast<float4*>(st + off) = z;

@@ -679,13 +679,16 @@ class EvacuationEnv:
         "% NOT evacuated".  Everything runs on the device (`evac_rollout` with the scripted `agent`); create the env
         with auto_reset=False so that finished episodes stay at N escaped.
 
-        `agent` may also be a trained `FusedRPOLinearPolicy` (gravity encoding): it acts with the clipped actor mean, on the
-        observation normalised by `normalizer` (a `VectorNormalizer`, used frozen; None = the raw observation), in
-        `evac_rollout_policy` launches of `chunk` steps that record the status counts."""
+        `agent` may also be a trained fused policy (`FusedRPOTransformerPolicy` or `FusedRPOLinearPolicy`): it acts with the clipped
+        actor mean, on the observation normalised by `normalizer` (a `VectorNormalizer`, used frozen; None = the raw observation), in
+        chunks of `chunk` steps that record the status counts.  The gravity-encoding linear policy on a one-warp handle (float32,
+        N <= 64) runs one `evac_rollout_policy` launch per chunk; every other pair runs `rollout.evaluate_policy`, one replayed
+        CUDA graph of policy forward + step per step."""
         self.reset()
         fused = not isinstance(agent, str)
         if fused:
-            from .rollout import fused_policy_rollout
+            from .rollout import evaluate_policy, fused_policy_rollout, one_launch_evaluation_supported
+            one_launch = one_launch_evaluation_supported(self, agent)
             next_done = torch.zeros(self.num_envs, dtype=torch.float32, device=self.device)
         means, stds = [], []
         done = 0
@@ -693,8 +696,11 @@ class EvacuationEnv:
             k = min(chunk, num_steps - done)
             if fused:
                 trace = torch.empty((k, self.num_envs, 4), dtype=torch.int16, device=self.device)
-                fused_policy_rollout(self, agent, k, next_done, normalizer=normalizer, norm_update=False, normalize_reward=False,
-                                     sample=False, status_counts=trace)
+                if one_launch:
+                    fused_policy_rollout(self, agent, k, next_done, normalizer=normalizer, norm_update=False, normalize_reward=False,
+                                         sample=False, status_counts=trace)
+                else:
+                    evaluate_policy(self, agent, k, normalizer=normalizer, status_counts=trace)
                 self._host_statuses = None
                 self.last_status_counts = trace
             else:

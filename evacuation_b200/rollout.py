@@ -16,7 +16,8 @@ batched equivalent of that glue so that the loop never leaves the GPU:
   and flat-observation configs), restated the same way;
 * `FusedRPOTransformerPolicy` / `FusedRPOLinearPolicy` -- their forward passes as the library's kernels;
 * `PolicyRollout`      -- policy -> step -> normalise, one iteration captured in a CUDA graph
-  and replayed (the tiny-GEMM policy is otherwise launch-bound).
+  and replayed (the tiny-GEMM policy is otherwise launch-bound);
+* `evaluate_policy`    -- a trained fused policy evaluated (actor mean, frozen normaliser) on any handle, the same way.
 
 The environment step is the CUDA path; there is no CPU fallback here either.
 """
@@ -286,8 +287,11 @@ class _FusedRPOPolicy:
         return t.data_ptr()
 
     def forward(self, obs, *, embedding=None, mean=None, value=None, action=None, action_clipped=None, logprob=None, entropy=None,
-                given_action=None, sample=True, normalizer: Optional["VectorNormalizer"] = None, obs_norm=None, advance=True):
-        """One fused forward on the current stream; every output is an optional preallocated tensor."""
+                given_action=None, sample=True, normalizer: Optional["VectorNormalizer"] = None, obs_norm=None, advance=True,
+                norm_update=True):
+        """One fused forward on the current stream; every output is an optional preallocated tensor.  `norm_update=False` uses
+        `normalizer`'s statistics frozen (evaluation): they and `normalizer.obs_count` stay as they are, `obs_norm` is still written.
+        Frozen together with `training` on the transformer policy raises NotImplementedError (evaluation runs without dropout)."""
         E = obs.shape[0]
         if obs.numel() != E * self.obs_dim:
             raise ValueError(f"obs must hold [E, {self.obs_dim}] values, got {tuple(obs.shape)}")
@@ -297,6 +301,7 @@ class _FusedRPOPolicy:
             io.norm_mean, io.norm_var = self._ptr(normalizer.obs_mean), self._ptr(normalizer.obs_var)
             io.norm_count, io.obs_norm = self._ptr(normalizer.obs_count, torch.float64), self._ptr(obs_norm)
             io.norm_eps, io.norm_clip = normalizer.epsilon, normalizer.obs_clip
+            io.norm_frozen = int(not norm_update)
         io.embedding, io.mean, io.value = self._ptr(embedding), self._ptr(mean), self._ptr(value)
         io.action, io.action_clipped = self._ptr(action), self._ptr(action_clipped)
         io.logprob, io.entropy, io.given_action = self._ptr(logprob), self._ptr(entropy), self._ptr(given_action)
@@ -305,7 +310,7 @@ class _FusedRPOPolicy:
         io.env_index_offset = self.env_index_offset
         st = torch.cuda.current_stream(self.device).cuda_stream
         self._nat.check(self._lib.evac_policy_forward(self._h, self._C.byref(io), self._C.c_void_p(st)))
-        if normalizer is not None:
+        if normalizer is not None and norm_update:
             normalizer.obs_count.add_(1.0)
         if advance:
             self.calls.add_(1)
@@ -483,6 +488,123 @@ def fused_policy_rollout(env, policy: "FusedRPOLinearPolicy", num_steps: int, ne
     nat.check(nat.load().evac_rollout_policy(u._handle(), policy._h, int(num_steps), C.byref(io), C.c_void_p(st)))
 
 
+def one_launch_evaluation_supported(env, policy) -> bool:
+    """Whether `evac_rollout_policy` runs `policy` on `env` (include/evac_b200.h): a handle of the one-warp step kernel (float32,
+    N <= 64) with positions = grav, and a `FusedRPOLinearPolicy` on its 6 values with action_dim 2.  Device-free."""
+    u = env.unwrapped
+    return (u.precision == "fp32" and u.cfg.number_of_pedestrians <= 64 and u._positions == "grav"
+            and isinstance(policy, FusedRPOLinearPolicy) and policy.obs_dim == 6 and policy.A == 2)
+
+
+def check_evaluation_args(num_envs: int, obs_dim: int, policy, num_steps: int, normalizer: Optional["VectorNormalizer"] = None,
+                          **outputs) -> None:
+    """What `evaluate_policy` needs before it touches a device: a fused policy (NotImplementedError otherwise) on the env's
+    obs_dim values with 2 actions, num_steps >= 1, and the normaliser and the per-step outputs of `check_policy_rollout_tensors`,
+    each output with num_steps rows (ValueError otherwise)."""
+    if not isinstance(policy, _FusedRPOPolicy):
+        raise NotImplementedError(f"evaluate_policy runs a fused policy (FusedRPOTransformerPolicy, FusedRPOLinearPolicy), "
+                                  f"not {type(policy).__name__}")
+    if policy.obs_dim != int(obs_dim) or policy.A != 2:
+        raise ValueError(f"the policy reads {policy.obs_dim} values and acts with {policy.A}; the env has obs_dim {obs_dim} and 2 actions")
+    if int(num_steps) < 1:
+        raise ValueError(f"num_steps must be >= 1, got {num_steps}")
+    check_policy_rollout_tensors(num_envs, obs_dim, normalizer, **outputs)
+    for k, t in outputs.items():
+        if t is not None and t.shape[0] != num_steps:
+            raise ValueError(f"{k}: expected {num_steps} steps, got {t.shape[0]}")
+
+
+def _snapshot(env, tensors):
+    """The env's checkpoint image and copies of `tensors`: what one captured iteration mutates, for `_restore`."""
+    return env.unwrapped.save_state(), [(t, t.clone()) for t in tensors]
+
+
+def _restore(env, snap):
+    image, tensors = snap
+    env.unwrapped.load_state(image)
+    for t, saved in tensors:
+        t.copy_(saved)
+
+
+def _capture_graph(env, iteration, tensors, count):
+    """One `iteration()` recorded into a CUDA graph -> (graph, kernels counted by `count()` while recording).
+
+    The warm-up outside the capture (lazy initialisation: function attributes, library autotuning) and the capture itself execute /
+    record real iterations, so the env state and `tensors` (everything else an iteration mutates) are snapshotted and restored: the
+    first replay starts exactly where the caller left the environments."""
+    device = env.unwrapped.device
+    snap = _snapshot(env, tensors)
+    rng_state = torch.cuda.get_rng_state(device)
+    side = torch.cuda.Stream(device=device)
+    side.wait_stream(torch.cuda.current_stream(device))
+    with torch.cuda.stream(side):
+        for _ in range(2):
+            iteration()
+    torch.cuda.current_stream(device).wait_stream(side)
+    torch.cuda.synchronize(device)
+    graph = torch.cuda.CUDAGraph()
+    before = count()
+    with torch.cuda.graph(graph):
+        iteration()
+    launches = count() - before
+    _restore(env, snap)
+    torch.cuda.set_rng_state(rng_state, device)
+    torch.cuda.synchronize(device)
+    return graph, launches
+
+
+@torch.no_grad()
+def evaluate_policy(env, policy, num_steps: int, *, normalizer: Optional["VectorNormalizer"] = None, obs_norm=None, action=None,
+                    status_counts=None) -> None:
+    """`num_steps` evaluation steps of a trained fused policy (`FusedRPOTransformerPolicy` or `FusedRPOLinearPolicy`) on every
+    environment of `env`, whatever kernel its handle runs (one-warp, CTA cell list, cluster, float64).
+
+    Per step: `evac_policy_forward` on the env's raw observation with training off, the actor mean as the action and `normalizer`'s
+    statistics frozen (None = the raw observation), then one table-agent step (`evac_rollout`) on the clipped action.  One step is
+    captured in a CUDA graph and replayed; the capture does not advance the environments.  The per-step outputs are optional
+    [num_steps, E, ...] tensors: `obs_norm` the observation the policy saw, `action` the actor mean before ClipAction,
+    `status_counts` (int16) the escaped / exiting / following / viscek counts after the step.  `policy.calls`, `policy.training` and
+    the normaliser are left as they are."""
+    u = env.unwrapped
+    E, D = u.num_envs, u.obs_dim
+    T = int(num_steps)
+    check_evaluation_args(E, D, policy, T, normalizer, obs_norm=obs_norm, action=action, status_counts=status_counts)
+    from . import _native as nat
+
+    lib, dev = nat.load(), u.device
+    policy.reserve(E)  # the transformer's embedding scratch, allocated before the capture
+    x = u.flat_observation  # the raw observation: every step rewrites this buffer in place
+    step_act = torch.empty((E, 2), device=dev) if action is not None else None
+    step_clip = torch.empty((E, 2), device=dev)
+    step_norm = torch.empty((E, D), device=dev) if obs_norm is not None and normalizer is not None else None
+    step_counts = torch.empty((1, E, 4), dtype=torch.int16, device=dev) if status_counts is not None else None
+    p = lambda t: None if t is None else t.data_ptr()
+
+    def iteration():
+        policy.forward(x, action=step_act, action_clipped=step_clip, sample=False, normalizer=normalizer, obs_norm=step_norm,
+                       norm_update=False, advance=False)
+        nat.check(lib.evac_rollout(u._handle(), 1, nat.AGENT["table"], p(step_clip), None, p(x), 0, p(u._reward), p(u._terminated),
+                                   p(u._truncated), p(step_counts), u._stream()))
+
+    training = policy.training
+    policy.training = False
+    try:
+        graph, _ = _capture_graph(env, iteration, [x, u._reward, u._terminated, u._truncated], lambda: 0)
+    finally:
+        policy.training = training
+    for t in range(T):
+        if obs_norm is not None and normalizer is None:
+            obs_norm[t].copy_(x)  # without a normaliser the policy sees the raw observation
+        graph.replay()
+        if step_norm is not None:
+            obs_norm[t].copy_(step_norm)
+        if action is not None:
+            action[t].copy_(step_act)
+        if status_counts is not None:
+            status_counts[t].copy_(step_counts[0])
+    u._host_statuses = None
+
+
 # ---------------------------------------------------------------------------------------------
 class PolicyRollout:
     """policy forward -> ClipAction -> fused env step (same-step auto-reset) -> normalise, `num_steps` times.
@@ -537,47 +659,24 @@ class PolicyRollout:
         self.next_obs.copy_(self.norm.observation(self.env.unwrapped.flat_observation))
         self.next_done.copy_(torch.logical_or(term, trunc).to(self.next_done.dtype))
 
-    def _snapshot(self):
-        """Everything one `_iteration()` mutates: env state (checkpoint image), normaliser statistics, the loop's carried
-        tensors, the policy's stream offset and the observation buffer."""
+    def _mutated(self):
+        """Everything one `_iteration()` mutates besides the env state: normaliser statistics, the loop's carried tensors, the
+        policy's stream offset and the observation buffer."""
         u = self.env.unwrapped
         tensors = [self.next_obs, self.next_done, u.flat_observation, *self.out.values(), self._act_clipped,
                    self.norm.obs_mean, self.norm.obs_var, self.norm.obs_count, self.norm.returns, self.norm.ret_mean, self.norm.ret_var, self.norm.ret_count]
         if self.fused:
             tensors.append(self.policy.calls)
-        return u.save_state(), [(t, t.clone()) for t in tensors]
-
-    def _restore(self, snap):
-        image, tensors = snap
-        self.env.unwrapped.load_state(image)
-        for t, saved in tensors:
-            t.copy_(saved)
+        return tensors
 
     def _capture(self):
-        # warm-up outside the capture (lazy initialisation: function attributes, library autotuning) and the capture itself
-        # execute / record real iterations -> the state they touch is snapshotted and restored, so that the first run()
-        # starts exactly where reset() left the environments (ADVICE r1: the warm-up used to advance them by two steps)
-        snap = self._snapshot()
-        rng_state = torch.cuda.get_rng_state(self.device)
-        side = torch.cuda.Stream(device=self.device)
-        side.wait_stream(torch.cuda.current_stream(self.device))
-        with torch.cuda.stream(side):
-            for _ in range(2):
-                self._iteration()
-        torch.cuda.current_stream(self.device).wait_stream(side)
-        torch.cuda.synchronize(self.device)
-        self._graph = torch.cuda.CUDAGraph()
+        # the first run() starts exactly where reset() left the environments (ADVICE r1: the warm-up used to advance them by two steps)
         count = lambda: self.env.unwrapped.launch_count + (self.policy.launch_count if self.fused else 0)
-        before = count()
-        with torch.cuda.graph(self._graph):
-            self._iteration()
+        self._graph, launches = _capture_graph(self.env, self._iteration, self._mutated(), count)
         # kernels of THIS library recorded into one graph replay: the handles count launches at capture time; the fused loop's
         # evac_normalize_reward is a handle-less entry point (+1)
-        self.launches_per_iteration = count() - before + (1 if self.fused else 0)
+        self.launches_per_iteration = launches + (1 if self.fused else 0)
         self._graph_params_mode = self.env.unwrapped._env_params_mode
-        self._restore(snap)
-        torch.cuda.set_rng_state(rng_state, self.device)
-        torch.cuda.synchronize(self.device)
 
     def run(self, num_steps: int, steps_per_launch: int = 1):
         """Returns the storage dict ([T, E, ...]) when `store`, else None.
@@ -635,4 +734,4 @@ class PolicyRollout:
 
 
 __all__ = ["VectorNormalizer", "RPOTransformerPolicy", "RPOLinearPolicy", "FusedRPOTransformerPolicy", "FusedRPOLinearPolicy", "PolicyRollout",
-           "flatten_policy_weights", "normalize_reward_fused", "fused_policy_rollout"]
+           "flatten_policy_weights", "normalize_reward_fused", "fused_policy_rollout", "evaluate_policy"]

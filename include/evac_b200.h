@@ -55,7 +55,7 @@
 extern "C" {
 #endif
 
-#define EVAC_ABI_VERSION 5
+#define EVAC_ABI_VERSION 6
 
 enum {
   EVAC_OK = 0,
@@ -340,6 +340,15 @@ typedef struct EvacPolicyIO {
   const uint64_t* offset_device; /* ... or point this at a DEVICE counter that is added to `offset` (NULL = unused): a
                                     forward captured in a CUDA graph then draws fresh numbers on every replay */
   int64_t env_index_offset;  /* global index of env 0 (sharding-invariant streams, like evac_create) */
+  /* != 0: evaluation -- the normaliser's statistics are used frozen, like gymnasium's NormalizeObservation at test time.
+   * norm_mean, norm_var and *norm_count are only read and stay bit for bit as they were (norm_count must still be given with
+   * them); obs_norm, when given, still receives the normalised clipped observation.  Per element, op for op the one-warp
+   * kernel's frozen normaliser (evac_rollout_policy with norm_update = 0):
+   *     z = clip(__fmul_rn(__fsub_rn(x, mean), rsqrtf(__fadd_rn(var, norm_eps))), -norm_clip, norm_clip)
+   * with NaN-propagating min / max (a NaN observation or statistic stays NaN and poisons only its own environment).
+   * Evaluation runs without dropout: norm_frozen together with training != 0 on a transformer policy (num_blocks > 0) fails
+   * with EVAC_ERR_UNSUPPORTED.  0 (a zero-initialised struct) updates the statistics as described above. */
+  int32_t norm_frozen;
 } EvacPolicyIO;
 
 /* embedding kernel (+ heads kernel if any head output is requested), asynchronous on `stream`.  The heads -- the 372 x 128 and
@@ -348,7 +357,10 @@ typedef struct EvacPolicyIO {
  * the environment at evac_policy_create, on the CUDA cores.  Both agree with a float64 evaluation to 3e-6.
  * Linear policy (num_blocks = 0): ONE launch, the heads kernel on `obs` (always, so that the normaliser runs even without head
  * outputs); the NormalizeObservation update + clip runs in the heads' load of X, and `obs` (plus norm_mean / norm_var / obs_norm
- * when K is a multiple of 4) must be 16-byte aligned. */
+ * when K is a multiple of 4) must be 16-byte aligned.
+ * Frozen normaliser (io->norm_frozen): the embedding kernel's prologue, or the heads' load of X, reads the statistics and writes only
+ * obs_norm; on the tensor cores the frozen load takes the normaliser-free kernel's column tiling (64 columns below 296 row tiles of
+ * 128 environments, 128 above), where the updating load always takes 128. */
 int evac_policy_forward(EvacPolicy* p, const EvacPolicyIO* io, void* stream);
 int64_t evac_policy_launch_count(const EvacPolicy* p);
 
